@@ -2,6 +2,7 @@
 """bench.py -- M^3PC plans/sec on B200 (BASELINE.json metric), one JSON line on rank 0.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--mode env|cand] [--envs E]
+                    [--dump-outputs DIR]
 
 A plan is one pass of the hot path (pass 1, candidate sampling, pass 2 at B=candidates, critic / return scoring, softmax
 selection) for one environment state.  A "step" plans ``--envs`` E lock-step environments (default 8, each with its own
@@ -18,6 +19,10 @@ candidates per plan, horizon 4, shipped MTM (D=512, 4 heads, 2+1 layers, T=8), r
   roofline  tensor-core GEMMs (the dominant kernel): algorithmic FLOPs of the GEMM launches / their summed per-launch
             CUDA-event time in a profiling pass of the same plan, against MEASURED_PEAKS.json (sustained bf16).
   cpu_baseline  the oracle port of the reference planner (torch CPU fp32, all host threads), same workload, bounded sample.
+
+``--dump-outputs DIR`` writes what the timed device-resident path returned in its last timed step -- the eval and sample
+actions, (E, A) -- as ``DIR/<name>.npy`` (float32; the one-window call's under ``single_env_*``).  Weights, histories and
+noise seeds are fixed, so two builds run with the same arguments can be compared output for output.
 
 Multi-GPU (launched by torchrun, one rank per GPU): ``--mode env`` (default) gives every rank its own environment --
 independent plans, no data-path collective, weak scaling; ``--mode cand`` shards the candidates of ONE plan across
@@ -223,7 +228,7 @@ def run_reference(args, w, shape, rank):
     if rank != 0:
         return
     steps, warmup = args.steps, args.warmup
-    val, times, threads, kind = time_cpu(w, shape, steps, warmup, budget_s=240.0)
+    val, times, threads, kind = time_cpu(w, shape, steps, warmup)
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": len(times), "warmup": warmup,
         "ms_per_step": 1e3 * sum(times) / len(times), "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -240,6 +245,14 @@ def run_reference(args, w, shape, rank):
 
 
 # ------------------------------------------------------------------------------------------------ ours
+def dump_outputs(out_dir, arrays):
+    """``out_dir/<name>.npy`` (float32) for every tensor of ``arrays``."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def build_learner(w, shape, n_local, E, dev, args, cand_offset=0):
     import torch
     from m3pc_b200 import synthetic as syn
@@ -293,7 +306,7 @@ def measure(L, w, shape, E, K, W, dev, flush, barrier, hist_base=1000, shard=Non
         ev, sm, _ = eng.plan(guidance=w["guidance"], horizon=h, n_cand=n_local, win_states=ws, win_actions=wa, win_rewards=wr,
                              win_returns_tok=wt, discount=0.99, temperature=w["temperature"], lmbda=0.6, seed=7 + i, cand_offset=lo,
                              n_env=E, exchange=shard is not None)
-        return ev
+        return ev, sm
 
     # ---- device-resident timing: K steps, one CUDA-event pair each, L2 flushed between steps ----
     for i in range(W):
@@ -305,11 +318,12 @@ def measure(L, w, shape, E, K, W, dev, flush, barrier, hist_base=1000, shard=Non
         flush.fill_(float(i))
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        plan_resident(W + i)
+        last = plan_resident(W + i)
         e1.record()
         pairs.append((e0, e1))
     torch.cuda.synchronize(); barrier()
     wall_resident = time.perf_counter() - t_wall0
+    outputs = {"eval_action": last[0].clone(), "sample_action": last[1].clone()}  # engine-owned: the next plan overwrites them
     per_step_ms = [a.elapsed_time(b) for a, b in pairs]
     launches = eng.last_launch_count()
 
@@ -339,10 +353,10 @@ def measure(L, w, shape, E, K, W, dev, flush, barrier, hist_base=1000, shard=Non
     torch.cuda.synchronize(); barrier()
     e2e_s = time.perf_counter() - t0
     return SimpleNamespace(E=E, dev_s=sum(per_step_ms) / 1e3, per_step_ms=per_step_ms, wall=wall_resident, launches=launches, e2e_s=e2e_s,
-                           lat=lat, plan_resident=plan_resident)
+                           lat=lat, plan_resident=plan_resident, outputs=outputs)
 
 
-def measure_cand_shard(args, dev, rank, world, flush, barrier, reduce_max):
+def measure_cand_shard(args, dev, rank, world, flush, barrier, reduce_max, K, W):
     """BASELINE.json configs[2] on the driver's own scaling run: ONE halfcheetah rtg plan of 16 384 candidates sharded over the
     `world` GPUs of the node (rank g owns [lo, hi); pass 1 replicated; Philox noise keyed by global candidate id), the shard
     records exchanged + merged inside the select kernel over NVLink peer memory.  Strong scaling; rank 0 also times the same
@@ -352,7 +366,6 @@ def measure_cand_shard(args, dev, rank, world, flush, barrier, reduce_max):
     name = "halfcheetah_rtg_16384"
     w = WORKLOADS[name]
     shape = model_shape(w)
-    K, W = min(args.steps, 50), 5
     n_total = w["n_cand"]
     lo, hi = mdist.shard_range(n_total, rank, world)
     L = build_learner(w, shape, hi - lo, 1, dev, args, cand_offset=lo)
@@ -381,7 +394,7 @@ def measure_cand_shard(args, dev, rank, world, flush, barrier, reduce_max):
         if rank == 0:
             out["n1_value_same_run"] = n1
             out["efficiency_vs_n1_same_run"] = out["value"] / (world * n1)
-    return out
+    return out, m.outputs
 
 
 def run_ours(args, w, shape, rank, local_rank, world):
@@ -405,9 +418,11 @@ def run_ours(args, w, shape, rank, local_rank, world):
         return [float(x) for x in t.tolist()]
 
     if cand_mode:  # explicit --mode cand: the candidate-sharded plan IS the headline of this run
-        cs = measure_cand_shard(args, dev, rank, world, flush, barrier, reduce_max)
+        cs, outputs = measure_cand_shard(args, dev, rank, world, flush, barrier, reduce_max, K, W)
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         if rank == 0:
-            emit({"metric": METRIC, "value": cs["value"], "unit": UNIT, "n_gpus": world, "steps": cs["steps"], "warmup": 5,
+            emit({"metric": METRIC, "value": cs["value"], "unit": UNIT, "n_gpus": world, "steps": cs["steps"], "warmup": W,
                   "ms_per_step": cs["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "bf16",
                   "data": "synthetic", "config": {"workload": cs["workload"], "parallelism": f"cand-shard x{world}", "collective": cs["collective"]},
                   "e2e": {"value": cs["e2e_value"], "unit": UNIT, "h2d_bytes_per_step": 4 * 8 * (17 + 6 + 2), "d2h_bytes_per_step": 4 * 6},
@@ -429,6 +444,11 @@ def run_ours(args, w, shape, rank, local_rank, world):
     single = measure(L, w, shape, 1, K, W, dev, flush, barrier, hist_base=base)  # the reference's call shape: one window per plan
     head = measure(L, w, shape, E_head, K, W, dev, flush, barrier, hist_base=base) if E_head > 1 else single
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        outputs = dict(head.outputs)
+        if E_head > 1:
+            outputs.update({f"single_env_{k}": v for k, v in single.outputs.items()})
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- roofline pass: same step with one event pair per GEMM launch ----
     eng.set_profile(True)
@@ -466,7 +486,7 @@ def run_ours(args, w, shape, rank, local_rank, world):
     if not args.lean and (world > 1 or args.cand_shard):
         del L, eng  # free the workspaces of the head workload first
         torch.cuda.empty_cache()
-        cs = measure_cand_shard(args, dev, rank, world, flush, barrier, reduce_max)
+        cs, _ = measure_cand_shard(args, dev, rank, world, flush, barrier, reduce_max, min(K, 50), 5)  # bounded side measurement
     if rank != 0:
         return
     peaks = {}
@@ -572,7 +592,10 @@ def main():
                     help="m3pc_set_option applied to every engine (A/B between result-equivalent launch sequences), e.g. fused_mlp=0")
     ap.add_argument("--lean", action="store_true", help="headline workload only: no north-star hopper key, no library baseline, no cand_shard")
     ap.add_argument("--cand-shard", action="store_true", help="also run the candidate-sharded config (halfcheetah 16384) on a single GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the actions of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     global _REAL_STDOUT
     sys.stdout.flush()
     _REAL_STDOUT = os.fdopen(os.dup(1), "w")  # keep the real stdout for the JSON line ...

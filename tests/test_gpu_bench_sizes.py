@@ -284,3 +284,35 @@ def test_scaled_model_1024_candidates():
     _report(case="scaled model (D=1024, 4+2 layers, T=16, h=8) N=1024, oracle on a 96-candidate slice", J=eJ, cand=eC,
             J_scale=float(ref["expect_return"].abs().max()))
     assert eJ < TOL and eC < 3.5 * TOL
+
+
+# ------------------------------------------------------------------------------------------------ bench.py --dump-outputs
+def test_bench_dumps_the_actions_of_the_last_timed_step(tmp_path):
+    """``bench.py --steps K --dump-outputs DIR`` times K steps and writes the actions the timed path returned in the last one:
+    they equal a fresh plan of the last timed step's windows and seed, and differ from the step before it."""
+    import subprocess
+    import sys
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    K, W = 3, 3
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", str(K), "--warmup", str(W), "--lean", "--no-cpu-baseline",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == K
+    dumped = {f.name: np.load(f) for f in tmp_path.glob("*.npy")}
+    assert sorted(dumped) == ["eval_action.npy", "sample_action.npy", "single_env_eval_action.npy", "single_env_sample_action.npy"]
+    assert all(a.dtype == np.float32 for a in dumped.values())
+    # the same learner, windows and seeds as the bench's default workload (rank 0)
+    w = bench.WORKLOADS["walker2d_critic_1024"]
+    shape = bench.model_shape(w)
+    dev = torch.device("cuda:0")
+    L = bench.build_learner(w, shape, w["n_cand"], 8, dev, SimpleNamespace(precision="bf16", chunk=0))
+    flush = torch.empty(1024, device=dev)
+    for E, prefix in ((1, "single_env_"), (8, "")):
+        m = bench.measure(L, w, shape, E, K, W, dev, flush, lambda: None, hist_base=1000)
+        last = [t.cpu().numpy() for t in m.plan_resident(W + K - 1)]
+        before = [t.cpu().numpy() for t in m.plan_resident(W + K - 2)]
+        assert dumped[prefix + "eval_action.npy"].shape == ((E, shape.act_dim) if E > 1 else (shape.act_dim,))
+        np.testing.assert_array_equal(dumped[prefix + "eval_action.npy"], last[0])
+        np.testing.assert_array_equal(dumped[prefix + "sample_action.npy"], last[1])
+        assert not np.array_equal(last[0], before[0])

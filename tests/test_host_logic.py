@@ -181,9 +181,10 @@ def test_bench_reference_arm_prints_contract_line():
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "0",
                           "--workload", "hopper_rtg_625"], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["metric"] == "plans_per_sec" and line["unit"] == "plans/s"
+    assert line["steps"] == 2  # --steps sets the number of timed plans
     assert line["cpu_baseline"]["kind"] in ("reference", "port") and line["e2e"]["h2d_bytes_per_step"] == 0 and line["value"] > 0
