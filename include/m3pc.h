@@ -98,13 +98,9 @@ int m3pc_finalize_params(m3pc_handle_t h);
 /* Selects between RESULT-EQUIVALENT launch sequences of the handle (parity tests compare them; none changes what is
  * computed).  Unknown names fail with M3PC_ERR_INVALID.  Names and defaults:
  *   "graphs" 1                 capture m3pc_plan into a CUDA graph and replay it (0: launch every kernel eagerly)
- *   "pdl" 1                    programmatic dependent launch between consecutive kernels (process-wide)
  *   "fused_b1" 1               one cooperative kernel for a B = 1 forward (0: one launch per op)
- *   "fused_ln" 1               residual GEMM + LayerNorm in one kernel (0: GEMM, then LayerNorm kernel)
- *   "fused_mlp" 0              1: linear1 + GELU + linear2 + residual in one kernel with the hidden kept on chip (m3pc_mlp_fused_bf16);
- *                              0: two GEMM launches.  Off by default: the on-chip variant is bound by the L2 -> SM operand stream
- *                              (weights re-streamed per 128 rows) and measured 4 % slower per plan step (DESIGN.md section 5)
- *   "fused_ln_min_rows" 1024   smallest GEMM (rows) the fused kernel is used for (>= 129)
+ *   "fused_ln_min_rows" 1024   smallest GEMM (rows) the fused residual GEMM + LayerNorm kernel is used for (>= 129; below, the
+ *                              GEMM is followed by a LayerNorm kernel)
  *   "restrict_deep_decoder" 1  decoders with > 1 layer: last layer on the consumed rows only (0: every row)
  *   "split_residual_min_rows" 0  restricted decoder layer, out-projection + residual + LayerNorm of the consumed rows: from this
  *                              many rows up the residual is read in place (batch-constant mask-token rows as a table, kept
@@ -112,7 +108,6 @@ int m3pc_finalize_params(m3pc_handle_t h);
  *                              a residual copy + one problem (bit-identical results)
  *   "grouped_ln" 1             problems of the fused residual GEMM + LayerNorm kernel that share K, bias and LayerNorm parameters
  *                              go into one launch (0: one launch per problem; bit-identical results)
- *   "dedupe_history" 1         first encoder block: history tokens once per environment (0: once per candidate)
  *   "gemm_ln_unit_rows" 0      rows per CTA-pair unit of the fused residual GEMM + LayerNorm kernel: 128 = two accumulators in
  *                              tensor memory (the epilogue of a unit overlaps the MMAs of the next), 256 = one accumulator with
  *                              1/3 less operand traffic per FLOP, 0 = chosen per launch from K and the row count
@@ -256,11 +251,6 @@ int m3pc_gemm_bf16_grouped(int32_t n, const void* const* A, const void* const* W
  * X = table[row / rows_per_group] + A W^T + bias; Y[M,512] (bf16) = LayerNorm(X; gamma, beta), eps 1e-5.  A, W bf16. */
 int m3pc_gemm_ln_bf16(const void* A, const void* W, const float* bias, float* X, void* Y, const float* gamma, const float* beta,
                       const float* table, int32_t rows_per_group, int32_t M, int32_t K, void* stream);
-/* Fused transformer MLP (n_embd 512, hidden 2048; mtm_model.py:379-409 linear1 -> GELU -> linear2 + residual):
- * X[M,512] (fp32, in place) += GELU(Y[M,512] W1[2048,512]^T + b1) W2[512,2048]^T + b2 with Y, W1, W2 bf16 and the hidden
- * activation kept in shared / tensor memory.  Bit-identical to m3pc_gemm_bf16(flags 1) into a bf16 hidden followed by
- * m3pc_gemm_bf16(flags 2). */
-int m3pc_mlp_fused_bf16(const void* Y, const void* W1, const float* b1, const void* W2, const float* b2, float* X, int32_t M, void* stream);
 /* y = LayerNorm(x) over the last dim (eps 1e-5); x fp32 (M,D); y bf16 (out_bf16=1) or fp32. */
 int m3pc_layernorm(const float* x, const float* gamma, const float* beta, void* y, int32_t M, int32_t D,
                    int32_t out_bf16, void* stream);

@@ -11,9 +11,7 @@ import subprocess
 from typing import Optional
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-#: M3PC_LIB=tuning selects the -DM3PC_TUNING build (``make -C m3pc_b200/csrc tuning``) that tools/ use for A/B experiments;
-#: it is the only place environment switches exist.  Everything else -- tests, bench.py, smoke() -- loads the release library.
-LIB_PATH = os.path.join(HERE, "libm3pc_tuning.so" if os.environ.get("M3PC_LIB") == "tuning" else "libm3pc.so")
+LIB_PATH = os.path.join(HERE, "libm3pc.so")
 CSRC = os.path.join(HERE, "csrc")
 
 OK = 0
@@ -33,7 +31,7 @@ GUIDANCE = {
 #: every symbol include/m3pc.h declares (tests/test_abi.py checks the header against this list and the .so)
 SYMBOLS = (
     "m3pc_last_error", "m3pc_version", "m3pc_create", "m3pc_destroy", "m3pc_set_param", "m3pc_finalize_params", "m3pc_set_option",
-    "m3pc_forward", "m3pc_plan", "m3pc_merge_partials", "m3pc_exchange_local", "m3pc_exchange_connect", "m3pc_exchange_status", "m3pc_backward_plan", "m3pc_backward_plan_draws", "m3pc_ring_append", "m3pc_ring_windows", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16", "m3pc_mlp_fused_bf16", "m3pc_gemm_fp32",
+    "m3pc_forward", "m3pc_plan", "m3pc_merge_partials", "m3pc_exchange_local", "m3pc_exchange_connect", "m3pc_exchange_status", "m3pc_backward_plan", "m3pc_backward_plan_draws", "m3pc_ring_append", "m3pc_ring_windows", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16", "m3pc_gemm_fp32",
     "m3pc_layernorm", "m3pc_attention", "m3pc_embed_gather", "m3pc_decoder_scatter_embed", "m3pc_block_forward", "m3pc_heads", "m3pc_sample_candidates", "m3pc_twinq",
     "m3pc_score_select", "m3pc_last_device_ms", "m3pc_last_launch_count", "m3pc_set_profile", "m3pc_get_profile",
 )
@@ -68,8 +66,7 @@ _lib: Optional[C.CDLL] = None
 
 def build(verbose: bool = False) -> str:
     """Compile the library in-tree with nvcc for sm_100a (``make -C m3pc_b200/csrc``)."""
-    target = ["tuning"] if os.environ.get("M3PC_LIB") == "tuning" else []
-    res = subprocess.run(["make", "-C", CSRC, "-j8"] + target, capture_output=True, text=True)
+    res = subprocess.run(["make", "-C", CSRC, "-j8"], capture_output=True, text=True)
     if verbose or res.returncode != 0:
         print(res.stdout[-4000:])
         print(res.stderr[-4000:])
@@ -111,7 +108,6 @@ def lib() -> C.CDLL:
     L.m3pc_gemm_bf16.argtypes = [vp, vp, f32p, vp, i32, i32, i32, i32, vp]
     L.m3pc_gemm_bf16_grouped.argtypes = [i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.m3pc_gemm_ln_bf16.argtypes = [vp, vp, f32p, f32p, vp, f32p, f32p, f32p, i32, i32, i32, vp]
-    L.m3pc_mlp_fused_bf16.argtypes = [vp, vp, f32p, vp, f32p, f32p, i32, vp]
     L.m3pc_gemm_fp32.argtypes = [f32p, f32p, f32p, f32p, i32, i32, i32, i32, vp]
     L.m3pc_layernorm.argtypes = [f32p, f32p, f32p, vp, i32, i32, i32, vp]
     L.m3pc_attention.argtypes = [vp, vp, i32, i32, i32, i32, vp]

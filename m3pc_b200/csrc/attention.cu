@@ -139,7 +139,6 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 __device__ __forceinline__ uint32_t swz(int r, int c) { return static_cast<uint32_t>(r * 256 + ((c ^ (r & 7)) << 4)); }
 
 constexpr int MMA_WARPS = 4;  // (b, head) pairs per CTA
-const bool g_attn_shared = tune_env("M3PC_ATTN_SHARED") == nullptr || tune_env("M3PC_ATTN_SHARED")[0] != '0';  // tuning build, M3PC_ATTN_SHARED=0: legacy staging
 
 // NTQ = ceil(n_q / 16) query tiles, NTK = ceil(n_kv / 16) key tiles
 template <int NTQ, int NTK>
@@ -563,7 +562,7 @@ int dispatch_q(const AttnParams& p, cudaStream_t st) {
 int launch_attention_gather(const AttnParams& p, bool bf16, cudaStream_t st) {
   M3PC_REQUIRE(p.B > 0 && p.n_q > 0 && p.n_kv > 0 && p.n_q <= MAX_TOK && p.n_kv <= MAX_TOK && p.n_head > 0, "attention: bad shape (<= 64 tokens)");
   if (!bf16) return launch_simple(p, st);
-  if (g_attn_shared && p.n_kv_batch > 0 && p.n_q <= 16 && p.B >= 64) {  // batch keys first, constant keys after (see AttnParams)
+  if (p.n_kv_batch > 0 && p.n_q <= 16 && p.B >= 64) {  // batch keys first, constant keys after (see AttnParams)
     const int n_c = p.n_kv - p.n_kv_batch, ntb = (p.n_kv_batch + 15) / 16, ntc = (n_c + 15) / 16;
     bool ok = n_c >= 8 && ntb <= 2 && ntc <= 3;
     for (int j = 0; j < p.n_kv && ok; ++j)

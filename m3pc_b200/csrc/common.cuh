@@ -146,15 +146,6 @@ struct PerDevice {
 };
 int device_num_sms();  // multiprocessors of the current device (cached per device; engine.cu)
 
-// Tuning switches (environment variables that pick between result-equivalent kernels, or that time a kernel with parts
-// skipped) exist only in the -DM3PC_TUNING build used by tools/; the release library reads no environment variable at all.
-// What tests and callers may legitimately choose between goes through m3pc_set_option (include/m3pc.h).
-#ifdef M3PC_TUNING
-inline const char* tune_env(const char* name) { return getenv(name); }
-#else
-inline const char* tune_env(const char*) { return nullptr; }
-#endif
-
 // ---- programmatic dependent launch (PDL) -------------------------------------------------------------------------------
 // Every kernel of a plan is launched with cudaLaunchAttributeProgrammaticStreamSerialization: it may be scheduled while
 // its predecessor in the stream is still draining, runs its private prologue, and blocks in griddepcontrol.wait until the
@@ -162,7 +153,6 @@ inline const char* tune_env(const char*) { return nullptr; }
 // global-memory access and before it can exit (a grid that finished without waiting would release ITS dependents early).
 // The trigger is issued right after the wait, so at most one dependent grid is pre-staged at a time.
 extern int g_ln_unit_rows;  // gemm_ln.cu
-extern bool g_use_pdl;  // m3pc_set_option "pdl" = 0 turns the attribute off (the device-side instructions are then no-ops)
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
@@ -183,7 +173,7 @@ inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = g_use_pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 #endif
@@ -208,9 +198,6 @@ struct LnJob {
   const float* R;       // residual rows when they are not X itself (and table is null), or null
 };
 int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const float* gamma, const float* beta, int K, cudaStream_t st);
-// mlp_fused.cu: X (M,512) fp32 += GELU(Y W1^T + b1) W2^T + b2, the 2048-wide hidden kept on chip
-int mlp_fused_bf16(const __nv_bfloat16* Y, const __nv_bfloat16* W1, const float* b1, const __nv_bfloat16* W2, const float* b2, float* X, int M,
-                   cudaStream_t st);
 // several independent bf16 GEMMs in one launch of the CTA-pair kernel (decoder embedding runs, K/V + Q, heads, twin critics)
 struct GemmProblem {
   const __nv_bfloat16* A;

@@ -18,7 +18,6 @@
 namespace m3pc {
 
 thread_local int g_launch_count = 0;
-bool g_use_pdl = true;
 static thread_local std::string g_error;
 void set_error(const std::string& msg) { g_error = msg; }
 
@@ -137,14 +136,11 @@ struct m3pc_engine {
   // workspaces (per chunk)
   DevBuf X, XS, Y, Y2, QKV, QSEL, ATT, HID, ENC;
   DevBuf XT, YT, QKVT;  // shared-history tables of the first encoder block (TAB_ROWS rows)
-  bool dedupe_history = true;  // option "dedupe_history"
   DevBuf fb_xd, fb_bar;  // fused B = 1 path: decoder-embedding scratch, grid-barrier state
   bool use_fused_b1 = true;
-  bool fuse_mlp = false;      // linear1 + GELU + linear2 + residual in one kernel, hidden on chip (mlp_fused.cu); option "fused_mlp".
-                              // Off by default: measured 4 % slower per step than the two launches (profiles/r2l_fused_mlp.txt)
   bool group_ln = true;       // several fused residual GEMM + LayerNorm problems per launch; option "grouped_ln" (0: one launch each)
-  bool fuse_ln = true;        // residual GEMM + LayerNorm in one kernel (gemm_ln.cu); option "fused_ln"
-  int fuse_ln_min_rows = 1024;  // option "fused_ln_min_rows" (the kernel-level parity tests call the kernel at any size)
+  int fuse_ln_min_rows = 1024;  // residual GEMM + LayerNorm in one kernel (gemm_ln.cu) from this many rows up; option "fused_ln_min_rows"
+                                // (the kernel-level parity tests call the kernel at any size)
   bool restrict_deep = true;  // decoders with > 1 layer: last layer on the consumed rows only; option "restrict_deep_decoder"
   int split_residual_min_rows = 0;  // restricted decoder, out-projection: from this many needed rows up the residual is read in place, one
                                     // problem per residual source in a grouped launch (no residual copy: -6 KB of HBM traffic per row);
@@ -489,25 +485,32 @@ int build_const_rows(m3pc_engine* e) {
   return M3PC_OK;
 }
 
+// Runs `launch` (one GEMM-family launch); with profiling on (m3pc_set_profile) it is bracketed by an event pair and `flops`
+// are booked against it for m3pc_get_profile.
+template <typename Launch>
+int profiled(m3pc_engine* e, double flops, cudaStream_t st, Launch&& launch) {
+  if (!e->profile) return launch();
+  const size_t slot = e->prof_used++;
+  if (slot >= e->prof_events.size()) {
+    cudaEvent_t a, b;
+    M3PC_CHECK_CUDA(cudaEventCreate(&a));
+    M3PC_CHECK_CUDA(cudaEventCreate(&b));
+    e->prof_events.push_back({a, b});
+    e->prof_flops.push_back(0.0);
+  }
+  e->prof_flops[slot] = flops;
+  M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].first, st));
+  M3PC_TRY(launch());
+  M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].second, st));
+  return M3PC_OK;
+}
+
 int gemm(m3pc_engine* e, const void* A, const float* w32, const __nv_bfloat16* w16, void* C, int M, int N, int K, const GemmEpilogue& epi,
          cudaStream_t st) {
-  size_t slot = 0;
-  if (e->profile) {
-    slot = e->prof_used++;
-    if (slot >= e->prof_events.size()) {
-      cudaEvent_t a, b;
-      M3PC_CHECK_CUDA(cudaEventCreate(&a));
-      M3PC_CHECK_CUDA(cudaEventCreate(&b));
-      e->prof_events.push_back({a, b});
-      e->prof_flops.push_back(0.0);
-    }
-    e->prof_flops[slot] = 2.0 * M * static_cast<double>(N) * K;
-    M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].first, st));
-  }
-  const int rc = e->bf16 ? gemm_bf16_tcgen05(reinterpret_cast<const __nv_bfloat16*>(A), w16, C, M, N, K, epi, st)
-                         : gemm_fp32(reinterpret_cast<const float*>(A), w32, reinterpret_cast<float*>(C), M, N, K, epi, st);
-  if (e->profile && rc == M3PC_OK) M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].second, st));
-  return rc;
+  return profiled(e, 2.0 * M * static_cast<double>(N) * K, st, [&] {
+    return e->bf16 ? gemm_bf16_tcgen05(reinterpret_cast<const __nv_bfloat16*>(A), w16, C, M, N, K, epi, st)
+                   : gemm_fp32(reinterpret_cast<const float*>(A), w32, reinterpret_cast<float*>(C), M, N, K, epi, st);
+  });
 }
 
 // Several independent GEMMs as ONE launch where the CTA-pair tensor-core kernel applies (bf16 mode), else one launch each.
@@ -534,21 +537,7 @@ int gemm_group(m3pc_engine* e, const GemmJob* jobs, int n, cudaStream_t st) {
       pr[i] = GemmProblem{reinterpret_cast<const __nv_bfloat16*>(j.A), j.w16, j.C, j.M, j.N, j.K, j.epi};
       flops += 2.0 * j.M * static_cast<double>(j.N) * j.K;
     }
-    size_t slot = 0;
-    if (e->profile) {
-      slot = e->prof_used++;
-      if (slot >= e->prof_events.size()) {
-        cudaEvent_t a, b;
-        M3PC_CHECK_CUDA(cudaEventCreate(&a));
-        M3PC_CHECK_CUDA(cudaEventCreate(&b));
-        e->prof_events.push_back({a, b});
-        e->prof_flops.push_back(0.0);
-      }
-      e->prof_flops[slot] = flops;
-      M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].first, st));
-    }
-    M3PC_TRY(gemm_bf16_grouped(pr, m, st));
-    if (e->profile) M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].second, st));
+    M3PC_TRY(profiled(e, flops, st, [&] { return gemm_bf16_grouped(pr, m, st); }));
   }
   return M3PC_OK;
 }
@@ -562,23 +551,10 @@ int gemm_res_ln(m3pc_engine* e, const void* A, const float* w32, const __nv_bflo
   // one CTA pair per 256 rows: not for the few hundred rows of pass 1 of a multi-environment plan, where a single pair would do
   // the work of 4 .. 16.  (The switch is kept well below any pass-2 chunk or candidate shard, so the kernel choice -- and with it
   // the bit pattern of the scores -- does not depend on how candidates are chunked or sharded.)
-  if (allow_fused && e->bf16 && e->fuse_ln && D == 512 && M >= e->fuse_ln_min_rows) {
-    size_t slot = 0;
-    if (e->profile) {
-      slot = e->prof_used++;
-      if (slot >= e->prof_events.size()) {
-        cudaEvent_t a, c;
-        M3PC_CHECK_CUDA(cudaEventCreate(&a));
-        M3PC_CHECK_CUDA(cudaEventCreate(&c));
-        e->prof_events.push_back({a, c});
-        e->prof_flops.push_back(0.0);
-      }
-      e->prof_flops[slot] = 2.0 * M * static_cast<double>(D) * K;
-      M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].first, st));
-    }
-    M3PC_TRY(gemm_ln_bf16(reinterpret_cast<const __nv_bfloat16*>(A), w16, bias, X, reinterpret_cast<__nv_bfloat16*>(Y), g, b, table, rpg, M, K, st, res_src));
-    if (e->profile) M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].second, st));
-    return M3PC_OK;
+  if (allow_fused && e->bf16 && D == 512 && M >= e->fuse_ln_min_rows) {
+    return profiled(e, 2.0 * M * static_cast<double>(D) * K, st, [&] {
+      return gemm_ln_bf16(reinterpret_cast<const __nv_bfloat16*>(A), w16, bias, X, reinterpret_cast<__nv_bfloat16*>(Y), g, b, table, rpg, M, K, st, res_src);
+    });
   }
   M3PC_REQUIRE(res_src == nullptr, "gemm_res_ln: a separate residual source needs the fused kernel");
   GemmEpilogue ep;
@@ -616,7 +592,7 @@ struct ResLnJob {
 };
 int gemm_res_ln_group(m3pc_engine* e, const ResLnJob* jobs, int n, const float* bias, const float* g, const float* b, int K, cudaStream_t st) {
   const int D = e->D;
-  bool fused = e->bf16 && e->fuse_ln && D == 512 && e->group_ln;
+  bool fused = e->bf16 && D == 512 && e->group_ln;
   for (int i = 0; i < n; ++i) fused = fused && jobs[i].M >= e->fuse_ln_min_rows;
   if (!fused || n == 1) {
     for (int i = 0; i < n; ++i)
@@ -633,21 +609,7 @@ int gemm_res_ln_group(m3pc_engine* e, const ResLnJob* jobs, int n, const float* 
       lj[i] = LnJob{reinterpret_cast<const __nv_bfloat16*>(j.A), j.w16, j.X, reinterpret_cast<__nv_bfloat16*>(j.Y), j.table, j.rpg, j.M, j.res_src};
       flops += 2.0 * j.M * static_cast<double>(D) * K;
     }
-    size_t slot = 0;
-    if (e->profile) {
-      slot = e->prof_used++;
-      if (slot >= e->prof_events.size()) {
-        cudaEvent_t a, c;
-        M3PC_CHECK_CUDA(cudaEventCreate(&a));
-        M3PC_CHECK_CUDA(cudaEventCreate(&c));
-        e->prof_events.push_back({a, c});
-        e->prof_flops.push_back(0.0);
-      }
-      e->prof_flops[slot] = flops;
-      M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].first, st));
-    }
-    M3PC_TRY(gemm_ln_bf16_grouped(lj, m, bias, g, b, K, st));
-    if (e->profile) M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].second, st));
+    M3PC_TRY(profiled(e, flops, st, [&] { return gemm_ln_bf16_grouped(lj, m, bias, g, b, K, st); }));
   }
   return M3PC_OK;
 }
@@ -659,47 +621,9 @@ struct PostLn {
   void* y = nullptr;
 };
 
-// X += W2 GELU(W1 Y + b1) + b2 in ONE kernel with the 4D-wide hidden kept on chip (mlp_fused.cu), where it applies: bf16 mode,
-// n_embd 512, and -- like the fused residual + LayerNorm kernel -- from fuse_ln_min_rows rows up, so that the kernel choice does not
-// depend on how candidates are chunked or sharded.  Returns M3PC_OK + *done = true when it ran.
-int mlp_fused(m3pc_engine* e, const LayerW& w, const void* Y, float* X, int rows, cudaStream_t st, bool* done) {
-  *done = false;
-  if (!(e->bf16 && e->fuse_mlp && e->D == 512 && e->F == 2048 && rows >= e->fuse_ln_min_rows)) return M3PC_OK;
-  size_t slot = 0;
-  if (e->profile) {
-    slot = e->prof_used++;
-    if (slot >= e->prof_events.size()) {
-      cudaEvent_t a, c;
-      M3PC_CHECK_CUDA(cudaEventCreate(&a));
-      M3PC_CHECK_CUDA(cudaEventCreate(&c));
-      e->prof_events.push_back({a, c});
-      e->prof_flops.push_back(0.0);
-    }
-    e->prof_flops[slot] = 2.0 * 2.0 * rows * static_cast<double>(e->D) * e->F;
-    M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].first, st));
-  }
-  M3PC_TRY(mlp_fused_bf16(reinterpret_cast<const __nv_bfloat16*>(Y), w.l1_w16, w.l1_b, w.l2_w16, w.l2_b, X, rows, st));
-  if (e->profile) M3PC_CHECK_CUDA(cudaEventRecord(e->prof_events[slot].second, st));
-  *done = true;
-  return M3PC_OK;
-}
-
 // second half of a pre-LN transformer block on `rows` token-major rows: expects Y = LN2(X); X += MLP(Y); then `post` (optional)
 int mlp_half(m3pc_engine* e, const LayerW& w, int rows, cudaStream_t st, const PostLn& post) {
   const int D = e->D, F = e->F;
-  bool fused = false;
-  M3PC_TRY(mlp_fused(e, w, e->Y.p, e->X.as<float>(), rows, st, &fused));
-  if (fused) {
-    if (post.y == nullptr) return M3PC_OK;
-    LnParams ln{};
-    ln.x = e->X.as<float>();
-    ln.rows = rows;
-    ln.g1 = post.g;
-    ln.b1 = post.b;
-    ln.y1 = post.y;
-    ln.rows_per_group = 1;
-    return launch_layernorm(ln, D, e->bf16, st);
-  }
   GemmEpilogue ep;
   ep.bias = w.l1_b;
   ep.flags = EPI_GELU;
@@ -988,7 +912,7 @@ int restricted_last_layer(m3pc_engine* e, const FwdIO& io, const LayerW& w, cons
     }
     qi += len;
   }
-  bool per_run = e->bf16 && e->fuse_ln && D == 512 && rows >= e->split_residual_min_rows;  // and every run large enough for the fused kernel
+  bool per_run = e->bf16 && D == 512 && rows >= e->split_residual_min_rows;  // and every run large enough for the fused kernel
   for (int r = 0; r < n_runs; ++r) per_run = per_run && static_cast<long>(runs[r].len) * Bc >= e->fuse_ln_min_rows;
   if (per_run) {
     ResLnJob jobs[MAX_TOK];
@@ -1016,18 +940,14 @@ int restricted_last_layer(m3pc_engine* e, const FwdIO& io, const LayerW& w, cons
     M3PC_TRY(launch_fill_rows(fp, D, e->XS.as<float>(), st));
     M3PC_TRY(gemm_res_ln(e, e->ATT.p, w.out_w, w.out_w16, w.out_b, e->XS.as<float>(), e->Y.p, w.n2_w, w.n2_b, nullptr, 1, rows, D, st));
   }
-  bool fused_mlp_done = false;
-  M3PC_TRY(mlp_fused(e, w, e->Y.p, e->XS.as<float>(), rows, st, &fused_mlp_done));
-  if (!fused_mlp_done) {
-    ge = GemmEpilogue{};
-    ge.bias = w.l1_b;
-    ge.flags = EPI_GELU;
-    M3PC_TRY(gemm(e, e->Y.p, w.l1_w, w.l1_w16, e->HID.p, rows, F, D, ge, st));
-    ge = GemmEpilogue{};
-    ge.bias = w.l2_b;
-    ge.flags = EPI_RESIDUAL;
-    M3PC_TRY(gemm(e, e->HID.p, w.l2_w, w.l2_w16, e->XS.p, rows, D, F, ge, st));
-  }
+  ge = GemmEpilogue{};
+  ge.bias = w.l1_b;
+  ge.flags = EPI_GELU;
+  M3PC_TRY(gemm(e, e->Y.p, w.l1_w, w.l1_w16, e->HID.p, rows, F, D, ge, st));
+  ge = GemmEpilogue{};
+  ge.bias = w.l2_b;
+  ge.flags = EPI_RESIDUAL;
+  M3PC_TRY(gemm(e, e->HID.p, w.l2_w, w.l2_w16, e->XS.p, rows, D, F, ge, st));
   // (h) norms + heads
   M3PC_TRY(final_norms(e, e->XS.as<float>(), need.n, need.tok, Bc, st, io.out_mu != nullptr && need.nt[M3PC_ACTIONS] > 0));
   return heads(e, io, need, e->Y.p, e->Y2.p, b0, Bc, st);
@@ -1048,7 +968,7 @@ int decode_restricted(m3pc_engine* e, const FwdIO& io, const void* enc_out, cons
     j += len;
   }
   // every run must be large enough for the fused kernel, so that one batch size always takes one path
-  if (e->bf16 && e->fuse_ln && D == 512 && static_cast<long>(min_run) * Bc >= e->fuse_ln_min_rows) {
+  if (e->bf16 && D == 512 && static_cast<long>(min_run) * Bc >= e->fuse_ln_min_rows) {
     // (a) + (b) in one kernel per run of kept tokens of a modality: X = dec_cvec[token] + enc_out W_dec^T (compact, encoder order),
     // Y = LN1(X) -- the table-residual form of the fused residual GEMM + LayerNorm kernel (no residual traffic at all)
     const size_t ab = act_bytes(e);
@@ -1236,7 +1156,6 @@ int forward_chunk(m3pc_engine* e, const FwdIO& io, int b0, int Bc, cudaStream_t 
     fp.QKV = e->QKV.as<__nv_bfloat16>(); fp.ATT = e->ATT.as<__nv_bfloat16>(); fp.HID = e->HID.as<__nv_bfloat16>();
     fp.Y = e->Y.as<__nv_bfloat16>(); fp.Y2 = e->Y2.as<__nv_bfloat16>();
     fp.bar = e->fb_bar.as<unsigned>();
-    { static const bool tr = tune_env("M3PC_FB_TRACE") != nullptr; fp.trace = tr ? 1 : 0; }
     // the actor head is folded into the kernel's last phase; the MLP heads of the other modalities keep their own launches
     FwdIO io_rest = io;
     if (io.out_mu != nullptr && need.nt[M3PC_ACTIONS] > 0) {
@@ -1256,7 +1175,7 @@ int forward_chunk(m3pc_engine* e, const FwdIO& io, int b0, int Bc, cudaStream_t 
   // shared-history analysis: the leading encoder tokens whose source row is shared by whole groups of batch rows (one window
   // for the whole batch: bstride 0; one window per environment: bdiv rows each) -- the chunk must hold whole groups
   int n_sh = 0, grp = 0;
-  if (e->dedupe_history && e->Le >= 1 && Bc >= 64) {
+  if (e->Le >= 1 && Bc >= 64) {
     for (int s = 0; s < S; ++s) {
       const EmbedTok& tk = ep.tok[s];
       const int g = tk.bdiv > 0 ? tk.bdiv : (tk.bstride == 0 ? Bc : 0);
@@ -1646,13 +1565,6 @@ int create(m3pc_handle_t* out, const m3pc_config_t* cfg) {
   M3PC_TRY(e->fb_xd.alloc(static_cast<size_t>(FB_MAX_ROWS) * D * 4));
   M3PC_TRY(e->fb_bar.alloc(16));
   M3PC_CHECK_CUDA(cudaMemset(e->fb_bar.p, 0, 16));
-  if (const char* g = tune_env("M3PC_NO_FUSED_B1")) e->use_fused_b1 = !(g[0] == '1');
-  if (const char* g = tune_env("M3PC_NO_FUSED_LN")) e->fuse_ln = !(g[0] == '1');
-  if (const char* g = tune_env("M3PC_FUSED_LN_MIN_ROWS")) e->fuse_ln_min_rows = std::max(129, atoi(g));
-  if (const char* g = tune_env("M3PC_DEC_FULL")) e->restrict_deep = !(g[0] == '1');
-  if (const char* g = tune_env("M3PC_NO_DEDUPE")) e->dedupe_history = !(g[0] == '1');
-  if (const char* g = tune_env("M3PC_NO_GRAPHS")) e->use_graphs = !(g[0] == '1');
-  if (const char* g = tune_env("M3PC_NO_PDL")) g_use_pdl = !(g[0] == '1');
   M3PC_CHECK_CUDA(cudaEventCreate(&e->ev0));
   M3PC_CHECK_CUDA(cudaEventCreate(&e->ev1));
   M3PC_CHECK_CUDA(cudaDeviceSynchronize());
@@ -1703,15 +1615,11 @@ int m3pc_set_option(m3pc_handle_t h, const char* name, int32_t value) {
   const std::string n(name);
   h->drop_graphs();  // the launch sequence a graph froze may no longer be the selected one
   if (n == "graphs") h->use_graphs = value != 0;
-  else if (n == "pdl") m3pc::g_use_pdl = value != 0;
   else if (n == "fused_b1") h->use_fused_b1 = value != 0;
-  else if (n == "fused_ln") h->fuse_ln = value != 0;
-  else if (n == "fused_mlp") h->fuse_mlp = value != 0;
   else if (n == "grouped_ln") h->group_ln = value != 0;
   else if (n == "fused_ln_min_rows") h->fuse_ln_min_rows = std::max(129, static_cast<int>(value));
   else if (n == "restrict_deep_decoder") h->restrict_deep = value != 0;
   else if (n == "split_residual_min_rows") h->split_residual_min_rows = std::max(0, static_cast<int>(value));
-  else if (n == "dedupe_history") h->dedupe_history = value != 0;
   else if (n == "gemm_ln_unit_rows") {
     M3PC_REQUIRE(value == 0 || value == 128 || value == 256, "gemm_ln_unit_rows must be 0 (per launch), 128 or 256");
     m3pc::g_ln_unit_rows = value;
@@ -1898,11 +1806,6 @@ int m3pc_gemm_ln_bf16(const void* A, const void* W, const float* bias, float* X,
                       const float* table, int32_t rows_per_group, int32_t M, int32_t K, void* stream) {
   return m3pc::gemm_ln_bf16(reinterpret_cast<const __nv_bfloat16*>(A), reinterpret_cast<const __nv_bfloat16*>(W), bias, X,
                             reinterpret_cast<__nv_bfloat16*>(Y), gamma, beta, table, rows_per_group, M, K, reinterpret_cast<cudaStream_t>(stream));
-}
-
-int m3pc_mlp_fused_bf16(const void* Y, const void* W1, const float* b1, const void* W2, const float* b2, float* X, int32_t M, void* stream) {
-  return m3pc::mlp_fused_bf16(reinterpret_cast<const __nv_bfloat16*>(Y), reinterpret_cast<const __nv_bfloat16*>(W1), b1,
-                              reinterpret_cast<const __nv_bfloat16*>(W2), b2, X, M, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_gemm_fp32(const float* A, const float* W, const float* bias, float* C, int32_t M, int32_t N, int32_t K, int32_t flags, void* stream) {

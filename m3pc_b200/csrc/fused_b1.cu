@@ -268,17 +268,6 @@ __device__ __forceinline__ void attend_pair(QF qf, KF kf, VF vf, int n_kv, int l
   }
 }
 
-#define FB_STAMP()                                                                                      \
-  do {                                                                                                  \
-    if (p.trace && blockIdx.x == 0 && threadIdx.x == 0 && n_stamp < 48) stamps[n_stamp++] = clock64(); \
-  } while (0)
-#define FB_SYNC()      \
-  do {                 \
-    FB_STAMP();        \
-    grid_sync(p.bar, bar_target);  \
-    FB_STAMP();        \
-  } while (0)
-
 template <int NJ>
 __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_constant__ FusedB1Params p) {
   constexpr int D = NJ * 128, F = 4 * D, H = D / 128;
@@ -289,12 +278,9 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int G = gridDim.x;
   const int S = p.S;
-  long long stamps[48];
-  int n_stamp = 0;
   WSlab ws;
   unsigned bar_target = 0;
   PDL_PROLOGUE();  // launched without the PDL attribute (cooperative), but its successor may be pre-staged
-  FB_STAMP();
   // weights of this CTA's first work item of the next GEMM phase: in flight while the activation prologue runs
   auto prefetch = [&](const __nv_bfloat16* W, int K, int N) {
     const bool mine = static_cast<int>(blockIdx.x) < N / 8;
@@ -345,7 +331,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
     rows_gemm(a_s, LD1, 0, S, D, w.in_w, 3 * D, w.in_b, nullptr, 0, red, ws, pf, [&](int m, int n, float v, float) {
       p.QKV[static_cast<size_t>(m) * 3 * D + n] = __float2bfloat16_rn(v);
     });
-    FB_SYNC();
+    grid_sync(p.bar, bar_target);
     // ---- phase B: self-attention, one (row, head) pair per warp ----
     pf = prefetch(w.out_w, D, D);
     for (int pr = warp * G + blockIdx.x; pr < S * H; pr += FB_WARPS * G) {
@@ -356,7 +342,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
                   [&](int j) { return p.QKV + static_cast<size_t>(j) * 3 * D + 2 * D + h * 128; }, S, lane, o);
       *reinterpret_cast<uint2*>(p.ATT + static_cast<size_t>(r) * D + h * 128 + lane * 4) = f4_to_bf4(o);
     }
-    FB_SYNC();
+    grid_sync(p.bar, bar_target);
     // ---- phase C: x += att W_out^T + b ----
     copy_rows_to_smem(p.ATT, S, D, a_s);
     __syncthreads();
@@ -364,7 +350,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
       p.X[static_cast<size_t>(m) * D + n] = r + v;
     });
     pf = prefetch(w.l1_w, D, F);
-    FB_SYNC();
+    grid_sync(p.bar, bar_target);
     // ---- phase D: hid = gelu(LN2(x) W1^T + b1) ----
     ln_rows_to_smem<NJ>(p.X, S, w.n2_w, w.n2_b, a_s, LD1);
     __syncthreads();
@@ -372,14 +358,14 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
       p.HID[static_cast<size_t>(m) * F + n] = __float2bfloat16_rn(gelu_erf_fast(v));
     });
     pf = prefetch(w.l2_w, F, D);
-    FB_SYNC();
+    grid_sync(p.bar, bar_target);
     // ---- phase E: x += hid W2^T + b2 ----
     copy_rows_to_smem(p.HID, S, F, a_s);
     __syncthreads();
     rows_gemm(a_s, LD4, 0, S, F, w.l2_w, D, w.l2_b, p.X, D, red, ws, pf, [&](int m, int n, float v, float r) {
       p.X[static_cast<size_t>(m) * D + n] = r + v;
     });
-    FB_SYNC();
+    grid_sync(p.bar, bar_target);
   }
 
   // ================================================================= decoder (single layer, needed rows only)
@@ -396,14 +382,14 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
       });
   }
   bool pf = prefetch(w.in_w, D, 3 * D);
-  FB_SYNC();
+  grid_sync(p.bar, bar_target);
   // ---- phase G: [Q | K | V] of the kept tokens = LN1(xd) W_in^T + b ----
   ln_rows_to_smem<NJ>(p.Xd, S, w.n1_w, w.n1_b, a_s, LD1);
   __syncthreads();
   rows_gemm(a_s, LD1, 0, S, D, w.in_w, 3 * D, w.in_b, nullptr, 0, red, ws, pf, [&](int m, int n, float v, float) {
     p.QKV[static_cast<size_t>(m) * 3 * D + n] = __float2bfloat16_rn(v);
   });
-  FB_SYNC();
+  grid_sync(p.bar, bar_target);
   // ---- phase H: needed queries x all 4T keys (mask-token rows from the batch-constant table); residual rows -> XS ----
   pf = prefetch(w.out_w, D, D);
   for (int pr = warp * G + blockIdx.x; pr < NQ * H; pr += FB_WARPS * G) {
@@ -420,7 +406,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
     const float* res = sq < 0 ? p.dec_maskrow + static_cast<size_t>(jq) * D : p.Xd + static_cast<size_t>(sq) * D;
     *reinterpret_cast<float4*>(p.XS + static_cast<size_t>(qi) * D + h * 128 + lane * 4) = ldcg4(res + h * 128 + lane * 4);
   }
-  FB_SYNC();
+  grid_sync(p.bar, bar_target);
   // ---- phase I: xs += att W_out^T + b ----
   copy_rows_to_smem(p.ATT, NQ, D, a_s);
   __syncthreads();
@@ -428,7 +414,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
     p.XS[static_cast<size_t>(m) * D + n] = r + v;
   });
   pf = prefetch(w.l1_w, D, F);
-  FB_SYNC();
+  grid_sync(p.bar, bar_target);
   // ---- phase J: hid = gelu(LN2(xs) W1^T + b1) ----
   ln_rows_to_smem<NJ>(p.XS, NQ, w.n2_w, w.n2_b, a_s, LD1);
   __syncthreads();
@@ -436,14 +422,14 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
     p.HID[static_cast<size_t>(m) * F + n] = __float2bfloat16_rn(gelu_erf_fast(v));
   });
   pf = prefetch(w.l2_w, F, D);
-  FB_SYNC();
+  grid_sync(p.bar, bar_target);
   // ---- phase K: xs += hid W2^T + b2 ----
   copy_rows_to_smem(p.HID, NQ, F, a_s);
   __syncthreads();
   rows_gemm(a_s, LD4, 0, NQ, F, w.l2_w, D, w.l2_b, p.XS, D, red, ws, pf, [&](int m, int n, float v, float r) {
     p.XS[static_cast<size_t>(m) * D + n] = r + v;
   });
-  FB_SYNC();
+  grid_sync(p.bar, bar_target);
   // ---- phase L: y = final decoder norm, y2 = the consuming head's own LayerNorm of y (mtm_model.py:397-409, 428-433) ----
   for (int qi = warp * G + blockIdx.x; qi < NQ; qi += FB_WARPS * G) {
     float4 v[NJ], o[NJ];
@@ -495,12 +481,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
       }
     }
   }
-  FB_STAMP();
   grid_finish(p.bar);
-  if (p.trace && blockIdx.x == 0 && threadIdx.x == 0) {
-    for (int i = 1; i < n_stamp; ++i) printf("fb_trace %2d %s %6lld cycles\n", i, (i & 1) ? "work" : "sync", stamps[i] - stamps[i - 1]);
-    printf("fb_trace total %lld cycles\n", stamps[n_stamp - 1] - stamps[0]);
-  }
 }
 
 }  // namespace

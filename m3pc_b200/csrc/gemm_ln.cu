@@ -67,8 +67,6 @@ struct LnGemmParams {
   const float* gamma;
   const float* beta;
   int n, num_kb, n_units;
-  int tune;  // tuning build only (timing experiments, results are garbage): bit 0 = no residual loads, bit 1 = no X store,
-             // bit 2 = no Y store (pass 2 only drains TMEM), bit 3 = epilogue only hands the accumulator back
 };
 static_assert(sizeof(LnGemmParams) <= 4000, "kernel parameter space");
 
@@ -240,11 +238,6 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
     uint32_t rph = 0;  // bit b: parity of rbar[b]
     const uint32_t acc_empty_leader = mapa_u32(smem_u32(&acc_empty[0]), 0);
     const uint32_t sw = static_cast<uint32_t>((lane >> 1) & 3);  // SWIZZLE_64B: 16-byte chunk j of row r lives at j ^ ((r >> 1) & 3)
-#ifdef M3PC_TUNING
-    const int tune = P.tune;
-#else
-    constexpr int tune = 0;
-#endif
     const float* sbias = sconst;
     const float* sgamma = sconst + LN_N;
     const float* sbeta = sconst + 2 * LN_N;
@@ -259,10 +252,10 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
     for (int u = pair; u < P.n_units; u += n_pairs, ++it) {
       const uint32_t buf = static_cast<uint32_t>(it % NACC);
       const LnProblem& Q = P.p[ln_problem_of(P, u)];
-      const bool from_x = Q.table == nullptr && !(tune & 1);
+      const bool from_x = Q.table == nullptr;
       const int row0 = ((u - Q.unit0) * 2 + static_cast<int>(crank)) * (ROWS / 2) + rowq * 32;
       const int row = row0 + lane;
-      const bool live = row0 < Q.M && !(tune & 8);
+      const bool live = row0 < Q.M;
       const uint32_t tacc = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + buf * ACC_COLS + tcol;
       // residual boxes travel to shared memory while the MMAs of this unit (and the epilogue of the previous one) still run
       if (from_x) ns = 0;
@@ -320,7 +313,7 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
           fence_proxy_async();
           __syncwarp();
           if (lane == 0) {
-            if (!(tune & 2)) tma_store_2d(&Q.tx, bx, col0, row0);
+            tma_store_2d(&Q.tx, bx, col0, row0);
             bulk_commit();
             if (from_x && ci + NBOX < NB1) {  // this buffer is needed again for a later residual box of the unit
               bulk_wait_read<0>();
@@ -387,7 +380,7 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
           fence_proxy_async();
           __syncwarp();
           if (lane == 0) {
-            if (!(tune & 4)) tma_store_2d(&Q.ty, bx, col0, row0);
+            tma_store_2d(&Q.ty, bx, col0, row0);
             bulk_commit();
           }
           ++ns;
@@ -438,7 +431,7 @@ int launch_ln(LnGemmParams& P, cudaStream_t st) {
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = g_use_pdl ? 2 : 1;
+  cfg.numAttrs = 2;
   M3PC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, P));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
@@ -459,7 +452,6 @@ int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const floa
   M3PC_REQUIRE(gamma && beta, "gemm_ln: null operand");
   M3PC_TRY(gemm_init_driver_api());
   int rows = g_ln_unit_rows;
-  if (const char* t = tune_env("M3PC_LN_UNIT_ROWS")) rows = atoi(t);  // tuning build: A/B without a handle
   if (rows != 128 && rows != 256) {
     const int pairs = std::max(1, device_num_sms() / 2);
     int u256 = 0, u128 = 0;
@@ -491,7 +483,6 @@ int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const floa
   }
   P.bias = bias; P.gamma = gamma; P.beta = beta;
   P.num_kb = K / BK;
-  if (const char* t = tune_env("M3PC_TUNE_LN")) P.tune = atoi(t);
   return rows == 128 ? launch_ln<128, 3, 2>(P, st) : launch_ln<256, 3, 2>(P, st);
 }
 

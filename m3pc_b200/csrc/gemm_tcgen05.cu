@@ -25,7 +25,6 @@
 #include <cuda.h>
 
 #include <cmath>
-#include <cstdlib>
 
 #include "common.cuh"
 #include "tcgen05.cuh"
@@ -42,15 +41,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 EncodeTiledFn g_encode_tiled = nullptr;
-int g_force_bn = 0, g_force_cl = 0;  // tuning build: M3PC_GEMM_CONFIG="<bn>x<cl>" pins one single-CTA configuration (tuning / tests)
-#ifdef M3PC_TUNING
-int g_debug_skip_epi = 0;             // tuning build only, M3PC_GEMM_DEBUG_SKIP_EPI=1: the epilogue warps only hand the accumulator back (results are garbage)
-constexpr int EPI_DEBUG_SKIP = 1 << 30;
-#else
-constexpr int g_debug_skip_epi = 0;
-constexpr int EPI_DEBUG_SKIP = 0;     // the release library has no result-corrupting switch
-#endif
-int g_use_2sm = 1;                   // tuning build: M3PC_GEMM_2SM=0 disables the CTA-pair kernel
 
 struct EpiParams {
   const float* bias;
@@ -329,9 +319,7 @@ struct Smem2 {
 
 // Grouped launches: up to MAX_GROUP independent problems (own operands, output, epilogue, shapes) share one launch; the pair's
 // unit range simply runs across problem boundaries, so several small GEMMs of the decoder / heads / critic cost one kernel
-// boundary instead of one each.  Split-K (ksplit = 2, residual epilogue only): a unit is one K half of an output tile and
-// both halves are reduce-added into the fp32 residual stream by the TMA (bias / row table ride on half 0) -- used where
-// whole tiles would leave most pairs idle in the last round (N = D GEMMs with K = 4 D at ~1024 batch rows).
+// boundary instead of one each.
 constexpr int MAX_GROUP = 4;
 struct alignas(64) GroupProblem {
   CUtensorMap ta, tw, tc;
@@ -339,18 +327,15 @@ struct alignas(64) GroupProblem {
   const float* table;
   int rows_per_group, flags;
   int M, n_tiles;  // rows; N / 256
-  int num_kb;      // k-blocks per unit (K / 64 / ksplit)
-  int ksplit;      // 1 or 2
+  int num_kb;      // k-blocks (K / 64)
   int unit0;       // first unit of this problem in the launch-wide unit order
 };
 struct GroupParams {
   GroupProblem p[MAX_GROUP];
   int n, total_units;
   int strided;  // 1: pair p works on units p, p + n_pairs, ... (see launch_2sm) instead of one contiguous range
-  int tune;     // tuning build only (timing experiments, results are garbage): bit 0 = load A for a pair's first unit only,
-                // bit 1 = load W for a pair's first unit only
 };
-struct UnitCoord { int g, mp, nt, ks; };
+struct UnitCoord { int g, mp, nt; };
 __device__ __forceinline__ UnitCoord decode_unit(const GroupParams& gp, int u) {
   UnitCoord c;
   c.g = 0;
@@ -358,11 +343,11 @@ __device__ __forceinline__ UnitCoord decode_unit(const GroupParams& gp, int u) {
   for (int i = 1; i < MAX_GROUP; ++i)
     if (i < gp.n && u >= gp.p[i].unit0) c.g = i;
   const GroupProblem& P = gp.p[c.g];
-  int lu = u - P.unit0;
-  c.ks = 0;
-  if (P.ksplit == 2) { c.ks = lu & 1; lu >>= 1; }
-  c.mp = lu / P.n_tiles;
-  c.nt = lu - c.mp * P.n_tiles;
+  // unsigned: a unit index is never negative, and the signed division's sign fix-up costs registers the epilogue warps need
+  // for their per-unit state (with it, ptxas spills that state to local memory)
+  const unsigned lu = static_cast<unsigned>(u - P.unit0), nt = static_cast<unsigned>(P.n_tiles);
+  c.mp = static_cast<int>(lu / nt);
+  c.nt = static_cast<int>(lu - static_cast<unsigned>(c.mp) * nt);
   return c;
 }
 
@@ -429,19 +414,13 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
         const UnitCoord uc = decode_unit(gp, u);
         const GroupProblem& P = gp.p[uc.g];
         const int m0 = (uc.mp * 2 + static_cast<int>(crank)) * BM, n0 = uc.nt * BN + static_cast<int>(crank) * 128;
-        const int num_kb = P.num_kb, k0 = uc.ks * num_kb;
-#ifdef M3PC_TUNING
-        const bool load_a = !(gp.tune & 1) || u == u_lo, load_w = !(gp.tune & 2) || u == u_lo;
-#else
-        constexpr bool load_a = true, load_w = true;
-#endif
-        for (int kb = 0; kb < num_kb; ++kb) {
+        for (int kb = 0; kb < P.num_kb; ++kb) {
           mbar_wait(&empty_bar[s], ph ^ 1);
-          if (leader) mbar_arrive_expect_tx(&full_bar[s], 2u * ((load_a ? L::kABlk : 0) + (load_w ? L::kBBlk : 0)));
+          if (leader) mbar_arrive_expect_tx(&full_bar[s], 2u * L::kStageBytes);
           uint8_t* dst = smem + s * L::kStageBytes;
           const uint32_t bar = full_leader + 8u * static_cast<uint32_t>(s);
-          if (load_a) tma_load_2d_2sm(dst, &P.ta, bar, (k0 + kb) * BK, m0);
-          if (load_w) tma_load_2d_2sm(dst + L::kABlk, &P.tw, bar, (k0 + kb) * BK, n0);
+          tma_load_2d_2sm(dst, &P.ta, bar, kb * BK, m0);
+          tma_load_2d_2sm(dst + L::kABlk, &P.tw, bar, kb * BK, n0);
           if (++s == STAGES) { s = 0; ph ^= 1; }
         }
       }
@@ -489,11 +468,9 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
       const GroupProblem& P = gp.p[uc.g];
       const CUtensorMap* tmap_c = &P.tc;
       const int M = P.M, N = P.n_tiles * BN;
-      const bool first_k = uc.ks == 0;  // split-K: bias and row table are added by the first K half only
-      EpiParams ep{first_k ? P.bias : nullptr, first_k ? P.table : nullptr, P.rows_per_group, P.flags};
+      EpiParams ep{P.bias, P.table, P.rows_per_group, P.flags};
       const bool do_gelu = ep.flags & EPI_GELU, do_relu = ep.flags & EPI_RELU, do_res = ep.flags & EPI_RESIDUAL;
       const bool out_f32 = do_res || (ep.flags & EPI_OUT_F32);
-      const bool skip = ep.flags & EPI_DEBUG_SKIP;
       const int cw = out_f32 ? 16 : 32;  // columns per staged chunk (64 bytes of output)
       const int row0 = (uc.mp * 2 + static_cast<int>(crank)) * BM + quarter * 32;
       const int colw = uc.nt * BN + cgrp * 64;  // first column of this warp's share
@@ -508,7 +485,7 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
       const uint32_t aph = (it >> 1) & 1;
       mbar_wait(&acc_full[a], aph);
       tc_fence_after();
-      const bool live = row0 < M && !skip;
+      const bool live = row0 < M;
       const int row = row0 + lane;
       const uint32_t tacc = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + static_cast<uint32_t>(a * BN + cgrp * 64);
       if (live) {
@@ -601,7 +578,7 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
           }
           ++nstore;
         }
-      } else {  // nothing to store (rows beyond M, or the tuning switch): just release the accumulator
+      } else {  // nothing to store (rows beyond M): just release the accumulator
         tc_fence_before();
         if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * static_cast<uint32_t>(a));
       }
@@ -663,7 +640,7 @@ int launch(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, int M, int N
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = g_use_pdl ? 2 : 1;
+  cfg.numAttrs = 2;
   M3PC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_kernel<BN, STAGES, CL>, ta, tw, C, M, N, K, ep));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
@@ -688,9 +665,6 @@ int make_tmap_out(CUtensorMap* map, void* ptr, uint64_t rows, uint64_t cols, boo
 }
 namespace {
 
-int g_use_strided = 1;  // tuning build: M3PC_GEMM_STRIDED=0 restores contiguous unit ranges for every problem
-int g_use_splitk = 0;  // tuning build: M3PC_GEMM_SPLITK=1 enables split-K (measured +0.4% plans/s at 1024 candidates; off by default: the reduce-add order of the two halves is not reproducible run to run)
-
 // One launch of the CTA-pair kernel over `n` problems (n <= MAX_GROUP; every N a multiple of 256).
 template <int STAGES>
 int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
@@ -709,34 +683,23 @@ int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
   for (int g = 0; g < n; ++g) {
     const GemmProblem& q = probs[g];
     GroupProblem& P = gp.p[g];
-    const bool res = (q.epi.flags & EPI_RESIDUAL) != 0;
-    const bool out_f32 = res || (q.epi.flags & EPI_OUT_F32) != 0;
+    const bool out_f32 = (q.epi.flags & (EPI_RESIDUAL | EPI_OUT_F32)) != 0;
     M3PC_TRY(make_tmap(&P.ta, q.A, static_cast<uint64_t>(q.M), static_cast<uint64_t>(q.K), BM));
     M3PC_TRY(make_tmap(&P.tw, q.W, static_cast<uint64_t>(q.N), static_cast<uint64_t>(q.K), 128));
     M3PC_TRY(make_tmap_out(&P.tc, q.C, static_cast<uint64_t>(q.M), static_cast<uint64_t>(q.N), out_f32));
     P.bias = q.epi.bias;
     P.table = q.epi.table;
     P.rows_per_group = q.epi.rows_per_group > 0 ? q.epi.rows_per_group : 1;
-    P.flags = q.epi.flags | (g_debug_skip_epi ? EPI_DEBUG_SKIP : 0);
+    P.flags = q.epi.flags;
     P.M = q.M;
     P.n_tiles = q.N / 256;
-    const int tiles = P.n_tiles * ceil_div(q.M, 2 * BM);
-    // split K in two where whole tiles quantise badly: single-problem residual GEMMs with a long K whose last round would
-    // leave most pairs idle (e.g. 104 tiles on 74 pairs: 2 rounds of whole tiles vs 3 rounds of half tiles)
-    P.ksplit = 1;
-    if (g_use_splitk && n == 1 && res && q.K >= 1024 && (q.K / BK) % 2 == 0) {
-      const double r1 = std::ceil(static_cast<double>(tiles) / n_pairs_max);
-      const double r2 = 0.5 * std::ceil(2.0 * tiles / n_pairs_max);
-      if (r2 + 0.25 <= r1) P.ksplit = 2;
-    }
-    P.num_kb = q.K / BK / P.ksplit;
+    P.num_kb = q.K / BK;
     P.unit0 = units;
-    units += tiles * P.ksplit;
+    units += P.n_tiles * ceil_div(q.M, 2 * BM);
   }
   gp.total_units = units;
-  if (const char* t = tune_env("M3PC_TUNE_GEMM")) gp.tune = atoi(t);
   const int pairs = std::min(units, n_pairs_max);
-  gp.strided = g_use_strided && n == 1 && gp.p[0].n_tiles == 2 && gp.p[0].ksplit == 1 && probs[0].K >= 1024 && pairs % 2 == 0 && units >= 2 * pairs;
+  gp.strided = n == 1 && gp.p[0].n_tiles == 2 && probs[0].K >= 1024 && pairs % 2 == 0 && units >= 2 * pairs;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(2 * pairs);
   cfg.blockDim = dim3(GEMM_THREADS_2SM);
@@ -750,7 +713,7 @@ int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = g_use_pdl ? 2 : 1;
+  cfg.numAttrs = 2;
   M3PC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_2sm_kernel<STAGES>, gp));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
@@ -781,16 +744,6 @@ int gemm_init_driver_api() {
     return M3PC_ERR_CUDA;
   }
   g_encode_tiled = reinterpret_cast<EncodeTiledFn>(fn);
-  if (const char* f = tune_env("M3PC_GEMM_2SM")) g_use_2sm = atoi(f);
-  if (const char* f = tune_env("M3PC_GEMM_SPLITK")) g_use_splitk = atoi(f);
-  if (const char* f = tune_env("M3PC_GEMM_STRIDED")) g_use_strided = atoi(f);
-#ifdef M3PC_TUNING
-  if (const char* f = tune_env("M3PC_GEMM_DEBUG_SKIP_EPI")) g_debug_skip_epi = atoi(f);
-#endif
-  if (const char* f = tune_env("M3PC_GEMM_CONFIG")) {
-    if (sscanf(f, "%dx%d", &g_force_bn, &g_force_cl) != 2 || (g_force_bn != 128 && g_force_bn != 256) || (g_force_cl != 1 && g_force_cl != 2))
-      g_force_bn = g_force_cl = 0;
-  }
   return M3PC_OK;
 }
 
@@ -805,7 +758,7 @@ int gemm_bf16_tcgen05(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, i
   M3PC_TRY(gemm_init_driver_api());
   if (M <= 32 && static_cast<size_t>(M) * K * 2 <= 160 * 1024) return gemm_bf16_skinny(A, W, C, M, N, K, epi, st);
   // CTA-pair kernel wherever a pair has two row tiles to work on and N splits into 256-wide tiles
-  if (g_use_2sm && !g_force_bn && N % 256 == 0 && M > BM) {
+  if (N % 256 == 0 && M > BM) {
     const GemmProblem q{A, W, C, M, N, K, epi};
     return launch_2sm<4>(&q, 1, st);
   }
@@ -815,7 +768,6 @@ int gemm_bf16_tcgen05(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, i
   double best_t = 1e30;
   for (int i = 0; i < 4; ++i) {
     if (N % cands[i].bn != 0) continue;
-    if (g_force_bn && (cands[i].bn != g_force_bn || cands[i].cl != g_force_cl)) continue;
     const double t = model_time(M, N, K, cands[i].bn, cands[i].cl);
     if (t < best_t * 0.98) { best_t = t; best = i; }
   }
@@ -828,11 +780,11 @@ int gemm_bf16_tcgen05(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, i
 }
 
 // Several independent GEMMs in one launch (see GroupParams).  Falls back to one launch per problem where the CTA-pair
-// kernel does not apply (a problem with N % 256 != 0, only tiny M, pinned tuning configurations).
+// kernel does not apply (a problem with N % 256 != 0, only tiny M).
 int gemm_bf16_grouped(const GemmProblem* probs, int n, cudaStream_t st) {
   M3PC_REQUIRE(n >= 1, "gemm_bf16_grouped: no problems");
   M3PC_TRY(gemm_init_driver_api());
-  bool ok = g_use_2sm && !g_force_bn && n <= MAX_GROUP;
+  bool ok = n <= MAX_GROUP;
   int max_m = 0;
   for (int g = 0; g < n && ok; ++g) {
     const GemmProblem& q = probs[g];

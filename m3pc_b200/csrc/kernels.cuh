@@ -68,7 +68,6 @@ struct FusedB1Params {
   float *out_mu, *out_std;
   int act_dim;
   unsigned* bar;        // grid barrier state {count, generation}, zero-initialised once
-  int trace;            // debug: CTA 0 prints per-phase cycle counts (tuning build: M3PC_FB_TRACE=1)
 };
 size_t fused_b1_smem_bytes(int D, int S, int n_need);
 int launch_fused_b1(const FusedB1Params& p, int D, cudaStream_t st);

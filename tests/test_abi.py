@@ -66,8 +66,8 @@ def test_invalid_arguments_are_rejected_without_a_gpu(lib):
 
 
 def test_release_library_reads_no_environment_switch(lib):
-    """Tuning switches (kernel A/B selection, timing-only variants that corrupt results) exist only in the -DM3PC_TUNING build
-    (libm3pc_tuning.so); the shipped library holds no M3PC_* environment variable name and therefore reads none."""
+    """Launch choices go through m3pc_set_option only: the library holds no M3PC_* environment variable name and therefore
+    reads none."""
     assert nat.LIB_PATH.endswith("libm3pc.so")
     blob = open(nat.LIB_PATH, "rb").read()
     names = set(re.findall(rb"\x00(M3PC_[A-Z][A-Z0-9_]{3,})\x00", blob))  # a getenv() argument is a string of its own

@@ -221,28 +221,3 @@ def test_k8_score_select(nat, kind, temp, h):
     assert idx.tolist() == [int(torch.argmax(Jd)), int(torch.argmax(w / expq.double()))]
     assert torch.equal(sm.cpu(), cand[idx[1].item(), 0])
     assert float(part[0]) == float(Jd.max()) and abs(float(part[1]) - float(w.sum())) < 1e-3 * float(w.sum())
-
-
-@pytest.mark.parametrize("M", [129, 300, 1000, 13312, 106496 + 77])
-def test_fused_mlp_matches_the_two_launch_path(nat, M):
-    """m3pc_mlp_fused_bf16 (linear1 + GELU + linear2 + residual, hidden kept on chip) against the two tensor-core launches it
-    replaces -- bit for bit: same k order, same bf16 rounding of the hidden, same fp32 residual add -- and against fp64."""
-    L = nat.lib()
-    g = torch.Generator(device="cuda").manual_seed(M)
-    Y = torch.randn(M, 512, device="cuda", generator=g).bfloat16()
-    W1 = (torch.randn(2048, 512, device="cuda", generator=g) / 512 ** 0.5).bfloat16()
-    W2 = (torch.randn(512, 2048, device="cuda", generator=g) / 2048 ** 0.5).bfloat16()
-    b1, b2 = torch.randn(2048, device="cuda", generator=g), torch.randn(512, device="cuda", generator=g)
-    X0 = torch.randn(M, 512, device="cuda", generator=g)
-    hid = torch.full((M, 2048), float("nan"), device="cuda", dtype=torch.bfloat16)
-    Xa = X0.clone()
-    nat.check(L.m3pc_gemm_bf16(Y.data_ptr(), W1.data_ptr(), b1.data_ptr(), hid.data_ptr(), M, 2048, 512, 1, None))
-    nat.check(L.m3pc_gemm_bf16(hid.data_ptr(), W2.data_ptr(), b2.data_ptr(), Xa.data_ptr(), M, 512, 2048, 2, None))
-    Xb = X0.clone()
-    nat.check(L.m3pc_mlp_fused_bf16(Y.data_ptr(), W1.data_ptr(), b1.data_ptr(), W2.data_ptr(), b2.data_ptr(), Xb.data_ptr(), M, None))
-    torch.cuda.synchronize()
-    assert torch.isfinite(Xb).all()
-    ref = X0.double() + torch.nn.functional.gelu(Y.double() @ W1.double().T + b1.double()).bfloat16().double() @ W2.double().T + b2.double()
-    assert rel(Xb, ref) < 5e-3
-    assert rel(Xb, Xa) < 1e-6, "fused and two-launch results differ by more than fp32 rounding"
-    assert torch.equal(Xa, Xb)

@@ -867,16 +867,6 @@ def test_gemm_ln_unit_sizes_are_bit_identical(nat, M, K, table_rows):
     assert torch.equal(outs[0][0], outs[256][0]) and torch.equal(outs[0][1], outs[256][1])
 
 
-def test_plan_with_the_fused_mlp_kernel(monkeypatch):
-    """Option "fused_mlp" = 1 routes every MLP of pass 2 (encoder blocks, restricted decoder layer) through the on-chip-hidden kernel
-    (mlp_fused.cu, off by default because it is slower); the plan must still match the float64 oracle."""
-    from m3pc_b200.engine import PlanEngine
-    monkeypatch.setitem(PlanEngine.default_options, "fused_mlp", 1)
-    monkeypatch.setitem(PlanEngine.default_options, "fused_ln_min_rows", 129)
-    test_plan_internals_vs_fp64_oracle("bf16", "walker2d", "critic_lambda_guiding", 1.0, 130, 50)
-    test_plan_internals_vs_fp64_oracle("bf16", "hopper", "rtg_guiding", 0.01, 200, 50)
-
-
 def test_restricted_decoder_residual_sources_are_bit_identical():
     """The restricted decoder's out-projection takes its residual either from a copied row block (small batches) or, per run of
     needed tokens, straight from the batch-constant mask-token table / the kept token's residual-stream rows (large batches:

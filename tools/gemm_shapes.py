@@ -2,8 +2,7 @@
 """Hot GEMM shapes of one bench step (8 environments x 1024 candidates), hand-written kernels vs cuBLAS (torch.matmul /
 F.linear on the same bf16 operands), warm, CUDA events, L2 flushed between repetitions.
 
-    python tools/gemm_shapes.py [--json out.json]           release library
-    M3PC_LIB=tuning M3PC_TUNE_GEMM=1 python tools/gemm_shapes.py   tuning build: timing experiments (garbage results)
+    python tools/gemm_shapes.py [--json out.json]
 
 cuBLAS is the LIBRARY bar here (VERDICT r1 "What's missing" #1): it computes only the plain product (+ bias through
 F.linear); the fused epilogues (GELU, residual, LayerNorm) of the hand-written kernels would cost it extra launches.
@@ -75,4 +74,4 @@ for M in args.rows:
         rows.append(rec)
         print(" ".join(f"{k}={v:.1f}" if isinstance(v, float) else f"{k}={v}" for k, v in rec.items()), flush=True)
 if args.json:
-    json.dump({"tune_env": {k: v for k, v in os.environ.items() if k.startswith("M3PC_")}, "rows": rows}, open(args.json, "w"), indent=1)
+    json.dump({"rows": rows}, open(args.json, "w"), indent=1)

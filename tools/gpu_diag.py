@@ -97,12 +97,11 @@ def sec_gemm_bf16():
 
 
 def sec_gemm_bench():
-    """Time the tensor-core GEMM on the plan's shapes (CUDA events, warm L2, 20 reps) under the current M3PC_GEMM_CONFIG."""
+    """Time the tensor-core GEMM on the plan's shapes (CUDA events, warm L2, 20 reps)."""
     import torch
     from m3pc_b200 import _native as nat
     L = nat.lib()
     torch.manual_seed(0)
-    print("M3PC_GEMM_CONFIG =", os.environ.get("M3PC_GEMM_CONFIG", "(model)"))
     shapes = [("enc qkv", 13312, 1536, 512, 0), ("enc out", 13312, 512, 512, 2), ("enc ffn1", 13312, 2048, 512, 1), ("enc ffn2", 13312, 512, 2048, 2),
               ("dec kv", 13312, 1024, 512, 0), ("dec ffn1", 7168, 2048, 512, 1), ("dec ffn2", 7168, 512, 2048, 2), ("full dec qkv", 32768, 1536, 512, 0),
               ("big ffn1", 65536, 2048, 512, 1), ("odd", 625 * 13, 1536, 512, 0)]

@@ -102,7 +102,6 @@ def sec_envs():
 def sec_gemm():
     from m3pc_b200 import _native as nat
     L = nat.lib()
-    print("M3PC_GEMM_CONFIG =", os.environ.get("M3PC_GEMM_CONFIG"))
     shapes = [(13312, 1536, 512, 0, "enc qkv"), (13312, 512, 512, 2, "enc out-proj +res"), (13312, 2048, 512, 1, "enc lin1 gelu"),
               (13312, 512, 2048, 2, "enc lin2 +res"), (13312, 1024, 512, 0, "dec kv"), (7168, 2048, 512, 1, "dec lin1"), (7168, 512, 2048, 2, "dec lin2"),
               (4096, 256, 256, 4, "critic l2"), (65536, 2048, 512, 1, "big lin1"), (65536, 512, 2048, 2, "big lin2"), (8192, 8192, 8192, 0, "square 8k")]
