@@ -106,9 +106,7 @@ struct m3pc_engine {
   bool finalized = false;
   std::map<std::string, std::vector<float>> staged;
 
-  DevBuf arena_f32, arena_bf16;            // packed parameters
-  std::map<std::string, size_t> off_f32;   // name -> float offset in arena_f32
-  std::map<std::string, size_t> off_bf16;  // name -> element offset in arena_bf16
+  DevBuf arena_f32, arena_bf16;  // packed parameters
 
   // derived device pointers
   const float* enc_wt[4] = {};    // W_enc^T (d, D)
@@ -222,72 +220,55 @@ int need(m3pc_engine* e, const std::string& name, size_t count, const std::vecto
   return M3PC_OK;
 }
 
+// Lays the parameters out in the fp32 arena and (bf16 mode) the bf16 arena, and records for every tensor the engine field that
+// receives its device pointer; finalize() writes those fields once the arenas are uploaded.
 struct Packer {
+  bool bf16 = false;  // bf16 mode: tensors given a bf16 slot also get a bf16 copy
   std::vector<float> f32;
-  std::vector<std::pair<size_t, size_t>> bf16_src;  // (offset in f32, count) of tensors that also get a bf16 copy
-  std::map<std::string, size_t>* off;
-  std::map<std::string, size_t>* off16;
+  struct Slot { size_t off; const float** p; };
+  struct Slot16 { size_t src, n, off; const __nv_bfloat16** p; };  // bf16 copy of f32[src, src + n) at element `off`
+  std::vector<Slot> slots;
+  std::vector<Slot16> slots16;
   size_t n16 = 0;
-  size_t add(const std::string& name, const float* data, size_t n, bool also_bf16 = false) {
+  void add(const float* data, size_t n, const float** slot, const __nv_bfloat16** slot16 = nullptr) {
     // 64-float (256 B) alignment keeps every tensor TMA/float4 friendly
     while (f32.size() % 64) f32.push_back(0.f);
     const size_t o = f32.size();
     f32.insert(f32.end(), data, data + n);
-    (*off)[name] = o;
-    if (also_bf16) {
+    if (slot != nullptr) slots.push_back({o, slot});
+    if (bf16 && slot16 != nullptr) {
       while (n16 % 128) ++n16;
-      (*off16)[name] = n16;
-      bf16_src.push_back({o, n});
+      slots16.push_back({o, n, n16, slot16});
       n16 += n;
     }
-    return o;
   }
 };
 
-int pack_stack(m3pc_engine* e, Packer& pk, const std::string& prefix, int n_layer) {
-  const size_t D = e->D, F = e->F;
+// packs the staged parameter `name` of `n` values
+int pack(m3pc_engine* e, Packer& pk, const std::string& name, size_t n, const float** slot, const __nv_bfloat16** slot16 = nullptr) {
   const std::vector<float>* v;
-  for (int l = 0; l < n_layer; ++l) {
-    const std::string p = prefix + ".layers." + std::to_string(l);
-    struct Item { const char* suffix; size_t n; bool mat; } items[] = {
-        {".self_attn.in_proj_weight", 3 * D * D, true}, {".self_attn.in_proj_bias", 3 * D, false},
-        {".self_attn.out_proj.weight", D * D, true},    {".self_attn.out_proj.bias", D, false},
-        {".linear1.weight", F * D, true},               {".linear1.bias", F, false},
-        {".linear2.weight", D * F, true},               {".linear2.bias", D, false},
-        {".norm1.weight", D, false},                    {".norm1.bias", D, false},
-        {".norm2.weight", D, false},                    {".norm2.bias", D, false}};
-    for (auto& it : items) {
-      M3PC_TRY(need(e, p + it.suffix, it.n, &v));
-      pk.add(p + it.suffix, v->data(), it.n, it.mat && e->bf16);
-    }
-  }
-  M3PC_TRY(need(e, prefix + ".norm.weight", D, &v));
-  pk.add(prefix + ".norm.weight", v->data(), D);
-  M3PC_TRY(need(e, prefix + ".norm.bias", D, &v));
-  pk.add(prefix + ".norm.bias", v->data(), D);
+  M3PC_TRY(need(e, name, n, &v));
+  pk.add(v->data(), n, slot, slot16);
   return M3PC_OK;
 }
 
-void bind_stack(m3pc_engine* e, StackW& s, const std::string& prefix, int n_layer) {
-  const float* base = e->arena_f32.as<float>();
-  const __nv_bfloat16* base16 = e->arena_bf16.as<__nv_bfloat16>();
-  auto f = [&](const std::string& n) { return base + e->off_f32.at(n); };
-  auto h = [&](const std::string& n) -> const __nv_bfloat16* { return e->bf16 ? base16 + e->off_bf16.at(n) : nullptr; };
-  s.layers.resize(n_layer);
+int pack_stack(m3pc_engine* e, Packer& pk, StackW& s, const std::string& prefix, int n_layer) {
+  const size_t D = e->D, F = e->F;
+  s.layers.resize(n_layer);  // before packing: the slots point into it
   for (int l = 0; l < n_layer; ++l) {
     const std::string p = prefix + ".layers." + std::to_string(l);
     LayerW& w = s.layers[l];
-    w.in_w = f(p + ".self_attn.in_proj_weight"); w.in_b = f(p + ".self_attn.in_proj_bias");
-    w.out_w = f(p + ".self_attn.out_proj.weight"); w.out_b = f(p + ".self_attn.out_proj.bias");
-    w.l1_w = f(p + ".linear1.weight"); w.l1_b = f(p + ".linear1.bias");
-    w.l2_w = f(p + ".linear2.weight"); w.l2_b = f(p + ".linear2.bias");
-    w.n1_w = f(p + ".norm1.weight"); w.n1_b = f(p + ".norm1.bias");
-    w.n2_w = f(p + ".norm2.weight"); w.n2_b = f(p + ".norm2.bias");
-    w.in_w16 = h(p + ".self_attn.in_proj_weight"); w.out_w16 = h(p + ".self_attn.out_proj.weight");
-    w.l1_w16 = h(p + ".linear1.weight"); w.l2_w16 = h(p + ".linear2.weight");
+    struct Item { const char* suffix; size_t n; const float** slot; const __nv_bfloat16** slot16; } items[] = {
+        {".self_attn.in_proj_weight", 3 * D * D, &w.in_w, &w.in_w16}, {".self_attn.in_proj_bias", 3 * D, &w.in_b, nullptr},
+        {".self_attn.out_proj.weight", D * D, &w.out_w, &w.out_w16},   {".self_attn.out_proj.bias", D, &w.out_b, nullptr},
+        {".linear1.weight", F * D, &w.l1_w, &w.l1_w16},                {".linear1.bias", F, &w.l1_b, nullptr},
+        {".linear2.weight", D * F, &w.l2_w, &w.l2_w16},                {".linear2.bias", D, &w.l2_b, nullptr},
+        {".norm1.weight", D, &w.n1_w, nullptr},                        {".norm1.bias", D, &w.n1_b, nullptr},
+        {".norm2.weight", D, &w.n2_w, nullptr},                        {".norm2.bias", D, &w.n2_b, nullptr}};
+    for (auto& it : items) M3PC_TRY(pack(e, pk, p + it.suffix, it.n, it.slot, it.slot16));
   }
-  s.norm_w = f(prefix + ".norm.weight");
-  s.norm_b = f(prefix + ".norm.bias");
+  M3PC_TRY(pack(e, pk, prefix + ".norm.weight", D, &s.norm_w));
+  return pack(e, pk, prefix + ".norm.bias", D, &s.norm_b);
 }
 
 int build_const_rows(m3pc_engine* e);
@@ -299,10 +280,7 @@ int finalize(m3pc_engine* e) {
   M3PC_CHECK_CUDA(cudaDeviceSynchronize());
   e->drop_graphs();
   Packer pk;
-  pk.off = &e->off_f32;
-  pk.off16 = &e->off_bf16;
-  e->off_f32.clear();
-  e->off_bf16.clear();
+  pk.bf16 = e->bf16;
   const std::vector<float>* v;
   const std::vector<float>* pos;
   M3PC_TRY(need(e, "pos_embed", T * D, &pos));
@@ -323,8 +301,8 @@ int finalize(m3pc_engine* e) {
     std::vector<float> wt(d * D);
     for (size_t c = 0; c < D; ++c)
       for (size_t i = 0; i < d; ++i) wt[i * D + c] = (*ew)[c * d + i];
-    pk.add("enc_wt." + m, wt.data(), wt.size());
-    pk.add("decoder_embed_dict." + m + ".weight", dw->data(), D * D, e->bf16);
+    pk.add(wt.data(), wt.size(), &e->enc_wt[k]);
+    pk.add(dw->data(), D * D, &e->dec_w[k], &e->dec_w16[k]);
     // W_dec mask_token (fp64 accumulate, rounded once)
     std::vector<float> wm(D);
     for (size_t c = 0; c < D; ++c) {
@@ -340,37 +318,33 @@ int finalize(m3pc_engine* e) {
         dec_maskrow[o] = ((wm[c] + (*db)[c]) + (*dpd)[c]) + (*pos)[t * D + c];
       }
   }
-  pk.add("enc_cvec", enc_cvec.data(), enc_cvec.size());
-  pk.add("dec_cvec", dec_cvec.data(), dec_cvec.size());
-  pk.add("dec_maskrow", dec_maskrow.data(), dec_maskrow.size());
-  M3PC_TRY(pack_stack(e, pk, "encoder", e->Le));
-  M3PC_TRY(pack_stack(e, pk, "decoder", e->Ld));
+  pk.add(enc_cvec.data(), enc_cvec.size(), &e->enc_cvec);
+  pk.add(dec_cvec.data(), dec_cvec.size(), &e->dec_cvec);
+  pk.add(dec_maskrow.data(), dec_maskrow.size(), &e->dec_maskrow);
+  M3PC_TRY(pack_stack(e, pk, e->enc, "encoder", e->Le));
+  M3PC_TRY(pack_stack(e, pk, e->dec, "decoder", e->Ld));
   for (int k = 0; k < 4; ++k) {
     const std::string m = kMod[k];
     const size_t d = e->dims[k];
     if (k == M3PC_ACTIONS) {
-      const char* names[4] = {"output_head_dict.actions.mu.weight", "output_head_dict.actions.mu.bias",
-                              "output_head_dict.actions.log_std.weight", "output_head_dict.actions.log_std.bias"};
-      const size_t counts[4] = {d * D, d, d * D, d};
-      for (int i = 0; i < 4; ++i) {
-        M3PC_TRY(need(e, names[i], counts[i], &v));
-        pk.add(names[i], v->data(), counts[i]);
-      }
+      M3PC_TRY(pack(e, pk, "output_head_dict.actions.mu.weight", d * D, &e->mu_w));
+      M3PC_TRY(pack(e, pk, "output_head_dict.actions.mu.bias", d, &e->mu_b));
+      M3PC_TRY(pack(e, pk, "output_head_dict.actions.log_std.weight", d * D, &e->ls_w));
+      M3PC_TRY(pack(e, pk, "output_head_dict.actions.log_std.bias", d, &e->ls_b));
     } else {
       const std::string p = "output_head_dict." + m;
-      struct Item { const char* suffix; size_t n; bool mat; } items[] = {{".0.weight", D, false}, {".0.bias", D, false},
-                                                                       {".1.weight", D * D, true}, {".1.bias", D, false},
-                                                                       {".3.weight", d * D, false}, {".3.bias", d, false}};
-      for (auto& it : items) {
-        M3PC_TRY(need(e, p + it.suffix, it.n, &v));
-        pk.add(p + it.suffix, v->data(), it.n, it.mat && e->bf16);
-      }
+      M3PC_TRY(pack(e, pk, p + ".0.weight", D, &e->head_ln_w[k]));
+      M3PC_TRY(pack(e, pk, p + ".0.bias", D, &e->head_ln_b[k]));
+      M3PC_TRY(pack(e, pk, p + ".1.weight", D * D, &e->head_w1[k], &e->head_w1_16[k]));
+      M3PC_TRY(pack(e, pk, p + ".1.bias", D, &e->head_b1[k]));
+      M3PC_TRY(pack(e, pk, p + ".3.weight", d * D, &e->head_w3[k]));
+      M3PC_TRY(pack(e, pk, p + ".3.bias", d, &e->head_b3[k]));
       // tokenizer statistics (decode needs them for all three; encode for states/rewards)
       M3PC_TRY(need(e, "tokenizer." + m + ".mean", d, &v));
-      pk.add("tokenizer." + m + ".mean", v->data(), d);
+      pk.add(v->data(), d, &e->tok_mean[k]);
       if (d == 1) e->h_tok_mean[k] = (*v)[0];
       M3PC_TRY(need(e, "tokenizer." + m + ".std", d, &v));
-      pk.add("tokenizer." + m + ".std", v->data(), d);
+      pk.add(v->data(), d, &e->tok_std[k]);
       if (d == 1) e->h_tok_std[k] = (*v)[0];
     }
   }
@@ -384,76 +358,32 @@ int finalize(m3pc_engine* e) {
       for (int l = 0; l < 3; ++l) {
         const std::string p = "critic.q" + std::to_string(q + 1) + ".net." + std::to_string(2 * l);
         M3PC_TRY(need(e, p + ".weight", wn[l], &v));
-        pk.add(p + ".weight", v->data(), wn[l], l == 1 && e->critic_tc);
+        pk.add(v->data(), wn[l], &e->q_w[q][l], l == 1 && e->critic_tc ? &e->q_w16[q][1] : nullptr);
         if (l == 0 && e->critic_tc) {  // zero-pad the input dimension to a TMA/UMMA friendly multiple of 64
           std::vector<float> wp(Hq * e->q_kp, 0.f);
           for (size_t r = 0; r < Hq; ++r)
             for (size_t c = 0; c < in; ++c) wp[r * e->q_kp + c] = (*v)[r * in + c];
-          pk.add(p + ".weight.padded", wp.data(), wp.size(), true);
+          pk.add(wp.data(), wp.size(), nullptr, &e->q_w16[q][0]);
         }
-        M3PC_TRY(need(e, p + ".bias", bn[l], &v));
-        pk.add(p + ".bias", v->data(), bn[l]);
+        M3PC_TRY(pack(e, pk, p + ".bias", bn[l], &e->q_b[q][l]));
       }
-    M3PC_TRY(need(e, "critic.obs_mean", e->obs, &v));
-    pk.add("critic.obs_mean", v->data(), e->obs);
-    M3PC_TRY(need(e, "critic.obs_std", e->obs, &v));
-    pk.add("critic.obs_std", v->data(), e->obs);
+    M3PC_TRY(pack(e, pk, "critic.obs_mean", e->obs, &e->obs_mean));
+    M3PC_TRY(pack(e, pk, "critic.obs_std", e->obs, &e->obs_std));
     e->has_critic = true;
   }
 
-  // upload
+  // upload, then point every slot into the arenas
   M3PC_TRY(e->arena_f32.alloc(pk.f32.size() * sizeof(float)));
   M3PC_CHECK_CUDA(cudaMemcpy(e->arena_f32.p, pk.f32.data(), pk.f32.size() * sizeof(float), cudaMemcpyHostToDevice));
+  for (const Packer::Slot& s : pk.slots) *s.p = e->arena_f32.as<float>() + s.off;
   if (e->bf16) {
     M3PC_TRY(e->arena_bf16.alloc((pk.n16 + 128) * sizeof(__nv_bfloat16)));
     M3PC_CHECK_CUDA(cudaMemset(e->arena_bf16.p, 0, e->arena_bf16.bytes));
-    size_t o16 = 0;
-    for (auto& pr : pk.bf16_src) {
-      while (o16 % 128) ++o16;
-      M3PC_TRY(launch_f32_to_bf16(e->arena_f32.as<float>() + pr.first, e->arena_bf16.as<__nv_bfloat16>() + o16, pr.second, 0));
-      o16 += pr.second;
+    for (const Packer::Slot16& s : pk.slots16) {
+      M3PC_TRY(launch_f32_to_bf16(e->arena_f32.as<float>() + s.src, e->arena_bf16.as<__nv_bfloat16>() + s.off, s.n, 0));
+      *s.p = e->arena_bf16.as<__nv_bfloat16>() + s.off;
     }
     M3PC_CHECK_CUDA(cudaDeviceSynchronize());
-  }
-
-  // bind
-  const float* base = e->arena_f32.as<float>();
-  const __nv_bfloat16* base16 = e->arena_bf16.as<__nv_bfloat16>();
-  auto f = [&](const std::string& n) { return base + e->off_f32.at(n); };
-  auto h16 = [&](const std::string& n) -> const __nv_bfloat16* { return e->bf16 ? base16 + e->off_bf16.at(n) : nullptr; };
-  e->enc_cvec = f("enc_cvec");
-  e->dec_cvec = f("dec_cvec");
-  e->dec_maskrow = f("dec_maskrow");
-  for (int k = 0; k < 4; ++k) {
-    const std::string m = kMod[k];
-    e->enc_wt[k] = f("enc_wt." + m);
-    e->dec_w[k] = f("decoder_embed_dict." + m + ".weight");
-    e->dec_w16[k] = h16("decoder_embed_dict." + m + ".weight");
-    if (k != M3PC_ACTIONS) {
-      const std::string p = "output_head_dict." + m;
-      e->head_ln_w[k] = f(p + ".0.weight"); e->head_ln_b[k] = f(p + ".0.bias");
-      e->head_w1[k] = f(p + ".1.weight"); e->head_b1[k] = f(p + ".1.bias");
-      e->head_w1_16[k] = h16(p + ".1.weight");
-      e->head_w3[k] = f(p + ".3.weight"); e->head_b3[k] = f(p + ".3.bias");
-      e->tok_mean[k] = f("tokenizer." + m + ".mean");
-      e->tok_std[k] = f("tokenizer." + m + ".std");
-    }
-  }
-  e->mu_w = f("output_head_dict.actions.mu.weight"); e->mu_b = f("output_head_dict.actions.mu.bias");
-  e->ls_w = f("output_head_dict.actions.log_std.weight"); e->ls_b = f("output_head_dict.actions.log_std.bias");
-  bind_stack(e, e->enc, "encoder", e->Le);
-  bind_stack(e, e->dec, "decoder", e->Ld);
-  if (e->has_critic) {
-    for (int q = 0; q < 2; ++q)
-      for (int l = 0; l < 3; ++l) {
-        const std::string p = "critic.q" + std::to_string(q + 1) + ".net." + std::to_string(2 * l);
-        e->q_w[q][l] = f(p + ".weight");
-        e->q_b[q][l] = f(p + ".bias");
-        if (e->critic_tc && l == 0) e->q_w16[q][0] = h16(p + ".weight.padded");
-        if (e->critic_tc && l == 1) e->q_w16[q][1] = h16(p + ".weight");
-      }
-    e->obs_mean = f("critic.obs_mean");
-    e->obs_std = f("critic.obs_std");
   }
   e->finalized = true;  // `staged` is kept: a later m3pc_set_param of a subset + finalize re-packs (include/m3pc.h)
   if (e->Ld == 1) M3PC_TRY(build_const_rows(e));
@@ -464,20 +394,25 @@ int finalize(m3pc_engine* e) {
 int gemm(m3pc_engine* e, const void* A, const float* w32, const __nv_bfloat16* w16, void* C, int M, int N, int K, const GemmEpilogue& epi,
          cudaStream_t st);
 
+// y = LayerNorm(x; gamma, beta) on `rows` rows of D features, y in bf16 or fp32
+int layernorm(const float* x, int rows, const float* gamma, const float* beta, void* y, int D, bool y_bf16, cudaStream_t st) {
+  LnParams ln{};
+  ln.x = x;
+  ln.rows = rows;
+  ln.rows_per_group = 1;
+  ln.g1 = gamma;
+  ln.b1 = beta;
+  ln.y1 = y;
+  return launch_layernorm(ln, D, y_bf16, st);
+}
+
 // Batch-constant decoder rows.  With a single decoder layer, a masked token's decoder input is the same vector for every
 // batch row: decoder_embed(mask_token) + per-dim + pos[t] (dec_maskrow, mtm_model.py:646-696).  Its LayerNorm and its Q / K / V
 // projections are therefore constants of the weights: computed once here, with the same kernels the per-batch rows use.
 int build_const_rows(m3pc_engine* e) {
   const int D = e->D, rows = 4 * e->T;
   const LayerW& w = e->dec.layers[0];
-  LnParams ln{};
-  ln.x = e->dec_maskrow;
-  ln.rows = rows;
-  ln.rows_per_group = 1;
-  ln.g1 = w.n1_w;
-  ln.b1 = w.n1_b;
-  ln.y1 = e->Y.p;
-  M3PC_TRY(launch_layernorm(ln, D, e->bf16, 0));
+  M3PC_TRY(layernorm(e->dec_maskrow, rows, w.n1_w, w.n1_b, e->Y.p, D, e->bf16, 0));
   GemmEpilogue ge;
   ge.bias = w.in_b;
   M3PC_TRY(gemm(e, e->Y.p, w.in_w, w.in_w16, e->const_qkv.p, rows, 3 * D, D, ge, 0));
@@ -567,14 +502,7 @@ int gemm_res_ln(m3pc_engine* e, const void* A, const float* w32, const __nv_bflo
     ep.flags = EPI_RESIDUAL;
   }
   M3PC_TRY(gemm(e, A, w32, w16, X, M, D, K, ep, st));
-  LnParams ln{};
-  ln.x = X;
-  ln.rows = M;
-  ln.g1 = g;
-  ln.b1 = b;
-  ln.y1 = Y;
-  ln.rows_per_group = 1;
-  return launch_layernorm(ln, D, e->bf16, st);
+  return layernorm(X, M, g, b, Y, D, e->bf16, st);
 }
 
 // Several residual GEMM + LayerNorm problems that share K, bias and the LayerNorm parameters: ONE launch of the fused kernel where
@@ -698,18 +626,42 @@ struct NeedSet {
   int t0[4] = {0, 0, 0, 0}, nt[4] = {0, 0, 0, 0};
 };
 
-// decoder_embed of the encoder outputs: one grouped GEMM per run of kept tokens of one modality (mtm_model.py:646-661).
-// `compact`: write rows in encoder-token order (row block = dec_src[j]); otherwise in decoder order (row block = j).
-int decoder_embed(m3pc_engine* e, const void* enc_out, const int* dec_src, int Bc, bool compact, cudaStream_t st, float* xout = nullptr) {
-  const int D = e->D, T = e->T;
-  const size_t ab = act_bytes(e);
-  GemmJob jobs[MAX_TOK];
-  int n = 0;
+// Calls fn(j, k, len) for every run of kept tokens of one modality k: decoder tokens j .. j+len-1, whose encoder rows
+// dec_src[j] .. dec_src[j]+len-1 are consecutive too.
+template <typename Fn>
+void for_each_kept_run(const int* dec_src, int T, Fn&& fn) {
   for (int j = 0; j < 4 * T;) {
     if (dec_src[j] < 0) { ++j; continue; }
     const int k = j / T;
     int len = 1;
     while (j + len < (k + 1) * T && dec_src[j + len] == dec_src[j] + len) ++len;
+    fn(j, k, len);
+    j += len;
+  }
+}
+
+// the masked decoder tokens of a layout, each broadcast from its batch-constant row dec_maskrow[j] into row block j
+FillParams mask_rows(const m3pc_engine* e, const int* dec_src, int Bc) {
+  FillParams fp{};
+  fp.B = Bc;
+  for (int j = 0; j < 4 * e->T; ++j)
+    if (dec_src[j] < 0) {
+      fp.row[fp.n] = e->dec_maskrow + static_cast<size_t>(j) * e->D;
+      fp.bstride[fp.n] = 0;
+      fp.tok[fp.n] = j;
+      ++fp.n;
+    }
+  return fp;
+}
+
+// decoder_embed of the encoder outputs: one grouped GEMM per run of kept tokens of one modality (mtm_model.py:646-661).
+// `compact`: write rows in encoder-token order (row block = dec_src[j]); otherwise in decoder order (row block = j).
+int decoder_embed(m3pc_engine* e, const void* enc_out, const int* dec_src, int Bc, bool compact, cudaStream_t st, float* xout = nullptr) {
+  const int D = e->D;
+  const size_t ab = act_bytes(e);
+  GemmJob jobs[MAX_TOK];
+  int n = 0;
+  for_each_kept_run(dec_src, e->T, [&](int j, int k, int len) {
     GemmEpilogue ge;
     ge.table = e->dec_cvec + static_cast<size_t>(j) * D;
     ge.rows_per_group = Bc;
@@ -717,8 +669,7 @@ int decoder_embed(m3pc_engine* e, const void* enc_out, const int* dec_src, int B
     const char* a = reinterpret_cast<const char*>(enc_out) + static_cast<size_t>(dec_src[j]) * Bc * D * ab;
     float* c = (xout != nullptr ? xout : e->X.as<float>()) + static_cast<size_t>(compact ? dec_src[j] : j) * Bc * D;
     jobs[n++] = GemmJob{a, e->dec_w[k], e->dec_w16[k], c, len * Bc, D, D, ge};
-    j += len;
-  }
+  });
   return gemm_group(e, jobs, n, st);  // the runs of all modalities in one launch
 }
 
@@ -790,40 +741,12 @@ int final_norms(m3pc_engine* e, const float* x, int n_tok, const int* tok, int B
   return launch_layernorm(ln, e->D, e->bf16, st);
 }
 
-// Full decoder: every one of the 4T rows goes through every layer (mtm_model.py:663-716).
-int decode_full(m3pc_engine* e, const FwdIO& io, const void* enc_out, const int* dec_src, const NeedSet& need_in, int b0, int Bc,
-                cudaStream_t st) {
-  const int D = e->D, T = e->T;
-  FillParams fp{};
-  fp.B = Bc;
-  for (int j = 0; j < 4 * T; ++j)
-    if (dec_src[j] < 0) {
-      fp.row[fp.n] = e->dec_maskrow + static_cast<size_t>(j) * D;
-      fp.bstride[fp.n] = 0;
-      fp.tok[fp.n] = j;
-      ++fp.n;
-    }
-  M3PC_TRY(launch_fill_rows(fp, D, e->X.as<float>(), st));
-  M3PC_TRY(decoder_embed(e, enc_out, dec_src, Bc, false, st));
-  const int Sd = 4 * T;
-  LnParams ln{};
-  ln.x = e->X.as<float>();
-  ln.rows = Sd * Bc;
-  ln.rows_per_group = Bc;
-  ln.g1 = e->dec.layers[0].n1_w;
-  ln.b1 = e->dec.layers[0].n1_b;
-  ln.y1 = e->Y.p;
-  M3PC_TRY(launch_layernorm(ln, D, e->bf16, st));
-  for (int l = 0; l < e->Ld; ++l) {
-    PostLn post;  // the next layer's norm1 rides on this layer's linear2
-    if (l + 1 < e->Ld) post = PostLn{e->dec.layers[l + 1].n1_w, e->dec.layers[l + 1].n1_b, e->Y.p};
-    M3PC_TRY(block(e, e->dec.layers[l], Bc, Sd, st, post));
-  }
-  // heads over all rows: token blocks in decoder order
+// final norms + heads over all 4T decoder rows of `x` (token blocks in decoder order); reads need.t0 / need.nt
+int heads_all_rows(m3pc_engine* e, const FwdIO& io, const float* x, NeedSet need, int b0, int Bc, cudaStream_t st) {
+  const int T = e->T;
   int all_tok[MAX_TOK];
-  for (int j = 0; j < Sd; ++j) all_tok[j] = j;
-  M3PC_TRY(final_norms(e, e->X.as<float>(), Sd, all_tok, Bc, st));
-  NeedSet need = need_in;
+  for (int j = 0; j < 4 * T; ++j) all_tok[j] = j;
+  M3PC_TRY(final_norms(e, x, 4 * T, all_tok, Bc, st));
   for (int k = 0; k < 4; ++k) need.q0[k] = k * T + need.t0[k];  // row block of (k, t0) in decoder order
   return heads(e, io, need, e->Y.p, e->Y2.p, b0, Bc, st);
 }
@@ -960,13 +883,7 @@ int decode_restricted(m3pc_engine* e, const FwdIO& io, const void* enc_out, cons
   const LayerW& w = e->dec.layers[0];
   const int D = e->D, T = e->T;
   int min_run = 1 << 30;  // shortest run of consecutive kept tokens of one modality
-  for (int j = 0; j < 4 * T;) {
-    if (dec_src[j] < 0) { ++j; continue; }
-    int len = 1;
-    while (j + len < (j / T + 1) * T && dec_src[j + len] == dec_src[j] + len) ++len;
-    min_run = std::min(min_run, len);
-    j += len;
-  }
+  for_each_kept_run(dec_src, T, [&](int, int, int len) { min_run = std::min(min_run, len); });
   // every run must be large enough for the fused kernel, so that one batch size always takes one path
   if (e->bf16 && D == 512 && static_cast<long>(min_run) * Bc >= e->fuse_ln_min_rows) {
     // (a) + (b) in one kernel per run of kept tokens of a modality: X = dec_cvec[token] + enc_out W_dec^T (compact, encoder order),
@@ -974,59 +891,37 @@ int decode_restricted(m3pc_engine* e, const FwdIO& io, const void* enc_out, cons
     const size_t ab = act_bytes(e);
     ResLnJob jobs[MAX_TOK];
     int nj = 0;
-    for (int j = 0; j < 4 * T;) {
-      if (dec_src[j] < 0) { ++j; continue; }
-      const int k = j / T;
-      int len = 1;
-      while (j + len < (k + 1) * T && dec_src[j + len] == dec_src[j] + len) ++len;
+    for_each_kept_run(dec_src, T, [&](int j, int k, int len) {
       const size_t r0 = static_cast<size_t>(dec_src[j]) * Bc;
       jobs[nj++] = ResLnJob{reinterpret_cast<const char*>(enc_out) + r0 * D * ab, e->dec_w[k], e->dec_w16[k], e->X.as<float>() + r0 * D,
                             reinterpret_cast<char*>(e->Y.p) + r0 * D * ab, e->dec_cvec + static_cast<size_t>(j) * D, Bc, len * Bc, nullptr};
-      j += len;
-    }
+    });
     M3PC_TRY(gemm_res_ln_group(e, jobs, nj, nullptr, w.n1_w, w.n1_b, D, st));
     return restricted_last_layer(e, io, w, dec_src, S, need, b0, Bc, st);
   }
   // (a) decoder embedding of the kept tokens, compact (encoder order) -> X[0 : S*Bc)
   M3PC_TRY(decoder_embed(e, enc_out, dec_src, Bc, true, st));
   // (b) LN1 -> Y
-  LnParams ln{};
-  ln.x = e->X.as<float>();
-  ln.rows = S * Bc;
-  ln.rows_per_group = Bc;
-  ln.g1 = w.n1_w;
-  ln.b1 = w.n1_b;
-  ln.y1 = e->Y.p;
-  M3PC_TRY(launch_layernorm(ln, D, e->bf16, st));
+  M3PC_TRY(layernorm(e->X.as<float>(), S * Bc, w.n1_w, w.n1_b, e->Y.p, D, e->bf16, st));
   return restricted_last_layer(e, io, w, dec_src, S, need, b0, Bc, st);
 }
 
-// Deeper decoders: layers 0 .. Ld-2 run on all 4T rows (after the first layer no row is batch-constant any more), the last
-// layer only on the rows the caller consumes (mtm_model.py:663-716 computes every row of every layer).
-int decode_deep_restricted(m3pc_engine* e, const FwdIO& io, const void* enc_out, const int* dec_src, const NeedSet& need, int b0, int Bc,
-                           cudaStream_t st) {
-  const int D = e->D, T = e->T, Sd = 4 * T;
-  FillParams fp{};
-  fp.B = Bc;
-  for (int j = 0; j < Sd; ++j)
-    if (dec_src[j] < 0) {
-      fp.row[fp.n] = e->dec_maskrow + static_cast<size_t>(j) * D;
-      fp.bstride[fp.n] = 0;
-      fp.tok[fp.n] = j;
-      ++fp.n;
-    }
-  M3PC_TRY(launch_fill_rows(fp, D, e->X.as<float>(), st));
+// Decoder on all 4T rows (mtm_model.py:663-716 computes every row of every layer).  `restrict_last` (deeper decoders; after the
+// first layer no row is batch-constant any more): layers 0 .. Ld-2 run on all rows, the last layer only on the rows the caller
+// consumes.  Otherwise every layer and the heads run on all rows.
+int decode_full(m3pc_engine* e, const FwdIO& io, const void* enc_out, const int* dec_src, const NeedSet& need, int b0, int Bc,
+                bool restrict_last, cudaStream_t st) {
+  const int D = e->D, Sd = 4 * e->T;
+  M3PC_TRY(launch_fill_rows(mask_rows(e, dec_src, Bc), D, e->X.as<float>(), st));
   M3PC_TRY(decoder_embed(e, enc_out, dec_src, Bc, false, st));
-  LnParams ln{};
-  ln.x = e->X.as<float>();
-  ln.rows = Sd * Bc;
-  ln.rows_per_group = Bc;
-  ln.y1 = e->Y.p;
-  ln.g1 = e->dec.layers[0].n1_w;
-  ln.b1 = e->dec.layers[0].n1_b;
-  M3PC_TRY(launch_layernorm(ln, D, e->bf16, st));
-  for (int l = 0; l + 1 < e->Ld; ++l)  // the next layer's norm1 rides on this layer's linear2
-    M3PC_TRY(block(e, e->dec.layers[l], Bc, Sd, st, PostLn{e->dec.layers[l + 1].n1_w, e->dec.layers[l + 1].n1_b, e->Y.p}));
+  M3PC_TRY(layernorm(e->X.as<float>(), Sd * Bc, e->dec.layers[0].n1_w, e->dec.layers[0].n1_b, e->Y.p, D, e->bf16, st));
+  const int n_full = restrict_last ? e->Ld - 1 : e->Ld;
+  for (int l = 0; l < n_full; ++l) {
+    PostLn post;  // the next layer's norm1 rides on this layer's linear2
+    if (l + 1 < e->Ld) post = PostLn{e->dec.layers[l + 1].n1_w, e->dec.layers[l + 1].n1_b, e->Y.p};
+    M3PC_TRY(block(e, e->dec.layers[l], Bc, Sd, st, post));
+  }
+  if (!restrict_last) return heads_all_rows(e, io, e->X.as<float>(), need, b0, Bc, st);
   int ident[MAX_TOK];
   for (int j = 0; j < Sd; ++j) ident[j] = j;
   return restricted_last_layer(e, io, e->dec.layers[e->Ld - 1], ident, Sd, need, b0, Bc, st);
@@ -1089,7 +984,7 @@ int forward_chunk(m3pc_engine* e, const FwdIO& io, int b0, int Bc, cudaStream_t 
   const size_t ab = act_bytes(e);
   const TokTables tt = token_tables(io.mask, T);
   const int S = tt.S;
-  const int *enc_mod = tt.enc_mod, *enc_t = tt.enc_t, *dec_src = tt.dec_src;
+  const int* dec_src = tt.dec_src;
   M3PC_REQUIRE(S > 0, "forward: every token is masked");
 
   // ---- which head rows does the caller consume? ----
@@ -1105,6 +1000,7 @@ int forward_chunk(m3pc_engine* e, const FwdIO& io, int b0, int Bc, cudaStream_t 
     need.nt[k] = nt;
     for (int t = t0; t < t0 + nt; ++t) need.tok[need.n++] = k * T + t;
   }
+  const EmbedParams ep = embed_params(e, io, tt, b0, Bc);  // the encoder tokens, for K1 or the fused B = 1 kernel
 
   // ---- B = 1: the whole encoder + restricted decoder in one cooperative kernel (fused_b1.cu) ----
   bool grouped_src = false;
@@ -1128,23 +1024,10 @@ int forward_chunk(m3pc_engine* e, const FwdIO& io, int b0, int Bc, cudaStream_t 
     }
     fp.dec_cvec = e->dec_cvec; fp.dec_maskrow = e->dec_maskrow;
     fp.const_qkv = e->const_qkv.as<__nv_bfloat16>();
-    for (int k = 0; k <= 4; ++k) fp.mod_row0[k] = 0;
-    for (int s = 0; s < S; ++s) {
-      const int k = enc_mod[s], t = enc_t[s], d = e->dims[k];
-      const ModSrc& ms = io.src[k];
-      EmbedTok& tk = fp.tok[s];
-      if (ms.base2 != nullptr && t >= ms.t_split) {
-        tk.src = ms.base2 + static_cast<size_t>(b0) * ms.bstride2 + static_cast<size_t>(t - ms.t_split) * d;
-      } else {
-        tk.src = ms.base + static_cast<size_t>(b0) * ms.bstride + static_cast<size_t>(t) * d;
-      }
-      tk.bstride = 0;
-      tk.wt = e->enc_wt[k];
-      tk.cvec = e->enc_cvec + (static_cast<size_t>(k) * T + t) * D;
-      tk.nmean = ms.normalize ? e->tok_mean[k] : nullptr;
-      tk.nstd = ms.normalize ? e->tok_std[k] : nullptr;
-      tk.d = d;
-      fp.enc_dectok[s] = static_cast<unsigned char>(k * T + t);
+    for (int s = 0; s < S; ++s) {  // the kernel reads src, wt, cvec, nmean, nstd and d of a token (the single batch row's source)
+      const int k = tt.enc_mod[s];
+      fp.tok[s] = ep.tok[s];
+      fp.enc_dectok[s] = static_cast<unsigned char>(k * T + tt.enc_t[s]);
       for (int kk = k + 1; kk <= 4; ++kk) fp.mod_row0[kk] = s + 1;
     }
     for (int j = 0; j < 4 * T; ++j) fp.dec_src[j] = static_cast<signed char>(dec_src[j]);
@@ -1170,7 +1053,6 @@ int forward_chunk(m3pc_engine* e, const FwdIO& io, int b0, int Bc, cudaStream_t 
   }
 
   // ---- K1: embed + gather + first LayerNorm ----
-  const EmbedParams ep = embed_params(e, io, tt, b0, Bc);
   const LayerW& first = e->Le > 0 ? e->enc.layers[0] : e->dec.layers[0];
   // shared-history analysis: the leading encoder tokens whose source row is shared by whole groups of batch rows (one window
   // for the whole batch: bstride 0; one window per environment: bdiv rows each) -- the chunk must hold whole groups
@@ -1226,8 +1108,7 @@ int forward_chunk(m3pc_engine* e, const FwdIO& io, int b0, int Bc, cudaStream_t 
 
   if (need.n == 0) return M3PC_OK;
   if (e->Ld == 1 && need.n < 4 * T) return decode_restricted(e, io, enc_out, dec_src, S, need, b0, Bc, st);
-  if (e->Ld > 1 && need.n < 4 * T && e->restrict_deep) return decode_deep_restricted(e, io, enc_out, dec_src, need, b0, Bc, st);
-  return decode_full(e, io, enc_out, dec_src, need, b0, Bc, st);
+  return decode_full(e, io, enc_out, dec_src, need, b0, Bc, e->Ld > 1 && need.n < 4 * T && e->restrict_deep, st);
 }
 
 int forward(m3pc_engine* e, const FwdIO& io, int B, cudaStream_t st) {
@@ -1278,16 +1159,9 @@ int critic(m3pc_engine* e, int N, int h, cudaStream_t st, const float* states_pr
     GemmEpilogue ge;
     ge.bias = e->q_b[q][0];
     ge.flags = EPI_RELU;
-    if (e->critic_tc) {
-      M3PC_TRY(gemm(e, e->sa.p, nullptr, e->q_w16[q][0], e->qa.p, rows, Hq, e->q_kp, ge, st));
-      ge.bias = e->q_b[q][1];
-      ge.flags = EPI_RELU | EPI_OUT_F32;
-      M3PC_TRY(gemm(e, e->qa.p, nullptr, e->q_w16[q][1], outs[q], rows, Hq, Hq, ge, st));
-    } else {
-      M3PC_TRY(gemm_fp32(e->sa.as<float>(), e->q_w[q][0], e->qa.as<float>(), rows, Hq, in, ge, st));
-      ge.bias = e->q_b[q][1];
-      M3PC_TRY(gemm_fp32(e->qa.as<float>(), e->q_w[q][1], outs[q], rows, Hq, Hq, ge, st));
-    }
+    M3PC_TRY(gemm_fp32(e->sa.as<float>(), e->q_w[q][0], e->qa.as<float>(), rows, Hq, in, ge, st));
+    ge.bias = e->q_b[q][1];
+    M3PC_TRY(gemm_fp32(e->qa.as<float>(), e->q_w[q][1], outs[q], rows, Hq, Hq, ge, st));
   }
   return launch_critic_out(outs[0], outs[1], e->q_w[0][2], e->q_b[0][2], e->q_w[1][2], e->q_b[1][2], qv, rows, Hq, st);
 }
@@ -1298,6 +1172,21 @@ void set_window_sources(m3pc_engine* e, FwdIO& io, const float* ws, const float*
   io.src[M3PC_ACTIONS] = ModSrc{wa, stride_mul * T * e->act, false};
   io.src[M3PC_REWARDS] = ModSrc{wr, stride_mul * T, true};
   io.src[M3PC_RETURNS] = ModSrc{wrt, stride_mul * T, false};
+}
+
+// sources and mask of a forward on already tokenised (batch, T, d) inputs
+int io_from_tokens(const m3pc_engine* e, FwdIO& io, const float* ts, const float* ta, const float* tr, const float* tt, const uint8_t* masks) {
+  M3PC_REQUIRE(masks != nullptr, "null masks");
+  const int T = e->T;
+  io.src[M3PC_STATES] = ModSrc{ts, static_cast<long>(T) * e->obs, false};
+  io.src[M3PC_ACTIONS] = ModSrc{ta, static_cast<long>(T) * e->act, false};
+  io.src[M3PC_REWARDS] = ModSrc{tr, static_cast<long>(T), false};
+  io.src[M3PC_RETURNS] = ModSrc{tt, static_cast<long>(T), false};
+  for (int i = 0; i < 4 * T; ++i) {
+    M3PC_REQUIRE(masks[i] <= 1, "mask entries must be 0 or 1");
+    io.mask[i] = masks[i];
+  }
+  return M3PC_OK;
 }
 
 int plan_body(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
@@ -1642,15 +1531,7 @@ int m3pc_forward(m3pc_handle_t h, int32_t batch, const float* tok_states, const 
   M3PC_REQUIRE(h != nullptr && masks != nullptr, "null argument");
   M3PC_REQUIRE(tok_states && tok_actions && tok_rewards && tok_returns, "all four modalities must be given");
   m3pc::FwdIO io{};
-  const int T = h->T;
-  io.src[M3PC_STATES] = m3pc::ModSrc{tok_states, static_cast<long>(T) * h->obs, false};
-  io.src[M3PC_ACTIONS] = m3pc::ModSrc{tok_actions, static_cast<long>(T) * h->act, false};
-  io.src[M3PC_REWARDS] = m3pc::ModSrc{tok_rewards, static_cast<long>(T), false};
-  io.src[M3PC_RETURNS] = m3pc::ModSrc{tok_returns, static_cast<long>(T), false};
-  for (int i = 0; i < 4 * T; ++i) {
-    M3PC_REQUIRE(masks[i] <= 1, "mask entries must be 0 or 1");
-    io.mask[i] = masks[i];
-  }
+  M3PC_TRY(m3pc::io_from_tokens(h, io, tok_states, tok_actions, tok_rewards, tok_returns, masks));
   io.out_states = out_states; io.out_mu = out_act_mu; io.out_std = out_act_std;
   io.out_rewards = out_rewards; io.out_returns = out_returns;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -1819,9 +1700,7 @@ int m3pc_gemm_fp32(const float* A, const float* W, const float* bias, float* C, 
 
 int m3pc_layernorm(const float* x, const float* gamma, const float* beta, void* y, int32_t M, int32_t D, int32_t out_bf16, void* stream) {
   M3PC_REQUIRE(x && gamma && beta && y, "null argument");
-  m3pc::LnParams p{};
-  p.x = x; p.rows = M; p.g1 = gamma; p.b1 = beta; p.y1 = y; p.rows_per_group = 1;
-  return m3pc::launch_layernorm(p, D, out_bf16 != 0, reinterpret_cast<cudaStream_t>(stream));
+  return m3pc::layernorm(x, M, gamma, beta, y, D, out_bf16 != 0, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_attention(const void* qkv, void* out, int32_t B, int32_t S, int32_t n_head, int32_t is_bf16, void* stream) {
@@ -1830,28 +1709,12 @@ int m3pc_attention(const void* qkv, void* out, int32_t B, int32_t S, int32_t n_h
 }
 
 // ---- kernel-level entries K1 / K4 / K5 / K6 / K7 / K8 (SURVEY.md section 8b): the same launchers m3pc_forward / m3pc_plan use ----
-namespace {
-int io_from_tokens(m3pc_handle_t h, m3pc::FwdIO& io, const float* ts, const float* ta, const float* tr, const float* tt, const uint8_t* masks) {
-  M3PC_REQUIRE(h != nullptr && h->finalized, "kernel-level call before m3pc_finalize_params");
-  M3PC_REQUIRE(masks != nullptr, "null masks");
-  const int T = h->T;
-  io.src[M3PC_STATES] = m3pc::ModSrc{ts, static_cast<long>(T) * h->obs, false};
-  io.src[M3PC_ACTIONS] = m3pc::ModSrc{ta, static_cast<long>(T) * h->act, false};
-  io.src[M3PC_REWARDS] = m3pc::ModSrc{tr, static_cast<long>(T), false};
-  io.src[M3PC_RETURNS] = m3pc::ModSrc{tt, static_cast<long>(T), false};
-  for (int i = 0; i < 4 * T; ++i) {
-    M3PC_REQUIRE(masks[i] <= 1, "mask entries must be 0 or 1");
-    io.mask[i] = masks[i];
-  }
-  return M3PC_OK;
-}
-}  // namespace
-
 int m3pc_embed_gather(m3pc_handle_t h, int32_t batch, const float* tok_states, const float* tok_actions, const float* tok_rewards,
                       const float* tok_returns, const uint8_t* masks, float* x_out, void* y_out, void* stream) {
   M3PC_REQUIRE(tok_states && tok_actions && tok_rewards && tok_returns && x_out && y_out, "null argument");
+  M3PC_REQUIRE(h != nullptr && h->finalized, "kernel-level call before m3pc_finalize_params");
   m3pc::FwdIO io{};
-  M3PC_TRY(io_from_tokens(h, io, tok_states, tok_actions, tok_rewards, tok_returns, masks));
+  M3PC_TRY(m3pc::io_from_tokens(h, io, tok_states, tok_actions, tok_rewards, tok_returns, masks));
   M3PC_REQUIRE(batch >= 1 && batch <= h->cfg.max_batch, "batch exceeds cfg.max_batch");
   const m3pc::TokTables tt = m3pc::token_tables(io.mask, h->T);
   M3PC_REQUIRE(tt.S > 0, "every token is masked");
@@ -1871,9 +1734,7 @@ int m3pc_block_forward(m3pc_handle_t h, int32_t stack, int32_t layer, int32_t ba
   const size_t rows = static_cast<size_t>(batch) * n_tok, D = h->D, ab = m3pc::act_bytes(h);
   const m3pc::LayerW& w = sw.layers[layer];
   M3PC_CHECK_CUDA(cudaMemcpyAsync(h->X.p, x, rows * D * 4, cudaMemcpyDeviceToDevice, st));
-  m3pc::LnParams ln{};
-  ln.x = h->X.as<float>(); ln.rows = static_cast<int>(rows); ln.g1 = w.n1_w; ln.b1 = w.n1_b; ln.y1 = h->Y.p; ln.rows_per_group = 1;
-  M3PC_TRY(m3pc::launch_layernorm(ln, h->D, h->bf16, st));
+  M3PC_TRY(m3pc::layernorm(h->X.as<float>(), static_cast<int>(rows), w.n1_w, w.n1_b, h->Y.p, h->D, h->bf16, st));
   m3pc::PostLn post;
   if (y_next != nullptr)
     post = layer + 1 < n_layer ? m3pc::PostLn{sw.layers[layer + 1].n1_w, sw.layers[layer + 1].n1_b, h->ENC.p} : m3pc::PostLn{sw.norm_w, sw.norm_b, h->ENC.p};
@@ -1886,20 +1747,11 @@ int m3pc_block_forward(m3pc_handle_t h, int32_t stack, int32_t layer, int32_t ba
 int m3pc_decoder_scatter_embed(m3pc_handle_t h, int32_t batch, const void* enc_out, const uint8_t* masks, float* x_out, void* stream) {
   M3PC_REQUIRE(h != nullptr && h->finalized && enc_out && masks && x_out, "bad argument");
   M3PC_REQUIRE(batch >= 1 && batch <= h->chunk, "batch exceeds the engine's chunk (workspace rows)");
-  const int T = h->T, D = h->D;
+  const int T = h->T;
   for (int i = 0; i < 4 * T; ++i) M3PC_REQUIRE(masks[i] <= 1, "mask entries must be 0 or 1");
   const m3pc::TokTables tt = m3pc::token_tables(masks, T);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  m3pc::FillParams fp{};
-  fp.B = batch;
-  for (int j = 0; j < 4 * T; ++j)
-    if (tt.dec_src[j] < 0) {
-      fp.row[fp.n] = h->dec_maskrow + static_cast<size_t>(j) * D;
-      fp.bstride[fp.n] = 0;
-      fp.tok[fp.n] = j;
-      ++fp.n;
-    }
-  if (fp.n > 0) M3PC_TRY(m3pc::launch_fill_rows(fp, D, x_out, st));
+  M3PC_TRY(m3pc::launch_fill_rows(m3pc::mask_rows(h, tt.dec_src, batch), h->D, x_out, st));  // no launch when every token is kept
   if (tt.S == 0) return M3PC_OK;
   return m3pc::decoder_embed(h, enc_out, tt.dec_src, batch, false, st, x_out);
 }
@@ -1909,22 +1761,12 @@ int m3pc_heads(m3pc_handle_t h, int32_t batch, const float* x_dec, float* out_st
   M3PC_REQUIRE(h != nullptr && h->finalized && x_dec, "bad argument");
   M3PC_REQUIRE(batch >= 1 && batch <= h->chunk, "batch exceeds the engine's chunk (workspace rows)");
   M3PC_REQUIRE((out_act_mu == nullptr) == (out_act_std == nullptr), "out_act_mu and out_act_std go together");
-  const int T = h->T, Sd = 4 * T;
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   m3pc::FwdIO io{};
   io.out_states = out_states; io.out_mu = out_act_mu; io.out_std = out_act_std; io.out_rewards = out_rewards; io.out_returns = out_returns;
   m3pc::NeedSet need;
   const float* outp[4] = {out_states, out_act_mu, out_rewards, out_returns};
-  int all_tok[m3pc::MAX_TOK];
-  for (int j = 0; j < Sd; ++j) all_tok[j] = j;
-  for (int k = 0; k < 4; ++k) {
-    need.q0[k] = k * T;  // row block of (k, t = 0) in decoder order
-    need.t0[k] = 0;
-    need.nt[k] = outp[k] != nullptr ? T : 0;
-  }
-  need.n = Sd;
-  M3PC_TRY(m3pc::final_norms(h, x_dec, Sd, all_tok, batch, st));
-  return m3pc::heads(h, io, need, h->Y.p, h->Y2.p, 0, batch, st);
+  for (int k = 0; k < 4; ++k) need.nt[k] = outp[k] != nullptr ? h->T : 0;
+  return m3pc::heads_all_rows(h, io, x_dec, need, 0, batch, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_sample_candidates(const float* mu, const float* std, const float* eps, uint64_t seed, int32_t n_cand, int32_t horizon, int32_t act_dim,
