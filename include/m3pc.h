@@ -170,7 +170,16 @@ typedef struct {
                                the GLOBAL result on every rank -- no collective launch, nothing outside the captured CUDA graph.
                                Every rank of the group must issue the same sequence of exchange plans. */
   int32_t reserved0;
-  void* reserved1[3];
+  const int32_t* env_horizons; /* HOST (max(n_env, 1)) or NULL: one horizon per environment, each in [1, traj_length]
+                                  (learner.py:342-345 clamps the horizon of an environment in its first T - h steps).  `horizon`
+                                  must equal the largest entry, which fixes the layouts: eps and dbg_candidates stay
+                                  (E*n_cand, horizon, A) and environment e uses the first env_horizons[e] steps of its rows.  All
+                                  entries equal: exactly the call with NULL.  Otherwise the environments are split into horizon
+                                  classes and each class is planned as the uniform call on its windows at n_env = E_c (bit for bit),
+                                  all in one launch sequence (one CUDA graph per horizon pattern).  Philox is keyed by the caller's
+                                  environment index, so an environment's draws do not depend on the other environments of the call.
+                                  Needs n_env <= 256; cannot be combined with exchange, out_partials or cand_offset. */
+  void* reserved1[2];
 } m3pc_plan_args_t;
 
 int m3pc_plan(m3pc_handle_t h, const m3pc_plan_args_t* args, void* stream);
@@ -231,6 +240,24 @@ int m3pc_ring_append(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_d
 int m3pc_ring_windows(const float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, int32_t path_length,
                       int32_t horizon, int32_t traj_length, int32_t future_obs, const float* rtg_tok, float* win_states,
                       float* win_actions, float* win_rewards, float* win_returns_tok, void* stream);
+
+/* The same ring with one clock per slot, for environments whose episodes end at different steps and whose slots start the next
+ * episode at once.  `slots` is a HOST list of n_slots slot indices (any length: it travels in kernel parameters, 256 per launch);
+ * per-slot inputs and outputs are in list order.  `t` / `path_length` are DEVICE (n_env) int32 tables indexed by slot.
+ *   m3pc_ring_reset          zeroes the whole history of the listed slots: a new episode (rollout.new_trajectory).  Without it the
+ *                            actions / rewards of the previous episode would show up in the windows of the next.
+ *   m3pc_ring_append_slots   listed slot k = slots[k] writes obs row k at step t[slot] and (when non-NULL) prev_action row k /
+ *                            prev_reward[k] at step t[slot] - 1; a slot with t outside [0, ring_len) writes nothing.
+ *   m3pc_ring_windows_slots  the (n_slots, T, .) windows of the listed slots, row k = m3pc_ring_windows of slot slots[k] at
+ *                            path_length[slot] with horizon horizons[k] (HOST list) and rtg_tok[k] (device (n_slots)). */
+int m3pc_ring_reset(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* slots, int32_t n_slots,
+                    void* stream);
+int m3pc_ring_append_slots(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* t, const int32_t* slots,
+                           int32_t n_slots, const float* obs, const float* prev_action, const float* prev_reward, void* stream);
+int m3pc_ring_windows_slots(const float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* path_length,
+                            const int32_t* slots, const int32_t* horizons, int32_t n_slots, int32_t traj_length, int32_t future_obs,
+                            const float* rtg_tok, float* win_states, float* win_actions, float* win_rewards, float* win_returns_tok,
+                            void* stream);
 
 /* ---- kernel-level entry points (unit parity tests and profiling; same kernels the calls above launch) ---- */
 

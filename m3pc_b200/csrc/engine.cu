@@ -5,6 +5,7 @@
 // HBM layout: all activations are token-major matrices, row = token * Bc + b for the Bc batch rows (candidates
 // or environments) of the current chunk.  A chunk is run through the whole network before the next one starts,
 // so its working set (<= ~80 bytes/feature/row) stays L2-resident; weights (22.7 MB bf16) stay L2-resident too.
+#include <algorithm>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -145,12 +146,15 @@ struct m3pc_engine {
                                     // below, a copy kernel + one problem.  Option "split_residual_min_rows" (tests force either form).
   // planner buffers
   DevBuf p1_mu, p1_std, cand, pred_states, pred_rewards, pred_returns, sa, qa, qb1, qb2, qvals, J, filled, e_mu, e_std;
+  // plans with one horizon per environment: every class's windows, noise rows and id table, gathered (launch_mix_gather)
+  DevBuf mix_ws, mix_wa, mix_wr, mix_wt, mix_eps, mix_expq, mix_id;
 
   // CUDA-graph replay of m3pc_plan (production path: on-device Philox noise, no debug outputs)
   struct PlanKey {
     int guidance, horizon, n_cand, cand_offset, n_env, exchange;
     float discount, temperature, lmbda;
     const void *ws, *wa, *wr, *wt, *ev, *sm, *pt;
+    unsigned char env_h[MIX_MAX_ENV];  // per-environment horizons of a mixed plan (all zero otherwise)
     bool operator<(const PlanKey& o) const { return std::memcmp(this, &o, sizeof(PlanKey)) < 0; }
   };
   struct PlanGraph {
@@ -1189,7 +1193,8 @@ int io_from_tokens(const m3pc_engine* e, FwdIO& io, const float* ts, const float
   return M3PC_OK;
 }
 
-int plan_body(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
+// env_id: null, or the device id table of a horizon class planned by plan_mixed (local environment -> the caller's index)
+int plan_body(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st, const int* env_id = nullptr) {
   M3PC_REQUIRE(e->finalized, "plan before m3pc_finalize_params");
   const int T = e->T, h = a->horizon, N = a->n_cand, A = e->act, idx = T - h;
   const int E = a->n_env > 1 ? a->n_env : 1;  // lock-step environments planned by this call
@@ -1223,7 +1228,7 @@ int plan_body(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
   M3PC_TRY(forward(e, io, E, st));
   if (a->guidance == M3PC_GUIDE_SAMPLING)
     return launch_sampling_tail(io.out_mu, io.out_std, a->eps, T, h, A, E, a->out_eval_action, a->out_sample_action, a->seed,
-                                e->seed_ptr_active, st);
+                                e->seed_ptr_active, st, 1, env_id);
 
   // ---- K6: candidates ----
   CandParams cp{};
@@ -1231,7 +1236,7 @@ int plan_body(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
   cp.N = static_cast<int>(R); cp.h = h; cp.A = A; cp.T = T;
   cp.n_per_env = E > 1 ? N : 0;
   cp.noise_mode = a->guidance == M3PC_GUIDE_NOISE_CRITIC ? 1 : 0;
-  cp.seed = a->seed; cp.cand_offset = a->cand_offset; cp.seed_ptr = e->seed_ptr_active;
+  cp.seed = a->seed; cp.cand_offset = a->cand_offset; cp.seed_ptr = e->seed_ptr_active; cp.env_id = env_id;
   M3PC_TRY(launch_candidates(cp, st));
   if (a->dbg_candidates)
     M3PC_CHECK_CUDA(cudaMemcpyAsync(a->dbg_candidates, cp.cand, sizeof(float) * R * h * A, cudaMemcpyDeviceToDevice, st));
@@ -1282,7 +1287,7 @@ int plan_body(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
   sl.n_env = E; sl.N = N; sl.h = h; sl.A = A;
   sl.temperature = a->temperature; sl.seed = a->seed; sl.cand_offset = a->cand_offset; sl.seed_ptr = e->seed_ptr_active;
   sl.eval_action = a->out_eval_action; sl.sample_action = a->out_sample_action;
-  sl.partials = a->out_partials; sl.indices = a->dbg_indices;
+  sl.partials = a->out_partials; sl.indices = a->dbg_indices; sl.env_id = env_id;
   if (a->exchange) {
     for (int g = 0; g < e->xch_world; ++g) sl.xch.peer[g] = e->xch_peer[g];
     sl.xch.rank = e->xch_rank;
@@ -1295,14 +1300,121 @@ int plan_body(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
   return M3PC_OK;
 }
 
+// Horizon classes of a plan with env_horizons: class c holds the environments of horizon h[c] (ascending), in the caller's order,
+// as gathered slots [off[c], off[c + 1]); src maps a gathered slot to the caller's environment.
+struct MixPlan {
+  int n_class = 0;
+  int h[M3PC_MAX_T] = {}, off[M3PC_MAX_T + 1] = {};
+  short src[MIX_MAX_ENV] = {};
+};
+
+// Validates env_horizons.  *mixed is false when it is null or all its entries are equal: the plan is then exactly the uniform one.
+int mix_classes(const m3pc_engine* e, const m3pc_plan_args_t* a, MixPlan& m, bool* mixed) {
+  *mixed = false;
+  if (a->env_horizons == nullptr) return M3PC_OK;
+  const int E = a->n_env > 1 ? a->n_env : 1;
+  M3PC_REQUIRE(a->n_env >= 0, "n_env must be >= 0");
+  M3PC_REQUIRE(a->exchange == 0 && a->out_partials == nullptr && a->cand_offset == 0, "env_horizons cannot be combined with candidate sharding");
+  int hmax = 0;
+  bool equal = true;
+  for (int i = 0; i < E; ++i) {
+    const int hi = a->env_horizons[i];
+    M3PC_REQUIRE(hi >= 1 && hi <= e->T, "env_horizons entries must be in [1, traj_length]");
+    hmax = std::max(hmax, hi);
+    equal = equal && hi == a->env_horizons[0];
+  }
+  M3PC_REQUIRE(a->horizon == hmax, "with env_horizons, horizon must equal its largest entry");
+  if (equal) return M3PC_OK;
+  M3PC_REQUIRE(E <= MIX_MAX_ENV, "env_horizons: more environments than one mixed plan takes (256)");
+  int n = 0;
+  for (int hh = 1; hh <= e->T; ++hh) {
+    const int start = n;
+    for (int i = 0; i < E; ++i)
+      if (a->env_horizons[i] == hh) m.src[n++] = static_cast<short>(i);
+    if (n > start) {
+      m.h[m.n_class] = hh;
+      m.off[m.n_class++] = start;
+    }
+  }
+  m.off[m.n_class] = n;
+  *mixed = true;
+  return M3PC_OK;
+}
+
+// A plan whose environments have different horizons: one gather launch, then per horizon class the uniform plan sequence at
+// n_env = E_c on the class's contiguous windows (and noise rows), with the class's id table so Philox keys and outputs use the
+// caller's environment index.  Each class computes exactly what the uniform call on its windows computes.
+int plan_mixed(m3pc_engine* e, const m3pc_plan_args_t* a, const MixPlan& m, cudaStream_t st) {
+  M3PC_REQUIRE(e->finalized, "plan before m3pc_finalize_params");
+  M3PC_REQUIRE(a->win_states && a->win_actions && a->win_rewards && a->win_returns_tok, "window pointers must be set");
+  const int T = e->T, A = e->act, N = a->n_cand, E = m.off[m.n_class], hmax = a->horizon;
+  const bool g3 = a->guidance == M3PC_GUIDE_SAMPLING;
+  M3PC_REQUIRE(E <= e->cfg.max_batch && (g3 || (N >= 1 && static_cast<long>(E) * N <= e->cfg.max_batch)), "n_env * n_cand exceeds cfg.max_batch");
+  MixGatherParams g{};
+  g.ws = a->win_states; g.wa = a->win_actions; g.wr = a->win_rewards; g.wt = a->win_returns_tok;
+  g.gs = e->mix_ws.as<float>(); g.ga = e->mix_wa.as<float>(); g.gr = e->mix_wr.as<float>(); g.gt = e->mix_wt.as<float>();
+  g.eps = a->eps; g.geps = e->mix_eps.as<float>();
+  g.expq = g3 ? nullptr : a->expq; g.gexpq = e->mix_expq.as<float>();
+  g.env_id = e->mix_id.as<int>();
+  g.E = E; g.T = T; g.obs = e->obs; g.A = A; g.N = g3 ? 0 : N;
+  g.eps_rows = g3 ? 1 : N;            // guidance 3: eps is (E, A)
+  g.eps_ld = g3 ? A : hmax * A;
+  for (int c = 0; c < m.n_class; ++c)
+    for (int s = m.off[c]; s < m.off[c + 1]; ++s) {
+      g.src[s] = m.src[s];
+      g.slot_of[m.src[s]] = static_cast<short>(s);
+      g.eps_off[s + 1] = g.eps_off[s] + g.eps_rows * (g3 ? A : m.h[c] * A);
+    }
+  M3PC_TRY(launch_mix_gather(g, st));
+  for (int c = 0; c < m.n_class; ++c) {
+    const int off = m.off[c], Ec = m.off[c + 1] - off, h = m.h[c];
+    m3pc_plan_args_t sub = *a;
+    sub.env_horizons = nullptr;
+    sub.n_env = Ec;
+    sub.horizon = h;
+    sub.win_states = g.gs + static_cast<size_t>(off) * T * e->obs;
+    sub.win_actions = g.ga + static_cast<size_t>(off) * T * A;
+    sub.win_rewards = g.gr + static_cast<size_t>(off) * T;
+    sub.win_returns_tok = g.gt + static_cast<size_t>(off) * T;
+    sub.eps = a->eps ? g.geps + g.eps_off[off] : nullptr;
+    sub.expq = g.expq ? g.gexpq + static_cast<size_t>(off) * N : nullptr;
+    sub.dbg_expect_return = nullptr;
+    sub.dbg_candidates = nullptr;
+    M3PC_TRY(plan_body(e, &sub, st, g.env_id + off));
+    // debug outputs (eager calls only) in the caller's environment order; steps >= h of a candidate row are not written
+    for (int i = 0; i < Ec && !g3; ++i) {
+      const size_t ce = static_cast<size_t>(m.src[off + i]);
+      if (a->dbg_expect_return)
+        M3PC_CHECK_CUDA(cudaMemcpyAsync(a->dbg_expect_return + ce * N, e->J.as<float>() + static_cast<size_t>(i) * N, sizeof(float) * N,
+                                        cudaMemcpyDeviceToDevice, st));
+      if (a->dbg_candidates)
+        M3PC_CHECK_CUDA(cudaMemcpy2DAsync(a->dbg_candidates + ce * N * hmax * A, sizeof(float) * hmax * A,
+                                          e->cand.as<float>() + static_cast<size_t>(i) * N * h * A, sizeof(float) * h * A, sizeof(float) * h * A, N,
+                                          cudaMemcpyDeviceToDevice, st));
+    }
+  }
+  return M3PC_OK;
+}
+
 // m3pc_plan: eager for parity / debug calls (injected noise, debug outputs, profiling); otherwise the launch sequence is
 // captured once per (arguments, buffer addresses) into a CUDA graph and replayed -- ~70 dependent launches become one
 // submission, which is what bounds the B = 1 pass.  The Philox key travels through a device scalar so replays differ.
-int plan(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
+int plan(m3pc_engine* e, const m3pc_plan_args_t* args, cudaStream_t st) {
+  MixPlan mix;
+  bool mixed = false;
+  M3PC_TRY(mix_classes(e, args, mix, &mixed));
+  m3pc_plan_args_t uniform;
+  const m3pc_plan_args_t* a = args;
+  if (args->env_horizons != nullptr && !mixed) {  // all horizons equal: the uniform plan, launch for launch and graph for graph
+    uniform = *args;
+    uniform.env_horizons = nullptr;
+    a = &uniform;
+  }
+  auto body = [&](cudaStream_t s) { return mixed ? plan_mixed(e, a, mix, s) : plan_body(e, a, s); };
   const bool eager = !e->use_graphs || e->profile || a->eps || a->expq || a->dbg_expect_return || a->dbg_candidates || a->dbg_indices;
   if (eager) {
     e->seed_ptr_active = nullptr;
-    return plan_body(e, a, st);
+    return body(st);
   }
   m3pc_engine::PlanKey key;
   std::memset(&key, 0, sizeof(key));
@@ -1311,12 +1423,14 @@ int plan(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
   key.discount = a->discount; key.temperature = a->temperature; key.lmbda = a->lmbda;
   key.ws = a->win_states; key.wa = a->win_actions; key.wr = a->win_rewards; key.wt = a->win_returns_tok;
   key.ev = a->out_eval_action; key.sm = a->out_sample_action; key.pt = a->out_partials;
+  if (mixed)
+    for (int i = 0; i < mix.off[mix.n_class]; ++i) key.env_h[i] = static_cast<unsigned char>(a->env_horizons[i]);
   if (e->plan_graphs.size() > 64) e->drop_graphs();  // callers that keep changing buffers would otherwise grow the cache without bound
   m3pc_engine::PlanGraph& pg = e->plan_graphs[key];
   if (pg.exec == nullptr) {
     if (pg.seen++ < 1) {  // first sighting: run eagerly (also performs every lazy cudaFuncSetAttribute)
       e->seed_ptr_active = nullptr;
-      return plan_body(e, a, st);
+      return body(st);
     }
     // captured on a private stream: the caller's stream may be the legacy default stream, which cannot be captured;
     // the instantiated graph is then launched on the caller's stream
@@ -1325,7 +1439,7 @@ int plan(m3pc_engine* e, const m3pc_plan_args_t* a, cudaStream_t st) {
     e->seed_ptr_active = e->seed_scalar.as<unsigned long long>();
     M3PC_CHECK_CUDA(cudaStreamBeginCapture(e->cap_stream, cudaStreamCaptureModeThreadLocal));
     const int before = g_launch_count;
-    const int rc = plan_body(e, a, e->cap_stream);
+    const int rc = body(e->cap_stream);
     pg.launches = g_launch_count - before;
     const cudaError_t ce = cudaStreamEndCapture(e->cap_stream, &graph);
     e->seed_ptr_active = nullptr;
@@ -1443,6 +1557,14 @@ int create(m3pc_handle_t* out, const m3pc_config_t* cfg) {
   M3PC_TRY(e->filled.alloc(N * T * e->obs * 4));
   M3PC_TRY(e->e_mu.alloc(N * T * e->act * 4));
   M3PC_TRY(e->e_std.alloc(N * T * e->act * 4));
+  const size_t NE = std::min<size_t>(N, MIX_MAX_ENV);  // environments of a mixed plan
+  M3PC_TRY(e->mix_ws.alloc(NE * T * e->obs * 4));
+  M3PC_TRY(e->mix_wa.alloc(NE * T * e->act * 4));
+  M3PC_TRY(e->mix_wr.alloc(NE * T * 4));
+  M3PC_TRY(e->mix_wt.alloc(NE * T * 4));
+  M3PC_TRY(e->mix_eps.alloc(N * T * e->act * 4));  // sum_c E_c n_cand h_c A <= max_batch T A
+  M3PC_TRY(e->mix_expq.alloc(N * 4));
+  M3PC_TRY(e->mix_id.alloc(NE * 4));
   if (e->QH > 0) {
     M3PC_TRY(e->sa.alloc((N * T + 128) * static_cast<size_t>((e->obs + e->act + 63) / 64 * 64) * 4));
     M3PC_TRY(e->qa.alloc((N * T + 128) * e->QH * 4));
@@ -1646,6 +1768,25 @@ int m3pc_ring_append(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_d
                      const float* prev_action, const float* prev_reward, void* stream) {
   M3PC_REQUIRE(ring != nullptr && obs != nullptr, "null argument");
   return m3pc::launch_ring_append(ring, n_env, ring_len, obs_dim, act_dim, t, obs, prev_action, prev_reward, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int m3pc_ring_reset(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* slots, int32_t n_slots,
+                    void* stream) {
+  return m3pc::launch_ring_reset(ring, n_env, ring_len, obs_dim, act_dim, slots, n_slots, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int m3pc_ring_append_slots(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* t, const int32_t* slots,
+                           int32_t n_slots, const float* obs, const float* prev_action, const float* prev_reward, void* stream) {
+  return m3pc::launch_ring_append_slots(ring, n_env, ring_len, obs_dim, act_dim, t, slots, n_slots, obs, prev_action, prev_reward,
+                                        reinterpret_cast<cudaStream_t>(stream));
+}
+
+int m3pc_ring_windows_slots(const float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* path_length,
+                            const int32_t* slots, const int32_t* horizons, int32_t n_slots, int32_t traj_length, int32_t future_obs,
+                            const float* rtg_tok, float* win_states, float* win_actions, float* win_rewards, float* win_returns_tok,
+                            void* stream) {
+  return m3pc::launch_ring_windows_slots(ring, n_env, ring_len, obs_dim, act_dim, path_length, slots, horizons, n_slots, traj_length, future_obs,
+                                         rtg_tok, win_states, win_actions, win_rewards, win_returns_tok, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_ring_windows(const float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, int32_t path_length,

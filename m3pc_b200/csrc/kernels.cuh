@@ -153,6 +153,9 @@ struct CandParams {
   unsigned long long seed;
   int cand_offset;
   const unsigned long long* seed_ptr;  // if non-null the Philox key is read from device memory (CUDA-graph replay)
+  const int* env_id;  // (E) or null: device table local environment -> the caller's environment index.  Philox is then keyed by
+                      // the caller's index (gid = env_id * n_per_env + n), so an environment's draws do not depend on which other
+                      // environments share the call; null: gid = cand_offset + n
 };
 int launch_candidates(const CandParams& p, cudaStream_t st);
 
@@ -220,6 +223,7 @@ struct SelectParams {
   int* indices;          // (2) or null
   ExchangeParams xch;    // xch.world > 0 (n_env == 1 only): exchange + merge inside the kernel; the outputs are the GLOBAL result
   ScoreParams score;     // score.J == J: the TD(lambda) scores are computed by this launch first (one launch less per plan); null J: not
+  const int* env_id;     // (n_env) or null: as CandParams::env_id; the outputs of block e go to row env_id[e] (indices 2 env_id[e])
 };
 int launch_select(const SelectParams& p, cudaStream_t st);
 int launch_merge(const float* partials, int n_shards, int A, float temperature, float* eval_action, float* sample_action, int* indices,
@@ -227,8 +231,29 @@ int launch_merge(const float* partials, int n_shards, int A, float temperature, 
 
 // mtm_sampling tail (learner.py:103-115): eval = tanh(mu[T-h]), sample = tanh(mu[T-h] + std[T-h]*eps)
 // C > 1: C draws per environment, sample_action is (E, C, A) and eps (E, C, A)
+// env_id (E) or null: as CandParams::env_id (Philox keyed by, and outputs written to, the caller's environment index)
 int launch_sampling_tail(const float* mu, const float* std, const float* eps, int T, int h, int A, int E, float* eval_action,
-                         float* sample_action, unsigned long long seed, const unsigned long long* seed_ptr, cudaStream_t st, int C = 1);
+                         float* sample_action, unsigned long long seed, const unsigned long long* seed_ptr, cudaStream_t st, int C = 1,
+                         const int* env_id = nullptr);
+
+// ---- m3pc_plan with one horizon per environment: the environments of one horizon class are planned as one uniform sub-plan on
+// contiguous copies of their inputs.  One launch gathers every class at once (classes are disjoint, so nothing is overwritten
+// while a later class runs).  The class order is a kernel parameter: a captured plan holds no host-to-device copy. ----
+constexpr int MIX_MAX_ENV = 256;
+struct MixGatherParams {
+  const float *ws, *wa, *wr, *wt;  // caller windows (E, T, .)
+  float *gs, *ga, *gr, *gt;        // gathered windows (E, T, .), gathered slot s = caller environment src[s]
+  const float* eps;                // caller noise: eps_rows rows of eps_ld floats per environment, or null
+  float* geps;                     // gathered noise: slot s keeps the first (eps_off[s+1]-eps_off[s]) / eps_rows floats of each row
+  const float* expq;               // caller (E, N) or null
+  float* gexpq;                    // gathered (E, N)
+  int* env_id;                     // out (E): gathered slot -> caller environment (the sub-plans' id tables)
+  int E, T, obs, A, N, eps_rows, eps_ld;
+  short src[MIX_MAX_ENV];          // gathered slot -> caller environment
+  short slot_of[MIX_MAX_ENV];      // caller environment -> gathered slot
+  int eps_off[MIX_MAX_ENV + 1];    // first gathered noise float of each slot
+};
+int launch_mix_gather(const MixGatherParams& p, cudaStream_t st);
 int launch_set_seed(unsigned long long* dst, unsigned long long seed, cudaStream_t st);
 
 // zero-shot piid fill (zeroshot_omtm/learner.py:240-246): states[:, T-h+2:-1] and states[:, :T-h+1] <- decode(pred)
@@ -239,6 +264,13 @@ int launch_piid_fill(const float* win_states, const float* states_pred, const fl
 int launch_ring_append(float* ring, int E, int L, int obs, int act, int t, const float* o, const float* pa, const float* pr, cudaStream_t st);
 int launch_ring_windows(const float* ring, int E, int L, int obs, int act, int pl, int h, int T, int future_obs, const float* rtg_tok,
                         float* ws, float* wa, float* wr, float* wt, cudaStream_t st);
+// per-slot clocks (m3pc_ring_reset / m3pc_ring_append_slots / m3pc_ring_windows_slots): slots and horizons are host lists,
+// t / path_length device (E) tables indexed by slot; per-slot inputs and outputs are in list order
+int launch_ring_reset(float* ring, int E, int L, int obs, int act, const int* slots, int n, cudaStream_t st);
+int launch_ring_append_slots(float* ring, int E, int L, int obs, int act, const int* t, const int* slots, int n, const float* o, const float* pa,
+                             const float* pr, cudaStream_t st);
+int launch_ring_windows_slots(const float* ring, int E, int L, int obs, int act, const int* pl, const int* slots, const int* horizons, int n,
+                              int T, int future_obs, const float* rtg_tok, float* ws, float* wa, float* wr, float* wt, cudaStream_t st);
 
 // conversions
 int launch_f32_to_bf16(const float* in, __nv_bfloat16* out, size_t n, cudaStream_t st);

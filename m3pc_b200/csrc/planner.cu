@@ -7,6 +7,8 @@
 //   score_kernel        K8  TD(lambda) return per candidate, written as the reference's loop (learner.py:301-316).
 //   select_kernel       K8  softmax over candidates, weighted-mean action, exponential-race sample == torch.multinomial
 //                           (learner.py:318-325); emits the per-shard record merged by merge_kernel under sharding.
+#include <algorithm>
+
 #include "kernels.cuh"
 
 namespace m3pc {
@@ -44,7 +46,12 @@ __global__ void candidates_kernel(const __grid_constant__ CandParams p) {
   if (i >= p.N * per) return;
   const int n = i / per, e = i - n * per, j = e / p.A, a = e - j * p.A;
   const unsigned long long seed = p.seed_ptr ? *p.seed_ptr : p.seed;
-  const float eps = p.eps ? p.eps[i] : philox_normal(seed, static_cast<unsigned>(p.cand_offset + n), static_cast<unsigned>(e), 0u);
+  int gid = p.cand_offset + n;
+  if (p.env_id != nullptr) {  // key by the caller's environment index
+    const int n_env_c = p.n_per_env > 0 ? p.n_per_env : p.N, le = n / n_env_c;
+    gid = p.cand_offset + p.env_id[le] * n_env_c + (n - le * n_env_c);
+  }
+  const float eps = p.eps ? p.eps[i] : philox_normal(seed, static_cast<unsigned>(gid), static_cast<unsigned>(e), 0u);
   const int t = p.T - p.h + j;
   const int ms = ((p.n_per_env > 0 ? n / p.n_per_env : 0) * p.T + t) * p.A + a;  // pass-1 distribution of the candidate's environment
   const float mu = p.mu[ms];
@@ -226,11 +233,13 @@ __global__ void __launch_bounds__(SEL_THREADS) select_kernel(const __grid_consta
   const unsigned long long seed = p.seed_ptr ? *p.seed_ptr : p.seed;
   // one block per environment: this block's slice of every per-candidate array
   const int env = blockIdx.x, row0 = env * p.N;
+  const int out_env = p.env_id ? p.env_id[env] : env;  // the caller's row of this environment
+  const int grow0 = out_env * p.N;                     // Philox id of its candidate 0 (before cand_offset)
   const float* Jv = p.J + row0;
   const float* __restrict__ candv = p.cand + static_cast<size_t>(row0) * stride_a0;
   const float* __restrict__ expq = p.expq ? p.expq + row0 : nullptr;
-  float* eval_action = p.eval_action + env * p.A;
-  float* sample_action = p.sample_action + env * p.A;
+  float* eval_action = p.eval_action + out_env * p.A;
+  float* sample_action = p.sample_action + out_env * p.A;
   // 0. scores of this environment's candidates, when the score pass rides in this launch (p.score.J == p.J)
   if (p.score.J != nullptr) {
     for (int n = tid; n < p.N; n += SEL_THREADS) p.score.J[row0 + n] = score_one(p.score, row0 + n);
@@ -250,7 +259,7 @@ __global__ void __launch_bounds__(SEL_THREADS) select_kernel(const __grid_consta
   for (int n = tid; n < p.N; n += SEL_THREADS) {
     const float w = expf(__fmul_rn(__fsub_rn(Jv[n], m), p.temperature));
     z += w;
-    const float q = expq ? expq[n] : philox_exp(seed, static_cast<unsigned>(p.cand_offset + row0 + n), 1u);
+    const float q = expq ? expq[n] : philox_exp(seed, static_cast<unsigned>(p.cand_offset + grow0 + n), 1u);
     const float key = w / q;
     if (key > kbest) { kbest = key; ki = n; }
   }
@@ -290,8 +299,8 @@ __global__ void __launch_bounds__(SEL_THREADS) select_kernel(const __grid_consta
     rec[6] = static_cast<float>(p.N);
     rec[7] = 0.f;
     if (p.indices && !exchange) {
-      p.indices[2 * env + 0] = p.cand_offset + mi;
-      p.indices[2 * env + 1] = p.cand_offset + ki;
+      p.indices[2 * out_env + 0] = p.cand_offset + mi;
+      p.indices[2 * out_env + 1] = p.cand_offset + ki;
     }
     xch_failed = 0;
   }
@@ -354,17 +363,18 @@ __global__ void set_seed_kernel(unsigned long long* dst, unsigned long long seed
 // C draws per environment: i = (e * C + c) * A + a.  C = 1 is the reference's single draw (zeroshot_omtm/learner.py:136-147).
 __global__ void sampling_tail_kernel(const float* __restrict__ mu, const float* __restrict__ std, const float* __restrict__ eps, int T, int h,
                                      int A, int E, int C, float* eval_action, float* sample_action, unsigned long long seed,
-                                     const unsigned long long* seed_ptr) {
+                                     const unsigned long long* seed_ptr, const int* __restrict__ env_id) {
   PDL_PROLOGUE();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= E * C * A) return;
   if (seed_ptr) seed = *seed_ptr;
   const int a = i % A, c = (i / A) % C, e = i / (A * C);
+  const int oe = env_id ? env_id[e] : e;  // the caller's row of environment e
   const size_t src = (static_cast<size_t>(e) * T + (T - h)) * A + a;
   const float m = mu[src];
-  const float z = eps ? eps[i] : philox_normal(seed, static_cast<unsigned>(e), static_cast<unsigned>(c * A + a), 2u);
-  if (c == 0) eval_action[e * A + a] = tanhf(m);
-  sample_action[i] = tanhf(__fadd_rn(m, __fmul_rn(std[src], z)));
+  const float z = eps ? eps[i] : philox_normal(seed, static_cast<unsigned>(oe), static_cast<unsigned>(c * A + a), 2u);
+  if (c == 0) eval_action[oe * A + a] = tanhf(m);
+  sample_action[(static_cast<size_t>(oe) * C + c) * A + a] = tanhf(__fadd_rn(m, __fmul_rn(std[src], z)));
 }
 
 __global__ void piid_fill_kernel(const float* __restrict__ win_states, const float* __restrict__ states_pred, const float* __restrict__ tok_mean,
@@ -398,14 +408,11 @@ __global__ void ring_append_kernel(float* __restrict__ ring, int E, int L, int o
   }
 }
 
-__global__ void ring_windows_kernel(const float* __restrict__ ring, int E, int L, int obs, int act, int pl, int h, int T, int future_obs,
-                                    const float* __restrict__ rtg_tok, float* __restrict__ ws, float* __restrict__ wa, float* __restrict__ wr,
-                                    float* __restrict__ wt) {
-  PDL_PROLOGUE();
+// element c of time step t of the window of ring slot `e` at step `pl` with horizon h, written to output window `o`
+__device__ __forceinline__ void ring_window_elem(const float* __restrict__ ring, int e, int o, int c, int t, int L, int obs, int act, int pl,
+                                                 int h, int T, int future_obs, const float* __restrict__ rtg_tok, float* __restrict__ ws,
+                                                 float* __restrict__ wa, float* __restrict__ wr, float* __restrict__ wt) {
   const int w = obs + act + 1;
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= E * T * w) return;
-  const int c = i % w, t = (i / w) % T, e = i / (w * T);
   const int hl = T - h + 1, lo = pl - hl + 1;  // learner.py:346-359
   int smart_T = T;                             // zeroshot_omtm/learner.py:77-79
   if (future_obs && pl + h > 1000) smart_T = T - (pl + h - 1000);
@@ -414,12 +421,105 @@ __global__ void ring_windows_kernel(const float* __restrict__ ring, int E, int L
   const float* row = ring + (static_cast<size_t>(e) * L + (in_ring ? step : 0)) * w;
   if (c < obs) {
     const bool take = future_obs ? (t < smart_T || t < hl) : (t < hl);
-    ws[(static_cast<size_t>(e) * T + t) * obs + c] = (take && in_ring) ? row[c] : 0.f;
+    ws[(static_cast<size_t>(o) * T + t) * obs + c] = (take && in_ring) ? row[c] : 0.f;
   } else if (c < obs + act) {
-    wa[(static_cast<size_t>(e) * T + t) * act + (c - obs)] = (t < hl && in_ring) ? row[c] : 0.f;
+    wa[(static_cast<size_t>(o) * T + t) * act + (c - obs)] = (t < hl && in_ring) ? row[c] : 0.f;
   } else {
-    wr[e * T + t] = (t < hl && in_ring) ? row[c] : 0.f;
-    wt[e * T + t] = rtg_tok[e];
+    wr[o * T + t] = (t < hl && in_ring) ? row[c] : 0.f;
+    wt[o * T + t] = rtg_tok[o];
+  }
+}
+
+__global__ void ring_windows_kernel(const float* __restrict__ ring, int E, int L, int obs, int act, int pl, int h, int T, int future_obs,
+                                    const float* __restrict__ rtg_tok, float* __restrict__ ws, float* __restrict__ wa, float* __restrict__ wr,
+                                    float* __restrict__ wt) {
+  PDL_PROLOGUE();
+  const int w = obs + act + 1;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= E * T * w) return;
+  const int c = i % w, t = (i / w) % T, e = i / (w * T);
+  ring_window_elem(ring, e, e, c, t, L, obs, act, pl, h, T, future_obs, rtg_tok, ws, wa, wr, wt);
+}
+
+// ---- per-slot clocks: a slot list (and the horizons of its windows) travels as a kernel parameter ----
+constexpr int RING_MAX_SLOTS = 256;  // per launch; the launchers split longer lists
+struct RingSlots {
+  int n;
+  int slot[RING_MAX_SLOTS];
+  unsigned char h[RING_MAX_SLOTS];
+};
+
+__global__ void ring_reset_kernel(float* __restrict__ ring, int L, int w, const __grid_constant__ RingSlots s) {
+  PDL_PROLOGUE();
+  const size_t per = static_cast<size_t>(L) * w;
+  const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= per * s.n) return;
+  const int k = static_cast<int>(i / per);
+  ring[static_cast<size_t>(s.slot[k]) * per + (i - k * per)] = 0.f;
+}
+
+// listed slot k writes its observation (o row k) at step t[slot] and, when given, the action / reward of step t[slot] - 1
+__global__ void ring_append_slots_kernel(float* __restrict__ ring, int L, int obs, int act, const int* __restrict__ tt, const __grid_constant__ RingSlots s,
+                                         const float* __restrict__ o, const float* __restrict__ pa, const float* __restrict__ pr) {
+  PDL_PROLOGUE();
+  const int w = obs + act + 1;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= s.n * w) return;
+  const int k = i / w, c = i - k * w, e = s.slot[k];
+  const int t = tt[e];
+  if (t < 0 || t >= L) return;  // an idle slot (clock < 0) or a step outside the ring: nothing to record
+  float* row_t = ring + (static_cast<size_t>(e) * L + t) * w;
+  if (c < obs) {
+    row_t[c] = o[k * obs + c];
+  } else if (t > 0) {
+    float* row_p = row_t - w;
+    if (c < obs + act) {
+      if (pa != nullptr) row_p[c] = pa[k * act + (c - obs)];
+    } else if (pr != nullptr) {
+      row_p[c] = pr[k];
+    }
+  }
+}
+
+__global__ void ring_windows_slots_kernel(const float* __restrict__ ring, int L, int obs, int act, const int* __restrict__ pl, int T, int future_obs,
+                                          const __grid_constant__ RingSlots s, const float* __restrict__ rtg_tok, float* __restrict__ ws,
+                                          float* __restrict__ wa, float* __restrict__ wr, float* __restrict__ wt) {
+  PDL_PROLOGUE();
+  const int w = obs + act + 1;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= s.n * T * w) return;
+  const int c = i % w, t = (i / w) % T, k = i / (w * T), e = s.slot[k];
+  ring_window_elem(ring, e, k, c, t, L, obs, act, pl[e], s.h[k], T, future_obs, rtg_tok, ws, wa, wr, wt);
+}
+
+// ---- mixed-horizon plans: every horizon class's windows, noise rows and id table, gathered in one launch ----
+__global__ void mix_gather_kernel(const __grid_constant__ MixGatherParams p) {
+  PDL_PROLOGUE();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (blockIdx.y == 0) {  // windows: per step [states | actions | reward | return token]
+    const int w = p.obs + p.A + 2;
+    if (i >= p.E * p.T * w) return;
+    const int s = i / (p.T * w), r = i - s * p.T * w, t = r / w, c = r - t * w;
+    const size_t src = static_cast<size_t>(p.src[s]) * p.T + t, dst = static_cast<size_t>(s) * p.T + t;
+    if (c < p.obs)
+      p.gs[dst * p.obs + c] = p.ws[src * p.obs + c];
+    else if (c < p.obs + p.A)
+      p.ga[dst * p.A + (c - p.obs)] = p.wa[src * p.A + (c - p.obs)];
+    else if (c == p.obs + p.A)
+      p.gr[dst] = p.wr[src];
+    else
+      p.gt[dst] = p.wt[src];
+  } else if (blockIdx.y == 1) {  // injected noise: the first h_e steps of each of environment e's rows
+    const int per = p.eps_rows * p.eps_ld;
+    if (p.eps == nullptr || i >= p.E * per) return;
+    const int e = i / per, r = (i - e * per) / p.eps_ld, c = i - e * per - r * p.eps_ld, s = p.slot_of[e];
+    const int wdt = (p.eps_off[s + 1] - p.eps_off[s]) / p.eps_rows;
+    if (c < wdt) p.geps[p.eps_off[s] + r * wdt + c] = p.eps[i];
+  } else {  // Exp(1) draws and the id table
+    if (i < p.E) p.env_id[i] = p.src[i];
+    if (p.expq == nullptr || i >= p.E * p.N) return;
+    const int e = i / p.N;
+    p.gexpq[p.slot_of[e] * p.N + (i - e * p.N)] = p.expq[i];
   }
 }
 
@@ -436,6 +536,67 @@ int launch_ring_windows(const float* ring, int E, int L, int obs, int act, int p
   M3PC_REQUIRE(E >= 1 && L >= 1 && pl >= 0 && pl < L && h >= 1 && h <= T && T <= M3PC_MAX_T, "ring_windows: bad shape / step");
   M3PC_CHECK_CUDA(launch_k(ring_windows_kernel, dim3(ceil_div(E * T * (obs + act + 1), 256)), dim3(256), 0, st, ring, E, L, obs, act, pl, h, T,
                            future_obs, rtg_tok, ws, wa, wr, wt));
+  M3PC_CHECK_LAUNCH();
+  return M3PC_OK;
+}
+
+template <typename Fn>
+int for_slot_chunks(const int* slots, const int* horizons, int n, int E, int T, Fn&& launch) {
+  for (int k0 = 0; k0 < n; k0 += RING_MAX_SLOTS) {
+    RingSlots s{};
+    s.n = std::min(RING_MAX_SLOTS, n - k0);
+    for (int k = 0; k < s.n; ++k) {
+      M3PC_REQUIRE(slots[k0 + k] >= 0 && slots[k0 + k] < E, "ring: slot index out of range");
+      if (horizons) {
+        M3PC_REQUIRE(horizons[k0 + k] >= 1 && horizons[k0 + k] <= T, "ring: horizon out of range");
+        s.h[k] = static_cast<unsigned char>(horizons[k0 + k]);
+      }
+      s.slot[k] = slots[k0 + k];
+    }
+    M3PC_TRY(launch(s, k0));
+  }
+  return M3PC_OK;
+}
+
+int launch_ring_reset(float* ring, int E, int L, int obs, int act, const int* slots, int n, cudaStream_t st) {
+  M3PC_REQUIRE(ring && E >= 1 && L >= 1 && obs >= 1 && act >= 1 && n >= 0 && (n == 0 || slots), "ring_reset: bad shape");
+  const int w = obs + act + 1;
+  M3PC_REQUIRE(static_cast<long>(L) * w <= 0x7fffffffL / RING_MAX_SLOTS, "ring_reset: ring too long");
+  return for_slot_chunks(slots, nullptr, n, E, 1, [&](const RingSlots& s, int) {
+    M3PC_CHECK_CUDA(launch_k(ring_reset_kernel, dim3(ceil_div(s.n * L * w, 256)), dim3(256), 0, st, ring, L, w, s));
+    M3PC_CHECK_LAUNCH();
+    return M3PC_OK;
+  });
+}
+int launch_ring_append_slots(float* ring, int E, int L, int obs, int act, const int* t, const int* slots, int n, const float* o, const float* pa,
+                             const float* pr, cudaStream_t st) {
+  M3PC_REQUIRE(ring && t && o && E >= 1 && L >= 1 && obs >= 1 && act >= 1 && n >= 0 && (n == 0 || slots), "ring_append_slots: bad shape");
+  const int w = obs + act + 1;
+  return for_slot_chunks(slots, nullptr, n, E, 1, [&](const RingSlots& s, int k0) {
+    M3PC_CHECK_CUDA(launch_k(ring_append_slots_kernel, dim3(ceil_div(s.n * w, 128)), dim3(128), 0, st, ring, L, obs, act, t, s, o + static_cast<size_t>(k0) * obs,
+                             pa ? pa + static_cast<size_t>(k0) * act : nullptr, pr ? pr + k0 : nullptr));
+    M3PC_CHECK_LAUNCH();
+    return M3PC_OK;
+  });
+}
+int launch_ring_windows_slots(const float* ring, int E, int L, int obs, int act, const int* pl, const int* slots, const int* horizons, int n,
+                              int T, int future_obs, const float* rtg_tok, float* ws, float* wa, float* wr, float* wt, cudaStream_t st) {
+  M3PC_REQUIRE(ring && pl && rtg_tok && ws && wa && wr && wt && horizons && E >= 1 && L >= 1 && n >= 0 && (n == 0 || slots) && T >= 1 &&
+                   T <= M3PC_MAX_T,
+               "ring_windows_slots: bad shape");
+  const int w = obs + act + 1;
+  return for_slot_chunks(slots, horizons, n, E, T, [&](const RingSlots& s, int k0) {
+    const size_t o = static_cast<size_t>(k0) * T;
+    M3PC_CHECK_CUDA(launch_k(ring_windows_slots_kernel, dim3(ceil_div(s.n * T * w, 256)), dim3(256), 0, st, ring, L, obs, act, pl, T, future_obs, s,
+                             rtg_tok + k0, ws + o * obs, wa + o * act, wr + o, wt + o));
+    M3PC_CHECK_LAUNCH();
+    return M3PC_OK;
+  });
+}
+int launch_mix_gather(const MixGatherParams& p, cudaStream_t st) {
+  M3PC_REQUIRE(p.E >= 1 && p.E <= MIX_MAX_ENV, "mixed horizons: too many environments");
+  const int n = std::max({p.E * p.T * (p.obs + p.A + 2), p.eps ? p.E * p.eps_rows * p.eps_ld : 0, p.E * p.N});
+  M3PC_CHECK_CUDA(launch_k(mix_gather_kernel, dim3(ceil_div(n, 256), 3), dim3(256), 0, st, p));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
 }
@@ -481,9 +642,11 @@ int launch_merge(const float* partials, int n_shards, int A, float temperature, 
   return M3PC_OK;
 }
 int launch_sampling_tail(const float* mu, const float* std, const float* eps, int T, int h, int A, int E, float* eval_action,
-                         float* sample_action, unsigned long long seed, const unsigned long long* seed_ptr, cudaStream_t st, int C) {
+                         float* sample_action, unsigned long long seed, const unsigned long long* seed_ptr, cudaStream_t st, int C,
+                         const int* env_id) {
   M3PC_REQUIRE(C >= 1, "sampling tail: n_draws must be >= 1");
-  M3PC_CHECK_CUDA(launch_k(sampling_tail_kernel, dim3(ceil_div(E * C * A, 128)), dim3(128), 0, st, mu, std, eps, T, h, A, E, C, eval_action, sample_action, seed, seed_ptr));
+  M3PC_CHECK_CUDA(launch_k(sampling_tail_kernel, dim3(ceil_div(E * C * A, 128)), dim3(128), 0, st, mu, std, eps, T, h, A, E, C, eval_action, sample_action, seed, seed_ptr,
+                           env_id));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
 }

@@ -148,7 +148,8 @@ class PlanEngine:
     def plan(self, *, guidance: str, horizon: int, n_cand: int, win_states: torch.Tensor, win_actions: torch.Tensor,
              win_rewards: torch.Tensor, win_returns_tok: torch.Tensor, discount: float, temperature: float, lmbda: float,
              eps: Optional[torch.Tensor] = None, expq: Optional[torch.Tensor] = None, seed: int = 0, cand_offset: int = 0,
-             debug: bool = False, want_partials: bool = False, n_env: int = 1, exchange: bool = False):
+             debug: bool = False, want_partials: bool = False, n_env: int = 1, exchange: bool = False,
+             env_horizons: Optional[Sequence[int]] = None):
         """One M^3PC plan on one window (learner.py:103-327).  All tensors are CUDA fp32, contiguous.
         Returns (eval_action, sample_action, dbg) -- the action tensors are engine-owned and overwritten by the next call.
 
@@ -158,7 +159,12 @@ class PlanEngine:
 
         ``exchange=True`` (after ``exchange_connect``): this call plans ONE SHARD (``n_cand`` candidates starting at global id
         ``cand_offset``); the selection kernel exchanges the shard records with every rank over peer memory and merges them, so
-        the returned actions (and ``dbg["indices"]``) are the GLOBAL result on every rank."""
+        the returned actions (and ``dbg["indices"]``) are the GLOBAL result on every rank.
+
+        ``env_horizons``: one planning horizon per environment (environments at different points of their episodes,
+        learner.py:342-345); ``horizon`` must be the largest.  ``eps`` / ``dbg["candidates"]`` keep the (E*n_cand, horizon, A)
+        layout and environment e uses the first ``env_horizons[e]`` steps of its rows.  Row e of the result is what the uniform
+        call on the environments of e's horizon returns for e; with all entries equal the call is exactly the one without."""
         if not self.finalized:
             self.finalize()
         E = int(n_env)
@@ -168,6 +174,11 @@ class PlanEngine:
             raise ValueError("n_env must be >= 1")
         if E > 1 and (want_partials or cand_offset):
             raise ValueError("n_env > 1 cannot be combined with candidate sharding")
+        hz = None
+        if env_horizons is not None:
+            hz = np.ascontiguousarray(np.asarray(env_horizons, dtype=np.int32).reshape(-1))
+            if hz.size != E:
+                raise ValueError(f"env_horizons has {hz.size} entries, expected n_env={E}")
         if E > 1:
             for t, d in ((win_states, self.obs), (win_actions, self.act), (win_rewards, 1), (win_returns_tok, 1)):
                 if t.numel() != E * self.T * d:
@@ -197,8 +208,10 @@ class PlanEngine:
         a.seed = int(seed) & (2 ** 64 - 1)
         a.out_eval_action, a.out_sample_action = ev_out.data_ptr(), sm_out.data_ptr()
         a.exchange = 1 if exchange else 0
+        if hz is not None:
+            a.env_horizons = hz.ctypes.data
         dbg = {}
-        if (want_partials or debug) and E == 1:
+        if (want_partials or debug) and E == 1 and hz is None:
             a.out_partials = self._partials.data_ptr()
             dbg["partials"] = self._partials
         if debug and guidance != "mtm_sampling":

@@ -114,13 +114,14 @@ class PlannerMixin:
         self.__dict__["_plan_counter"] = c + 1
         return (int(self.seed) << 32) ^ c
 
-    def _plan_device(self, guidance: str, h: int, lmbda: float, ws, wa, wr, wt, n_env: int = 1):
+    def _plan_device(self, guidance: str, h: int, lmbda: float, ws, wa, wr, wt, n_env: int = 1, env_horizons=None):
+        """``env_horizons``: one horizon per environment when they differ (``h`` is then their maximum), else None."""
         eng = self._engine()
         eps, q = self.injected_noise if self.injected_noise is not None else (None, None)
         ev, sm, dbg = eng.plan(guidance=guidance, horizon=h, n_cand=int(self.cfg.action_samples), win_states=ws, win_actions=wa,
                                win_rewards=wr, win_returns_tok=wt, discount=float(self.cfg.discount), temperature=float(self.cfg.temperature),
                                lmbda=float(lmbda), eps=eps, expq=q, seed=self._next_seed(), cand_offset=int(self.cand_offset),
-                               debug=self.debug_plans, n_env=n_env)
+                               debug=self.debug_plans, n_env=n_env, env_horizons=env_horizons)
         if self.debug_plans:
             self.last_plan_debug = {k: v.clone() for k, v in dbg.items()}
         return ev, sm
@@ -313,24 +314,22 @@ class PlannerMixin:
 
     def _stage_and_plan(self, histories, percentage, plan: bool, rtg, future_obs: bool = False):
         """Shared body of ``action_sample_batch`` / ``action_sample_async``: E windows into ONE pinned staging buffer
-        (learner.py:346-385 per window), one H2D copy, one ``m3pc_plan`` launch sequence.  Returns (eval (E,A), sample (E,A))
-        engine-owned device tensors."""
+        (learner.py:346-385 per window, each with its environment's own clamped horizon), one H2D copy, one ``m3pc_plan``
+        launch sequence.  Returns (eval (E,A), sample (E,A)) engine-owned device tensors."""
         E = len(histories)
         if E < 1:
             raise ValueError("need at least one history")
         if E > int(getattr(self, "max_envs", 1)):
             raise ValueError(f"{E} environments but the Learner was built with max_envs={getattr(self, 'max_envs', 1)}")
         self._engine()
-        horizons = {self._clamped_horizon(hist) for hist in histories}
-        if len(horizons) != 1:
-            raise ValueError("lock-step environments must share the planning horizon (same path_length regime)")
-        horizon = horizons.pop()
+        horizons = [self._clamped_horizon(hist) for hist in histories]
+        horizon = max(horizons)
         h0 = histories[0]
         wb, slot = self._window_buffers(h0["observations"].shape[-1], h0["actions"].shape[-1], n_env=E)
         for e_, hist in enumerate(histories):
             v = (slot.h_states, slot.h_actions, slot.h_rewards, slot.h_returns) if E == 1 else \
                 (slot.h_states[e_], slot.h_actions[e_], slot.h_rewards[e_], slot.h_returns[e_])
-            self._fill_window(*v, hist, horizon, percentage, self._rtg_of(rtg, e_), future_obs=future_obs)
+            self._fill_window(*v, hist, horizons[e_], percentage, self._rtg_of(rtg, e_), future_obs=future_obs)
         self._upload_window(wb, slot)
         if plan:
             assert self.cfg.plan_guidance in _PLAN_GUIDANCE
@@ -338,13 +337,15 @@ class PlannerMixin:
             guidance = self.cfg.plan_guidance
         else:
             lmbda, guidance = 0.0, "mtm_sampling"
-        return self._plan_device(guidance, horizon, lmbda, wb.d_states, wb.d_actions, wb.d_rewards, wb.d_returns, n_env=E)
+        mixed = horizons if min(horizons) != horizon else None
+        return self._plan_device(guidance, horizon, lmbda, wb.d_states, wb.d_actions, wb.d_rewards, wb.d_returns, n_env=E, env_horizons=mixed)
 
     @torch.no_grad()
     def action_sample_batch(self, histories, percentage=1.0, horizon=4, plan=True, eval=False, rtg=None):
         """``action_sample`` for E lock-step environments in one ``m3pc_plan`` launch sequence (SURVEY.md section 8f rank 1;
-        the reference plans one environment per call, learner.py:329-417).  ``histories`` is a sequence of E history dicts that
-        share the planning-horizon regime; ``rtg`` a scalar or one value per environment (list, tuple or ndarray).  Returns
+        the reference plans one environment per call, learner.py:329-417).  ``histories`` is a sequence of E history dicts, each
+        at any ``path_length`` (each window gets its own clamped horizon); ``rtg`` a scalar or one value per environment (list,
+        tuple or ndarray).  Returns
         (E, act): row e is what ``action_sample(histories[e], ...)`` returns (``eval_action`` if ``eval`` else
         ``sample_action``).  The E windows are built in one pinned staging buffer and travel in one H2D copy; E * act floats
         come back."""

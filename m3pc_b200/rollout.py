@@ -9,7 +9,8 @@ Both build ``current_trajectory`` (zero-filled (1000, d) arrays + ``path_length`
 action, ``env.step`` it and write action / reward back.  Here the same loop runs over E lock-step environments split into G
 groups: while group g's environments step on the host, the plans of the other groups run on the GPU
 (``Learner.action_sample_async`` tickets), so neither side waits for the other.  With G = 1 and E = 1 it degenerates to the
-reference's loop.  Environments use the reference's (old gym) protocol: ``reset() -> obs``, ``step(a) -> (obs, r, done, info)``.
+reference's loop.  ``evaluate_plan(..., refill=True)`` keeps every environment slot busy instead: when an episode ends, the next
+one starts in that slot at once, and each plan covers environments at different points of their episodes.  Environments use the reference's (old gym) protocol: ``reset() -> obs``, ``step(a) -> (obs, r, done, info)``.
 """
 from __future__ import annotations
 
@@ -96,31 +97,137 @@ def run_episodes(learner, envs: Sequence[Any], *, rtg: Optional[Callable[[int], 
 
 
 def evaluate_plan(learner, make_env: Callable[[], Any], num_episodes: int, episode_rtg_ref: np.ndarray, *, n_envs: Optional[int] = None,
-                  groups: int = 2, max_path_length: int = 1000) -> Dict[str, float]:
-    """``Learner.evaluate_plan`` (learner.py:648-720) over ``num_episodes`` episodes, ``n_envs`` at a time (default: the
-    Learner's ``max_envs``): plan=True, eval=True, rtg = episode_rtg_ref[timestep], actions clipped to [-1, 1]."""
+                  groups: int = 2, max_path_length: int = 1000, refill: bool = False, device_histories: bool = False, plan: bool = True,
+                  eval: bool = True) -> Dict[str, Any]:
+    """``Learner.evaluate_plan`` (learner.py:648-720) over ``num_episodes`` episodes on ``n_envs`` environment slots (default:
+    the Learner's ``max_envs``): rtg = episode_rtg_ref[timestep of the episode], actions clipped to [-1, 1].
+
+    refill=False: rounds of ``n_envs`` episodes that start together; a round lasts as long as its longest episode.
+    refill=True: the episodes stream through the slots -- when an episode ends, the next one (``make_env()`` is called in
+    episode order) starts in its slot at once, so no slot idles while episodes are queued.  Every episode runs exactly as it
+    would alone (its own timestep, its own clamped horizon); only the batching changes.  ``device_histories=True`` keeps the
+    histories in HBM (``DeviceEpisodes``) instead of re-slicing host arrays every step (refill only).
+
+    Returns the means plus per-episode ``returns`` / ``lengths`` / ``trajectories`` in episode order."""
     n_envs = int(n_envs or getattr(learner, "max_envs", 1))
-    rets: List[float] = []
-    lens: List[int] = []
-    while len(rets) < num_episodes:
-        k = min(n_envs, num_episodes - len(rets))
-        out = run_episodes(learner, [make_env() for _ in range(k)], rtg=lambda t: episode_rtg_ref[min(t, len(episode_rtg_ref) - 1)], plan=True,
-                           eval=True, max_path_length=max_path_length, groups=groups)
-        rets += out["returns"].tolist()
-        lens += out["lengths"].tolist()
-    return {"return_mean": float(np.mean(rets)), "return_std": float(np.std(rets)), "length_mean": float(np.mean(lens)), "episodes": len(rets)}
+    rtg = lambda t: episode_rtg_ref[min(t, len(episode_rtg_ref) - 1)]  # noqa: E731
+    if device_histories and not refill:
+        raise ValueError("device_histories needs refill=True")
+    if refill:
+        trajs = _stream_episodes(learner, make_env, num_episodes, rtg, n_envs=n_envs, groups=groups, max_path_length=max_path_length,
+                                 plan=plan, eval=eval, device=device_histories)
+    else:
+        trajs = []
+        while len(trajs) < num_episodes:
+            k = min(n_envs, num_episodes - len(trajs))
+            trajs += run_episodes(learner, [make_env() for _ in range(k)], rtg=rtg, plan=plan, eval=eval, max_path_length=max_path_length,
+                                  groups=groups)["trajectories"]
+    rets = [float(tr["total_return"]) for tr in trajs]
+    lens = [int(tr["path_length"]) for tr in trajs]
+    return {"return_mean": float(np.mean(rets)), "return_std": float(np.std(rets)), "length_mean": float(np.mean(lens)), "episodes": len(rets),
+            "returns": rets, "lengths": lens, "trajectories": trajs}
+
+
+def _stream_episodes(learner, make_env: Callable[[], Any], num_episodes: int, rtg: Callable[[int], float], *, n_envs: int, groups: int,
+                     max_path_length: int, plan: bool, eval: bool, device: bool, clip=(-1.0, 1.0)) -> List[Dict[str, Any]]:
+    """``num_episodes`` episodes through min(n_envs, num_episodes) slots split into G groups (the pipelining of ``run_episodes``);
+    a slot whose episode ends takes the next queued one before its group plans again.  Returns the trajectories in episode order."""
+    E = min(int(n_envs), int(num_episodes))
+    if E < 1:
+        raise ValueError("evaluate_plan needs at least one episode and one environment slot")
+    act_dim = int(learner.mtm.data_shapes["actions"][1])
+    done_trajs: List[Optional[Dict[str, Any]]] = [None] * num_episodes
+    episode: List[Optional[int]] = [None] * E  # episode index running in each slot (None: idle)
+    envs: List[Any] = [None] * E
+    trajs: List[Optional[Dict[str, Any]]] = [None] * E
+    queued = [0]  # next episode to start
+
+    def begin(s: int) -> Optional[np.ndarray]:
+        """Start the next queued episode in slot s; its first observation, or None when the queue is empty."""
+        if queued[0] >= num_episodes:
+            episode[s] = None
+            return None
+        episode[s], queued[0] = queued[0], queued[0] + 1
+        envs[s] = make_env()
+        obs = np.asarray(envs[s].reset(), dtype=np.float32)
+        trajs[s] = new_trajectory(obs.shape[-1], act_dim, max_path_length)
+        trajs[s]["observations"][0] = obs
+        return obs
+
+    first = [begin(s) for s in range(E)]
+    ep = None
+    if device:
+        ep = DeviceEpisodes(learner, n_env=E, max_path_length=max_path_length)
+        ep.start(np.stack(first))
+    parts = [list(r) for r in _split(E, groups)]
+    members: List[List[int]] = [[] for _ in parts]
+    tickets: List[Any] = [None] * len(parts)
+
+    def submit(g: int) -> None:
+        members[g] = [s for s in parts[g] if episode[s] is not None]
+        if not members[g]:
+            tickets[g] = None
+            return
+        r = [float(rtg(trajs[s]["path_length"])) for s in members[g]]
+        if ep is not None:
+            tickets[g] = ep.plan_async(plan=plan, eval=eval, rtg=r, slots=members[g])
+        else:
+            tickets[g] = learner.action_sample_async([trajs[s] for s in members[g]], plan=plan, eval=eval, rtg=r)
+
+    for g in range(len(parts)):
+        submit(g)
+    while any(t is not None for t in tickets):
+        for g in range(len(parts)):
+            if tickets[g] is None:
+                continue
+            actions = np.clip(tickets[g].result(), clip[0], clip[1])  # waits for THIS group's plan only
+            going, ended = [], []
+            for row, s in enumerate(members[g]):
+                tr = trajs[s]
+                t = tr["path_length"]
+                new_obs, reward, done, _info = envs[s].step(actions[row])
+                tr["actions"][t] = actions[row]
+                tr["rewards"][t] = reward
+                tr["total_return"] += float(reward)
+                tr["path_length"] += 1
+                if done or t + 1 >= max_path_length:
+                    done_trajs[episode[s]] = tr
+                    ended.append(s)
+                else:
+                    tr["observations"][t + 1] = np.asarray(new_obs, dtype=np.float32)
+                    going.append((row, s))
+            if ep is not None and going:
+                rows = [r_ for r_, _ in going]
+                ep.step(actions[rows], np.array([trajs[s]["rewards"][trajs[s]["path_length"] - 1, 0] for _, s in going], np.float32),
+                        np.stack([trajs[s]["observations"][trajs[s]["path_length"]] for _, s in going]), slots=[s for _, s in going])
+            for s in ended:
+                obs = begin(s)
+                if ep is not None:
+                    if obs is None:
+                        ep.release([s])
+                    else:
+                        ep.reset([s], obs[None])
+            submit(g)
+    return done_trajs
 
 
 class DeviceEpisodes:
-    """Device-resident histories of E lock-step episodes (SURVEY.md section 8f rank 1; ``m3pc_ring_*`` in include/m3pc.h).
+    """Device-resident histories of E episode slots (SURVEY.md section 8f rank 1; ``m3pc_ring_*`` in include/m3pc.h).
 
     The reference keeps each episode as zero-filled (1000, d) numpy arrays and re-slices a window out of them on the host at
-    every step (learner.py:346-366).  Here the arrays live in HBM: a step uploads only the new observation and the action /
-    reward just taken (E * (obs + act + 1) floats), and the planner's (E, T, .) windows are cut on the device.
+    every step (learner.py:346-366).  Here the arrays live in HBM: a step uploads only the new observations and the actions /
+    rewards just taken (obs + act + 1 floats per slot), and the planner's (E, T, .) windows are cut on the device.
+
+    Every slot has its own clock ``t[slot]`` (its episode's ``path_length``; -1 = idle), so the slots need not be in lock-step:
+    when an episode ends, ``reset`` starts the next one in its slot (or ``release`` leaves the slot idle) while the other slots
+    carry on.  Per-slot arguments and results are in the order of the slot list they come with; without a list, that is every
+    active slot in ascending order.
 
         ep = DeviceEpisodes(learner, n_env=E); ep.start(obs0)                     # obs0: (E, obs)
-        a = ep.plan_async(rtg=3.0, plan=True, eval=True).result()                 # (E, act)
+        a = ep.plan_async(rtg=3.0, plan=True, eval=True).result()                 # (n_active, act)
         ep.step(a, rewards, next_obs)                                             # then plan again
+        ep.reset([2], obs)                                                        # slot 2 starts a new episode
+        ep.release([5])                                                           # slot 5 stays idle
     """
 
     def __init__(self, learner, n_env: int, max_path_length: int = 1000):
@@ -140,15 +247,23 @@ class DeviceEpisodes:
         dev = learner.mtm.pos_embed.device
         w = self.obs + self.act + 1
         self.ring = torch.zeros(self.E, self.L, w, device=dev)
-        self.t = -1  # path_length of the current step; -1 before start()
-        self._stage = [SimpleNamespace(host=torch.zeros(self.E * (w + 1)).pin_memory(), event=torch.cuda.Event(), used=False) for _ in range(2)]
+        self.t = np.full(self.E, -1, dtype=np.int64)  # path_length of each slot's current step; -1 = idle
+        # staging: [clocks (E int32) | per-slot payload], one H2D copy per call
+        n_stage = self.E * (w + 2)
+        self._stage = [SimpleNamespace(host=torch.zeros(n_stage).pin_memory(), event=torch.cuda.Event(), used=False) for _ in range(2)]
         self._turn = 0
-        self._dev_stage = torch.zeros(self.E * (w + 1), device=dev)
+        self._dev_stage = torch.zeros(n_stage, device=dev)
+        self._clock = self._dev_stage[:self.E].view(torch.int32)
         E, T = self.E, self.T
         self.win_states = torch.zeros(E, T, self.obs, device=dev)
         self.win_actions = torch.zeros(E, T, self.act, device=dev)
         self.win_rewards = torch.zeros(E, T, device=dev)
         self.win_returns = torch.zeros(E, T, device=dev)
+
+    @property
+    def active(self) -> np.ndarray:
+        """Slots with a running episode, ascending."""
+        return np.flatnonzero(self.t >= 0)
 
     def _slot(self):
         s = self._stage[self._turn]
@@ -165,75 +280,110 @@ class DeviceEpisodes:
     def _stream(self):
         return self._torch.cuda.current_stream().cuda_stream
 
-    def start(self, obs0) -> None:
-        """Begin E episodes: clears the histories and stores the first observations (E, obs)."""
-        self.ring.zero_()
-        self.t = 0
-        self._append(np.asarray(obs0, dtype=np.float32), None, None)
+    def _slots(self, slots, need_active: bool) -> np.ndarray:
+        s = self.active if slots is None else np.asarray(list(slots), dtype=np.int64).reshape(-1)
+        if s.size and (s.min() < 0 or s.max() >= self.E or len(set(s.tolist())) != s.size):
+            raise ValueError(f"slots {s.tolist()} must be distinct and in [0, {self.E})")
+        if need_active and s.size and (self.t[s] < 0).any():
+            raise RuntimeError(f"slots {s[self.t[s] < 0].tolist()} have no running episode (start() / reset() first)")
+        return s.astype(np.int32)
 
-    def step(self, actions, rewards, next_obs) -> None:
-        """Record the actions taken at the current step and their rewards, and the observations of the next step."""
-        if self.t < 0:
-            raise RuntimeError("DeviceEpisodes.step() before start()")
-        if self.t + 1 >= self.L:
-            raise RuntimeError("episode longer than max_path_length")
-        self.t += 1
-        self._append(np.asarray(next_obs, dtype=np.float32), np.asarray(actions, dtype=np.float32), np.asarray(rewards, dtype=np.float32))
-
-    def _append(self, obs, act, rew) -> None:
-        E, o, a = self.E, self.obs, self.act
-        if obs.shape != (E, o):
-            raise ValueError(f"observations have shape {obs.shape}, expected {(E, o)}")
+    def _stage_clocks(self):
         slot = self._slot()
         h = slot.host.numpy()
-        h[:E * o] = obs.reshape(-1)
-        n = E * o
+        h[:self.E].view(np.int32)[:] = self.t
+        return slot, h
+
+    def start(self, obs0) -> None:
+        """Begin E episodes, one per slot: clears the histories and stores the first observations (E, obs)."""
+        self.reset(range(self.E), obs0)
+
+    def reset(self, slots, obs) -> None:
+        """Start a new episode in each of ``slots``: zero its history (nothing of the previous episode may reach the windows of
+        the next) and store its first observation (one row of ``obs`` per listed slot)."""
+        s = self._slots(slots, need_active=False)
+        obs = np.asarray(obs, dtype=np.float32).reshape(len(s), -1)
+        nat, C = self._nat, self._C
+        nat.check(nat.lib().m3pc_ring_reset(self.ring.data_ptr(), self.E, self.L, self.obs, self.act, s.ctypes.data_as(C.c_void_p), len(s),
+                                            self._stream()), "m3pc_ring_reset")
+        self.t[s] = 0
+        self._append(s, obs, None, None)
+
+    def release(self, slots) -> None:
+        """Leave ``slots`` idle: they are skipped by ``step`` and ``plan_async`` until ``reset``."""
+        self.t[self._slots(slots, need_active=False)] = -1
+
+    def step(self, actions, rewards, next_obs, slots=None) -> None:
+        """Record the actions taken at the current step of ``slots`` (default: every active slot) and their rewards, and the
+        observations of the next step; one row per listed slot."""
+        s = self._slots(slots, need_active=True)
+        if not s.size:
+            raise RuntimeError("DeviceEpisodes.step() without a running episode")
+        if (self.t[s] + 1 >= self.L).any():
+            raise RuntimeError("episode longer than max_path_length")
+        self.t[s] += 1
+        self._append(s, np.asarray(next_obs, dtype=np.float32), np.asarray(actions, dtype=np.float32), np.asarray(rewards, dtype=np.float32))
+
+    def _append(self, s: np.ndarray, obs, act, rew) -> None:
+        n, o, a = len(s), self.obs, self.act
+        if obs.shape != (n, o):
+            raise ValueError(f"observations have shape {obs.shape}, expected {(n, o)}")
+        slot, h = self._stage_clocks()
+        base = self.E
+        h[base:base + n * o] = obs.reshape(-1)
+        m = base + n * o
         pa = pr = None
         if act is not None:
-            h[n:n + E * a] = act.reshape(E * a)
-            h[n + E * a:n + E * a + E] = rew.reshape(E)
-            pa = self._dev_stage.data_ptr() + 4 * n
-            pr = pa + 4 * E * a
-            n += E * a + E
-        self._upload(slot, n)
-        nat = self._nat
-        nat.check(nat.lib().m3pc_ring_append(self.ring.data_ptr(), E, self.L, o, a, self.t, self._dev_stage.data_ptr(), pa, pr, self._stream()),
-                  "m3pc_ring_append")
+            h[m:m + n * a] = act.reshape(n * a)
+            h[m + n * a:m + n * a + n] = rew.reshape(n)
+            pa = self._dev_stage.data_ptr() + 4 * m
+            pr = pa + 4 * n * a
+            m += n * a + n
+        self._upload(slot, m)
+        nat, C = self._nat, self._C
+        nat.check(nat.lib().m3pc_ring_append_slots(self.ring.data_ptr(), self.E, self.L, o, a, self._clock.data_ptr(), s.ctypes.data_as(C.c_void_p),
+                                                   n, self._dev_stage.data_ptr() + 4 * base, pa, pr, self._stream()), "m3pc_ring_append_slots")
 
-    def plan_async(self, percentage: float = 1.0, plan: bool = True, eval: bool = False, rtg=None):
-        """``Learner.action_sample_async`` on the device-resident histories: returns a ticket for the (E, act) actions."""
+    def plan_async(self, percentage: float = 1.0, plan: bool = True, eval: bool = False, rtg=None, slots=None):
+        """``Learner.action_sample_async`` on the device-resident histories of ``slots`` (default: every active slot): returns a
+        ticket for their (n, act) actions, row k for slot k of the list.  Each slot plans at its own clock with its own clamped
+        horizon (learner.py:342-345); ``rtg`` is a scalar or one value per listed slot."""
         L = self.learner
         if eval == True:  # noqa: E712
             assert rtg is not None
-        if self.t < 0:
-            raise RuntimeError("DeviceEpisodes.plan_async() before start()")
-        E, T = self.E, self.T
-        horizon = L._clamped_horizon({"path_length": self.t})
+        s = self._slots(slots, need_active=True)
+        n, T = len(s), self.T
+        if n == 0:
+            raise RuntimeError("DeviceEpisodes.plan_async() without a running episode (start() / reset() first)")
+        horizons = np.array([L._clamped_horizon({"path_length": int(self.t[k])}) for k in s], dtype=np.int32)
         if rtg is not None:
-            r = np.broadcast_to(np.asarray(rtg, dtype=np.float64).reshape(-1), (E,)) if np.ndim(rtg) else np.full(E, float(rtg))
+            r = np.broadcast_to(np.asarray(rtg, dtype=np.float64).reshape(-1), (n,)) if np.ndim(rtg) else np.full(n, float(rtg))
         else:
             stats = L.tokenizer_manager.tokenizers["returns"].stats
-            r = np.full(E, float(np.asarray(stats.min + (stats.max - stats.min) * percentage).reshape(-1)[0]))
-        slot = self._slot()
-        slot.host.numpy()[:E] = L._returns_tok(r * np.ones(E)).reshape(E)
-        self._upload(slot, E)
-        nat = self._nat
-        nat.check(nat.lib().m3pc_ring_windows(self.ring.data_ptr(), E, self.L, self.obs, self.act, self.t, horizon, T,
-                                              1 if getattr(L, "_future_obs_windows", False) else 0, self._dev_stage.data_ptr(),
-                                              self.win_states.data_ptr(), self.win_actions.data_ptr(), self.win_rewards.data_ptr(),
-                                              self.win_returns.data_ptr(), self._stream()), "m3pc_ring_windows")
+            r = np.full(n, float(np.asarray(stats.min + (stats.max - stats.min) * percentage).reshape(-1)[0]))
+        slot, h = self._stage_clocks()
+        h[self.E:self.E + n] = L._returns_tok(r * np.ones(n)).reshape(n)
+        self._upload(slot, self.E + n)
+        nat, C = self._nat, self._C
+        nat.check(nat.lib().m3pc_ring_windows_slots(self.ring.data_ptr(), self.E, self.L, self.obs, self.act, self._clock.data_ptr(),
+                                                    s.ctypes.data_as(C.c_void_p), horizons.ctypes.data_as(C.c_void_p), n, T,
+                                                    1 if getattr(L, "_future_obs_windows", False) else 0, self._dev_stage.data_ptr() + 4 * self.E,
+                                                    self.win_states.data_ptr(), self.win_actions.data_ptr(), self.win_rewards.data_ptr(),
+                                                    self.win_returns.data_ptr(), self._stream()), "m3pc_ring_windows_slots")
         if plan:
             assert L.cfg.plan_guidance in ("critic_lambda_guiding", "rtg_guiding", "noise_adding_lambda")
             lmbda = 0.6 if L.cfg.plan_guidance == "rtg_guiding" else L.cfg.lmbda
             guidance = L.cfg.plan_guidance
         else:
             lmbda, guidance = 0.0, "mtm_sampling"
-        lead = (E,) if E > 1 else ()
-        ev, sm = L._plan_device(guidance, horizon, lmbda, self.win_states.view(*lead, T, self.obs), self.win_actions.view(*lead, T, self.act),
-                                self.win_rewards.view(*lead, T), self.win_returns.view(*lead, T), n_env=E)
+        lead = (n,) if n > 1 else ()
+        hmax = int(horizons.max())
+        ev, sm = L._plan_device(guidance, hmax, lmbda, self.win_states[:n].view(*lead, T, self.obs), self.win_actions[:n].view(*lead, T, self.act),
+                                self.win_rewards[:n].view(*lead, T), self.win_returns[:n].view(*lead, T), n_env=n,
+                                env_horizons=horizons.tolist() if int(horizons.min()) != hmax else None)
         from .learner import PlanTicket
-        pool = L.__dict__.setdefault("_tickets", {}).setdefault(E, [])
-        ticket = pool.pop() if pool else PlanTicket(E, self.act, pool)
+        pool = L.__dict__.setdefault("_tickets", {}).setdefault(n, [])
+        ticket = pool.pop() if pool else PlanTicket(n, self.act, pool)
         ticket._submit(ev if eval else sm)
         return ticket
 
