@@ -225,31 +225,24 @@ int m3pc_backward_plan_draws(m3pc_handle_t h, int32_t mode, int32_t n_env, int32
                              const float* win_actions, const float* win_rewards, const float* win_returns_tok, const float* eps,
                              uint64_t seed, float* out_eval_action, float* out_sample_actions, void* stream);
 
-/* Device-resident episode histories of E lock-step environments (SURVEY.md section 8f rank 1): what the reference keeps as
+/* Device-resident episode histories of n_env environment slots (SURVEY.md section 8f rank 1): what the reference keeps as
  * `current_trajectory` numpy arrays (replay_buffer.py:192-205, learner.py:663-675) and re-slices on the host every step
- * (learner.py:346-366).  ring: device fp32 (E, ring_len, obs+act+1), row = [observation | action | reward] of one time step,
- * zero-initialised by the caller at episode start.
- *   m3pc_ring_append   writes the observation of step t and (when non-NULL) the action / reward of step t-1 -- the per-step
- *                      host->device traffic is E*(obs+act+1) floats instead of E windows.
- *   m3pc_ring_windows  builds the (E,T,.) planner windows of step `path_length` exactly as learner.py:346-366 does (the last
- *                      T-horizon+1 steps, zero padded; zeroshot_omtm/learner.py:97-106 when future_obs: the states window
- *                      also holds the stored future waypoints) and fills the tokenised return-to-go (one scalar per
- *                      environment, rtg_tok (E), computed by the host as in m3pc_plan_args_t.win_returns_tok). */
-int m3pc_ring_append(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, int32_t t, const float* obs,
-                     const float* prev_action, const float* prev_reward, void* stream);
-int m3pc_ring_windows(const float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, int32_t path_length,
-                      int32_t horizon, int32_t traj_length, int32_t future_obs, const float* rtg_tok, float* win_states,
-                      float* win_actions, float* win_rewards, float* win_returns_tok, void* stream);
-
-/* The same ring with one clock per slot, for environments whose episodes end at different steps and whose slots start the next
- * episode at once.  `slots` is a HOST list of n_slots slot indices (any length: it travels in kernel parameters, 256 per launch);
- * per-slot inputs and outputs are in list order.  `t` / `path_length` are DEVICE (n_env) int32 tables indexed by slot.
+ * (learner.py:346-366).  Each step uploads n*(obs+act+1) floats instead of n windows.
+ *   ring: device fp32 (n_env, ring_len, obs+act+1); row t of a slot = [observation | action | reward] of step t of its episode.
+ *   Every slot has its own clock, so episodes may end at different steps and a slot may start the next episode at once.
+ *   `slots` is a HOST list of n_slots slot indices (any length: it travels in kernel parameters, 256 per launch); per-slot inputs
+ *   and outputs are in list order.  `t` / `path_length` are DEVICE (n_env) int32 tables indexed by slot.
  *   m3pc_ring_reset          zeroes the whole history of the listed slots: a new episode (rollout.new_trajectory).  Without it the
  *                            actions / rewards of the previous episode would show up in the windows of the next.
  *   m3pc_ring_append_slots   listed slot k = slots[k] writes obs row k at step t[slot] and (when non-NULL) prev_action row k /
  *                            prev_reward[k] at step t[slot] - 1; a slot with t outside [0, ring_len) writes nothing.
- *   m3pc_ring_windows_slots  the (n_slots, T, .) windows of the listed slots, row k = m3pc_ring_windows of slot slots[k] at
- *                            path_length[slot] with horizon horizons[k] (HOST list) and rtg_tok[k] (device (n_slots)). */
+ *   m3pc_ring_windows_slots  window k of the (n_slots, T, .) planner windows is slot s = slots[k] at step p = path_length[s] with
+ *                            horizon h = horizons[k] (HOST list, in [1, T]), exactly as learner.py:346-366 builds it: the states,
+ *                            actions and rewards of steps p-T+h .. p (the last T-h+1 steps, zero where before step 0), zero padded
+ *                            to T.  With future_obs the states window instead holds the T stored steps from p-T+h on, the future
+ *                            waypoints included (zeroshot_omtm/learner.py:77-79, :97-106); when p+h > 1000 only the first
+ *                            max(T-(p+h-1000), T-h+1) of them, the rest zero.  Every step of the return window is rtg_tok[k]
+ *                            (device (n_slots)), the tokenised return-to-go the host computes as for m3pc_plan_args_t.win_returns_tok. */
 int m3pc_ring_reset(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* slots, int32_t n_slots,
                     void* stream);
 int m3pc_ring_append_slots(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* t, const int32_t* slots,

@@ -1602,7 +1602,7 @@ int timed(m3pc_engine* e, cudaStream_t st, Fn&& fn) {
 extern "C" {
 
 const char* m3pc_last_error(void) { return m3pc::g_error.c_str(); }
-const char* m3pc_version(void) { return "m3pc-b200 0.2.0 (sm_100a)"; }
+const char* m3pc_version(void) { return "m3pc-b200 0.3.0 (sm_100a)"; }
 
 int m3pc_create(m3pc_handle_t* out, const m3pc_config_t* cfg) { return m3pc::create(out, cfg); }
 
@@ -1764,12 +1764,6 @@ int m3pc_backward_plan_draws(m3pc_handle_t h, int32_t mode, int32_t n_env, int32
   });
 }
 
-int m3pc_ring_append(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, int32_t t, const float* obs,
-                     const float* prev_action, const float* prev_reward, void* stream) {
-  M3PC_REQUIRE(ring != nullptr && obs != nullptr, "null argument");
-  return m3pc::launch_ring_append(ring, n_env, ring_len, obs_dim, act_dim, t, obs, prev_action, prev_reward, reinterpret_cast<cudaStream_t>(stream));
-}
-
 int m3pc_ring_reset(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* slots, int32_t n_slots,
                     void* stream) {
   return m3pc::launch_ring_reset(ring, n_env, ring_len, obs_dim, act_dim, slots, n_slots, reinterpret_cast<cudaStream_t>(stream));
@@ -1787,14 +1781,6 @@ int m3pc_ring_windows_slots(const float* ring, int32_t n_env, int32_t ring_len, 
                             void* stream) {
   return m3pc::launch_ring_windows_slots(ring, n_env, ring_len, obs_dim, act_dim, path_length, slots, horizons, n_slots, traj_length, future_obs,
                                          rtg_tok, win_states, win_actions, win_rewards, win_returns_tok, reinterpret_cast<cudaStream_t>(stream));
-}
-
-int m3pc_ring_windows(const float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, int32_t path_length,
-                      int32_t horizon, int32_t traj_length, int32_t future_obs, const float* rtg_tok, float* win_states,
-                      float* win_actions, float* win_rewards, float* win_returns_tok, void* stream) {
-  M3PC_REQUIRE(ring && rtg_tok && win_states && win_actions && win_rewards && win_returns_tok, "null argument");
-  return m3pc::launch_ring_windows(ring, n_env, ring_len, obs_dim, act_dim, path_length, horizon, traj_length, future_obs, rtg_tok, win_states,
-                                   win_actions, win_rewards, win_returns_tok, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_gemm_bf16(const void* A, const void* W, const float* bias, void* C, int32_t M, int32_t N, int32_t K, int32_t flags, void* stream) {

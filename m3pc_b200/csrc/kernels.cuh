@@ -260,12 +260,8 @@ int launch_set_seed(unsigned long long* dst, unsigned long long seed, cudaStream
 int launch_piid_fill(const float* win_states, const float* states_pred, const float* tok_mean, const float* tok_std, float* filled, int E,
                      int T, int h, int obs, cudaStream_t st);
 
-// device-resident episode ring (include/m3pc.h: m3pc_ring_append / m3pc_ring_windows)
-int launch_ring_append(float* ring, int E, int L, int obs, int act, int t, const float* o, const float* pa, const float* pr, cudaStream_t st);
-int launch_ring_windows(const float* ring, int E, int L, int obs, int act, int pl, int h, int T, int future_obs, const float* rtg_tok,
-                        float* ws, float* wa, float* wr, float* wt, cudaStream_t st);
-// per-slot clocks (m3pc_ring_reset / m3pc_ring_append_slots / m3pc_ring_windows_slots): slots and horizons are host lists,
-// t / path_length device (E) tables indexed by slot; per-slot inputs and outputs are in list order
+// device-resident episode ring (include/m3pc.h: m3pc_ring_reset / m3pc_ring_append_slots / m3pc_ring_windows_slots): slots and
+// horizons are host lists, t / path_length device (E) tables indexed by slot; per-slot inputs and outputs are in list order
 int launch_ring_reset(float* ring, int E, int L, int obs, int act, const int* slots, int n, cudaStream_t st);
 int launch_ring_append_slots(float* ring, int E, int L, int obs, int act, const int* t, const int* slots, int n, const float* o, const float* pa,
                              const float* pr, cudaStream_t st);

@@ -388,60 +388,8 @@ __global__ void piid_fill_kernel(const float* __restrict__ win_states, const flo
   filled[i] = from_pred ? __fadd_rn(__fmul_rn(states_pred[i], tok_std[c]), tok_mean[c]) : win_states[i];
 }
 
-// ---- device-resident episode ring (row = [obs | act | reward]) ----
-__global__ void ring_append_kernel(float* __restrict__ ring, int E, int L, int obs, int act, int t, const float* __restrict__ o,
-                                   const float* __restrict__ pa, const float* __restrict__ pr) {
-  const int w = obs + act + 1;
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= E * w) return;
-  const int e = i / w, c = i - e * w;
-  float* row_t = ring + (static_cast<size_t>(e) * L + t) * w;
-  if (c < obs) {
-    row_t[c] = o[e * obs + c];
-  } else if (t > 0) {
-    float* row_p = row_t - w;
-    if (c < obs + act) {
-      if (pa != nullptr) row_p[c] = pa[e * act + (c - obs)];
-    } else if (pr != nullptr) {
-      row_p[c] = pr[e];
-    }
-  }
-}
-
-// element c of time step t of the window of ring slot `e` at step `pl` with horizon h, written to output window `o`
-__device__ __forceinline__ void ring_window_elem(const float* __restrict__ ring, int e, int o, int c, int t, int L, int obs, int act, int pl,
-                                                 int h, int T, int future_obs, const float* __restrict__ rtg_tok, float* __restrict__ ws,
-                                                 float* __restrict__ wa, float* __restrict__ wr, float* __restrict__ wt) {
-  const int w = obs + act + 1;
-  const int hl = T - h + 1, lo = pl - hl + 1;  // learner.py:346-359
-  int smart_T = T;                             // zeroshot_omtm/learner.py:77-79
-  if (future_obs && pl + h > 1000) smart_T = T - (pl + h - 1000);
-  const int step = lo + t;
-  const bool in_ring = step >= 0 && step < L;
-  const float* row = ring + (static_cast<size_t>(e) * L + (in_ring ? step : 0)) * w;
-  if (c < obs) {
-    const bool take = future_obs ? (t < smart_T || t < hl) : (t < hl);
-    ws[(static_cast<size_t>(o) * T + t) * obs + c] = (take && in_ring) ? row[c] : 0.f;
-  } else if (c < obs + act) {
-    wa[(static_cast<size_t>(o) * T + t) * act + (c - obs)] = (t < hl && in_ring) ? row[c] : 0.f;
-  } else {
-    wr[o * T + t] = (t < hl && in_ring) ? row[c] : 0.f;
-    wt[o * T + t] = rtg_tok[o];
-  }
-}
-
-__global__ void ring_windows_kernel(const float* __restrict__ ring, int E, int L, int obs, int act, int pl, int h, int T, int future_obs,
-                                    const float* __restrict__ rtg_tok, float* __restrict__ ws, float* __restrict__ wa, float* __restrict__ wr,
-                                    float* __restrict__ wt) {
-  PDL_PROLOGUE();
-  const int w = obs + act + 1;
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= E * T * w) return;
-  const int c = i % w, t = (i / w) % T, e = i / (w * T);
-  ring_window_elem(ring, e, e, c, t, L, obs, act, pl, h, T, future_obs, rtg_tok, ws, wa, wr, wt);
-}
-
-// ---- per-slot clocks: a slot list (and the horizons of its windows) travels as a kernel parameter ----
+// ---- device-resident episode ring (row = [obs | act | reward]), one clock per slot: a slot list (and the horizons of its windows)
+// travels as a kernel parameter ----
 constexpr int RING_MAX_SLOTS = 256;  // per launch; the launchers split longer lists
 struct RingSlots {
   int n;
@@ -481,6 +429,7 @@ __global__ void ring_append_slots_kernel(float* __restrict__ ring, int L, int ob
   }
 }
 
+// element c of time step t of window k: listed slot e = slots[k] at its step pl[e] with horizon h[k]
 __global__ void ring_windows_slots_kernel(const float* __restrict__ ring, int L, int obs, int act, const int* __restrict__ pl, int T, int future_obs,
                                           const __grid_constant__ RingSlots s, const float* __restrict__ rtg_tok, float* __restrict__ ws,
                                           float* __restrict__ wa, float* __restrict__ wr, float* __restrict__ wt) {
@@ -489,7 +438,22 @@ __global__ void ring_windows_slots_kernel(const float* __restrict__ ring, int L,
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= s.n * T * w) return;
   const int c = i % w, t = (i / w) % T, k = i / (w * T), e = s.slot[k];
-  ring_window_elem(ring, e, k, c, t, L, obs, act, pl[e], s.h[k], T, future_obs, rtg_tok, ws, wa, wr, wt);
+  const int p = pl[e], h = s.h[k];
+  const int hl = T - h + 1, lo = p - hl + 1;  // learner.py:346-359
+  int smart_T = T;                            // zeroshot_omtm/learner.py:77-79
+  if (future_obs && p + h > 1000) smart_T = T - (p + h - 1000);
+  const int step = lo + t;
+  const bool in_ring = step >= 0 && step < L;
+  const float* row = ring + (static_cast<size_t>(e) * L + (in_ring ? step : 0)) * w;
+  if (c < obs) {
+    const bool take = future_obs ? (t < smart_T || t < hl) : (t < hl);
+    ws[(static_cast<size_t>(k) * T + t) * obs + c] = (take && in_ring) ? row[c] : 0.f;
+  } else if (c < obs + act) {
+    wa[(static_cast<size_t>(k) * T + t) * act + (c - obs)] = (t < hl && in_ring) ? row[c] : 0.f;
+  } else {
+    wr[k * T + t] = (t < hl && in_ring) ? row[c] : 0.f;
+    wt[k * T + t] = rtg_tok[k];
+  }
 }
 
 // ---- mixed-horizon plans: every horizon class's windows, noise rows and id table, gathered in one launch ----
@@ -524,21 +488,6 @@ __global__ void mix_gather_kernel(const __grid_constant__ MixGatherParams p) {
 }
 
 }  // namespace
-
-int launch_ring_append(float* ring, int E, int L, int obs, int act, int t, const float* o, const float* pa, const float* pr, cudaStream_t st) {
-  M3PC_REQUIRE(E >= 1 && L >= 1 && t >= 0 && t < L && obs >= 1 && act >= 1, "ring_append: bad shape / step");
-  M3PC_CHECK_CUDA(launch_k(ring_append_kernel, dim3(ceil_div(E * (obs + act + 1), 128)), dim3(128), 0, st, ring, E, L, obs, act, t, o, pa, pr));
-  M3PC_CHECK_LAUNCH();
-  return M3PC_OK;
-}
-int launch_ring_windows(const float* ring, int E, int L, int obs, int act, int pl, int h, int T, int future_obs, const float* rtg_tok,
-                        float* ws, float* wa, float* wr, float* wt, cudaStream_t st) {
-  M3PC_REQUIRE(E >= 1 && L >= 1 && pl >= 0 && pl < L && h >= 1 && h <= T && T <= M3PC_MAX_T, "ring_windows: bad shape / step");
-  M3PC_CHECK_CUDA(launch_k(ring_windows_kernel, dim3(ceil_div(E * T * (obs + act + 1), 256)), dim3(256), 0, st, ring, E, L, obs, act, pl, h, T,
-                           future_obs, rtg_tok, ws, wa, wr, wt));
-  M3PC_CHECK_LAUNCH();
-  return M3PC_OK;
-}
 
 template <typename Fn>
 int for_slot_chunks(const int* slots, const int* horizons, int n, int E, int T, Fn&& launch) {

@@ -19,7 +19,7 @@ this path and are not provided.
 from __future__ import annotations
 
 from types import SimpleNamespace
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -27,9 +27,6 @@ import torch
 from .critic import TwinQ
 from .mtm_model import omtm
 from .tokenizers import TokenizerManager
-
-_PLAN_GUIDANCE = ("critic_lambda_guiding", "rtg_guiding", "noise_adding_lambda")
-
 
 class PlannerMixin:
     """Needs: self.cfg (traj_length, device, action_samples, discount, temperature, horizon, plan_guidance, lmbda),
@@ -114,17 +111,32 @@ class PlannerMixin:
         self.__dict__["_plan_counter"] = c + 1
         return (int(self.seed) << 32) ^ c
 
-    def _plan_device(self, guidance: str, h: int, lmbda: float, ws, wa, wr, wt, n_env: int = 1, env_horizons=None):
-        """``env_horizons``: one horizon per environment when they differ (``h`` is then their maximum), else None."""
+    def _guidance(self, plan: bool) -> Tuple[str, float]:
+        """learner.py:388-412: (guidance, lmbda) of a plan; ``plan=False`` samples the model (``mtm_sampling``)."""
+        if not plan:
+            return "mtm_sampling", 0.0
+        assert self.cfg.plan_guidance in ("critic_lambda_guiding", "rtg_guiding", "noise_adding_lambda")
+        return self.cfg.plan_guidance, (0.6 if self.cfg.plan_guidance == "rtg_guiding" else self.cfg.lmbda)  # learner.py:405-407 drops cfg.lmbda
+
+    def _plan_device(self, guidance: str, horizons: Sequence[int], lmbda: float, ws, wa, wr, wt):
+        """One ``m3pc_plan`` on len(horizons) windows, window e planned with horizon ``horizons[e]``."""
         eng = self._engine()
+        h = max(horizons)
         eps, q = self.injected_noise if self.injected_noise is not None else (None, None)
         ev, sm, dbg = eng.plan(guidance=guidance, horizon=h, n_cand=int(self.cfg.action_samples), win_states=ws, win_actions=wa,
                                win_rewards=wr, win_returns_tok=wt, discount=float(self.cfg.discount), temperature=float(self.cfg.temperature),
                                lmbda=float(lmbda), eps=eps, expq=q, seed=self._next_seed(), cand_offset=int(self.cand_offset),
-                               debug=self.debug_plans, n_env=n_env, env_horizons=env_horizons)
+                               debug=self.debug_plans, n_env=len(horizons), env_horizons=horizons if min(horizons) != h else None)
         if self.debug_plans:
             self.last_plan_debug = {k: v.clone() for k, v in dbg.items()}
         return ev, sm
+
+    def _ticket(self, actions: torch.Tensor, n_env: int) -> "PlanTicket":
+        """A pooled ``PlanTicket`` that receives the (n_env, act) ``actions`` once the work queued before them is done."""
+        free = self.__dict__.setdefault("_tickets", {}).setdefault(n_env, [])
+        ticket = free.pop() if free else PlanTicket(n_env, actions.shape[-1], free)
+        ticket._submit(actions)
+        return ticket
 
     def _plan_from_trajectory(self, guidance: str, trajectory: Dict[str, torch.Tensor], h: int, lmbda: float):
         self._engine()
@@ -134,7 +146,7 @@ class PlannerMixin:
         wa = trajectory["actions"].reshape(T, -1).to(dev, torch.float32)
         wr = trajectory["rewards"].reshape(T).to(dev, torch.float32)
         wt = torch.from_numpy(self._returns_tok(trajectory["returns"].detach().reshape(T).cpu().numpy())).to(dev)
-        return self._plan_device(guidance, h, lmbda, ws, wa, wr, wt)
+        return self._plan_device(guidance, [h], lmbda, ws, wa, wr, wt)
 
     # -- the reference's planner entry points -------------------------------------------------------------
     @torch.no_grad()
@@ -265,19 +277,23 @@ class PlannerMixin:
             if end_idx + horizon > 1000:
                 smart_T = smart_T - (end_idx + horizon - 1000)
             states[:smart_T] = obs[lo:lo + T]
+        returns[:] = self._rtg_token(percentage, rtg)
+
+    def _rtg_token(self, percentage: float, rtg) -> np.float32:
+        """learner.py:368-385: the token of return-to-go ``rtg`` (None: the ``percentage`` point of the dataset's return range),
+        one scalar for the whole window: (rtg * 1.0 - mean) / std in float64, rounded once to fp32."""
         if rtg is not None:
             return_to_go = float(rtg)
         else:
             stats = self.tokenizer_manager.tokenizers["returns"].stats
             return_to_go = float(np.asarray(stats.min + (stats.max - stats.min) * percentage).reshape(-1)[0])
-        # the token of a constant return-to-go is one scalar: (rtg * 1.0 - mean) / std in float64, rounded once to fp32
         cache = self.__dict__.setdefault("_rtg_tok", {})
         tok = cache.get(return_to_go)
         if tok is None:
             if len(cache) > 4096:
                 cache.clear()
             tok = cache[return_to_go] = self._returns_tok(return_to_go * np.ones(1)).reshape(-1)[0]
-        returns[:] = tok
+        return tok
 
     def _clamped_horizon(self, sequence_history) -> int:
         """learner.py:342-345: early in an episode the planning horizon grows so the window stays full."""
@@ -288,20 +304,8 @@ class PlannerMixin:
 
     @torch.no_grad()
     def action_sample(self, sequence_history, percentage=1.0, horizon=4, plan=True, eval=False, rtg=None):
-        if eval == True:  # noqa: E712  (mirrors learner.py:339-340)
-            assert rtg is not None
-        self._engine()
-        horizon = self._clamped_horizon(sequence_history)
-        wb, slot = self._window_buffers(sequence_history["observations"].shape[-1], sequence_history["actions"].shape[-1])
-        self._fill_window(slot.h_states, slot.h_actions, slot.h_rewards, slot.h_returns, sequence_history, horizon, percentage, rtg)
-        self._upload_window(wb, slot)
-        if plan:
-            assert self.cfg.plan_guidance in _PLAN_GUIDANCE
-            lmbda = 0.6 if self.cfg.plan_guidance == "rtg_guiding" else self.cfg.lmbda  # learner.py:405-407 drops cfg.lmbda
-            ev, sm = self._plan_device(self.cfg.plan_guidance, horizon, lmbda, wb.d_states, wb.d_actions, wb.d_rewards, wb.d_returns)
-            return ev.clone() if eval else sm.clone()[None, :]
-        ev, sm = self._plan_device("mtm_sampling", horizon, 0.0, wb.d_states, wb.d_actions, wb.d_rewards, wb.d_returns)
-        return ev.clone()[None, :] if eval else sm.clone()[None, :]
+        action = self._stage_and_plan([sequence_history], percentage, plan, eval, rtg).clone()
+        return action if plan and eval else action[None, :]
 
     @staticmethod
     def _rtg_of(rtg, e: int):
@@ -312,10 +316,25 @@ class PlannerMixin:
             return rtg.reshape(-1)[e if rtg.size > 1 else 0]
         return rtg
 
-    def _stage_and_plan(self, histories, percentage, plan: bool, rtg, future_obs: bool = False):
-        """Shared body of ``action_sample_batch`` / ``action_sample_async``: E windows into ONE pinned staging buffer
-        (learner.py:346-385 per window, each with its environment's own clamped horizon), one H2D copy, one ``m3pc_plan``
-        launch sequence.  Returns (eval (E,A), sample (E,A)) engine-owned device tensors."""
+    def _stage_windows(self, histories, horizons, percentage, rtg, future_obs: bool = False):
+        """The E windows of ``histories`` (learner.py:346-385, window e with horizon ``horizons[e]``) in ONE pinned staging
+        buffer and one H2D copy; returns the device side of the window buffers."""
+        E = len(histories)
+        h0 = histories[0]
+        wb, slot = self._window_buffers(h0["observations"].shape[-1], h0["actions"].shape[-1], n_env=E)
+        for e, hist in enumerate(histories):
+            v = (slot.h_states, slot.h_actions, slot.h_rewards, slot.h_returns) if E == 1 else \
+                (slot.h_states[e], slot.h_actions[e], slot.h_rewards[e], slot.h_returns[e])
+            self._fill_window(*v, hist, horizons[e], percentage, self._rtg_of(rtg, e), future_obs=future_obs)
+        self._upload_window(wb, slot)
+        return wb
+
+    def _stage_and_plan(self, histories, percentage, plan: bool, eval: bool, rtg):
+        """Shared body of ``action_sample`` / ``action_sample_batch`` / ``action_sample_async``: the E windows, each with its
+        environment's own clamped horizon, and one ``m3pc_plan`` launch sequence.  Returns the engine-owned (E, A) device tensor
+        of the eval actions if ``eval`` else of the sampled actions."""
+        if eval == True:  # noqa: E712  (mirrors learner.py:339-340)
+            assert rtg is not None
         E = len(histories)
         if E < 1:
             raise ValueError("need at least one history")
@@ -323,22 +342,10 @@ class PlannerMixin:
             raise ValueError(f"{E} environments but the Learner was built with max_envs={getattr(self, 'max_envs', 1)}")
         self._engine()
         horizons = [self._clamped_horizon(hist) for hist in histories]
-        horizon = max(horizons)
-        h0 = histories[0]
-        wb, slot = self._window_buffers(h0["observations"].shape[-1], h0["actions"].shape[-1], n_env=E)
-        for e_, hist in enumerate(histories):
-            v = (slot.h_states, slot.h_actions, slot.h_rewards, slot.h_returns) if E == 1 else \
-                (slot.h_states[e_], slot.h_actions[e_], slot.h_rewards[e_], slot.h_returns[e_])
-            self._fill_window(*v, hist, horizons[e_], percentage, self._rtg_of(rtg, e_), future_obs=future_obs)
-        self._upload_window(wb, slot)
-        if plan:
-            assert self.cfg.plan_guidance in _PLAN_GUIDANCE
-            lmbda = 0.6 if self.cfg.plan_guidance == "rtg_guiding" else self.cfg.lmbda  # learner.py:405-407 drops cfg.lmbda
-            guidance = self.cfg.plan_guidance
-        else:
-            lmbda, guidance = 0.0, "mtm_sampling"
-        mixed = horizons if min(horizons) != horizon else None
-        return self._plan_device(guidance, horizon, lmbda, wb.d_states, wb.d_actions, wb.d_rewards, wb.d_returns, n_env=E, env_horizons=mixed)
+        wb = self._stage_windows(histories, horizons, percentage, rtg)
+        guidance, lmbda = self._guidance(plan)
+        ev, sm = self._plan_device(guidance, horizons, lmbda, wb.d_states, wb.d_actions, wb.d_rewards, wb.d_returns)
+        return ev if eval else sm
 
     @torch.no_grad()
     def action_sample_batch(self, histories, percentage=1.0, horizon=4, plan=True, eval=False, rtg=None):
@@ -349,10 +356,7 @@ class PlannerMixin:
         (E, act): row e is what ``action_sample(histories[e], ...)`` returns (``eval_action`` if ``eval`` else
         ``sample_action``).  The E windows are built in one pinned staging buffer and travel in one H2D copy; E * act floats
         come back."""
-        if eval == True:  # noqa: E712
-            assert rtg is not None
-        ev, sm = self._stage_and_plan(histories, percentage, plan, rtg)
-        return (ev if eval else sm).clone().reshape(len(histories), -1)
+        return self._stage_and_plan(histories, percentage, plan, eval, rtg).clone().reshape(len(histories), -1)
 
     @torch.no_grad()
     def action_sample_async(self, histories, percentage=1.0, plan=True, eval=False, rtg=None) -> "PlanTicket":
@@ -361,14 +365,7 @@ class PlannerMixin:
         ``ticket.result()`` waits for that copy only.  The reference's callers block in ``action.cpu()`` every step
         (replay_buffer.py:211-214, learner.py:681-689); with a ticket the caller can step other environments meanwhile
         (``m3pc_b200.rollout``)."""
-        if eval == True:  # noqa: E712
-            assert rtg is not None
-        ev, sm = self._stage_and_plan(histories, percentage, plan, rtg)
-        E = len(histories)
-        free = self.__dict__.setdefault("_tickets", {}).setdefault(E, [])
-        ticket = free.pop() if free else PlanTicket(E, ev.shape[-1], free)
-        ticket._submit(ev if eval else sm)
-        return ticket
+        return self._ticket(self._stage_and_plan(histories, percentage, plan, eval, rtg), len(histories))
 
 
 class PlanTicket:

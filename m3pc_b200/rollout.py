@@ -6,11 +6,13 @@ Reference loops (one environment, one blocking plan per step):
   Learner.evaluate_plan(num_episodes, episode_rtg_ref)              finetune_omtm/learner.py:648-720
 
 Both build ``current_trajectory`` (zero-filled (1000, d) arrays + ``path_length``), call ``action_sample`` on it, clip the
-action, ``env.step`` it and write action / reward back.  Here the same loop runs over E lock-step environments split into G
-groups: while group g's environments step on the host, the plans of the other groups run on the GPU
-(``Learner.action_sample_async`` tickets), so neither side waits for the other.  With G = 1 and E = 1 it degenerates to the
-reference's loop.  ``evaluate_plan(..., refill=True)`` keeps every environment slot busy instead: when an episode ends, the next
-one starts in that slot at once, and each plan covers environments at different points of their episodes.  Environments use the reference's (old gym) protocol: ``reset() -> obs``, ``step(a) -> (obs, r, done, info)``.
+action, ``env.step`` it and write action / reward back.  Here one loop (``_run``) runs episodes through E environment slots split
+into G groups: while group g's environments step on the host, the plans of the other groups run on the GPU
+(``Learner.action_sample_async`` tickets), so neither side waits for the other.  When an episode ends and more are queued, the
+next one starts in that slot at once, so a plan may cover environments at different points of their episodes.
+``run_episodes`` queues exactly one episode per slot, so its groups stay in lock-step; with G = 1 and E = 1 it degenerates to the
+reference's loop.  ``evaluate_plan`` runs rounds of ``run_episodes`` or, with ``refill=True``, streams all its episodes through
+the slots.  Environments use the reference's (old gym) protocol: ``reset() -> obs``, ``step(a) -> (obs, r, done, info)``.
 """
 from __future__ import annotations
 
@@ -47,51 +49,8 @@ def run_episodes(learner, envs: Sequence[Any], *, rtg: Optional[Callable[[int], 
     learner.py:685); None -> the ``percentage`` rule of learner.py:368-385.  An environment that reports ``done`` leaves its
     group (the others keep their lock-step).  Returns per-environment ``returns`` / ``lengths`` and the trajectories.
     """
-    E = len(envs)
-    if E < 1:
-        raise ValueError("run_episodes needs at least one environment")
-    obs0 = [np.asarray(env.reset(), dtype=np.float32) for env in envs]
-    obs_dim = obs0[0].shape[-1]
-    act_dim = int(learner.mtm.data_shapes["actions"][1])
-    trajs = [new_trajectory(obs_dim, act_dim, max_path_length) for _ in range(E)]
-    for e in range(E):
-        trajs[e]["observations"][0] = obs0[e]
-    alive = [list(r) for r in _split(E, groups)]
-    tickets: List[Any] = [None] * len(alive)
-    steps = [0] * len(alive)  # timestep of each group (groups advance independently, members of a group together)
-
-    def submit(g: int) -> None:
-        if not alive[g]:
-            tickets[g] = None
-            return
-        t = steps[g]
-        r = None if rtg is None else float(rtg(t))
-        tickets[g] = learner.action_sample_async([trajs[e] for e in alive[g]], percentage=percentage, plan=plan, eval=eval, rtg=r)
-
-    for g in range(len(alive)):
-        submit(g)
-    while any(alive):
-        for g in range(len(alive)):
-            if tickets[g] is None:
-                continue
-            actions = np.clip(tickets[g].result(), clip[0], clip[1])  # waits for THIS group's plan only
-            t = steps[g]
-            still = []
-            for row, e in enumerate(alive[g]):
-                new_obs, reward, done, _info = envs[e].step(actions[row])
-                tr = trajs[e]
-                tr["actions"][t] = actions[row]
-                tr["rewards"][t] = reward
-                tr["total_return"] += float(reward)
-                tr["path_length"] += 1
-                if on_step is not None:
-                    on_step(e, t, actions[row], float(reward), bool(done))
-                if not done and t + 1 < max_path_length:
-                    tr["observations"][t + 1] = np.asarray(new_obs, dtype=np.float32)
-                    still.append(e)
-            alive[g] = still
-            steps[g] = t + 1
-            submit(g)  # queued behind the other groups' plans; runs while the next group's environments step
+    trajs = _run(learner, lambda i: envs[i], len(envs), len(envs), rtg=rtg, plan=plan, eval=eval, max_path_length=max_path_length,
+                 groups=groups, percentage=percentage, clip=clip, on_step=on_step)
     return {"returns": np.array([tr["total_return"] for tr in trajs], dtype=np.float64),
             "lengths": np.array([tr["path_length"] for tr in trajs], dtype=np.int64), "trajectories": trajs}
 
@@ -114,8 +73,8 @@ def evaluate_plan(learner, make_env: Callable[[], Any], num_episodes: int, episo
     if device_histories and not refill:
         raise ValueError("device_histories needs refill=True")
     if refill:
-        trajs = _stream_episodes(learner, make_env, num_episodes, rtg, n_envs=n_envs, groups=groups, max_path_length=max_path_length,
-                                 plan=plan, eval=eval, device=device_histories)
+        trajs = _run(learner, lambda i: make_env(), num_episodes, n_envs, rtg=rtg, plan=plan, eval=eval, max_path_length=max_path_length,
+                     groups=groups, device=device_histories)
     else:
         trajs = []
         while len(trajs) < num_episodes:
@@ -128,13 +87,18 @@ def evaluate_plan(learner, make_env: Callable[[], Any], num_episodes: int, episo
             "returns": rets, "lengths": lens, "trajectories": trajs}
 
 
-def _stream_episodes(learner, make_env: Callable[[], Any], num_episodes: int, rtg: Callable[[int], float], *, n_envs: int, groups: int,
-                     max_path_length: int, plan: bool, eval: bool, device: bool, clip=(-1.0, 1.0)) -> List[Dict[str, Any]]:
-    """``num_episodes`` episodes through min(n_envs, num_episodes) slots split into G groups (the pipelining of ``run_episodes``);
-    a slot whose episode ends takes the next queued one before its group plans again.  Returns the trajectories in episode order."""
-    E = min(int(n_envs), int(num_episodes))
+def _run(learner, env_of: Callable[[int], Any], num_episodes: int, n_slots: int, *, rtg: Optional[Callable[[int], float]], plan: bool,
+         eval: bool, max_path_length: int, groups: int, percentage: float = 1.0, clip=(-1.0, 1.0), device: bool = False,
+         on_step: Optional[Callable[[int, int, np.ndarray, float, bool], None]] = None) -> List[Dict[str, Any]]:
+    """The episode loop of every entry point: ``num_episodes`` episodes (``env_of(i)`` is the environment of episode i, asked for
+    in episode order) through min(n_slots, num_episodes) slots split into G groups.  While group g's environments step on the
+    host, the plans of the other groups run on the GPU.  A slot whose episode ends takes the next queued one before its group
+    plans again; with as many slots as episodes none is refilled and every group stays in lock-step.  ``device`` keeps the
+    histories in a ``DeviceEpisodes``.  ``on_step(episode, t, action, reward, done)`` follows every environment step.  Returns the
+    trajectories in episode order."""
+    E = min(int(n_slots), int(num_episodes))
     if E < 1:
-        raise ValueError("evaluate_plan needs at least one episode and one environment slot")
+        raise ValueError("need at least one episode and one environment slot")
     act_dim = int(learner.mtm.data_shapes["actions"][1])
     done_trajs: List[Optional[Dict[str, Any]]] = [None] * num_episodes
     episode: List[Optional[int]] = [None] * E  # episode index running in each slot (None: idle)
@@ -148,7 +112,7 @@ def _stream_episodes(learner, make_env: Callable[[], Any], num_episodes: int, rt
             episode[s] = None
             return None
         episode[s], queued[0] = queued[0], queued[0] + 1
-        envs[s] = make_env()
+        envs[s] = env_of(episode[s])
         obs = np.asarray(envs[s].reset(), dtype=np.float32)
         trajs[s] = new_trajectory(obs.shape[-1], act_dim, max_path_length)
         trajs[s]["observations"][0] = obs
@@ -168,11 +132,14 @@ def _stream_episodes(learner, make_env: Callable[[], Any], num_episodes: int, rt
         if not members[g]:
             tickets[g] = None
             return
-        r = [float(rtg(trajs[s]["path_length"])) for s in members[g]]
+        steps = [trajs[s]["path_length"] for s in members[g]]
+        r = None  # a group in lock-step shares one return-to-go; otherwise one per member
+        if rtg is not None:
+            r = float(rtg(steps[0])) if len(set(steps)) == 1 else [float(rtg(t)) for t in steps]
         if ep is not None:
-            tickets[g] = ep.plan_async(plan=plan, eval=eval, rtg=r, slots=members[g])
+            tickets[g] = ep.plan_async(percentage=percentage, plan=plan, eval=eval, rtg=r, slots=members[g])
         else:
-            tickets[g] = learner.action_sample_async([trajs[s] for s in members[g]], plan=plan, eval=eval, rtg=r)
+            tickets[g] = learner.action_sample_async([trajs[s] for s in members[g]], percentage=percentage, plan=plan, eval=eval, rtg=r)
 
     for g in range(len(parts)):
         submit(g)
@@ -190,6 +157,8 @@ def _stream_episodes(learner, make_env: Callable[[], Any], num_episodes: int, rt
                 tr["rewards"][t] = reward
                 tr["total_return"] += float(reward)
                 tr["path_length"] += 1
+                if on_step is not None:
+                    on_step(episode[s], t, actions[row], float(reward), bool(done))
                 if done or t + 1 >= max_path_length:
                     done_trajs[episode[s]] = tr
                     ended.append(s)
@@ -207,7 +176,7 @@ def _stream_episodes(learner, make_env: Callable[[], Any], num_episodes: int, rt
                         ep.release([s])
                     else:
                         ep.reset([s], obs[None])
-            submit(g)
+            submit(g)  # queued behind the other groups' plans; runs while the next group's environments step
     return done_trajs
 
 
@@ -356,13 +325,8 @@ class DeviceEpisodes:
         if n == 0:
             raise RuntimeError("DeviceEpisodes.plan_async() without a running episode (start() / reset() first)")
         horizons = np.array([L._clamped_horizon({"path_length": int(self.t[k])}) for k in s], dtype=np.int32)
-        if rtg is not None:
-            r = np.broadcast_to(np.asarray(rtg, dtype=np.float64).reshape(-1), (n,)) if np.ndim(rtg) else np.full(n, float(rtg))
-        else:
-            stats = L.tokenizer_manager.tokenizers["returns"].stats
-            r = np.full(n, float(np.asarray(stats.min + (stats.max - stats.min) * percentage).reshape(-1)[0]))
         slot, h = self._stage_clocks()
-        h[self.E:self.E + n] = L._returns_tok(r * np.ones(n)).reshape(n)
+        h[self.E:self.E + n] = [L._rtg_token(percentage, L._rtg_of(rtg, k)) for k in range(n)]
         self._upload(slot, self.E + n)
         nat, C = self._nat, self._C
         nat.check(nat.lib().m3pc_ring_windows_slots(self.ring.data_ptr(), self.E, self.L, self.obs, self.act, self._clock.data_ptr(),
@@ -370,22 +334,11 @@ class DeviceEpisodes:
                                                     1 if getattr(L, "_future_obs_windows", False) else 0, self._dev_stage.data_ptr() + 4 * self.E,
                                                     self.win_states.data_ptr(), self.win_actions.data_ptr(), self.win_rewards.data_ptr(),
                                                     self.win_returns.data_ptr(), self._stream()), "m3pc_ring_windows_slots")
-        if plan:
-            assert L.cfg.plan_guidance in ("critic_lambda_guiding", "rtg_guiding", "noise_adding_lambda")
-            lmbda = 0.6 if L.cfg.plan_guidance == "rtg_guiding" else L.cfg.lmbda
-            guidance = L.cfg.plan_guidance
-        else:
-            lmbda, guidance = 0.0, "mtm_sampling"
+        guidance, lmbda = L._guidance(plan)
         lead = (n,) if n > 1 else ()
-        hmax = int(horizons.max())
-        ev, sm = L._plan_device(guidance, hmax, lmbda, self.win_states[:n].view(*lead, T, self.obs), self.win_actions[:n].view(*lead, T, self.act),
-                                self.win_rewards[:n].view(*lead, T), self.win_returns[:n].view(*lead, T), n_env=n,
-                                env_horizons=horizons.tolist() if int(horizons.min()) != hmax else None)
-        from .learner import PlanTicket
-        pool = L.__dict__.setdefault("_tickets", {}).setdefault(n, [])
-        ticket = pool.pop() if pool else PlanTicket(n, self.act, pool)
-        ticket._submit(ev if eval else sm)
-        return ticket
+        ev, sm = L._plan_device(guidance, horizons.tolist(), lmbda, self.win_states[:n].view(*lead, T, self.obs),
+                                self.win_actions[:n].view(*lead, T, self.act), self.win_rewards[:n].view(*lead, T), self.win_returns[:n].view(*lead, T))
+        return L._ticket(ev if eval else sm, n)
 
 
 class LinearEnv:

@@ -44,15 +44,7 @@ class Learner(PlannerMixin):
             raise ValueError("lock-step environments must share the planning horizon (same path_length regime)")
         horizon = horizons.pop()
         E = len(histories)
-        h0 = histories[0]
-        wb, slot = self._window_buffers(h0["observations"].shape[-1], h0["actions"].shape[-1], n_env=E)
-        for e, hist in enumerate(histories):
-            if E == 1:
-                views = (slot.h_states, slot.h_actions, slot.h_rewards, slot.h_returns)
-            else:
-                views = (slot.h_states[e], slot.h_actions[e], slot.h_rewards[e], slot.h_returns[e])
-            self._fill_window(*views, hist, horizon, percentage, self._rtg_of(rtg, e), future_obs=True)
-        self._upload_window(wb, slot)
+        wb = self._stage_windows(histories, [horizon] * E, percentage, rtg, future_obs=True)
         T = self.cfg.traj_length
         ev, sm, dbg = eng.backward_plan(mode=mode, horizon=horizon, win_states=wb.d_states.view(E, T, -1), win_actions=wb.d_actions.view(E, T, -1),
                                         win_rewards=wb.d_rewards.view(E, T), win_returns_tok=wb.d_returns.view(E, T), eps=self.injected_eps,

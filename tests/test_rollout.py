@@ -78,6 +78,25 @@ def test_evaluate_plan_batches_episodes():
     assert {c[2] for c in P.calls} == set(float(v) for v in ref)  # rtg = episode_rtg_ref[timestep]
 
 
+@pytest.mark.parametrize("groups", [1, 3])
+def test_run_episodes_is_the_refill_loop_with_one_episode_per_slot(groups):
+    """run_episodes(envs) and evaluate_plan(refill=True) with as many slots as episodes are one loop: the same planner calls
+    (sizes, lock-step path_length, rtg) in the same order and the same trajectories."""
+    E, obs, A, H = 5, 4, 2, 9
+    horizons = [H, 4, H, 7, H]
+    ref = np.linspace(1.0, 0.5, H)
+    mk = lambda: [ro.LinearEnv(obs, A, seed=20 + e, horizon=horizons[e]) for e in range(E)]  # noqa: E731
+    P, Q = _FakePlanner(A), _FakePlanner(A)
+    out = ro.run_episodes(P, mk(), rtg=lambda t: ref[min(t, H - 1)], max_path_length=H, groups=groups)
+    envs = iter(mk())
+    res = ro.evaluate_plan(Q, lambda: next(envs), num_episodes=E, episode_rtg_ref=ref, n_envs=E, groups=groups, max_path_length=H, refill=True)
+    assert P.calls == Q.calls and len(P.calls) >= H
+    assert out["lengths"].tolist() == res["lengths"] == horizons
+    for a, b in zip(out["trajectories"], res["trajectories"]):
+        for k in ("observations", "actions", "rewards", "values", "total_return", "path_length"):
+            np.testing.assert_array_equal(a[k], b[k], err_msg=k)
+
+
 # ------------------------------------------------------------------------------------------------ GPU
 def _gpu_learner(precision, n_cand, max_envs, guidance="critic_lambda_guiding"):
     from m3pc_b200.learner import Learner
@@ -140,9 +159,9 @@ def test_evaluate_plan_with_the_planner_and_tickets():
 
 @pytest.mark.gpu
 def test_device_resident_episodes_build_the_same_windows_and_actions():
-    """m3pc_ring_append / m3pc_ring_windows (SURVEY.md section 8f rank 1): windows cut on the device from HBM-resident histories
-    are bit-identical to the host window builder (learner.py:346-366 semantics) at every step, across the horizon-clamp regime
-    change, and the plans on them return the same actions."""
+    """DeviceEpisodes on m3pc_ring_reset / _append_slots / _windows_slots (SURVEY.md section 8f rank 1), every slot at the same
+    step: windows cut on the device from HBM-resident histories are bit-identical to the host window builder (learner.py:346-366
+    semantics) at every step, across the horizon-clamp regime change, and the plans on them return the same actions."""
     E, H = 5, 13
     shape, L = _gpu_learner("bf16", 32, E)
     envs = [ro.LinearEnv(shape.obs_dim, shape.act_dim, seed=70 + e, horizon=H) for e in range(E)]
