@@ -104,39 +104,121 @@ int launch_simple(const AttnParams& p, cudaStream_t st) {
   const size_t smem = (static_cast<size_t>(p.n_q) * QS + static_cast<size_t>(p.n_kv) * QS + static_cast<size_t>(p.n_kv) * HD +
                        static_cast<size_t>(p.n_q) * (p.n_kv + 1)) * sizeof(float);
   M3PC_REQUIRE(smem <= 200 * 1024, "attention: sequence too long for the shared-memory resident kernel");
-  static PerDevice<size_t> configured;
-  if (smem > configured.here()) {
-    M3PC_CHECK_CUDA(cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    configured.here() = smem;
-  }
+  static PerDevice<size_t> smem_limit;
+  M3PC_CHECK_CUDA(raise_smem_limit(attention_kernel, smem_limit, smem));
   M3PC_CHECK_CUDA(launch_k(attention_kernel, dim3(p.B * p.n_head), dim3(ATT_THREADS), smem, st, p));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ bf16 tensor-core path
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
 __device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
 }
 __device__ __forceinline__ void ldsm_x4_t(uint32_t addr, uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
 }
-__device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-  __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t*>(&p);
-}
 // byte offset of 16-byte chunk `c` (0..15) of row `r` in a [rows][256 B] tile, XOR-swizzled so that the 8 rows an
 // ldmatrix phase touches fall in 8 different 16-byte bank groups
 __device__ __forceinline__ uint32_t swz(int r, int c) { return static_cast<uint32_t>(r * 256 + ((c ^ (r & 7)) << 4)); }
+
+// Key tile jp (16 keys) of a warp's attention: the shared-memory addresses of the K and V buffers that hold it and its first row
+// there.  Its keys are numbered key0 .. key0 + 15 and those numbered end or higher are pad rows, masked out of the softmax.
+struct KvTile {
+  uint32_t k, v;
+  int row, key0, end;
+};
+
+extern __shared__ __align__(128) uint8_t smem_att[];  // dynamic shared memory of both tensor-core kernels
+
+// Query tile mt (rows 16 mt .. 16 mt + 15) of the warp's Q rows, which start q_off bytes into smem_att (uQ: their shared-memory
+// address), against NTK key tiles, kv(jp) -> KvTile: scores Q K^T on mma.sync (bf16 in, fp32 accumulate), softmax in the
+// accumulator registers with quad shuffles, O = P V, and O staged as bf16 into the tile's own Q rows (dead once the scores are in
+// registers), same swizzle.  kv is a lambda capturing by value, so jp stays a compile-time constant of the unrolled loops.
+// Q is addressed as the shared-memory symbol plus an offset, not through a pointer argument, and the per-row kernel numbers its
+// keys from 0 across tiles: with a pointer argument or per-tile key counts the compiler lays the kernels out differently (more
+// registers, or a spill).
+template <int NTK, class KvOf>
+__device__ __forceinline__ void attend_q_tile(size_t q_off, uint32_t uQ, int mt, KvOf kv, int lane) {
+  uint8_t* sQ = smem_att + q_off;
+  const int g = lane >> 2, t = lane & 3;
+  const float sl2 = 0.08838834764831845f * 1.4426950408889634f;  // 1/sqrt(128) * log2(e)
+  // ---- scores = Q K^T : 16 x 16 NTK, fp32 accumulators ----
+  float sc[2 * NTK][4];
+#pragma unroll
+  for (int j = 0; j < 2 * NTK; ++j) sc[j][0] = sc[j][1] = sc[j][2] = sc[j][3] = 0.f;
+#pragma unroll
+  for (int kk = 0; kk < HD / 16; ++kk) {
+    uint32_t a[4];
+    {
+      const int r = mt * 16 + (lane & 7) + 8 * ((lane >> 3) & 1), c = 2 * kk + (lane >> 4);
+      ldsm_x4(uQ + swz(r, c), a[0], a[1], a[2], a[3]);
+    }
+#pragma unroll
+    for (int jp = 0; jp < NTK; ++jp) {  // two key tiles (16 keys) per ldmatrix.x4
+      const KvTile tile = kv(jp);
+      uint32_t b0, b1, b2, b3;
+      const int r = tile.row + (lane & 7) + 8 * (lane >> 4), c = 2 * kk + ((lane >> 3) & 1);
+      ldsm_x4(tile.k + swz(r, c), b0, b1, b2, b3);
+      mma_bf16_16816(sc[2 * jp], a, b0, b1);
+      mma_bf16_16816(sc[2 * jp + 1], a, b2, b3);
+    }
+  }
+  // ---- softmax over keys (rows g and g+8 of the tile); pad keys of each key tile masked ----
+  float m0 = -INFINITY, m1 = -INFINITY;
+#pragma unroll
+  for (int j = 0; j < 2 * NTK; ++j) {
+    const KvTile tile = kv(j >> 1);
+    const int key = tile.key0 + 8 * (j & 1) + 2 * t;
+    if (key >= tile.end) sc[j][0] = sc[j][2] = -INFINITY;
+    if (key + 1 >= tile.end) sc[j][1] = sc[j][3] = -INFINITY;
+    m0 = fmaxf(m0, fmaxf(sc[j][0], sc[j][1]));
+    m1 = fmaxf(m1, fmaxf(sc[j][2], sc[j][3]));
+  }
+  m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1)); m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
+  m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1)); m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
+  float l0 = 0.f, l1 = 0.f;
+#pragma unroll
+  for (int j = 0; j < 2 * NTK; ++j) {
+    sc[j][0] = exp2f((sc[j][0] - m0) * sl2); sc[j][1] = exp2f((sc[j][1] - m0) * sl2);
+    sc[j][2] = exp2f((sc[j][2] - m1) * sl2); sc[j][3] = exp2f((sc[j][3] - m1) * sl2);
+    l0 += sc[j][0] + sc[j][1];
+    l1 += sc[j][2] + sc[j][3];
+  }
+  l0 += __shfl_xor_sync(0xffffffffu, l0, 1); l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
+  l1 += __shfl_xor_sync(0xffffffffu, l1, 1); l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
+  const float inv0 = 1.0f / l0, inv1 = 1.0f / l1;
+
+  // ---- O = P V : 16 x 128 ----
+  float o[HD / 8][4];
+#pragma unroll
+  for (int n = 0; n < HD / 8; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
+#pragma unroll
+  for (int kk = 0; kk < NTK; ++kk) {  // 16 keys per step; the score tiles (2kk, 2kk+1) are exactly the A fragment
+    uint32_t a[4];
+    a[0] = pack_bf16(sc[2 * kk][0] * inv0, sc[2 * kk][1] * inv0);
+    a[1] = pack_bf16(sc[2 * kk][2] * inv1, sc[2 * kk][3] * inv1);
+    a[2] = pack_bf16(sc[2 * kk + 1][0] * inv0, sc[2 * kk + 1][1] * inv0);
+    a[3] = pack_bf16(sc[2 * kk + 1][2] * inv1, sc[2 * kk + 1][3] * inv1);
+    const KvTile tile = kv(kk);
+#pragma unroll
+    for (int np = 0; np < HD / 16; ++np) {  // two 8-wide dim tiles per ldmatrix.x4.trans
+      uint32_t b0, b1, b2, b3;
+      const int r = tile.row + (lane & 7) + 8 * ((lane >> 3) & 1), c = 2 * np + (lane >> 4);
+      ldsm_x4_t(tile.v + swz(r, c), b0, b1, b2, b3);
+      mma_bf16_16816(o[2 * np], a, b0, b1);
+      mma_bf16_16816(o[2 * np + 1], a, b2, b3);
+    }
+  }
+  // ---- stage O into the tile's (now dead) Q rows ----
+  __syncwarp();
+#pragma unroll
+  for (int n = 0; n < HD / 8; ++n) {
+    const int r0 = mt * 16 + g, r1 = r0 + 8;
+    *reinterpret_cast<uint32_t*>(sQ + swz(r0, n) + 4 * t) = pack_bf16(o[n][0], o[n][1]);
+    *reinterpret_cast<uint32_t*>(sQ + swz(r1, n) + 4 * t) = pack_bf16(o[n][2], o[n][3]);
+  }
+}
 
 constexpr int MMA_WARPS = 4;  // (b, head) pairs per CTA
 
@@ -145,7 +227,6 @@ template <int NTQ, int NTK>
 __global__ void __launch_bounds__(MMA_WARPS * 32) attention_mma_kernel(const __grid_constant__ AttnParams p) {
   PDL_PROLOGUE();
   constexpr int QP = NTQ * 16, KP = NTK * 16;
-  extern __shared__ __align__(128) uint8_t smem_att[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int pair = blockIdx.x * MMA_WARPS + warp;
   if (pair >= p.B * p.n_head) return;
@@ -201,88 +282,12 @@ __global__ void __launch_bounds__(MMA_WARPS * 32) attention_mma_kernel(const __g
       *reinterpret_cast<uint4*>(sV + off) = make_uint4(0, 0, 0, 0);
     }
   }
-  asm volatile("cp.async.commit_group;" ::: "memory");
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_commit();
+  cp_async_wait_all();
   __syncwarp();
 
-  const int g = lane >> 2, t = lane & 3;
-  const float sl2 = 0.08838834764831845f * 1.4426950408889634f;  // 1/sqrt(128) * log2(e)
-
 #pragma unroll 1
-  for (int mt = 0; mt < NTQ; ++mt) {
-    // ---- scores = Q[mt] K^T : 16 x KP, fp32 accumulators ----
-    float sc[2 * NTK][4];
-#pragma unroll
-    for (int j = 0; j < 2 * NTK; ++j) sc[j][0] = sc[j][1] = sc[j][2] = sc[j][3] = 0.f;
-#pragma unroll
-    for (int kk = 0; kk < HD / 16; ++kk) {
-      uint32_t a[4];
-      {
-        const int r = mt * 16 + (lane & 7) + 8 * ((lane >> 3) & 1), c = 2 * kk + (lane >> 4);
-        ldsm_x4(uQ + swz(r, c), a[0], a[1], a[2], a[3]);
-      }
-#pragma unroll
-      for (int jp = 0; jp < NTK; ++jp) {  // two key tiles (16 keys) per ldmatrix.x4
-        uint32_t b0, b1, b2, b3;
-        const int r = jp * 16 + (lane & 7) + 8 * (lane >> 4), c = 2 * kk + ((lane >> 3) & 1);
-        ldsm_x4(uK + swz(r, c), b0, b1, b2, b3);
-        mma_bf16_16816(sc[2 * jp], a, b0, b1);
-        mma_bf16_16816(sc[2 * jp + 1], a, b2, b3);
-      }
-    }
-    // ---- softmax over keys (rows g and g+8 of this m-tile); pad keys masked ----
-    float m0 = -INFINITY, m1 = -INFINITY;
-#pragma unroll
-    for (int j = 0; j < 2 * NTK; ++j) {
-      const int key = 8 * j + 2 * t;
-      if (key >= S) sc[j][0] = sc[j][2] = -INFINITY;
-      if (key + 1 >= S) sc[j][1] = sc[j][3] = -INFINITY;
-      m0 = fmaxf(m0, fmaxf(sc[j][0], sc[j][1]));
-      m1 = fmaxf(m1, fmaxf(sc[j][2], sc[j][3]));
-    }
-    m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1)); m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
-    m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1)); m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
-    float l0 = 0.f, l1 = 0.f;
-#pragma unroll
-    for (int j = 0; j < 2 * NTK; ++j) {
-      sc[j][0] = exp2f((sc[j][0] - m0) * sl2); sc[j][1] = exp2f((sc[j][1] - m0) * sl2);
-      sc[j][2] = exp2f((sc[j][2] - m1) * sl2); sc[j][3] = exp2f((sc[j][3] - m1) * sl2);
-      l0 += sc[j][0] + sc[j][1];
-      l1 += sc[j][2] + sc[j][3];
-    }
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 1); l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 1); l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-    const float inv0 = 1.0f / l0, inv1 = 1.0f / l1;
-
-    // ---- O = P V : 16 x 128 ----
-    float o[HD / 8][4];
-#pragma unroll
-    for (int n = 0; n < HD / 8; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
-#pragma unroll
-    for (int kk = 0; kk < NTK; ++kk) {  // 16 keys per step; the score tiles (2kk, 2kk+1) are exactly the A fragment
-      uint32_t a[4];
-      a[0] = pack_bf16(sc[2 * kk][0] * inv0, sc[2 * kk][1] * inv0);
-      a[1] = pack_bf16(sc[2 * kk][2] * inv1, sc[2 * kk][3] * inv1);
-      a[2] = pack_bf16(sc[2 * kk + 1][0] * inv0, sc[2 * kk + 1][1] * inv0);
-      a[3] = pack_bf16(sc[2 * kk + 1][2] * inv1, sc[2 * kk + 1][3] * inv1);
-#pragma unroll
-      for (int np = 0; np < HD / 16; ++np) {  // two 8-wide dim tiles per ldmatrix.x4.trans
-        uint32_t b0, b1, b2, b3;
-        const int r = kk * 16 + (lane & 7) + 8 * ((lane >> 3) & 1), c = 2 * np + (lane >> 4);
-        ldsm_x4_t(uV + swz(r, c), b0, b1, b2, b3);
-        mma_bf16_16816(o[2 * np], a, b0, b1);
-        mma_bf16_16816(o[2 * np + 1], a, b2, b3);
-      }
-    }
-    // ---- stage O into this m-tile's (now dead) Q rows, same swizzle ----
-    __syncwarp();
-#pragma unroll
-    for (int n = 0; n < HD / 8; ++n) {
-      const int r0 = mt * 16 + g, r1 = r0 + 8;
-      *reinterpret_cast<uint32_t*>(sQ + swz(r0, n) + 4 * t) = pack_bf16(o[n][0], o[n][1]);
-      *reinterpret_cast<uint32_t*>(sQ + swz(r1, n) + 4 * t) = pack_bf16(o[n][2], o[n][3]);
-    }
-  }
+  for (int mt = 0; mt < NTQ; ++mt) attend_q_tile<NTK>(static_cast<size_t>(sQ - smem_att), uQ, mt, [=](int jp) { return KvTile{uK, uV, jp * 16, jp * 16, S}; }, lane);
   __syncwarp();
   // ---- coalesced copy-out: 16 lanes x 16 bytes per row ----
   __nv_bfloat16* out = reinterpret_cast<__nv_bfloat16*>(p.out);
@@ -304,7 +309,6 @@ template <int NTB, int NTC>
 __global__ void __launch_bounds__(SH_WARPS * 32) attention_mma_shared_kernel(const __grid_constant__ AttnParams p) {
   PDL_PROLOGUE();
   constexpr int NTK = NTB + NTC, BP = NTB * 16, CP = NTC * 16;
-  extern __shared__ __align__(128) uint8_t smem_att[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int h = blockIdx.y;
   const int n_q = p.n_q, n_b = p.n_kv_batch, n_c = p.n_kv - p.n_kv_batch;
@@ -314,8 +318,6 @@ __global__ void __launch_bounds__(SH_WARPS * 32) attention_mma_shared_kernel(con
   uint8_t* sKb = sQ + 16 * 256;
   uint8_t* sVb = sKb + BP * 256;
   const uint32_t uKc = smem_u32(sKc), uVc = smem_u32(sVc), uQ = smem_u32(sQ), uKb = smem_u32(sKb), uVb = smem_u32(sVb);
-  const int g = lane >> 2, t = lane & 3;
-  const float sl2 = 0.08838834764831845f * 1.4426950408889634f;  // 1/sqrt(128) * log2(e)
 
   // persistent over a contiguous range of 8-row blocks: the shared tiles are staged only when their source changes (never for
   // batch-constant rows, once per environment for per-group rows) and the CTA launch cost is paid once
@@ -423,84 +425,14 @@ __global__ void __launch_bounds__(SH_WARPS * 32) attention_mma_shared_kernel(con
         cp_async16(uVb + off, src + dv + cchunk * 16);
       }
     }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
+    cp_async_commit();
+    cp_async_wait_all();
     if (restage) __syncthreads(); else __syncwarp();
 
-    // ---- scores = Q K^T : 16 x (BP + CP), fp32 accumulators ----
-    float sc[2 * NTK][4];
-#pragma unroll
-    for (int j = 0; j < 2 * NTK; ++j) sc[j][0] = sc[j][1] = sc[j][2] = sc[j][3] = 0.f;
-#pragma unroll
-    for (int kk = 0; kk < HD / 16; ++kk) {
-      uint32_t a[4];
-      {
-        const int r = (lane & 7) + 8 * ((lane >> 3) & 1), c = 2 * kk + (lane >> 4);
-        ldsm_x4(uQ + swz(r, c), a[0], a[1], a[2], a[3]);
-      }
-#pragma unroll
-      for (int jp = 0; jp < NTK; ++jp) {
-        uint32_t b0, b1, b2, b3;
-        const uint32_t base = jp < NTB ? uKb : uKc;
-        const int r = (jp < NTB ? jp : jp - NTB) * 16 + (lane & 7) + 8 * (lane >> 4), c = 2 * kk + ((lane >> 3) & 1);
-        ldsm_x4(base + swz(r, c), b0, b1, b2, b3);
-        mma_bf16_16816(sc[2 * jp], a, b0, b1);
-        mma_bf16_16816(sc[2 * jp + 1], a, b2, b3);
-      }
-    }
-    // ---- softmax over keys; pad keys of each tile masked ----
-    float m0 = -INFINITY, m1 = -INFINITY;
-#pragma unroll
-    for (int j = 0; j < 2 * NTK; ++j) {
-      const int tile = j >> 1;
-      const int cnt = tile < NTB ? n_b - 16 * tile : n_c - 16 * (tile - NTB);  // valid keys in this tile
-      const int key = 8 * (j & 1) + 2 * t;
-      if (key >= cnt) sc[j][0] = sc[j][2] = -INFINITY;
-      if (key + 1 >= cnt) sc[j][1] = sc[j][3] = -INFINITY;
-      m0 = fmaxf(m0, fmaxf(sc[j][0], sc[j][1]));
-      m1 = fmaxf(m1, fmaxf(sc[j][2], sc[j][3]));
-    }
-    m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1)); m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
-    m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1)); m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
-    float l0 = 0.f, l1 = 0.f;
-#pragma unroll
-    for (int j = 0; j < 2 * NTK; ++j) {
-      sc[j][0] = exp2f((sc[j][0] - m0) * sl2); sc[j][1] = exp2f((sc[j][1] - m0) * sl2);
-      sc[j][2] = exp2f((sc[j][2] - m1) * sl2); sc[j][3] = exp2f((sc[j][3] - m1) * sl2);
-      l0 += sc[j][0] + sc[j][1];
-      l1 += sc[j][2] + sc[j][3];
-    }
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 1); l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 1); l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-    const float inv0 = 1.0f / l0, inv1 = 1.0f / l1;
-
-    // ---- O = P V : 16 x 128 ----
-    float o[HD / 8][4];
-#pragma unroll
-    for (int n = 0; n < HD / 8; ++n) o[n][0] = o[n][1] = o[n][2] = o[n][3] = 0.f;
-#pragma unroll
-    for (int kk = 0; kk < NTK; ++kk) {
-      uint32_t a[4];
-      a[0] = pack_bf16(sc[2 * kk][0] * inv0, sc[2 * kk][1] * inv0);
-      a[1] = pack_bf16(sc[2 * kk][2] * inv1, sc[2 * kk][3] * inv1);
-      a[2] = pack_bf16(sc[2 * kk + 1][0] * inv0, sc[2 * kk + 1][1] * inv0);
-      a[3] = pack_bf16(sc[2 * kk + 1][2] * inv1, sc[2 * kk + 1][3] * inv1);
-      const uint32_t base = kk < NTB ? uVb : uVc;
-#pragma unroll
-      for (int np = 0; np < HD / 16; ++np) {
-        uint32_t b0, b1, b2, b3;
-        const int r = (kk < NTB ? kk : kk - NTB) * 16 + (lane & 7) + 8 * ((lane >> 3) & 1), c = 2 * np + (lane >> 4);
-        ldsm_x4_t(base + swz(r, c), b0, b1, b2, b3);
-        mma_bf16_16816(o[2 * np], a, b0, b1);
-        mma_bf16_16816(o[2 * np + 1], a, b2, b3);
-      }
-    }
-    __syncwarp();
-#pragma unroll
-    for (int n = 0; n < HD / 8; ++n) {  // stage O into the (now dead) Q rows, same swizzle
-      *reinterpret_cast<uint32_t*>(sQ + swz(g, n) + 4 * t) = pack_bf16(o[n][0], o[n][1]);
-      *reinterpret_cast<uint32_t*>(sQ + swz(g + 8, n) + 4 * t) = pack_bf16(o[n][2], o[n][3]);
-    }
+    // per-batch key tiles first, then the shared ones
+    attend_q_tile<NTK>(static_cast<size_t>(sQ - smem_att), uQ, 0, [=](int jp) {
+      return jp < NTB ? KvTile{uKb, uVb, jp * 16, 0, n_b - 16 * jp} : KvTile{uKc, uVc, (jp - NTB) * 16, 0, n_c - 16 * (jp - NTB)};
+    }, lane);
     __syncwarp();
     if (live) {
       char* orow = reinterpret_cast<char*>(p.out) + ((static_cast<size_t>(rhalf) * p.B + b) * D_out + h * HD) * 2 + cchunk * 16;
@@ -518,11 +450,8 @@ __global__ void __launch_bounds__(SH_WARPS * 32) attention_mma_shared_kernel(con
 template <int NTB, int NTC>
 int launch_mma_shared(const AttnParams& p, cudaStream_t st) {
   constexpr int smem = 2 * NTC * 16 * 256 + SH_WARPS * (16 + 2 * NTB * 16) * 256;
-  static PerDevice<bool> configured;
-  if (!configured.here()) {
-    M3PC_CHECK_CUDA(cudaFuncSetAttribute(attention_mma_shared_kernel<NTB, NTC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    configured.here() = true;
-  }
+  static PerDevice<size_t> smem_limit;
+  M3PC_CHECK_CUDA(raise_smem_limit(attention_mma_shared_kernel<NTB, NTC>, smem_limit, smem));
   const int nblk = ceil_div(p.B, SH_WARPS);
   const int per_sm = std::max(1, (227 * 1024) / (smem + 1024));
   // one wave of resident CTAs, each walking a range of row blocks -- once there are enough blocks for the ranges to balance
@@ -537,11 +466,8 @@ int launch_mma_shared(const AttnParams& p, cudaStream_t st) {
 template <int NTQ, int NTK>
 int launch_mma(const AttnParams& p, cudaStream_t st) {
   constexpr int smem = MMA_WARPS * (NTQ + 2 * NTK) * 16 * 256;
-  static PerDevice<bool> configured;
-  if (!configured.here()) {
-    M3PC_CHECK_CUDA(cudaFuncSetAttribute(attention_mma_kernel<NTQ, NTK>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    configured.here() = true;
-  }
+  static PerDevice<size_t> smem_limit;
+  M3PC_CHECK_CUDA(raise_smem_limit(attention_mma_kernel<NTQ, NTK>, smem_limit, smem));
   M3PC_CHECK_CUDA(launch_k(attention_mma_kernel<NTQ, NTK>, dim3(ceil_div(p.B * p.n_head, MMA_WARPS)), dim3(MMA_WARPS * 32), smem, st, p));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;

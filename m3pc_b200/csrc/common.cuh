@@ -7,6 +7,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <string>
+#include <utility>
 
 #include "../../include/m3pc.h"
 
@@ -75,24 +76,35 @@ struct Act<__nv_bfloat16> {
   static __device__ __forceinline__ void st(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
 };
 
-// 4 consecutive activations <-> float4
-__device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
-__device__ __forceinline__ float4 ld4(const __nv_bfloat16* p) {
-  uint2 u = *reinterpret_cast<const uint2*>(p);
-  __nv_bfloat162 a = *reinterpret_cast<__nv_bfloat162*>(&u.x);
-  __nv_bfloat162 b = *reinterpret_cast<__nv_bfloat162*>(&u.y);
-  float2 fa = __bfloat1622float2(a), fb = __bfloat1622float2(b);
+// ---- bf16 packing (round to nearest even) ------------------------------------------------------------------------------------
+// two floats -> packed bf16x2 (lo in the low half)
+__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
+  __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<uint32_t*>(&p);
+}
+// four bf16 (8 bytes) <-> float4
+__device__ __forceinline__ float4 bf4_to_f4(uint2 u) {
+  const __nv_bfloat162 a = *reinterpret_cast<const __nv_bfloat162*>(&u.x), b = *reinterpret_cast<const __nv_bfloat162*>(&u.y);
+  const float2 fa = __bfloat1622float2(a), fb = __bfloat1622float2(b);
   return make_float4(fa.x, fa.y, fb.x, fb.y);
 }
-__device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
-__device__ __forceinline__ void st4(__nv_bfloat16* p, float4 v) {
-  __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y);
-  __nv_bfloat162 b = __floats2bfloat162_rn(v.z, v.w);
-  uint2 u;
-  u.x = *reinterpret_cast<uint32_t*>(&a);
-  u.y = *reinterpret_cast<uint32_t*>(&b);
-  *reinterpret_cast<uint2*>(p) = u;
+__device__ __forceinline__ uint2 f4_to_bf4(float4 v) { return make_uint2(pack_bf16(v.x, v.y), pack_bf16(v.z, v.w)); }
+// eight bf16 (16 bytes) -> floats
+__device__ __forceinline__ void bf16x8_to_float(const uint4& u, float (&f)[8]) {
+  const __nv_bfloat162* p = reinterpret_cast<const __nv_bfloat162*>(&u);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 t = __bfloat1622float2(p[i]);
+    f[2 * i] = t.x;
+    f[2 * i + 1] = t.y;
+  }
 }
+
+// 4 consecutive activations <-> float4
+__device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
+__device__ __forceinline__ float4 ld4(const __nv_bfloat16* p) { return bf4_to_f4(*reinterpret_cast<const uint2*>(p)); }
+__device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+__device__ __forceinline__ void st4(__nv_bfloat16* p, float4 v) { *reinterpret_cast<uint2*>(p) = f4_to_bf4(v); }
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
@@ -103,6 +115,52 @@ __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
+}
+
+// nn.LayerNorm epsilon (every norm of the model)
+constexpr float kLnEps = 1e-5f;
+
+// LayerNorm of one row of NJ * 128 columns held by a warp as lane-strided float4s: lane owns columns j*128 + lane*4 + {0..3}
+template <int NJ>
+__device__ __forceinline__ void warp_layernorm(const float4 (&v)[NJ], const float* __restrict__ gamma, const float* __restrict__ beta,
+                                               int lane, float4 (&o)[NJ]) {
+  constexpr float inv_d = 1.0f / (NJ * 128);
+  float s = 0.f;
+#pragma unroll
+  for (int j = 0; j < NJ; ++j) s += (v[j].x + v[j].y) + (v[j].z + v[j].w);
+  const float mean = warp_sum(s) * inv_d;
+  float q = 0.f;
+#pragma unroll
+  for (int j = 0; j < NJ; ++j) {
+    const float a = v[j].x - mean, b = v[j].y - mean, c = v[j].z - mean, d = v[j].w - mean;
+    q += (a * a + b * b) + (c * c + d * d);
+  }
+  const float rstd = 1.0f / sqrtf(warp_sum(q) * inv_d + kLnEps);
+#pragma unroll
+  for (int j = 0; j < NJ; ++j) {
+    const int c = j * 128 + lane * 4;
+    const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
+    const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
+    o[j].x = (v[j].x - mean) * rstd * g.x + b.x;
+    o[j].y = (v[j].y - mean) * rstd * g.y + b.y;
+    o[j].z = (v[j].z - mean) * rstd * g.z + b.z;
+    o[j].w = (v[j].w - mean) * rstd * g.w + b.w;
+  }
+}
+
+// ---- shared memory staging and mma.sync ------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
+// 16-byte global -> shared copy through L2 only (cp.async.cg); a thread's copies land after cp_async_commit + cp_async_wait_all
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
+// d (16 x 8, fp32) += a (16 x 16, bf16, row fragment) * b (16 x 8, bf16, column fragment b0, b1): mma.sync.m16n8k16
+__device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
 // nn.GELU() (erf form), evaluated in fp32.
@@ -131,7 +189,7 @@ static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
 // ---- per-device launch bookkeeping ---------------------------------------------------------------------------------------
 // cudaFuncSetAttribute and the SM count belong to a DEVICE, not to the process: a second handle on another GPU of the same
-// process must configure its own copy of every kernel.  Launchers keep `static PerDevice<...> configured;` and index it with
+// process must configure its own copy of every kernel.  Launchers keep `static PerDevice<...>` state and index it with
 // current_device().
 constexpr int kMaxDevices = 64;
 inline int current_device() {
@@ -145,6 +203,18 @@ struct PerDevice {
   T& here() { return v[current_device()]; }
 };
 int device_num_sms();  // multiprocessors of the current device (cached per device; engine.cu)
+
+// Raise `kernel`'s dynamic shared-memory limit on the current device to `bytes` when `limit` (what was set so far) is below it:
+// a launcher with a fixed size sets it once, one with a varying size only when the size grows.  `limit` is a static of the
+// launcher, one per kernel instance: all instances of a kernel template have one function type, so a static in here would be
+// shared between them.
+template <typename... KArgs>
+inline cudaError_t raise_smem_limit(void (*kernel)(KArgs...), PerDevice<size_t>& limit, size_t bytes) {
+  if (bytes <= limit.here()) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(bytes));
+  if (e == cudaSuccess) limit.here() = bytes;
+  return e;
+}
 
 // ---- programmatic dependent launch (PDL) -------------------------------------------------------------------------------
 // Every kernel of a plan is launched with cudaLaunchAttributeProgrammaticStreamSerialization: it may be scheduled while
@@ -162,19 +232,35 @@ __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.lau
     pdl_trigger();     \
   } while (0)
 
+// PDL launch of a grid whose CTAs form clusters of `cluster` CTAs along x (the cluster-dimension attribute comes first);
+// cluster = 0 launches without the cluster attribute.
 template <typename... KArgs, typename... Args>
-inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+inline cudaError_t launch_k_cluster(unsigned cluster, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                                    Args&&... args) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchAttribute attr[2];
+  unsigned n = 0;
+  if (cluster > 0) {
+    attr[n].id = cudaLaunchAttributeClusterDimension;
+    attr[n].val.clusterDim.x = cluster;
+    attr[n].val.clusterDim.y = 1;
+    attr[n].val.clusterDim.z = 1;
+    ++n;
+  }
+  attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[n].val.programmaticStreamSerializationAllowed = 1;
+  ++n;
   cfg.attrs = attr;
-  cfg.numAttrs = 1;
+  cfg.numAttrs = n;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+  return launch_k_cluster(0, kernel, grid, block, smem, st, std::forward<Args>(args)...);
 }
 #endif
 

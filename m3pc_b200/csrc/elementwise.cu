@@ -14,36 +14,6 @@
 namespace m3pc {
 namespace {
 
-constexpr float kLnEps = 1e-5f;
-
-// Each lane owns columns c = j*128 + lane*4 + {0,1,2,3}, j < D/128.
-template <int NJ>
-__device__ __forceinline__ void warp_layernorm(const float4 (&v)[NJ], const float* __restrict__ gamma, const float* __restrict__ beta,
-                                               int lane, float4 (&o)[NJ]) {
-  constexpr float inv_d = 1.0f / (NJ * 128);
-  float s = 0.f;
-#pragma unroll
-  for (int j = 0; j < NJ; ++j) s += (v[j].x + v[j].y) + (v[j].z + v[j].w);
-  const float mean = warp_sum(s) * inv_d;
-  float q = 0.f;
-#pragma unroll
-  for (int j = 0; j < NJ; ++j) {
-    const float a = v[j].x - mean, b = v[j].y - mean, c = v[j].z - mean, d = v[j].w - mean;
-    q += (a * a + b * b) + (c * c + d * d);
-  }
-  const float rstd = 1.0f / sqrtf(warp_sum(q) * inv_d + kLnEps);
-#pragma unroll
-  for (int j = 0; j < NJ; ++j) {
-    const int c = j * 128 + lane * 4;
-    const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
-    const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
-    o[j].x = (v[j].x - mean) * rstd * g.x + b.x;
-    o[j].y = (v[j].y - mean) * rstd * g.y + b.y;
-    o[j].z = (v[j].z - mean) * rstd * g.z + b.z;
-    o[j].w = (v[j].w - mean) * rstd * g.w + b.w;
-  }
-}
-
 template <int NJ, typename AT>
 __global__ void __launch_bounds__(256) embed_kernel(const __grid_constant__ EmbedParams p, float* __restrict__ x, AT* __restrict__ y,
                                                     const float* __restrict__ gamma, const float* __restrict__ beta) {

@@ -20,7 +20,6 @@ namespace {
 
 constexpr int FB_THREADS = 256;
 constexpr int FB_WARPS = FB_THREADS / 32;
-constexpr float kEps = 1e-5f;
 constexpr int FB_APAD = 32;  // bf16 elements of row padding in a_s: rows g and g + 1 land on disjoint bank halves
 
 // ---- grid barrier: bar[0] counts arrivals monotonically within a launch (barrier k completes at (k + 1) * G), bar[1] counts CTAs
@@ -47,55 +46,6 @@ __device__ __forceinline__ void grid_finish(unsigned* bar) {
 }
 
 __device__ __forceinline__ float4 ldcg4(const float* p) { return __ldcg(reinterpret_cast<const float4*>(p)); }
-__device__ __forceinline__ float4 bf4_to_f4(uint2 u) {
-  const __nv_bfloat162 a = *reinterpret_cast<const __nv_bfloat162*>(&u.x), b = *reinterpret_cast<const __nv_bfloat162*>(&u.y);
-  const float2 fa = __bfloat1622float2(a), fb = __bfloat1622float2(b);
-  return make_float4(fa.x, fa.y, fb.x, fb.y);
-}
-__device__ __forceinline__ uint2 f4_to_bf4(float4 v) {
-  const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
-  uint2 u;
-  u.x = *reinterpret_cast<const uint32_t*>(&a);
-  u.y = *reinterpret_cast<const uint32_t*>(&b);
-  return u;
-}
-__device__ __forceinline__ void bf16x8_to_float(const uint4& u, float (&f)[8]) {
-  const __nv_bfloat162* p = reinterpret_cast<const __nv_bfloat162*>(&u);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float2 t = __bfloat1622float2(p[i]);
-    f[2 * i] = t.x;
-    f[2 * i + 1] = t.y;
-  }
-}
-
-// LayerNorm of one row held as lane-strided float4s (lane owns columns j*128 + lane*4 + {0..3})
-template <int NJ>
-__device__ __forceinline__ void warp_ln(const float4 (&v)[NJ], const float* __restrict__ gamma, const float* __restrict__ beta, int lane,
-                                        float4 (&o)[NJ]) {
-  constexpr float inv_d = 1.0f / (NJ * 128);
-  float s = 0.f;
-#pragma unroll
-  for (int j = 0; j < NJ; ++j) s += (v[j].x + v[j].y) + (v[j].z + v[j].w);
-  const float mean = warp_sum(s) * inv_d;
-  float q = 0.f;
-#pragma unroll
-  for (int j = 0; j < NJ; ++j) {
-    const float a = v[j].x - mean, b = v[j].y - mean, c = v[j].z - mean, d = v[j].w - mean;
-    q += (a * a + b * b) + (c * c + d * d);
-  }
-  const float rstd = 1.0f / sqrtf(warp_sum(q) * inv_d + kEps);
-#pragma unroll
-  for (int j = 0; j < NJ; ++j) {
-    const int c = j * 128 + lane * 4;
-    const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
-    const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
-    o[j].x = (v[j].x - mean) * rstd * g.x + b.x;
-    o[j].y = (v[j].y - mean) * rstd * g.y + b.y;
-    o[j].z = (v[j].z - mean) * rstd * g.z + b.z;
-    o[j].w = (v[j].w - mean) * rstd * g.w + b.w;
-  }
-}
 
 // a_s[r][0:D] = bf16(LayerNorm(x[r]; gamma, beta)) for r < R, x fp32 (R, D) in global memory (written by other CTAs: L2 loads)
 template <int NJ>
@@ -118,7 +68,7 @@ __device__ __forceinline__ void ln_rows_to_smem(const float* x, int R, const flo
       const int r = rb + i * FB_WARPS;
       if (r < R) {
         float4 o[NJ];
-        warp_ln<NJ>(v[i], gamma, beta, lane, o);
+        warp_layernorm<NJ>(v[i], gamma, beta, lane, o);
 #pragma unroll
         for (int j = 0; j < NJ; ++j) *reinterpret_cast<uint2*>(a_s + static_cast<size_t>(r) * lda + j * 128 + lane * 4) = f4_to_bf4(o[j]);
       }
@@ -129,13 +79,13 @@ __device__ __forceinline__ void ln_rows_to_smem(const float* x, int R, const flo
 // a_s[r][0:K] = A[r][0:K] (bf16, global, written by other CTAs)
 __device__ __forceinline__ void copy_rows_to_smem(const __nv_bfloat16* A, int R, int K, __nv_bfloat16* a_s) {
   const int cpr = K / 8, chunks = R * cpr, lda = K + FB_APAD;
-  const uint32_t base = static_cast<uint32_t>(__cvta_generic_to_shared(a_s));
+  const uint32_t base = smem_u32(a_s);
   for (int i = threadIdx.x; i < chunks; i += FB_THREADS) {  // cp.async.cg: L2 -> shared memory, every chunk in flight at once
     const int r = i / cpr, cc = i - r * cpr;
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(base + 2u * static_cast<uint32_t>(r * lda + cc * 8)), "l"(reinterpret_cast<const uint4*>(A) + i) : "memory");
+    cp_async16(base + 2u * static_cast<uint32_t>(r * lda + cc * 8), reinterpret_cast<const uint4*>(A) + i);
   }
-  asm volatile("cp.async.commit_group;" ::: "memory");
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_commit();
+  cp_async_wait_all();
 }
 
 // Skinny GEMM phase on tensor cores (mma.sync.m16n8k16, bf16 in, fp32 accumulate):
@@ -150,12 +100,6 @@ __device__ __forceinline__ void copy_rows_to_smem(const __nv_bfloat16* A, int R,
 struct WSlab {
   uint4 w[8];  // this lane's share of the item's weight slab: up to 8 k-steps of 32
 };
-
-__device__ __forceinline__ void mma_bf16_16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
 
 // issue the weight loads of work item `item` (columns 8*item .. 8*item+7) for this warp's K slice
 __device__ __forceinline__ void wslab_load(WSlab& ws, const __nv_bfloat16* __restrict__ W, int K, int item, int lane, int warp) {
@@ -194,8 +138,9 @@ __device__ __forceinline__ void rows_gemm(const __nv_bfloat16* a_s, int lda, int
           if (mt * 16 < R) {  // warp-uniform
             const uint4 lo = ra < R ? *reinterpret_cast<const uint4*>(ap + static_cast<size_t>(ra) * lda + i * 32) : make_uint4(0, 0, 0, 0);
             const uint4 hi = rb < R ? *reinterpret_cast<const uint4*>(ap + static_cast<size_t>(rb) * lda + i * 32) : make_uint4(0, 0, 0, 0);
-            mma_bf16_16816(c[mt], lo.x, hi.x, lo.y, hi.y, ws.w[i].x, ws.w[i].y);
-            mma_bf16_16816(c[mt], lo.z, hi.z, lo.w, hi.w, ws.w[i].z, ws.w[i].w);
+            const uint32_t a0[4] = {lo.x, hi.x, lo.y, hi.y}, a1[4] = {lo.z, hi.z, lo.w, hi.w};
+            mma_bf16_16816(c[mt], a0, ws.w[i].x, ws.w[i].y);
+            mma_bf16_16816(c[mt], a1, ws.w[i].z, ws.w[i].w);
           }
         }
       }
@@ -317,7 +262,7 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
             }
           }
         }
-        warp_ln<NJ>(acc, w.n1_w, w.n1_b, lane, o);
+        warp_layernorm<NJ>(acc, w.n1_w, w.n1_b, lane, o);
 #pragma unroll
         for (int j = 0; j < NJ; ++j) {
           *reinterpret_cast<uint2*>(a_s + static_cast<size_t>(s) * LD1 + j * 128 + lane * 4) = f4_to_bf4(o[j]);
@@ -435,13 +380,13 @@ __global__ void __launch_bounds__(FB_THREADS, 1) fused_b1_kernel(const __grid_co
     float4 v[NJ], o[NJ];
 #pragma unroll
     for (int j = 0; j < NJ; ++j) v[j] = ldcg4(p.XS + static_cast<size_t>(qi) * D + j * 128 + lane * 4);
-    warp_ln<NJ>(v, p.fnorm_w, p.fnorm_b, lane, o);
+    warp_layernorm<NJ>(v, p.fnorm_w, p.fnorm_b, lane, o);
 #pragma unroll
     for (int j = 0; j < NJ; ++j) *reinterpret_cast<uint2*>(p.Y + static_cast<size_t>(qi) * D + j * 128 + lane * 4) = f4_to_bf4(o[j]);
     const int k = p.need_mod[qi];
     if (p.head_g[k] != nullptr) {
       float4 o2[NJ];
-      warp_ln<NJ>(o, p.head_g[k], p.head_b[k], lane, o2);
+      warp_layernorm<NJ>(o, p.head_g[k], p.head_b[k], lane, o2);
 #pragma unroll
       for (int j = 0; j < NJ; ++j) *reinterpret_cast<uint2*>(p.Y2 + static_cast<size_t>(qi) * D + j * 128 + lane * 4) = f4_to_bf4(o2[j]);
     } else if (p.out_mu != nullptr) {
@@ -496,14 +441,11 @@ int launch_fused_b1(const FusedB1Params& p, int D, cudaStream_t st) {
                "fused_b1: shape out of range");
   const size_t smem = fused_b1_smem_bytes(D, p.S, p.n_need);
   M3PC_REQUIRE(smem <= 200 * 1024, "fused_b1: activation panel does not fit shared memory");
-  static PerDevice<size_t> configured;  // the attribute and the SM count are per device, not per process
+  static PerDevice<size_t> smem_limit;  // the attribute and the SM count are per device, not per process
   auto kern = fused_b1_kernel<4>;
   const int num_sms = device_num_sms();
   M3PC_REQUIRE(num_sms > 0, "fused_b1: no device");
-  if (smem > configured.here()) {
-    M3PC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    configured.here() = smem;
-  }
+  M3PC_CHECK_CUDA(raise_smem_limit(kern, smem_limit, smem));
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(num_sms);  // one CTA per SM: all CTAs are co-resident (cooperative launch), the grid barrier cannot deadlock
   cfg.blockDim = dim3(FB_THREADS);

@@ -34,9 +34,6 @@
 
 namespace m3pc {
 
-int make_tmap(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows);
-int make_tmap_out(CUtensorMap* map, void* ptr, uint64_t rows, uint64_t cols, bool f32);
-
 int g_ln_unit_rows = 0;  // rows per CTA-pair unit of the fused kernel: 0 = chosen per launch (gemm_ln_bf16), or 128 / 256 forced; m3pc_set_option "gemm_ln_unit_rows"
 
 namespace {
@@ -87,9 +84,6 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const float (&v)[16]) 
       "r"(__float_as_uint(v[8])), "r"(__float_as_uint(v[9])), "r"(__float_as_uint(v[10])), "r"(__float_as_uint(v[11])),
       "r"(__float_as_uint(v[12])), "r"(__float_as_uint(v[13])), "r"(__float_as_uint(v[14])), "r"(__float_as_uint(v[15]))
       : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* map, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1) : "memory");
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void named_bar_sync(int id, int threads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory"); }
@@ -342,7 +336,7 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
         }
         mean = t1 * (1.0f / LN_N);
         const float var = fmaxf(t2 * (1.0f / LN_N) - mean * mean, 0.f);
-        rstd = rsqrtf(var + 1e-5f);
+        rstd = rsqrtf(var + kLnEps);
       }
       named_bar_sync(1 + rowq, 32 * NSHARE);  // everybody has read the statistics: the next unit may overwrite them
       if (live) {
@@ -368,14 +362,8 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
               const int c = col0 + 8 * j + e;
               y[e] = (__uint_as_float(r[8 * j + e]) - mean) * rstd * sgamma[c] + sbeta[c];
             }
-            __nv_bfloat162 p0 = __floats2bfloat162_rn(y[0], y[1]);
-            __nv_bfloat162 p1 = __floats2bfloat162_rn(y[2], y[3]);
-            __nv_bfloat162 p2 = __floats2bfloat162_rn(y[4], y[5]);
-            __nv_bfloat162 p3 = __floats2bfloat162_rn(y[6], y[7]);
-            uint4 o;
-            o.x = *reinterpret_cast<uint32_t*>(&p0); o.y = *reinterpret_cast<uint32_t*>(&p1);
-            o.z = *reinterpret_cast<uint32_t*>(&p2); o.w = *reinterpret_cast<uint32_t*>(&p3);
-            *reinterpret_cast<uint4*>(bx + lane * 64 + ((static_cast<uint32_t>(j) ^ sw) << 4)) = o;
+            *reinterpret_cast<uint4*>(bx + lane * 64 + ((static_cast<uint32_t>(j) ^ sw) << 4)) =
+                make_uint4(pack_bf16(y[0], y[1]), pack_bf16(y[2], y[3]), pack_bf16(y[4], y[5]), pack_bf16(y[6], y[7]));
           }
           fence_proxy_async();
           __syncwarp();
@@ -406,11 +394,8 @@ int launch_ln(LnGemmParams& P, cudaStream_t st) {
   using L = SmemLn<ROWS, STAGES, NBOX>;
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
   static_assert(L::kStoreOffset % 1024 == 0, "operand stages must keep 1024-byte alignment");
-  static PerDevice<bool> configured;
-  if (!configured.here()) {
-    M3PC_CHECK_CUDA(cudaFuncSetAttribute(gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-    configured.here() = true;
-  }
+  static PerDevice<size_t> smem_limit;
+  M3PC_CHECK_CUDA(raise_smem_limit(gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, smem_limit, L::kTotal));
   int units = 0;
   for (int g = 0; g < P.n; ++g) {
     P.p[g].unit0 = units;
@@ -418,21 +403,7 @@ int launch_ln(LnGemmParams& P, cudaStream_t st) {
   }
   P.n_units = units;
   const int pairs = std::min(P.n_units, device_num_sms() / 2);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(2 * pairs);
-  cfg.blockDim = dim3(LN_THREADS);
-  cfg.dynamicSmemBytes = L::kTotal;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  M3PC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, P));
+  M3PC_CHECK_CUDA(launch_k_cluster(2, gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, dim3(2 * pairs), dim3(LN_THREADS), L::kTotal, st, P));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
 }

@@ -14,16 +14,6 @@ constexpr int SK_THREADS = 256;      // 8 warps, one output column per warp
 constexpr int SK_MAX_M = 32;
 constexpr int SK_WREG = 8;           // 16-byte weight chunks a lane keeps in flight (covers K <= 2048 in one batch)
 
-__device__ __forceinline__ void bf16x8_to_float(const uint4& u, float (&f)[8]) {
-  const __nv_bfloat162* p = reinterpret_cast<const __nv_bfloat162*>(&u);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float2 t = __bfloat1622float2(p[i]);
-    f[2 * i] = t.x;
-    f[2 * i + 1] = t.y;
-  }
-}
-
 __global__ void __launch_bounds__(SK_THREADS) gemm_skinny_kernel(const __nv_bfloat16* __restrict__ A, const __nv_bfloat16* __restrict__ W,
                                                                  void* __restrict__ C, int M, int N, int K, const float* __restrict__ bias,
                                                                  const float* __restrict__ table, int rows_per_group, int flags) {
@@ -43,10 +33,9 @@ __global__ void __launch_bounds__(SK_THREADS) gemm_skinny_kernel(const __nv_bflo
   }
   // stage A (M*K bf16) with cp.async: every 16-byte chunk is in flight before the first one is waited for
   const int chunks = M * kchunks;
-  const uint32_t as_base = static_cast<uint32_t>(__cvta_generic_to_shared(As));
-  for (int i = threadIdx.x; i < chunks; i += SK_THREADS)
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(as_base + 16u * i), "l"(reinterpret_cast<const uint4*>(A) + i) : "memory");
-  asm volatile("cp.async.commit_group;" ::: "memory");
+  const uint32_t as_base = smem_u32(As);
+  for (int i = threadIdx.x; i < chunks; i += SK_THREADS) cp_async16(as_base + 16u * i, reinterpret_cast<const uint4*>(A) + i);
+  cp_async_commit();
   // epilogue operands are independent of the accumulation: fetch them now as well
   const int erow = lane < M ? lane : 0;
   float e_bias = 0.f, e_table = 0.f, e_res = 0.f;
@@ -55,7 +44,7 @@ __global__ void __launch_bounds__(SK_THREADS) gemm_skinny_kernel(const __nv_bflo
     if (table != nullptr) e_table = __ldg(table + static_cast<size_t>(erow / rows_per_group) * N + n);
     if (flags & EPI_RESIDUAL) e_res = reinterpret_cast<const float*>(C)[static_cast<size_t>(erow) * N + n];
   }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  cp_async_wait_all();
   __syncthreads();
   if (n >= N) return;
   const bool do_gelu = flags & EPI_GELU, do_relu = flags & EPI_RELU, do_res = flags & EPI_RESIDUAL;
@@ -117,11 +106,8 @@ int gemm_bf16_skinny(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, in
   M3PC_REQUIRE(M >= 1 && M <= SK_MAX_M && K % 8 == 0, "gemm_skinny: needs M <= 32 and K % 8 == 0");
   const size_t smem = static_cast<size_t>(M) * K * sizeof(__nv_bfloat16);
   M3PC_REQUIRE(smem <= 160 * 1024, "gemm_skinny: A panel does not fit shared memory");
-  static PerDevice<size_t> configured;
-  if (smem > configured.here()) {
-    M3PC_CHECK_CUDA(cudaFuncSetAttribute(gemm_skinny_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    configured.here() = smem;
-  }
+  static PerDevice<size_t> smem_limit;
+  M3PC_CHECK_CUDA(raise_smem_limit(gemm_skinny_kernel, smem_limit, smem));
   M3PC_CHECK_CUDA(launch_k(gemm_skinny_kernel, dim3(ceil_div(N, SK_THREADS / 32)), dim3(SK_THREADS), smem, st, A, W, C, M, N, K, epi.bias, epi.table,
                                                                           epi.rows_per_group > 0 ? epi.rows_per_group : 1, epi.flags));
   M3PC_CHECK_LAUNCH();

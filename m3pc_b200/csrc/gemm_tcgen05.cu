@@ -145,16 +145,8 @@ __device__ __forceinline__ void epilogue_tile(uint32_t tmem_acc, float* xp, void
           }
 #pragma unroll
           for (int j = 0; j < 8; ++j) v[j] = apply_act(v[j], do_gelu, do_relu);
-          uint4 o;
-          __nv_bfloat162 p0 = __floats2bfloat162_rn(v[0], v[1]);
-          __nv_bfloat162 p1 = __floats2bfloat162_rn(v[2], v[3]);
-          __nv_bfloat162 p2 = __floats2bfloat162_rn(v[4], v[5]);
-          __nv_bfloat162 p3 = __floats2bfloat162_rn(v[6], v[7]);
-          o.x = *reinterpret_cast<uint32_t*>(&p0);
-          o.y = *reinterpret_cast<uint32_t*>(&p1);
-          o.z = *reinterpret_cast<uint32_t*>(&p2);
-          o.w = *reinterpret_cast<uint32_t*>(&p3);
-          *reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(C) + static_cast<size_t>(row) * N + col0 + cc) = o;
+          *reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(C) + static_cast<size_t>(row) * N + col0 + cc) =
+              make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
         }
       }
     }
@@ -560,14 +552,9 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
             }
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
-              __nv_bfloat162 p0 = __floats2bfloat162_rn(v[8 * j + 0], v[8 * j + 1]);
-              __nv_bfloat162 p1 = __floats2bfloat162_rn(v[8 * j + 2], v[8 * j + 3]);
-              __nv_bfloat162 p2 = __floats2bfloat162_rn(v[8 * j + 4], v[8 * j + 5]);
-              __nv_bfloat162 p3 = __floats2bfloat162_rn(v[8 * j + 6], v[8 * j + 7]);
-              uint4 o;
-              o.x = *reinterpret_cast<uint32_t*>(&p0); o.y = *reinterpret_cast<uint32_t*>(&p1);
-              o.z = *reinterpret_cast<uint32_t*>(&p2); o.w = *reinterpret_cast<uint32_t*>(&p3);
-              *reinterpret_cast<uint4*>(buf + lane * 64 + ((static_cast<uint32_t>(j) ^ sw) << 4)) = o;
+              *reinterpret_cast<uint4*>(buf + lane * 64 + ((static_cast<uint32_t>(j) ^ sw) << 4)) =
+                  make_uint4(pack_bf16(v[8 * j + 0], v[8 * j + 1]), pack_bf16(v[8 * j + 2], v[8 * j + 3]), pack_bf16(v[8 * j + 4], v[8 * j + 5]),
+                             pack_bf16(v[8 * j + 6], v[8 * j + 7]));
             }
           }
           fence_proxy_async();  // my generic-proxy writes -> visible to the TMA (async proxy)
@@ -616,32 +603,15 @@ template <int BN, int STAGES, int CL>
 int launch(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, int M, int N, int K, const GemmEpilogue& epi, cudaStream_t st) {
   using L = SmemLayout<BN, STAGES>;
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
-  static PerDevice<bool> configured;
-  if (!configured.here()) {
-    M3PC_CHECK_CUDA(cudaFuncSetAttribute(gemm_bf16_kernel<BN, STAGES, CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-    configured.here() = true;
-  }
+  static PerDevice<size_t> smem_limit;
+  M3PC_CHECK_CUDA(raise_smem_limit(gemm_bf16_kernel<BN, STAGES, CL>, smem_limit, L::kTotal));
   CUtensorMap ta, tw;
   M3PC_TRY(make_tmap(&ta, A, static_cast<uint64_t>(M), static_cast<uint64_t>(K), BM));
   M3PC_TRY(make_tmap(&tw, W, static_cast<uint64_t>(N), static_cast<uint64_t>(K), BN / CL));
   EpiParams ep{epi.bias, epi.table, epi.rows_per_group > 0 ? epi.rows_per_group : 1, epi.flags};
   const int units = (N / BN) * ceil_div(ceil_div(M, BM), CL);
   const int clusters = std::min(units, device_num_sms() / CL);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(clusters * CL);
-  cfg.blockDim = dim3(GEMM_THREADS);
-  cfg.dynamicSmemBytes = L::kTotal;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  M3PC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_kernel<BN, STAGES, CL>, ta, tw, C, M, N, K, ep));
+  M3PC_CHECK_CUDA(launch_k_cluster(CL, gemm_bf16_kernel<BN, STAGES, CL>, dim3(clusters * CL), dim3(GEMM_THREADS), L::kTotal, st, ta, tw, C, M, N, K, ep));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
 }
@@ -671,11 +641,8 @@ int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
   using L = Smem2<STAGES>;
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
   static_assert(sizeof(GroupParams) <= 4000, "kernel parameter space");
-  static PerDevice<bool> configured;
-  if (!configured.here()) {
-    M3PC_CHECK_CUDA(cudaFuncSetAttribute(gemm_bf16_2sm_kernel<STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
-    configured.here() = true;
-  }
+  static PerDevice<size_t> smem_limit;
+  M3PC_CHECK_CUDA(raise_smem_limit(gemm_bf16_2sm_kernel<STAGES>, smem_limit, L::kTotal));
   const int n_pairs_max = device_num_sms() / 2;
   GroupParams gp{};
   gp.n = n;
@@ -700,21 +667,7 @@ int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
   gp.total_units = units;
   const int pairs = std::min(units, n_pairs_max);
   gp.strided = n == 1 && gp.p[0].n_tiles == 2 && probs[0].K >= 1024 && pairs % 2 == 0 && units >= 2 * pairs;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(2 * pairs);
-  cfg.blockDim = dim3(GEMM_THREADS_2SM);
-  cfg.dynamicSmemBytes = L::kTotal;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  M3PC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_2sm_kernel<STAGES>, gp));
+  M3PC_CHECK_CUDA(launch_k_cluster(2, gemm_bf16_2sm_kernel<STAGES>, dim3(2 * pairs), dim3(GEMM_THREADS_2SM), L::kTotal, st, gp));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
 }

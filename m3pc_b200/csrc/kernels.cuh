@@ -5,7 +5,6 @@
 namespace m3pc {
 
 constexpr int MAX_TOK = 64;  // 4 * traj_length, traj_length <= 16
-constexpr int LN_EPS_BITS = 0x3727c5ac;  // 1e-5f
 
 // ---- K1: tokenise + embed + positional/per-dim + unmasked gather (+ LayerNorm of the first block) -------
 struct EmbedTok {

@@ -1,4 +1,4 @@
-// tcgen05 / TMA / mbarrier PTX wrappers shared by the sm_100a tensor-core kernels (gemm_tcgen05.cu, encoder_mega.cu).
+// tcgen05 / TMA / mbarrier PTX wrappers shared by the sm_100a tensor-core kernels (gemm_tcgen05.cu, gemm_ln.cu).
 #pragma once
 #include <cuda.h>
 
@@ -11,8 +11,6 @@ constexpr int BK = 64;      // 64 bf16 = 128 bytes = one SWIZZLE_128B atom row
 constexpr int UMMA_K = 16;  // K of one tcgen05.mma (kind::f16)
 
 // ---------------------------------------------------------------- PTX wrappers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
 }
@@ -32,22 +30,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       "@p bra.uni WAIT_DONE;\n\t"
       "bra.uni WAIT_LOOP;\n\t"
       "WAIT_DONE:\n\t"
-      "}" ::"r"(addr),
-      "r"(parity)
-      : "memory");
-}
-// wait with cluster-scope acquire: the barrier was arrived on (release.cluster) by threads of the PEER CTA whose shared-memory
-// writes must be visible to what this thread does next
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t addr = smem_u32(bar);
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "WAIT_LOOP_C:\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra.uni WAIT_DONE_C;\n\t"
-      "bra.uni WAIT_LOOP_C;\n\t"
-      "WAIT_DONE_C:\n\t"
       "}" ::"r"(addr),
       "r"(parity)
       : "memory");
@@ -151,9 +133,6 @@ __device__ __forceinline__ void tma_load_2d_2sm(void* smem_dst, const CUtensorMa
       "l"(reinterpret_cast<uint64_t>(map)), "r"(bar_cluster_addr), "r"(c0), "r"(c1)
       : "memory");
 }
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster_addr) : "memory");
-}
 // D[tmem, 256 x N split over the pair: 128 lanes in each CTA] (+)= A[256 x 16: 128 rows from each CTA's smem] * B[N x 16: N/2 rows
 // from each CTA's smem]^T; issued by one thread of the leader CTA, descriptors are the leader's (same offsets in the peer).
 __device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
@@ -204,7 +183,6 @@ __device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* map, const 
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 // GELU(erf) for the bf16 epilogues in 8 instructions (one MUFU): 0.5 x (1 + tanh(x (c0 + c1 x^2 + c2 x^4))) with x^2 capped at 16;
 // coefficients fitted to the erf form (max |error| 2.5e-5 with an exact tanh; tanh.approx adds <= 2^-11 relative on tanh),
