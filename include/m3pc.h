@@ -102,12 +102,6 @@ int m3pc_finalize_params(m3pc_handle_t h);
  *   "fused_ln_min_rows" 1024   smallest GEMM (rows) the fused residual GEMM + LayerNorm kernel is used for (>= 129; below, the
  *                              GEMM is followed by a LayerNorm kernel)
  *   "restrict_deep_decoder" 1  decoders with > 1 layer: last layer on the consumed rows only (0: every row)
- *   "split_residual_min_rows" 0  restricted decoder layer, out-projection + residual + LayerNorm of the consumed rows: from this
- *                              many rows up the residual is read in place (batch-constant mask-token rows as a table, kept
- *                              tokens through their own tensor map), one problem per source in a grouped launch, instead of
- *                              a residual copy + one problem (bit-identical results)
- *   "grouped_ln" 1             problems of the fused residual GEMM + LayerNorm kernel that share K, bias and LayerNorm parameters
- *                              go into one launch (0: one launch per problem; bit-identical results)
  *   "gemm_ln_unit_rows" 0      rows per CTA-pair unit of the fused residual GEMM + LayerNorm kernel: 128 = two accumulators in
  *                              tensor memory (the epilogue of a unit overlaps the MMAs of the next), 256 = one accumulator with
  *                              1/3 less operand traffic per FLOP, 0 = chosen per launch from K and the row count

@@ -137,13 +137,9 @@ struct m3pc_engine {
   DevBuf XT, YT, QKVT;  // shared-history tables of the first encoder block (TAB_ROWS rows)
   DevBuf fb_xd, fb_bar;  // fused B = 1 path: decoder-embedding scratch, grid-barrier state
   bool use_fused_b1 = true;
-  bool group_ln = true;       // several fused residual GEMM + LayerNorm problems per launch; option "grouped_ln" (0: one launch each)
   int fuse_ln_min_rows = 1024;  // residual GEMM + LayerNorm in one kernel (gemm_ln.cu) from this many rows up; option "fused_ln_min_rows"
                                 // (the kernel-level parity tests call the kernel at any size)
   bool restrict_deep = true;  // decoders with > 1 layer: last layer on the consumed rows only; option "restrict_deep_decoder"
-  int split_residual_min_rows = 0;  // restricted decoder, out-projection: from this many needed rows up the residual is read in place, one
-                                    // problem per residual source in a grouped launch (no residual copy: -6 KB of HBM traffic per row);
-                                    // below, a copy kernel + one problem.  Option "split_residual_min_rows" (tests force either form).
   // planner buffers
   DevBuf p1_mu, p1_std, cand, pred_states, pred_rewards, pred_returns, sa, qa, qb1, qb2, qvals, J, filled, e_mu, e_std;
   // plans with one horizon per environment: every class's windows, noise rows and id table, gathered (launch_mix_gather)
@@ -481,36 +477,18 @@ int gemm_group(m3pc_engine* e, const GemmJob* jobs, int n, cudaStream_t st) {
   return M3PC_OK;
 }
 
-// X += A W^T + bias (or, with `table`, X = table[row / rpg] + A W^T + bias) followed by Y = LayerNorm(X; g, b): ONE tensor-core
-// kernel whose epilogue owns whole rows (gemm_ln.cu) where it applies (bf16 mode, n_embd 512), else GEMM + LayerNorm kernel.
-int gemm_res_ln(m3pc_engine* e, const void* A, const float* w32, const __nv_bfloat16* w16, const float* bias, float* X, void* Y,
-                const float* g, const float* b, const float* table, int rpg, int M, int K, cudaStream_t st, bool allow_fused = true,
-                const float* res_src = nullptr) {
-  const int D = e->D;
-  // one CTA pair per 256 rows: not for the few hundred rows of pass 1 of a multi-environment plan, where a single pair would do
-  // the work of 4 .. 16.  (The switch is kept well below any pass-2 chunk or candidate shard, so the kernel choice -- and with it
-  // the bit pattern of the scores -- does not depend on how candidates are chunked or sharded.)
-  if (allow_fused && e->bf16 && D == 512 && M >= e->fuse_ln_min_rows) {
-    return profiled(e, 2.0 * M * static_cast<double>(D) * K, st, [&] {
-      return gemm_ln_bf16(reinterpret_cast<const __nv_bfloat16*>(A), w16, bias, X, reinterpret_cast<__nv_bfloat16*>(Y), g, b, table, rpg, M, K, st, res_src);
-    });
-  }
-  M3PC_REQUIRE(res_src == nullptr, "gemm_res_ln: a separate residual source needs the fused kernel");
-  GemmEpilogue ep;
-  ep.bias = bias;
-  if (table != nullptr) {
-    ep.table = table;
-    ep.rows_per_group = rpg;
-    ep.flags = EPI_OUT_F32 | EPI_ROWTABLE;
-  } else {
-    ep.flags = EPI_RESIDUAL;
-  }
-  M3PC_TRY(gemm(e, A, w32, w16, X, M, D, K, ep, st));
-  return layernorm(X, M, g, b, Y, D, e->bf16, st);
-}
+// Whether the residual GEMM + LayerNorm of `rows` rows runs as ONE tensor-core kernel whose epilogue owns whole rows (gemm_ln.cu):
+// bf16 mode, n_embd 512, and one CTA pair per 256 rows -- not for the few hundred rows of pass 1 of a multi-environment plan,
+// where a single pair would do the work of 4 .. 16.  (The switch is kept well below any pass-2 chunk or candidate shard, so the
+// kernel choice -- and with it the bit pattern of the scores -- does not depend on how candidates are chunked or sharded.)
+// Which rows decide: a problem of its own decides on its own rows (a block, an MLP half, each part of the shared-history block);
+// the decoder embedding's runs of kept tokens fuse only when every run is large enough; the restricted decoder layer's runs, which
+// only split its needed rows by where their residual comes from, decide on their total: the fused kernel gives every row the same
+// bits whether those rows run as one problem or as one per residual source.
+bool fuse_ln(const m3pc_engine* e, int rows) { return e->bf16 && e->D == 512 && rows >= e->fuse_ln_min_rows; }
 
-// Several residual GEMM + LayerNorm problems that share K, bias and the LayerNorm parameters: ONE launch of the fused kernel where
-// it applies to every problem (the ~10 us fixed cost of a launch is paid once), else one gemm_res_ln per problem.
+// X = R + A W^T + bias, Y = LayerNorm(X; g, b), with the residual R = X itself (in place), table[row / rpg] (`table`) or the fp32
+// rows `res_src`
 struct ResLnJob {
   const void* A;
   const float* w32;
@@ -522,15 +500,38 @@ struct ResLnJob {
   int M;
   const float* res_src;
 };
-int gemm_res_ln_group(m3pc_engine* e, const ResLnJob* jobs, int n, const float* bias, const float* g, const float* b, int K, cudaStream_t st) {
+
+// `n` residual GEMM + LayerNorm jobs that share K, bias and the LayerNorm parameters.  `fused` (fuse_ln): the fused kernel, up to 4
+// jobs per launch (the ~10 us fixed cost of a launch is paid once per 4).  Otherwise one grouped GEMM over all jobs, each residual
+// added in its epilogue as (A W^T + bias) + R -- the same sum for an in-place residual and a row table -- and one LayerNorm launch
+// over the jobs' rows, which therefore must tile one row range of X and of Y in order.
+int gemm_res_ln(m3pc_engine* e, const ResLnJob* jobs, int n, const float* bias, const float* g, const float* b, int K, bool fused,
+                cudaStream_t st) {
   const int D = e->D;
-  bool fused = e->bf16 && D == 512 && e->group_ln;
-  for (int i = 0; i < n; ++i) fused = fused && jobs[i].M >= e->fuse_ln_min_rows;
-  if (!fused || n == 1) {
-    for (int i = 0; i < n; ++i)
-      M3PC_TRY(gemm_res_ln(e, jobs[i].A, jobs[i].w32, jobs[i].w16, bias, jobs[i].X, jobs[i].Y, g, b, jobs[i].table, jobs[i].rpg, jobs[i].M, K, st, true,
-                           jobs[i].res_src));
-    return M3PC_OK;
+  M3PC_REQUIRE(n >= 1 && n <= MAX_TOK, "gemm_res_ln: 1 .. MAX_TOK jobs");
+  if (!fused) {
+    const size_t ab = act_bytes(e);
+    GemmJob gj[MAX_TOK];
+    int rows = 0;
+    for (int i = 0; i < n; ++i) {
+      const ResLnJob& j = jobs[i];
+      M3PC_REQUIRE(j.X == jobs[0].X + static_cast<size_t>(rows) * D &&
+                       static_cast<char*>(j.Y) == static_cast<char*>(jobs[0].Y) + static_cast<size_t>(rows) * D * ab,
+                   "gemm_res_ln: the jobs must tile one row range of X and of Y in order");
+      GemmEpilogue ep;
+      ep.bias = bias;
+      if (j.table != nullptr || j.res_src != nullptr) {
+        ep.table = j.table != nullptr ? j.table : j.res_src;
+        ep.rows_per_group = j.table != nullptr ? j.rpg : 1;
+        ep.flags = EPI_OUT_F32 | EPI_ROWTABLE;
+      } else {
+        ep.flags = EPI_RESIDUAL;
+      }
+      gj[i] = GemmJob{j.A, j.w32, j.w16, j.X, j.M, D, K, ep};
+      rows += j.M;
+    }
+    M3PC_TRY(gemm_group(e, gj, n, st));
+    return layernorm(jobs[0].X, rows, g, b, jobs[0].Y, D, e->bf16, st);
   }
   for (int i0 = 0; i0 < n; i0 += 4) {
     const int m = std::min(4, n - i0);
@@ -560,7 +561,10 @@ int mlp_half(m3pc_engine* e, const LayerW& w, int rows, cudaStream_t st, const P
   ep.bias = w.l1_b;
   ep.flags = EPI_GELU;
   M3PC_TRY(gemm(e, e->Y.p, w.l1_w, w.l1_w16, e->HID.p, rows, F, D, ep, st));
-  if (post.y != nullptr) return gemm_res_ln(e, e->HID.p, w.l2_w, w.l2_w16, w.l2_b, e->X.as<float>(), post.y, post.g, post.b, nullptr, 1, rows, F, st);
+  if (post.y != nullptr) {
+    const ResLnJob l2{e->HID.p, w.l2_w, w.l2_w16, e->X.as<float>(), post.y, nullptr, 1, rows, nullptr};
+    return gemm_res_ln(e, &l2, 1, w.l2_b, post.g, post.b, F, fuse_ln(e, rows), st);
+  }
   ep = GemmEpilogue{};
   ep.bias = w.l2_b;
   ep.flags = EPI_RESIDUAL;
@@ -574,7 +578,8 @@ int block(m3pc_engine* e, const LayerW& w, int Bc, int S, cudaStream_t st, const
   ep.bias = w.in_b;
   M3PC_TRY(gemm(e, e->Y.p, w.in_w, w.in_w16, e->QKV.p, rows, 3 * D, D, ep, st));
   M3PC_TRY(launch_attention(e->QKV.p, e->ATT.p, Bc, S, e->H, e->bf16, st));
-  M3PC_TRY(gemm_res_ln(e, e->ATT.p, w.out_w, w.out_w16, w.out_b, e->X.as<float>(), e->Y.p, w.n2_w, w.n2_b, nullptr, 1, rows, D, st));
+  const ResLnJob outp{e->ATT.p, w.out_w, w.out_w16, e->X.as<float>(), e->Y.p, nullptr, 1, rows, nullptr};
+  M3PC_TRY(gemm_res_ln(e, &outp, 1, w.out_b, w.n2_w, w.n2_b, D, fuse_ln(e, rows), st));
   return mlp_half(e, w, rows, st, post);
 }
 
@@ -619,7 +624,12 @@ int block_shared_history(m3pc_engine* e, const LayerW& w, int Bc, int S, int n_s
       {e->ATT.p, w.out_w, w.out_w16, e->X.as<float>(), e->Y.p, e->XT.as<float>(), grp, static_cast<int>(off), nullptr},
       {reinterpret_cast<const char*>(e->ATT.p) + off * D * ab, w.out_w, w.out_w16, e->X.as<float>() + off * D, reinterpret_cast<char*>(e->Y.p) + off * D * ab,
        nullptr, 1, (S - n_sh) * Bc, nullptr}};
-  M3PC_TRY(gemm_res_ln_group(e, outp, 2, w.out_b, w.n2_w, w.n2_b, D, st));
+  const bool fused[2] = {fuse_ln(e, outp[0].M), fuse_ln(e, outp[1].M)};
+  if (fused[0] == fused[1]) {
+    M3PC_TRY(gemm_res_ln(e, outp, 2, w.out_b, w.n2_w, w.n2_b, D, fused[0], st));
+  } else {
+    for (int i = 0; i < 2; ++i) M3PC_TRY(gemm_res_ln(e, &outp[i], 1, w.out_b, w.n2_w, w.n2_b, D, fused[i], st));
+  }
   return mlp_half(e, w, S * Bc, st, post);
 }
 
@@ -658,9 +668,9 @@ FillParams mask_rows(const m3pc_engine* e, const int* dec_src, int Bc) {
   return fp;
 }
 
-// decoder_embed of the encoder outputs: one grouped GEMM per run of kept tokens of one modality (mtm_model.py:646-661).
-// `compact`: write rows in encoder-token order (row block = dec_src[j]); otherwise in decoder order (row block = j).
-int decoder_embed(m3pc_engine* e, const void* enc_out, const int* dec_src, int Bc, bool compact, cudaStream_t st, float* xout = nullptr) {
+// decoder_embed of the encoder outputs: one grouped GEMM per run of kept tokens of one modality (mtm_model.py:646-661), rows in
+// decoder order (row block = decoder token j).
+int decoder_embed(m3pc_engine* e, const void* enc_out, const int* dec_src, int Bc, cudaStream_t st, float* xout = nullptr) {
   const int D = e->D;
   const size_t ab = act_bytes(e);
   GemmJob jobs[MAX_TOK];
@@ -671,7 +681,7 @@ int decoder_embed(m3pc_engine* e, const void* enc_out, const int* dec_src, int B
     ge.rows_per_group = Bc;
     ge.flags = EPI_OUT_F32 | EPI_ROWTABLE;
     const char* a = reinterpret_cast<const char*>(enc_out) + static_cast<size_t>(dec_src[j]) * Bc * D * ab;
-    float* c = (xout != nullptr ? xout : e->X.as<float>()) + static_cast<size_t>(compact ? dec_src[j] : j) * Bc * D;
+    float* c = (xout != nullptr ? xout : e->X.as<float>()) + static_cast<size_t>(j) * Bc * D;
     jobs[n++] = GemmJob{a, e->dec_w[k], e->dec_w16[k], c, len * Bc, D, D, ge};
   });
   return gemm_group(e, jobs, n, st);  // the runs of all modalities in one launch
@@ -824,49 +834,25 @@ int restricted_last_layer(m3pc_engine* e, const FwdIO& io, const LayerW& w, cons
   // A run = needed tokens with consecutive row blocks whose residual comes from one place: masked tokens take the batch-constant
   // row dec_maskrow[token] (consecutive tokens of a modality are consecutive table rows), kept tokens their own residual-stream rows.
   const int rows = need.n * Bc;
-  struct Run { int q0, len; const float* table; const float* res; };
-  Run runs[MAX_TOK];
+  ResLnJob jobs[MAX_TOK];
   int n_runs = 0;
   for (int qi = 0; qi < need.n;) {
     const int j = need.tok[qi];
     int len = 1;
+    const float *table = nullptr, *res = nullptr;
     if (src[j] < 0) {
       while (qi + len < need.n && need.tok[qi + len] == j + len && src[j + len] < 0) ++len;
-      runs[n_runs++] = Run{qi, len, e->dec_maskrow + static_cast<size_t>(j) * D, nullptr};
+      table = e->dec_maskrow + static_cast<size_t>(j) * D;
     } else {
       while (qi + len < need.n && src[need.tok[qi + len]] == src[j] + len) ++len;
-      runs[n_runs++] = Run{qi, len, nullptr, e->X.as<float>() + static_cast<size_t>(src[j]) * Bc * D};
+      res = e->X.as<float>() + static_cast<size_t>(src[j]) * Bc * D;
     }
+    const size_t off = static_cast<size_t>(qi) * Bc;
+    jobs[n_runs++] = ResLnJob{reinterpret_cast<const char*>(e->ATT.p) + off * D * ab, w.out_w, w.out_w16, e->XS.as<float>() + off * D,
+                              reinterpret_cast<char*>(e->Y.p) + off * D * ab, table, Bc, len * Bc, res};
     qi += len;
   }
-  bool per_run = e->bf16 && D == 512 && rows >= e->split_residual_min_rows;  // and every run large enough for the fused kernel
-  for (int r = 0; r < n_runs; ++r) per_run = per_run && static_cast<long>(runs[r].len) * Bc >= e->fuse_ln_min_rows;
-  if (per_run) {
-    ResLnJob jobs[MAX_TOK];
-    for (int r = 0; r < n_runs; ++r) {
-      const size_t off = static_cast<size_t>(runs[r].q0) * Bc;
-      jobs[r] = ResLnJob{reinterpret_cast<const char*>(e->ATT.p) + off * D * ab, w.out_w, w.out_w16, e->XS.as<float>() + off * D,
-                         reinterpret_cast<char*>(e->Y.p) + off * D * ab, runs[r].table, Bc, runs[r].len * Bc, runs[r].res};
-    }
-    M3PC_TRY(gemm_res_ln_group(e, jobs, n_runs, w.out_b, w.n2_w, w.n2_b, D, st));
-  } else {
-    // small batches: residual rows -> XS by a copy kernel, then one out-projection accumulates into them (same arithmetic, same bits)
-    FillParams fp{};
-    fp.B = Bc;
-    for (int qi = 0; qi < need.n; ++qi) {
-      const int j = need.tok[qi];
-      if (src[j] < 0) {
-        fp.row[fp.n] = e->dec_maskrow + static_cast<size_t>(j) * D;
-        fp.bstride[fp.n] = 0;
-      } else {
-        fp.row[fp.n] = e->X.as<float>() + static_cast<size_t>(src[j]) * Bc * D;
-        fp.bstride[fp.n] = D;
-      }
-      fp.tok[fp.n++] = qi;
-    }
-    M3PC_TRY(launch_fill_rows(fp, D, e->XS.as<float>(), st));
-    M3PC_TRY(gemm_res_ln(e, e->ATT.p, w.out_w, w.out_w16, w.out_b, e->XS.as<float>(), e->Y.p, w.n2_w, w.n2_b, nullptr, 1, rows, D, st));
-  }
+  M3PC_TRY(gemm_res_ln(e, jobs, n_runs, w.out_b, w.n2_w, w.n2_b, D, fuse_ln(e, rows), st));
   ge = GemmEpilogue{};
   ge.bias = w.l1_b;
   ge.flags = EPI_GELU;
@@ -885,28 +871,19 @@ int restricted_last_layer(m3pc_engine* e, const FwdIO& io, const LayerW& w, cons
 int decode_restricted(m3pc_engine* e, const FwdIO& io, const void* enc_out, const int* dec_src, int S, const NeedSet& need, int b0, int Bc,
                       cudaStream_t st) {
   const LayerW& w = e->dec.layers[0];
-  const int D = e->D, T = e->T;
-  int min_run = 1 << 30;  // shortest run of consecutive kept tokens of one modality
-  for_each_kept_run(dec_src, T, [&](int, int, int len) { min_run = std::min(min_run, len); });
-  // every run must be large enough for the fused kernel, so that one batch size always takes one path
-  if (e->bf16 && D == 512 && static_cast<long>(min_run) * Bc >= e->fuse_ln_min_rows) {
-    // (a) + (b) in one kernel per run of kept tokens of a modality: X = dec_cvec[token] + enc_out W_dec^T (compact, encoder order),
-    // Y = LN1(X) -- the table-residual form of the fused residual GEMM + LayerNorm kernel (no residual traffic at all)
-    const size_t ab = act_bytes(e);
-    ResLnJob jobs[MAX_TOK];
-    int nj = 0;
-    for_each_kept_run(dec_src, T, [&](int j, int k, int len) {
-      const size_t r0 = static_cast<size_t>(dec_src[j]) * Bc;
-      jobs[nj++] = ResLnJob{reinterpret_cast<const char*>(enc_out) + r0 * D * ab, e->dec_w[k], e->dec_w16[k], e->X.as<float>() + r0 * D,
-                            reinterpret_cast<char*>(e->Y.p) + r0 * D * ab, e->dec_cvec + static_cast<size_t>(j) * D, Bc, len * Bc, nullptr};
-    });
-    M3PC_TRY(gemm_res_ln_group(e, jobs, nj, nullptr, w.n1_w, w.n1_b, D, st));
-    return restricted_last_layer(e, io, w, dec_src, S, need, b0, Bc, st);
-  }
-  // (a) decoder embedding of the kept tokens, compact (encoder order) -> X[0 : S*Bc)
-  M3PC_TRY(decoder_embed(e, enc_out, dec_src, Bc, true, st));
-  // (b) LN1 -> Y
-  M3PC_TRY(layernorm(e->X.as<float>(), S * Bc, w.n1_w, w.n1_b, e->Y.p, D, e->bf16, st));
+  const int D = e->D;
+  const size_t ab = act_bytes(e);
+  // (a) + (b), one job per run of kept tokens of a modality: X = dec_cvec[token] + enc_out W_dec^T (compact, encoder order:
+  // X[0 : S*Bc)), Y = LN1(X) -- the table-residual form of the residual GEMM + LayerNorm (no residual traffic at all)
+  ResLnJob jobs[MAX_TOK];
+  int nj = 0, min_rows = 1 << 30;
+  for_each_kept_run(dec_src, e->T, [&](int j, int k, int len) {
+    const size_t r0 = static_cast<size_t>(dec_src[j]) * Bc;
+    jobs[nj++] = ResLnJob{reinterpret_cast<const char*>(enc_out) + r0 * D * ab, e->dec_w[k], e->dec_w16[k], e->X.as<float>() + r0 * D,
+                          reinterpret_cast<char*>(e->Y.p) + r0 * D * ab, e->dec_cvec + static_cast<size_t>(j) * D, Bc, len * Bc, nullptr};
+    min_rows = std::min(min_rows, len * Bc);
+  });
+  M3PC_TRY(gemm_res_ln(e, jobs, nj, nullptr, w.n1_w, w.n1_b, D, fuse_ln(e, min_rows), st));
   return restricted_last_layer(e, io, w, dec_src, S, need, b0, Bc, st);
 }
 
@@ -917,7 +894,7 @@ int decode_full(m3pc_engine* e, const FwdIO& io, const void* enc_out, const int*
                 bool restrict_last, cudaStream_t st) {
   const int D = e->D, Sd = 4 * e->T;
   M3PC_TRY(launch_fill_rows(mask_rows(e, dec_src, Bc), D, e->X.as<float>(), st));
-  M3PC_TRY(decoder_embed(e, enc_out, dec_src, Bc, false, st));
+  M3PC_TRY(decoder_embed(e, enc_out, dec_src, Bc, st));
   M3PC_TRY(layernorm(e->X.as<float>(), Sd * Bc, e->dec.layers[0].n1_w, e->dec.layers[0].n1_b, e->Y.p, D, e->bf16, st));
   const int n_full = restrict_last ? e->Ld - 1 : e->Ld;
   for (int l = 0; l < n_full; ++l) {
@@ -1627,10 +1604,8 @@ int m3pc_set_option(m3pc_handle_t h, const char* name, int32_t value) {
   h->drop_graphs();  // the launch sequence a graph froze may no longer be the selected one
   if (n == "graphs") h->use_graphs = value != 0;
   else if (n == "fused_b1") h->use_fused_b1 = value != 0;
-  else if (n == "grouped_ln") h->group_ln = value != 0;
   else if (n == "fused_ln_min_rows") h->fuse_ln_min_rows = std::max(129, static_cast<int>(value));
   else if (n == "restrict_deep_decoder") h->restrict_deep = value != 0;
-  else if (n == "split_residual_min_rows") h->split_residual_min_rows = std::max(0, static_cast<int>(value));
   else if (n == "gemm_ln_unit_rows") {
     M3PC_REQUIRE(value == 0 || value == 128 || value == 256, "gemm_ln_unit_rows must be 0 (per launch), 128 or 256");
     m3pc::g_ln_unit_rows = value;
@@ -1880,7 +1855,7 @@ int m3pc_decoder_scatter_embed(m3pc_handle_t h, int32_t batch, const void* enc_o
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   M3PC_TRY(m3pc::launch_fill_rows(m3pc::mask_rows(h, tt.dec_src, batch), h->D, x_out, st));  // no launch when every token is kept
   if (tt.S == 0) return M3PC_OK;
-  return m3pc::decoder_embed(h, enc_out, tt.dec_src, batch, false, st, x_out);
+  return m3pc::decoder_embed(h, enc_out, tt.dec_src, batch, st, x_out);
 }
 
 int m3pc_heads(m3pc_handle_t h, int32_t batch, const float* x_dec, float* out_states, float* out_act_mu, float* out_act_std,
