@@ -265,14 +265,13 @@ inline cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
 #endif
 
 // ---- kernel launchers implemented across the .cu files -----------------------------------------------
+// Problems that share one launch of a grouped tensor-core kernel (gemm_bf16, gemm_ln_bf16_grouped): each launch carries their
+// parameters in its kernel parameter space
+constexpr int kMaxGroup = 4;
 // gemm_tcgen05.cu
-int gemm_bf16_tcgen05(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, int M, int N, int K,
-                      const GemmEpilogue& epi, cudaStream_t st);
 int gemm_init_driver_api();
 // gemm_ln.cu: X (M,512) fp32 <- R + A W^T + bias (R = X in place, the fp32 rows `R`, or table[row / rows_per_group]); Y (M,512) bf16 <- LayerNorm(X)
-int gemm_ln_bf16(const __nv_bfloat16* A, const __nv_bfloat16* W, const float* bias, float* X, __nv_bfloat16* Y, const float* gamma,
-                 const float* beta, const float* table, int rows_per_group, int M, int K, cudaStream_t st, const float* R = nullptr);
-// several such problems in ONE launch (at most 4; same K, bias, gamma, beta): own A / W / X / Y / residual source each
+// for 1 .. kMaxGroup such problems in ONE launch (same K, bias, gamma, beta): own A / W / X / Y / residual source each
 struct LnJob {
   const __nv_bfloat16* A;
   const __nv_bfloat16* W;
@@ -284,7 +283,8 @@ struct LnJob {
   const float* R;       // residual rows when they are not X itself (and table is null), or null
 };
 int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const float* gamma, const float* beta, int K, cudaStream_t st);
-// several independent bf16 GEMMs in one launch of the CTA-pair kernel (decoder embedding runs, K/V + Q, heads, twin critics)
+// n >= 1 independent bf16 GEMMs C = epilogue(A W^T); up to kMaxGroup of them share one launch of the CTA-pair kernel where it
+// applies (decoder embedding runs, K/V + Q, heads, twin critics)
 struct GemmProblem {
   const __nv_bfloat16* A;
   const __nv_bfloat16* W;
@@ -292,7 +292,7 @@ struct GemmProblem {
   int M, N, K;
   GemmEpilogue epi;
 };
-int gemm_bf16_grouped(const GemmProblem* probs, int n, cudaStream_t st);
+int gemm_bf16(const GemmProblem* probs, int n, cudaStream_t st);
 // gemm_skinny.cu: M <= 32 rows (B = 1 passes): a latency-optimised CUDA-core kernel, same epilogues
 int gemm_bf16_skinny(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, int M, int N, int K, const GemmEpilogue& epi, cudaStream_t st);
 // sgemm.cu

@@ -440,15 +440,8 @@ int profiled(m3pc_engine* e, double flops, cudaStream_t st, Launch&& launch) {
   return M3PC_OK;
 }
 
-int gemm(m3pc_engine* e, const void* A, const float* w32, const __nv_bfloat16* w16, void* C, int M, int N, int K, const GemmEpilogue& epi,
-         cudaStream_t st) {
-  return profiled(e, 2.0 * M * static_cast<double>(N) * K, st, [&] {
-    return e->bf16 ? gemm_bf16_tcgen05(reinterpret_cast<const __nv_bfloat16*>(A), w16, C, M, N, K, epi, st)
-                   : gemm_fp32(reinterpret_cast<const float*>(A), w32, reinterpret_cast<float*>(C), M, N, K, epi, st);
-  });
-}
-
-// Several independent GEMMs as ONE launch where the CTA-pair tensor-core kernel applies (bf16 mode), else one launch each.
+// Independent GEMMs C = epilogue(A W^T) with the weights in both precisions.  bf16 mode: kMaxGroup at a time, each such group one
+// launch of the CTA-pair tensor-core kernel where it applies (gemm_bf16) and booked as one profile entry; fp32 mode: one launch each.
 struct GemmJob {
   const void* A;
   const float* w32;
@@ -458,23 +451,29 @@ struct GemmJob {
   GemmEpilogue epi;
 };
 int gemm_group(m3pc_engine* e, const GemmJob* jobs, int n, cudaStream_t st) {
-  if (!e->bf16 || n == 1) {
-    for (int i = 0; i < n; ++i) M3PC_TRY(gemm(e, jobs[i].A, jobs[i].w32, jobs[i].w16, jobs[i].C, jobs[i].M, jobs[i].N, jobs[i].K, jobs[i].epi, st));
-    return M3PC_OK;
-  }
-  constexpr int kMax = 4;
-  for (int i0 = 0; i0 < n; i0 += kMax) {
-    const int m = std::min(kMax, n - i0);
-    GemmProblem pr[kMax];
+  const int group = e->bf16 ? kMaxGroup : 1;
+  for (int i0 = 0; i0 < n; i0 += group) {
+    const int m = std::min(group, n - i0);
+    GemmProblem pr[kMaxGroup];
     double flops = 0.0;
     for (int i = 0; i < m; ++i) {
       const GemmJob& j = jobs[i0 + i];
       pr[i] = GemmProblem{reinterpret_cast<const __nv_bfloat16*>(j.A), j.w16, j.C, j.M, j.N, j.K, j.epi};
       flops += 2.0 * j.M * static_cast<double>(j.N) * j.K;
     }
-    M3PC_TRY(profiled(e, flops, st, [&] { return gemm_bf16_grouped(pr, m, st); }));
+    const GemmJob& j = jobs[i0];
+    M3PC_TRY(profiled(e, flops, st, [&] {
+      return e->bf16 ? gemm_bf16(pr, m, st)
+                     : gemm_fp32(reinterpret_cast<const float*>(j.A), j.w32, reinterpret_cast<float*>(j.C), j.M, j.N, j.K, j.epi, st);
+    }));
   }
   return M3PC_OK;
+}
+
+int gemm(m3pc_engine* e, const void* A, const float* w32, const __nv_bfloat16* w16, void* C, int M, int N, int K, const GemmEpilogue& epi,
+         cudaStream_t st) {
+  const GemmJob job{A, w32, w16, C, M, N, K, epi};
+  return gemm_group(e, &job, 1, st);
 }
 
 // Whether the residual GEMM + LayerNorm of `rows` rows runs as ONE tensor-core kernel whose epilogue owns whole rows (gemm_ln.cu):
@@ -501,10 +500,10 @@ struct ResLnJob {
   const float* res_src;
 };
 
-// `n` residual GEMM + LayerNorm jobs that share K, bias and the LayerNorm parameters.  `fused` (fuse_ln): the fused kernel, up to 4
-// jobs per launch (the ~10 us fixed cost of a launch is paid once per 4).  Otherwise one grouped GEMM over all jobs, each residual
-// added in its epilogue as (A W^T + bias) + R -- the same sum for an in-place residual and a row table -- and one LayerNorm launch
-// over the jobs' rows, which therefore must tile one row range of X and of Y in order.
+// `n` residual GEMM + LayerNorm jobs that share K, bias and the LayerNorm parameters.  `fused` (fuse_ln): the fused kernel, up to
+// kMaxGroup jobs per launch (the ~10 us fixed cost of a launch is paid once per group).  Otherwise one grouped GEMM over all jobs,
+// each residual added in its epilogue as (A W^T + bias) + R -- the same sum for an in-place residual and a row table -- and one
+// LayerNorm launch over the jobs' rows, which therefore must tile one row range of X and of Y in order.
 int gemm_res_ln(m3pc_engine* e, const ResLnJob* jobs, int n, const float* bias, const float* g, const float* b, int K, bool fused,
                 cudaStream_t st) {
   const int D = e->D;
@@ -533,9 +532,9 @@ int gemm_res_ln(m3pc_engine* e, const ResLnJob* jobs, int n, const float* bias, 
     M3PC_TRY(gemm_group(e, gj, n, st));
     return layernorm(jobs[0].X, rows, g, b, jobs[0].Y, D, e->bf16, st);
   }
-  for (int i0 = 0; i0 < n; i0 += 4) {
-    const int m = std::min(4, n - i0);
-    LnJob lj[4];
+  for (int i0 = 0; i0 < n; i0 += kMaxGroup) {
+    const int m = std::min(kMaxGroup, n - i0);
+    LnJob lj[kMaxGroup];
     double flops = 0.0;
     for (int i = 0; i < m; ++i) {
       const ResLnJob& j = jobs[i0 + i];
@@ -1764,8 +1763,8 @@ int m3pc_gemm_bf16(const void* A, const void* W, const float* bias, void* C, int
   m3pc::GemmEpilogue ep;
   ep.bias = bias;
   ep.flags = flags;
-  return m3pc::gemm_bf16_tcgen05(reinterpret_cast<const __nv_bfloat16*>(A), reinterpret_cast<const __nv_bfloat16*>(W), C, M, N, K, ep,
-                                 reinterpret_cast<cudaStream_t>(stream));
+  const m3pc::GemmProblem pr{reinterpret_cast<const __nv_bfloat16*>(A), reinterpret_cast<const __nv_bfloat16*>(W), C, M, N, K, ep};
+  return m3pc::gemm_bf16(&pr, 1, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_gemm_bf16_grouped(int32_t n, const void* const* A, const void* const* W, const float* const* bias, void* const* C, const int32_t* M,
@@ -1780,15 +1779,14 @@ int m3pc_gemm_bf16_grouped(int32_t n, const void* const* A, const void* const* W
     ep.flags = flags[i];
     pr[i] = m3pc::GemmProblem{reinterpret_cast<const __nv_bfloat16*>(A[i]), reinterpret_cast<const __nv_bfloat16*>(W[i]), C[i], M[i], N[i], K[i], ep};
   }
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  for (int i0 = 0; i0 < n; i0 += 4) M3PC_TRY(m3pc::gemm_bf16_grouped(pr + i0, std::min(4, n - i0), st));
-  return M3PC_OK;
+  return m3pc::gemm_bf16(pr, n, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_gemm_ln_bf16(const void* A, const void* W, const float* bias, float* X, void* Y, const float* gamma, const float* beta,
                       const float* table, int32_t rows_per_group, int32_t M, int32_t K, void* stream) {
-  return m3pc::gemm_ln_bf16(reinterpret_cast<const __nv_bfloat16*>(A), reinterpret_cast<const __nv_bfloat16*>(W), bias, X,
-                            reinterpret_cast<__nv_bfloat16*>(Y), gamma, beta, table, rows_per_group, M, K, reinterpret_cast<cudaStream_t>(stream));
+  const m3pc::LnJob job{reinterpret_cast<const __nv_bfloat16*>(A), reinterpret_cast<const __nv_bfloat16*>(W), X,
+                        reinterpret_cast<__nv_bfloat16*>(Y), table, rows_per_group, M, nullptr};
+  return m3pc::gemm_ln_bf16_grouped(&job, 1, bias, gamma, beta, K, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_gemm_fp32(const float* A, const float* W, const float* bias, float* C, int32_t M, int32_t N, int32_t K, int32_t flags, void* stream) {

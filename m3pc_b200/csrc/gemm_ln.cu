@@ -10,7 +10,7 @@
 // updated rows in TMEM (tcgen05.st), exchanges the row statistics between the warps that share a row, and writes the
 // normalised bf16 operand of the next GEMM.  6 KB of HBM traffic per row and one launch instead of 8 KB and two.
 //
-// Two unit sizes (template parameter ROWS, chosen per launch in gemm_ln_bf16):
+// Two unit sizes (template parameter ROWS, chosen per launch in gemm_ln_bf16_grouped):
 //   ROWS = 256  M = 256 MMAs; the unit's accumulator is the pair's whole tensor memory (128 lanes x 512 columns per CTA), so the
 //               epilogue of a unit and the MMAs of the next take turns.  Least operand traffic per FLOP: right for long K.
 //   ROWS = 128  M = 128 MMAs (cta_group::2).  Each CTA's 64 x N slice of D is stored as 128 lanes x N/2 columns (lanes 0-63:
@@ -34,15 +34,15 @@
 
 namespace m3pc {
 
-int g_ln_unit_rows = 0;  // rows per CTA-pair unit of the fused kernel: 0 = chosen per launch (gemm_ln_bf16), or 128 / 256 forced; m3pc_set_option "gemm_ln_unit_rows"
+// rows per CTA-pair unit of the fused kernel: 0 = chosen per launch (gemm_ln_bf16_grouped), or 128 / 256 forced; m3pc_set_option
+// "gemm_ln_unit_rows"
+int g_ln_unit_rows = 0;
 
 namespace {
 
 constexpr int LN_N = 512;
 constexpr int LN_EPI_WARPS = 16;
 constexpr int LN_THREADS = 32 * (2 + LN_EPI_WARPS);
-
-constexpr int LN_MAX_GROUP = 4;
 
 // One problem of a launch: X[M,512] <- R + A W^T + bias, Y <- LayerNorm(X).  Several problems share a launch (same K, bias, gamma,
 // beta; own operands, outputs and residual source): the fixed cost of a launch -- barrier set-up, tensor-memory allocation,
@@ -59,22 +59,13 @@ struct LnProblem {
 };
 
 struct LnGemmParams {
-  LnProblem p[LN_MAX_GROUP];
+  LnProblem p[kMaxGroup];
   const float* bias;
   const float* gamma;
   const float* beta;
   int n, num_kb, n_units;
 };
 static_assert(sizeof(LnGemmParams) <= 4000, "kernel parameter space");
-
-// problem of unit u (a launch has at most LN_MAX_GROUP problems, ordered by unit0)
-__device__ __forceinline__ int ln_problem_of(const LnGemmParams& P, int u) {
-  int g = 0;
-#pragma unroll
-  for (int i = 1; i < LN_MAX_GROUP; ++i)
-    if (i < P.n && u >= P.p[i].unit0) g = i;
-  return g;
-}
 
 __device__ __forceinline__ void tmem_st16(uint32_t taddr, const float (&v)[16]) {
   asm volatile(
@@ -112,14 +103,10 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
   // Row statistics are accumulated in a CANONICAL order that does not depend on ROWS: (sum, sum of squares) over each group of 64
   // consecutive columns, ascending, then the eight groups added in column order -- so both unit sizes produce identical bits.
   constexpr int NSLICE = 8;
+  using Pipe = TcPipeline<STAGES, NACC, ACC_COLS, 2, 2>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + L::kBarOffset);  // leader's copy is the one waited on
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* acc_full = empty_bar + STAGES;   // [2]
-  uint64_t* acc_empty = acc_full + 2;        // [2]; leader's copy counts both CTAs' epilogue warps
-  uint64_t* res_bar = acc_empty + 2;         // [LN_EPI_WARPS][NBOX]: residual box landed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(res_bar + NBOX * LN_EPI_WARPS);
+  uint64_t* res_bar = reinterpret_cast<uint64_t*>(smem + L::kBarOffset + Pipe::kBarBytes);  // [LN_EPI_WARPS][NBOX]: residual box landed
   float* sconst = reinterpret_cast<float*>(smem + L::kConstOffset);
   float2* sstats = reinterpret_cast<float2*>(smem + L::kStatsOffset);
 
@@ -129,7 +116,13 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
   const bool leader = crank == 0;
   const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
 
-  if (warp == 0 && lane == 0) {
+  for (int i = threadIdx.x; i < LN_N; i += LN_THREADS) {
+    sconst[i] = P.bias != nullptr ? __ldg(P.bias + i) : 0.f;
+    sconst[LN_N + i] = __ldg(P.gamma + i);
+    sconst[2 * LN_N + i] = __ldg(P.beta + i);
+  }
+  // all 512 TMEM columns: two accumulators of 256 columns (one 128-row x 512-column unit each) or one of 512
+  const Pipe pipe = Pipe::setup(smem + L::kBarOffset, LN_EPI_WARPS, [&] {
     for (int g = 0; g < P.n; ++g) {
       prefetch_tmap(&P.p[g].ta);
       prefetch_tmap(&P.p[g].tw);
@@ -137,83 +130,43 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
       prefetch_tmap(&P.p[g].ty);
       prefetch_tmap(&P.p[g].tr);
     }
-#pragma unroll
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], 1);
-    }
-    for (int b = 0; b < NACC; ++b) {
-      mbar_init(&acc_full[b], 1);
-      mbar_init(&acc_empty[b], 2 * LN_EPI_WARPS);
-    }
     for (int i = 0; i < NBOX * LN_EPI_WARPS; ++i) mbar_init(&res_bar[i], 1);
-    fence_barrier_init();
-    fence_proxy_async();
-  }
-  if (warp == 1) {  // all 512 TMEM columns: two accumulators of 256 columns (one 128-row x 512-column unit each)
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(LN_N) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  for (int i = threadIdx.x; i < LN_N; i += LN_THREADS) {
-    sconst[i] = P.bias != nullptr ? __ldg(P.bias + i) : 0.f;
-    sconst[LN_N + i] = __ldg(P.gamma + i);
-    sconst[2 * LN_N + i] = __ldg(P.beta + i);
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  PDL_PROLOGUE();
+  });
 
   if (warp == 0) {
     if (lane == 0) {
       // ---- TMA producer (both CTAs): own 64 rows of A, own 128 rows of each 256-row half of W ----
-      const uint32_t full_leader = mapa_u32(smem_u32(&full_bar[0]), 0);
-      int s = 0;
-      uint32_t ph = 0;
-      for (int u = pair; u < P.n_units; u += n_pairs) {
-        const LnProblem& Q = P.p[ln_problem_of(P, u)];
-        const int m0 = ((u - Q.unit0) * 2 + static_cast<int>(crank)) * (ROWS / 2);
-        for (int kb = 0; kb < P.num_kb; ++kb) {
-          mbar_wait(&empty_bar[s], ph ^ 1);
-          if (leader) mbar_arrive_expect_tx(&full_bar[s], 2u * L::kStageBytes);
-          uint8_t* dst = smem + s * L::kStageBytes;
-          const uint32_t bar = full_leader + 8u * static_cast<uint32_t>(s);
-          tma_load_2d_2sm(dst, &Q.ta, bar, kb * BK, m0);
-          tma_load_2d_2sm(dst + L::kABlk, &Q.tw, bar, kb * BK, static_cast<int>(crank) * 128);
-          tma_load_2d_2sm(dst + L::kABlk + L::kBBlk, &Q.tw, bar, kb * BK, 256 + static_cast<int>(crank) * 128);
-          if (++s == STAGES) { s = 0; ph ^= 1; }
-        }
-      }
+      const uint32_t full_leader = mapa_u32(smem_u32(&pipe.full[0]), 0);
+      const LnProblem* Q = nullptr;
+      int m0 = 0;
+      pipe.produce(pair, P.n_units, n_pairs, [&](int u) -> const int& {
+        Q = &P.p[problem_of(P, u)];
+        m0 = ((u - Q->unit0) * 2 + static_cast<int>(crank)) * (ROWS / 2);
+        return P.num_kb;
+      }, [&](int kb, int s) {
+        if (leader) mbar_arrive_expect_tx(&pipe.full[s], 2u * L::kStageBytes);
+        uint8_t* dst = smem + s * L::kStageBytes;
+        const uint32_t bar = full_leader + 8u * static_cast<uint32_t>(s);
+        tma_load_2d_2sm(dst, &Q->ta, bar, kb * BK, m0);
+        tma_load_2d_2sm(dst + L::kABlk, &Q->tw, bar, kb * BK, static_cast<int>(crank) * 128);
+        tma_load_2d_2sm(dst + L::kABlk + L::kBBlk, &Q->tw, bar, kb * BK, 256 + static_cast<int>(crank) * 128);
+      });
     }
   } else if (warp == 1) {
     if (lane == 0 && leader) {
       // ---- MMA issuer (leader only): M = ROWS across the pair, both N = 256 halves per k-step, accumulators alternate ----
       constexpr uint32_t idesc = make_idesc_mn(ROWS, 256);
-      int s = 0, it = 0;
-      uint32_t ph = 0;
-      for (int u = pair; u < P.n_units; u += n_pairs, ++it) {
-        const uint32_t buf = static_cast<uint32_t>(it % NACC);
-        mbar_wait(&acc_empty[buf], (static_cast<uint32_t>(it / NACC) & 1u) ^ 1u);
-        tc_fence_after();
-        const uint32_t d0 = tmem_base + buf * ACC_COLS;
-        for (int kb = 0; kb < P.num_kb; ++kb) {
-          mbar_wait(&full_bar[s], ph);
-          tc_fence_after();
-          const uint32_t a_addr = smem_u32(smem + s * L::kStageBytes);
-          const uint32_t b0_addr = a_addr + L::kABlk, b1_addr = b0_addr + L::kBBlk;
+      pipe.issue(pair, P.n_units, n_pairs, [&](int) -> const int& { return P.num_kb; }, [&](uint32_t d0, int kb, int s) {
+        const uint32_t a_addr = smem_u32(smem + s * L::kStageBytes);
+        const uint32_t b0_addr = a_addr + L::kABlk, b1_addr = b0_addr + L::kBBlk;
 #pragma unroll
-          for (int k = 0; k < BK / UMMA_K; ++k) {
-            const uint32_t acc = (kb | k) != 0 ? 1u : 0u;
-            const uint64_t da = make_smem_desc(a_addr + k * UMMA_K * 2);
-            umma_bf16_2sm(d0, da, make_smem_desc(b0_addr + k * UMMA_K * 2), idesc, acc);
-            umma_bf16_2sm(d0 + ACC_COLS / 2, da, make_smem_desc(b1_addr + k * UMMA_K * 2), idesc, acc);
-          }
-          umma_commit_2sm(&empty_bar[s]);
-          if (++s == STAGES) { s = 0; ph ^= 1; }
+        for (int k = 0; k < BK / UMMA_K; ++k) {
+          const uint32_t acc = (kb | k) != 0 ? 1u : 0u;
+          const uint64_t da = make_smem_desc(a_addr + k * UMMA_K * 2);
+          umma_bf16_2sm(d0, da, make_smem_desc(b0_addr + k * UMMA_K * 2), idesc, acc);
+          umma_bf16_2sm(d0 + ACC_COLS / 2, da, make_smem_desc(b1_addr + k * UMMA_K * 2), idesc, acc);
         }
-        umma_commit_2sm(&acc_full[buf]);
-      }
+      });
     }
   } else {
     // ---- epilogue warps (both CTAs): 32 rows x WCOLS columns each ----
@@ -230,7 +183,6 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
     uint8_t* sbuf = smem + L::kStoreOffset + ew * NBOX * L::kBoxBytes;
     uint64_t* rbar = res_bar + NBOX * ew;
     uint32_t rph = 0;  // bit b: parity of rbar[b]
-    const uint32_t acc_empty_leader = mapa_u32(smem_u32(&acc_empty[0]), 0);
     const uint32_t sw = static_cast<uint32_t>((lane >> 1) & 3);  // SWIZZLE_64B: 16-byte chunk j of row r lives at j ^ ((r >> 1) & 3)
     const float* sbias = sconst;
     const float* sgamma = sconst + LN_N;
@@ -238,19 +190,17 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
     constexpr int NB1 = WCOLS / 16;             // residual / X boxes per warp per unit (16 fp32 columns each)
     constexpr int NB2 = WCOLS / 32;             // Y boxes (32 bf16 columns each)
     constexpr int NPRE = NBOX < NB1 ? NBOX : NB1;  // boxes requested before the accumulator is waited for
-    int it = 0;
+    uint32_t it = 0;
     // Box buffers are used strictly round-robin (buffer = ns % NBOX for the ns-th bulk group this warp commits), which is what makes
     // "wait until at most NBOX - 1 groups are still being read" the condition for reusing one.  With the residual coming through the
     // TMA every unit starts from a drained state (ns = 0, all buffers free).
     uint32_t ns = 0;
     for (int u = pair; u < P.n_units; u += n_pairs, ++it) {
-      const uint32_t buf = static_cast<uint32_t>(it % NACC);
-      const LnProblem& Q = P.p[ln_problem_of(P, u)];
+      const LnProblem& Q = P.p[problem_of(P, u)];
       const bool from_x = Q.table == nullptr;
       const int row0 = ((u - Q.unit0) * 2 + static_cast<int>(crank)) * (ROWS / 2) + rowq * 32;
       const int row = row0 + lane;
       const bool live = row0 < Q.M;
-      const uint32_t tacc = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + buf * ACC_COLS + tcol;
       // residual boxes travel to shared memory while the MMAs of this unit (and the epilogue of the previous one) still run
       if (from_x) ns = 0;
       if (from_x && live && lane == 0) {
@@ -261,8 +211,8 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
           tma_load_2d(sbuf + b * L::kBoxBytes, &Q.tr, &rbar[b], colw + b * 16, row0);
         }
       }
-      mbar_wait(&acc_full[buf], static_cast<uint32_t>(it / NACC) & 1u);
-      tc_fence_after();
+      const uint32_t buf = pipe.acc_wait(it);
+      const uint32_t tacc = pipe.tmem_base + (static_cast<uint32_t>(q * 32) << 16) + buf * ACC_COLS + tcol;
       float s1 = 0.f, s2 = 0.f;
       if (live) {
         // ---- pass 1: x = acc + bias + residual -> X (TMA store) and back into TMEM; row sums ----
@@ -350,10 +300,7 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
           if (lane == 0) bulk_wait_read<NBOX - 1>();
           __syncwarp();
           tmem_ld_wait();
-          if (ci == NB2 - 1) {  // the accumulator has been drained: the MMA warp may reuse it
-            tc_fence_before();
-            if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * buf);
-          }
+          if (ci == NB2 - 1) pipe.acc_release(buf);  // the accumulator has been drained: the MMA warp may reuse it
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
             float y[8];
@@ -374,19 +321,13 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
           ++ns;
         }
       } else {
-        tc_fence_before();
-        if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * buf);
+        pipe.acc_release(buf);
       }
     }
     if (lane == 0) bulk_wait_read<0>();  // shared memory may be released once the stores have been read; the writes complete with the grid
   }
 
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(LN_N) : "memory");
-  }
+  pipe.teardown();
 }
 
 template <int ROWS, int STAGES, int NBOX>
@@ -395,30 +336,21 @@ int launch_ln(LnGemmParams& P, cudaStream_t st) {
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
   static_assert(L::kStoreOffset % 1024 == 0, "operand stages must keep 1024-byte alignment");
   static PerDevice<size_t> smem_limit;
-  M3PC_CHECK_CUDA(raise_smem_limit(gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, smem_limit, L::kTotal));
-  int units = 0;
-  for (int g = 0; g < P.n; ++g) {
-    P.p[g].unit0 = units;
-    units += ceil_div(P.p[g].M, ROWS);
-  }
-  P.n_units = units;
-  const int pairs = std::min(P.n_units, device_num_sms() / 2);
-  M3PC_CHECK_CUDA(launch_k_cluster(2, gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, dim3(2 * pairs), dim3(LN_THREADS), L::kTotal, st, P));
-  M3PC_CHECK_LAUNCH();
-  return M3PC_OK;
+  return launch_pair(gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, smem_limit, L::kTotal, LN_THREADS, P,
+                     [](const LnProblem& Q) { return ceil_div(Q.M, ROWS); }, [](int) {}, st);
 }
 
 }  // namespace
 
 // X (M, 512) fp32 in place (or other fp32 rows / table rows as the residual), Y (M, 512) bf16 = LayerNorm(X).  K % 64 == 0.
-// Up to LN_MAX_GROUP problems per launch (shared K, bias, gamma, beta).
+// Up to kMaxGroup problems per launch (shared K, bias, gamma, beta).
 // Unit size (rows per CTA pair; bit-identical results, tests/test_gpu_parity.py::test_gemm_ln_unit_sizes_are_bit_identical):
 //   K <= 512   128-row units: the launch is bound by its epilogue traffic (6 KB per row), which then runs under the next unit's MMAs
 //              (measured at 106 496 rows: 125 us vs 135 us with 256-row units; profiles/r2g_gemm_ln_variants.txt)
 //   K  > 512   256-row units feed the tensor pipe with 1/3 less operand traffic per FLOP (238 vs 264 us) -- unless the launch is so
 //              small that whole 256-row units quantise badly on the 74 CTA pairs (26 624 rows: 104 units = 2 rounds, vs 3 half rounds)
 int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const float* gamma, const float* beta, int K, cudaStream_t st) {
-  M3PC_REQUIRE(n >= 1 && n <= LN_MAX_GROUP, "gemm_ln: 1 .. 4 problems per launch");
+  M3PC_REQUIRE(n >= 1 && n <= kMaxGroup, "gemm_ln: 1 .. kMaxGroup problems per launch");
   M3PC_REQUIRE(K > 0 && K % BK == 0, "gemm_ln: K must be a positive multiple of 64");
   M3PC_REQUIRE(gamma && beta, "gemm_ln: null operand");
   M3PC_TRY(gemm_init_driver_api());
@@ -455,12 +387,6 @@ int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const floa
   P.bias = bias; P.gamma = gamma; P.beta = beta;
   P.num_kb = K / BK;
   return rows == 128 ? launch_ln<128, 3, 2>(P, st) : launch_ln<256, 3, 2>(P, st);
-}
-
-int gemm_ln_bf16(const __nv_bfloat16* A, const __nv_bfloat16* W, const float* bias, float* X, __nv_bfloat16* Y, const float* gamma,
-                 const float* beta, const float* table, int rows_per_group, int M, int K, cudaStream_t st, const float* R) {
-  const LnJob job{A, W, X, Y, table, rows_per_group, M, R};
-  return gemm_ln_bf16_grouped(&job, 1, bias, gamma, beta, K, st);
 }
 
 }  // namespace m3pc

@@ -162,11 +162,6 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_bf16_kernel(const __grid
   extern __shared__ uint8_t smem_raw[];
   // SWIZZLE_128B tiles need 1024-byte alignment
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + L::kBarOffset);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* acc_full = empty_bar + STAGES;
-  uint64_t* acc_empty = acc_full + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -176,84 +171,45 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_bf16_kernel(const __grid
   const int total_tiles = n_tiles * (((M + BM - 1) / BM + CL - 1) / CL);
   const uint32_t crank = CL > 1 ? cluster_ctarank() : 0u;
   const int unit0 = blockIdx.x / CL, unit_step = gridDim.x / CL;
-  constexpr uint16_t kMask = static_cast<uint16_t>((1u << CL) - 1u);
 
-  if (warp == 0 && lane == 0) {
+  const auto pipe = TcPipeline<STAGES, 2, BN, 1, CL>::setup(smem + L::kBarOffset, NUM_EPI_WARPS, [&] {
     prefetch_tmap(&tmap_a);
     prefetch_tmap(&tmap_w);
-#pragma unroll
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], CL);  // one tcgen05.commit arrival from every CTA of the cluster
-    }
-    mbar_init(&acc_full[0], 1);
-    mbar_init(&acc_full[1], 1);
-    mbar_init(&acc_empty[0], NUM_EPI_WARPS);
-    mbar_init(&acc_empty[1], NUM_EPI_WARPS);
-    fence_barrier_init();
-    fence_proxy_async();
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(2 * BN) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  if (CL > 1) cluster_sync_all(); else __syncthreads();  // peers must see initialised barriers before any multicast lands
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  PDL_PROLOGUE();  // everything above is private to this CTA; operands of the previous kernel are touched only below
+  });
 
   if (warp == 0) {
     if (lane == 0) {
-      int s = 0;
-      uint32_t ph = 0;
-      for (int tile = unit0; tile < total_tiles; tile += unit_step) {
-        const int m0 = ((tile / n_tiles) * CL + static_cast<int>(crank)) * BM, n0 = (tile % n_tiles) * BN;
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&empty_bar[s], ph ^ 1);  // every CTA of the cluster has consumed this slot
-          mbar_arrive_expect_tx(&full_bar[s], L::kStageBytes);
-          uint8_t* sa = smem + s * L::kStageBytes;
-          tma_load_2d(sa, &tmap_a, &full_bar[s], kb * BK, m0);
-          if (CL == 1) {
-            tma_load_2d(sa + L::kABytes, &tmap_w, &full_bar[s], kb * BK, n0);
-          } else {  // my 1/CL slice of the W k-block, delivered to every CTA of the cluster
-            constexpr int kSliceRows = BN / CL;
-            tma_load_2d_mc(sa + L::kABytes + crank * (kSliceRows * BK * 2), &tmap_w, &full_bar[s], kb * BK,
-                           n0 + static_cast<int>(crank) * kSliceRows, kMask);
-          }
-          if (++s == STAGES) { s = 0; ph ^= 1; }
+      int m0 = 0, n0 = 0;
+      pipe.produce(unit0, total_tiles, unit_step, [&](int tile) {
+        m0 = ((tile / n_tiles) * CL + static_cast<int>(crank)) * BM;
+        n0 = (tile % n_tiles) * BN;
+        return num_kb;
+      }, [&](int kb, int s) {
+        mbar_arrive_expect_tx(&pipe.full[s], L::kStageBytes);
+        uint8_t* sa = smem + s * L::kStageBytes;
+        tma_load_2d(sa, &tmap_a, &pipe.full[s], kb * BK, m0);
+        if (CL == 1) {
+          tma_load_2d(sa + L::kABytes, &tmap_w, &pipe.full[s], kb * BK, n0);
+        } else {  // my 1/CL slice of the W k-block, delivered to every CTA of the cluster
+          constexpr int kSliceRows = BN / CL;
+          tma_load_2d_mc(sa + L::kABytes + crank * (kSliceRows * BK * 2), &tmap_w, &pipe.full[s], kb * BK,
+                         n0 + static_cast<int>(crank) * kSliceRows, static_cast<uint16_t>((1u << CL) - 1u));
         }
-      }
+      });
     }
   } else if (warp == 1) {
     if (lane == 0) {
       constexpr uint32_t idesc = make_idesc(BN);
-      int s = 0;
-      uint32_t ph = 0;
-      int it = 0;
-      for (int tile = unit0; tile < total_tiles; tile += unit_step, ++it) {
-        const int a = it & 1;
-        const uint32_t aph = (it >> 1) & 1;
-        mbar_wait(&acc_empty[a], aph ^ 1);  // epilogue has drained this accumulator (first use passes immediately)
-        tc_fence_after();
-        const uint32_t tmem_d = tmem_base + static_cast<uint32_t>(a * BN);
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&full_bar[s], ph);
-          tc_fence_after();
-          const uint32_t a_addr = smem_u32(smem + s * L::kStageBytes);
-          const uint32_t b_addr = a_addr + L::kABytes;
+      pipe.issue(unit0, total_tiles, unit_step, [&](int) { return num_kb; }, [&](uint32_t tmem_d, int kb, int s) {
+        const uint32_t a_addr = smem_u32(smem + s * L::kStageBytes);
+        const uint32_t b_addr = a_addr + L::kABytes;
 #pragma unroll
-          for (int k = 0; k < BK / UMMA_K; ++k) {
-            // advance inside the 128-byte swizzle atom: +32 bytes per K=16 step
-            umma_bf16(tmem_d, make_smem_desc(a_addr + k * UMMA_K * 2), make_smem_desc(b_addr + k * UMMA_K * 2), idesc,
-                      (kb | k) != 0 ? 1u : 0u);
-          }
-          // slot reusable once these MMAs have read it -- in every CTA of the cluster, since peers multicast into it
-          if (CL == 1) umma_commit(&empty_bar[s]); else umma_commit_mc(&empty_bar[s], kMask);
-          if (++s == STAGES) { s = 0; ph ^= 1; }
+        for (int k = 0; k < BK / UMMA_K; ++k) {
+          // advance inside the 128-byte swizzle atom: +32 bytes per K=16 step
+          umma_bf16(tmem_d, make_smem_desc(a_addr + k * UMMA_K * 2), make_smem_desc(b_addr + k * UMMA_K * 2), idesc,
+                    (kb | k) != 0 ? 1u : 0u);
         }
-        umma_commit(&acc_full[a]);  // accumulator complete
-      }
+      });
     }
   } else {
     // ---- epilogue warps: TMEM -> registers -> smem transpose -> coalesced global ----
@@ -261,26 +217,15 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_bf16_kernel(const __grid
     const int quarter = warp & 3;       // TMEM lanes [32*quarter, 32*quarter+32) are the ones this warp may read
     const int half = ew >> 2;           // which half of the BN columns
     float* xp = reinterpret_cast<float*>(smem + L::kXposeOffset + ew * L::kXposeBytesPerWarp);
-    int it = 0;
+    uint32_t it = 0;
     for (int tile = unit0; tile < total_tiles; tile += unit_step, ++it) {
       const int m0 = ((tile / n_tiles) * CL + static_cast<int>(crank)) * BM, n0 = (tile % n_tiles) * BN;
-      const int a = it & 1;
-      const uint32_t aph = (it >> 1) & 1;
-      mbar_wait(&acc_full[a], aph);
-      tc_fence_after();
-      epilogue_tile<BN>(tmem_base + static_cast<uint32_t>(a * BN), xp, C, M, N, m0, n0, quarter, half, lane, ep);
-      // all of this warp's TMEM reads are complete (tcgen05.wait::ld above): hand the accumulator back
-      tc_fence_before();
-      if (lane == 0) mbar_arrive(&acc_empty[a]);
+      const uint32_t a = pipe.acc_wait(it);
+      epilogue_tile<BN>(pipe.tmem_base + a * BN, xp, C, M, N, m0, n0, quarter, half, lane, ep);
+      pipe.acc_release(a);
     }
   }
-
-  tc_fence_before();
-  if (CL > 1) cluster_sync_all(); else __syncthreads();  // no CTA may exit while a peer can still multicast into / arrive on it
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(2 * BN) : "memory");
-  }
+  pipe.teardown();
 }
 
 
@@ -309,10 +254,9 @@ struct Smem2 {
   static constexpr int kTotal = kBarOffset + 256 + 1024;
 };
 
-// Grouped launches: up to MAX_GROUP independent problems (own operands, output, epilogue, shapes) share one launch; the pair's
+// Grouped launches: up to kMaxGroup independent problems (own operands, output, epilogue, shapes) share one launch; the pair's
 // unit range simply runs across problem boundaries, so several small GEMMs of the decoder / heads / critic cost one kernel
 // boundary instead of one each.
-constexpr int MAX_GROUP = 4;
 struct alignas(64) GroupProblem {
   CUtensorMap ta, tw, tc;
   const float* bias;
@@ -323,17 +267,14 @@ struct alignas(64) GroupProblem {
   int unit0;       // first unit of this problem in the launch-wide unit order
 };
 struct GroupParams {
-  GroupProblem p[MAX_GROUP];
-  int n, total_units;
+  GroupProblem p[kMaxGroup];
+  int n, n_units;
   int strided;  // 1: pair p works on units p, p + n_pairs, ... (see launch_2sm) instead of one contiguous range
 };
 struct UnitCoord { int g, mp, nt; };
 __device__ __forceinline__ UnitCoord decode_unit(const GroupParams& gp, int u) {
   UnitCoord c;
-  c.g = 0;
-#pragma unroll
-  for (int i = 1; i < MAX_GROUP; ++i)
-    if (i < gp.n && u >= gp.p[i].unit0) c.g = i;
+  c.g = problem_of(gp, u);
   const GroupProblem& P = gp.p[c.g];
   // unsigned: a unit index is never negative, and the signed division's sign fix-up costs registers the epilogue warps need
   // for their per-unit state (with it, ptxas spills that state to local memory)
@@ -343,106 +284,97 @@ __device__ __forceinline__ UnitCoord decode_unit(const GroupParams& gp, int u) {
   return c;
 }
 
+// Epilogue values of CW columns of one row: accumulator words r + bias (staged in shared memory at sbias) + row table, then GELU
+// and ReLU as the flags ask.
+template <int CW>
+__device__ __forceinline__ void epilogue_values(const uint32_t (&r)[32], const float* sbias, const EpiParams& ep, int row, int M, int N,
+                                                int col0, bool do_gelu, bool do_relu, float (&v)[CW]) {
+#pragma unroll
+  for (int j = 0; j < CW / 4; ++j) {
+    const float4 b4 = *reinterpret_cast<const float4*>(sbias + 4 * j);
+    v[4 * j + 0] = __uint_as_float(r[4 * j + 0]) + b4.x;
+    v[4 * j + 1] = __uint_as_float(r[4 * j + 1]) + b4.y;
+    v[4 * j + 2] = __uint_as_float(r[4 * j + 2]) + b4.z;
+    v[4 * j + 3] = __uint_as_float(r[4 * j + 3]) + b4.w;
+  }
+  if (ep.table != nullptr && row < M) {
+    const float* tr = ep.table + static_cast<size_t>(row / ep.rows_per_group) * N + col0;
+#pragma unroll
+    for (int j = 0; j < CW / 4; ++j) {
+      const float4 t4 = __ldg(reinterpret_cast<const float4*>(tr + 4 * j));
+      v[4 * j + 0] += t4.x; v[4 * j + 1] += t4.y; v[4 * j + 2] += t4.z; v[4 * j + 3] += t4.w;
+    }
+  }
+  if (do_gelu) {
+#pragma unroll
+    for (int j = 0; j < CW; ++j) v[j] = gelu_erf_tanh(v[j]);
+  }
+  if (do_relu) {
+#pragma unroll
+    for (int j = 0; j < CW; ++j) v[j] = fmaxf(v[j], 0.0f);
+  }
+}
+
 template <int STAGES>
 __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(const __grid_constant__ GroupParams gp) {
   constexpr int BN = 256;
   using L = Smem2<STAGES>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + L::kBarOffset);  // waited on by the leader's MMA thread only
-  uint64_t* empty_bar = full_bar + STAGES;                                 // ring slot free (signalled in both CTAs)
-  uint64_t* acc_full = empty_bar + STAGES;
-  uint64_t* acc_empty = acc_full + 2;                                      // leader's copy counts both CTAs' epilogue warps
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const uint32_t crank = cluster_ctarank();
   const bool leader = crank == 0;
-  const int total_units = gp.total_units;
+  const int n_units = gp.n_units;
   const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
   // units are ordered m-major and split contiguously: a pair mostly stays on one row block, whose A slab stays hot in L2
   // strided (N = 512 problems with a long K): neighbouring pairs take the two column tiles of the SAME row block at the same
   // time, so its A slab is fetched from HBM once and the second reader hits L2 (contiguous ranges re-read it ~150 MB later)
   const int u_step = gp.strided ? n_pairs : 1;
-  const int u_lo = gp.strided ? pair : static_cast<int>(static_cast<long long>(pair) * total_units / n_pairs);
-  const int u_hi = gp.strided ? total_units : static_cast<int>(static_cast<long long>(pair + 1) * total_units / n_pairs);
+  const int u_lo = gp.strided ? pair : static_cast<int>(static_cast<long long>(pair) * n_units / n_pairs);
+  const int u_hi = gp.strided ? n_units : static_cast<int>(static_cast<long long>(pair + 1) * n_units / n_pairs);
 
-  if (warp == 0 && lane == 0) {
+  // 2 accumulators of 256 fp32 columns = all of TMEM; the leader's acc_empty counts both CTAs' epilogue warps
+  const auto pipe = TcPipeline<STAGES, 2, BN, 2, 2>::setup(smem + L::kBarOffset, NUM_EPI_WARPS_2SM, [&] {
     for (int g = 0; g < gp.n; ++g) {
       prefetch_tmap(&gp.p[g].ta);
       prefetch_tmap(&gp.p[g].tw);
       prefetch_tmap(&gp.p[g].tc);
     }
-#pragma unroll
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], 1);
-    }
-    mbar_init(&acc_full[0], 1);
-    mbar_init(&acc_full[1], 1);
-    mbar_init(&acc_empty[0], 2 * NUM_EPI_WARPS_2SM);
-    mbar_init(&acc_empty[1], 2 * NUM_EPI_WARPS_2SM);
-    fence_barrier_init();
-    fence_proxy_async();
-  }
-  if (warp == 1) {  // the same warp of both CTAs allocates (2 accumulators of 256 fp32 columns = all of TMEM)
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(2 * BN) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  PDL_PROLOGUE();  // everything above is private to this CTA pair; operands of the previous kernel are touched only below
+  });
 
   if (warp == 0) {
     if (lane == 0) {
       // ---- TMA producer (both CTAs): own half of every operand slab, completion signalled on the LEADER's barrier ----
-      const uint32_t full_leader = mapa_u32(smem_u32(&full_bar[0]), 0);
-      int s = 0;
-      uint32_t ph = 0;
-      for (int u = u_lo; u < u_hi; u += u_step) {
+      const uint32_t full_leader = mapa_u32(smem_u32(&pipe.full[0]), 0);
+      const GroupProblem* P = nullptr;
+      int m0 = 0, n0 = 0;
+      pipe.produce(u_lo, u_hi, u_step, [&](int u) -> const int& {
         const UnitCoord uc = decode_unit(gp, u);
-        const GroupProblem& P = gp.p[uc.g];
-        const int m0 = (uc.mp * 2 + static_cast<int>(crank)) * BM, n0 = uc.nt * BN + static_cast<int>(crank) * 128;
-        for (int kb = 0; kb < P.num_kb; ++kb) {
-          mbar_wait(&empty_bar[s], ph ^ 1);
-          if (leader) mbar_arrive_expect_tx(&full_bar[s], 2u * L::kStageBytes);
-          uint8_t* dst = smem + s * L::kStageBytes;
-          const uint32_t bar = full_leader + 8u * static_cast<uint32_t>(s);
-          tma_load_2d_2sm(dst, &P.ta, bar, kb * BK, m0);
-          tma_load_2d_2sm(dst + L::kABlk, &P.tw, bar, kb * BK, n0);
-          if (++s == STAGES) { s = 0; ph ^= 1; }
-        }
-      }
+        P = &gp.p[uc.g];
+        m0 = (uc.mp * 2 + static_cast<int>(crank)) * BM;
+        n0 = uc.nt * BN + static_cast<int>(crank) * 128;
+        return P->num_kb;
+      }, [&](int kb, int s) {
+        if (leader) mbar_arrive_expect_tx(&pipe.full[s], 2u * L::kStageBytes);
+        uint8_t* dst = smem + s * L::kStageBytes;
+        const uint32_t bar = full_leader + 8u * static_cast<uint32_t>(s);
+        tma_load_2d_2sm(dst, &P->ta, bar, kb * BK, m0);
+        tma_load_2d_2sm(dst + L::kABlk, &P->tw, bar, kb * BK, n0);
+      });
     }
   } else if (warp == 1) {
     if (lane == 0 && leader) {
       // ---- MMA issuer (leader only) ----
       constexpr uint32_t idesc = make_idesc_mn(2 * BM, BN);
-      int s = 0, it = 0;
-      uint32_t ph = 0;
-      for (int u = u_lo; u < u_hi; u += u_step, ++it) {
-        const int a = it & 1;
-        const uint32_t aph = (it >> 1) & 1;
-        mbar_wait(&acc_empty[a], aph ^ 1);
-        tc_fence_after();
-        const uint32_t tmem_d = tmem_base + static_cast<uint32_t>(a * BN);
-        const int num_kb = gp.p[decode_unit(gp, u).g].num_kb;
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(&full_bar[s], ph);
-          tc_fence_after();
-          const uint32_t a_addr = smem_u32(smem + s * L::kStageBytes);
-          const uint32_t b_addr = a_addr + L::kABlk;
+      pipe.issue(u_lo, u_hi, u_step, [&](int u) { return gp.p[decode_unit(gp, u).g].num_kb; }, [&](uint32_t tmem_d, int kb, int s) {
+        const uint32_t a_addr = smem_u32(smem + s * L::kStageBytes);
+        const uint32_t b_addr = a_addr + L::kABlk;
 #pragma unroll
-          for (int k = 0; k < BK / UMMA_K; ++k)
-            umma_bf16_2sm(tmem_d, make_smem_desc(a_addr + k * UMMA_K * 2), make_smem_desc(b_addr + k * UMMA_K * 2), idesc, (kb | k) != 0 ? 1u : 0u);
-          umma_commit_2sm(&empty_bar[s]);
-          if (++s == STAGES) { s = 0; ph ^= 1; }
-        }
-        umma_commit_2sm(&acc_full[a]);
-      }
+        for (int k = 0; k < BK / UMMA_K; ++k)
+          umma_bf16_2sm(tmem_d, make_smem_desc(a_addr + k * UMMA_K * 2), make_smem_desc(b_addr + k * UMMA_K * 2), idesc, (kb | k) != 0 ? 1u : 0u);
+      });
     }
   } else {
     // ---- epilogue warps (both CTAs): 32 rows (TMEM lane quarter) x 64 columns of this CTA's 128 x 256 tile each ----
@@ -451,9 +383,8 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
     const int cgrp = ew >> 2;      // which 64 of the tile's 256 columns
     uint8_t* sbuf = smem + L::kStoreOffset + ew * 2 * L::kStoreBufBytes;
     float* sbias = reinterpret_cast<float*>(smem + L::kBiasOffset) + ew * 64;
-    const uint32_t acc_empty_leader = mapa_u32(smem_u32(&acc_empty[0]), 0);
     const uint32_t sw = static_cast<uint32_t>((lane >> 1) & 3);  // SWIZZLE_64B: 16-byte chunk j of row r lives at j ^ ((r >> 1) & 3)
-    int it = 0;
+    uint32_t it = 0;
     uint32_t nstore = 0;  // chunks staged so far (selects the staging buffer)
     for (int u = u_lo; u < u_hi; u += u_step, ++it) {
       const UnitCoord uc = decode_unit(gp, u);
@@ -473,13 +404,10 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
         *reinterpret_cast<float2*>(sbias + 2 * lane) = b2;
         __syncwarp();
       }
-      const int a = it & 1;
-      const uint32_t aph = (it >> 1) & 1;
-      mbar_wait(&acc_full[a], aph);
-      tc_fence_after();
+      const uint32_t a = pipe.acc_wait(it);
       const bool live = row0 < M;
       const int row = row0 + lane;
-      const uint32_t tacc = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + static_cast<uint32_t>(a * BN + cgrp * 64);
+      const uint32_t tacc = pipe.tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + a * BN + static_cast<uint32_t>(cgrp * 64);
       if (live) {
 #pragma unroll 1
         for (int c = 0; c < 64; c += cw) {
@@ -491,65 +419,16 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
           if (lane == 0) bulk_wait_read<1>();
           __syncwarp();
           tmem_ld_wait();
-          if (c + cw == 64) {  // every TMEM read of this tile has landed in registers: hand the accumulator back to the MMA warp
-            tc_fence_before();
-            if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * static_cast<uint32_t>(a));
-          }
+          if (c + cw == 64) pipe.acc_release(a);  // every TMEM read of this tile has landed in registers
           if (out_f32) {
             float v[16];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float4 b4 = *reinterpret_cast<const float4*>(sbias + c + 4 * j);
-              v[4 * j + 0] = __uint_as_float(r[4 * j + 0]) + b4.x;
-              v[4 * j + 1] = __uint_as_float(r[4 * j + 1]) + b4.y;
-              v[4 * j + 2] = __uint_as_float(r[4 * j + 2]) + b4.z;
-              v[4 * j + 3] = __uint_as_float(r[4 * j + 3]) + b4.w;
-            }
-            if (ep.table != nullptr && row < M) {
-              const float* tr = ep.table + static_cast<size_t>(row / ep.rows_per_group) * N + col0;
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const float4 t4 = __ldg(reinterpret_cast<const float4*>(tr + 4 * j));
-                v[4 * j + 0] += t4.x; v[4 * j + 1] += t4.y; v[4 * j + 2] += t4.z; v[4 * j + 3] += t4.w;
-              }
-            }
-            if (do_gelu) {
-#pragma unroll
-              for (int j = 0; j < 16; ++j) v[j] = gelu_erf_tanh(v[j]);
-            }
-            if (do_relu) {
-#pragma unroll
-              for (int j = 0; j < 16; ++j) v[j] = fmaxf(v[j], 0.0f);
-            }
+            epilogue_values<16>(r, sbias + c, ep, row, M, N, col0, do_gelu, do_relu, v);
 #pragma unroll
             for (int j = 0; j < 4; ++j)
               *reinterpret_cast<float4*>(buf + lane * 64 + ((static_cast<uint32_t>(j) ^ sw) << 4)) = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
           } else {
             float v[32];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              const float4 b4 = *reinterpret_cast<const float4*>(sbias + c + 4 * j);
-              v[4 * j + 0] = __uint_as_float(r[4 * j + 0]) + b4.x;
-              v[4 * j + 1] = __uint_as_float(r[4 * j + 1]) + b4.y;
-              v[4 * j + 2] = __uint_as_float(r[4 * j + 2]) + b4.z;
-              v[4 * j + 3] = __uint_as_float(r[4 * j + 3]) + b4.w;
-            }
-            if (ep.table != nullptr && row < M) {
-              const float* tr = ep.table + static_cast<size_t>(row / ep.rows_per_group) * N + col0;
-#pragma unroll
-              for (int j = 0; j < 8; ++j) {
-                const float4 t4 = __ldg(reinterpret_cast<const float4*>(tr + 4 * j));
-                v[4 * j + 0] += t4.x; v[4 * j + 1] += t4.y; v[4 * j + 2] += t4.z; v[4 * j + 3] += t4.w;
-              }
-            }
-            if (do_gelu) {
-#pragma unroll
-              for (int j = 0; j < 32; ++j) v[j] = gelu_erf_tanh(v[j]);
-            }
-            if (do_relu) {
-#pragma unroll
-              for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j], 0.0f);
-            }
+            epilogue_values<32>(r, sbias + c, ep, row, M, N, col0, do_gelu, do_relu, v);
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
               *reinterpret_cast<uint4*>(buf + lane * 64 + ((static_cast<uint32_t>(j) ^ sw) << 4)) =
@@ -566,19 +445,12 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
           ++nstore;
         }
       } else {  // nothing to store (rows beyond M): just release the accumulator
-        tc_fence_before();
-        if (lane == 0) mbar_arrive_remote(acc_empty_leader + 8u * static_cast<uint32_t>(a));
+        pipe.acc_release(a);
       }
     }
     if (lane == 0) bulk_wait_read<0>();  // shared memory may be released once the stores have been READ; the writes complete with the grid
   }
-
-  tc_fence_before();
-  cluster_sync_all();  // no CTA may exit while its peer can still read its shared memory or arrive on its barriers
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(2 * BN) : "memory");
-  }
+  pipe.teardown();  // no CTA may exit while its peer can still read its shared memory or arrive on its barriers
 }
 
 }  // namespace
@@ -600,18 +472,19 @@ int make_tmap(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, u
 namespace {
 
 template <int BN, int STAGES, int CL>
-int launch(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, int M, int N, int K, const GemmEpilogue& epi, cudaStream_t st) {
+int launch(const GemmProblem& q, cudaStream_t st) {
   using L = SmemLayout<BN, STAGES>;
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
   static PerDevice<size_t> smem_limit;
   M3PC_CHECK_CUDA(raise_smem_limit(gemm_bf16_kernel<BN, STAGES, CL>, smem_limit, L::kTotal));
   CUtensorMap ta, tw;
-  M3PC_TRY(make_tmap(&ta, A, static_cast<uint64_t>(M), static_cast<uint64_t>(K), BM));
-  M3PC_TRY(make_tmap(&tw, W, static_cast<uint64_t>(N), static_cast<uint64_t>(K), BN / CL));
-  EpiParams ep{epi.bias, epi.table, epi.rows_per_group > 0 ? epi.rows_per_group : 1, epi.flags};
-  const int units = (N / BN) * ceil_div(ceil_div(M, BM), CL);
+  M3PC_TRY(make_tmap(&ta, q.A, static_cast<uint64_t>(q.M), static_cast<uint64_t>(q.K), BM));
+  M3PC_TRY(make_tmap(&tw, q.W, static_cast<uint64_t>(q.N), static_cast<uint64_t>(q.K), BN / CL));
+  const EpiParams ep{q.epi.bias, q.epi.table, q.epi.rows_per_group > 0 ? q.epi.rows_per_group : 1, q.epi.flags};
+  const int units = (q.N / BN) * ceil_div(ceil_div(q.M, BM), CL);
   const int clusters = std::min(units, device_num_sms() / CL);
-  M3PC_CHECK_CUDA(launch_k_cluster(CL, gemm_bf16_kernel<BN, STAGES, CL>, dim3(clusters * CL), dim3(GEMM_THREADS), L::kTotal, st, ta, tw, C, M, N, K, ep));
+  M3PC_CHECK_CUDA(launch_k_cluster(CL, gemm_bf16_kernel<BN, STAGES, CL>, dim3(clusters * CL), dim3(GEMM_THREADS), L::kTotal, st, ta, tw, q.C,
+                                   q.M, q.N, q.K, ep));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
 }
@@ -635,18 +508,15 @@ int make_tmap_out(CUtensorMap* map, void* ptr, uint64_t rows, uint64_t cols, boo
 }
 namespace {
 
-// One launch of the CTA-pair kernel over `n` problems (n <= MAX_GROUP; every N a multiple of 256).
+// One launch of the CTA-pair kernel over `n` problems (n <= kMaxGroup; every N a multiple of 256).
 template <int STAGES>
 int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
   using L = Smem2<STAGES>;
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
   static_assert(sizeof(GroupParams) <= 4000, "kernel parameter space");
   static PerDevice<size_t> smem_limit;
-  M3PC_CHECK_CUDA(raise_smem_limit(gemm_bf16_2sm_kernel<STAGES>, smem_limit, L::kTotal));
-  const int n_pairs_max = device_num_sms() / 2;
   GroupParams gp{};
   gp.n = n;
-  int units = 0;
   for (int g = 0; g < n; ++g) {
     const GemmProblem& q = probs[g];
     GroupProblem& P = gp.p[g];
@@ -661,15 +531,12 @@ int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
     P.M = q.M;
     P.n_tiles = q.N / 256;
     P.num_kb = q.K / BK;
-    P.unit0 = units;
-    units += P.n_tiles * ceil_div(q.M, 2 * BM);
   }
-  gp.total_units = units;
-  const int pairs = std::min(units, n_pairs_max);
-  gp.strided = n == 1 && gp.p[0].n_tiles == 2 && probs[0].K >= 1024 && pairs % 2 == 0 && units >= 2 * pairs;
-  M3PC_CHECK_CUDA(launch_k_cluster(2, gemm_bf16_2sm_kernel<STAGES>, dim3(2 * pairs), dim3(GEMM_THREADS_2SM), L::kTotal, st, gp));
-  M3PC_CHECK_LAUNCH();
-  return M3PC_OK;
+  return launch_pair(gemm_bf16_2sm_kernel<STAGES>, smem_limit, L::kTotal, GEMM_THREADS_2SM, gp,
+                     [](const GroupProblem& P) { return P.n_tiles * ceil_div(P.M, 2 * BM); },
+                     [&](int pairs) {
+                       gp.strided = n == 1 && gp.p[0].n_tiles == 2 && probs[0].K >= 1024 && pairs % 2 == 0 && gp.n_units >= 2 * pairs;
+                     }, st);
 }
 
 // Modelled time of one configuration: the slower of the tensor pipe (rounds of the persistent grid x MMA cycles per tile)
@@ -683,6 +550,28 @@ double model_time(int M, int N, int K, int bn, int cl) {
   const double t_mma = rounds * kb * 4.0 * (bn / 2.0) / 1.7e9 + 2.0e-6;                          // 64 / 128 cycles per K=16 step
   const double bytes = static_cast<double>(units) * cl * kb * (BM * BK * 2.0 + bn * BK * 2.0 / cl);  // per CTA: own A + 1/cl of W
   return std::max(t_mma, bytes / 10.5e12);
+}
+
+// One problem in a launch of its own: the skinny kernel for a few rows, the CTA-pair kernel wherever a pair has two row tiles to
+// work on and N splits into 256-wide tiles, else the single-CTA kernel.
+int gemm_bf16_one(const GemmProblem& q, cudaStream_t st) {
+  if (q.M <= 32 && static_cast<size_t>(q.M) * q.K * 2 <= 160 * 1024) return gemm_bf16_skinny(q.A, q.W, q.C, q.M, q.N, q.K, q.epi, st);
+  if (q.N % 256 == 0 && q.M > BM) return launch_2sm<4>(&q, 1, st);
+  // pick tile width and cluster size by the modelled time (ties: wider tile, larger cluster = less L2 traffic)
+  struct Cand { int bn, cl; } cands[] = {{256, 2}, {256, 1}, {128, 2}, {128, 1}};
+  int best = -1;
+  double best_t = 1e30;
+  for (int i = 0; i < 4; ++i) {
+    if (q.N % cands[i].bn != 0) continue;
+    const double t = model_time(q.M, q.N, q.K, cands[i].bn, cands[i].cl);
+    if (t < best_t * 0.98) { best_t = t; best = i; }
+  }
+  switch (best) {
+    case 0: return launch<256, 3, 2>(q, st);
+    case 1: return launch<256, 3, 1>(q, st);
+    case 2: return launch<128, 4, 2>(q, st);
+    default: return launch<128, 4, 1>(q, st);
+  }
 }
 
 }  // namespace
@@ -700,53 +589,34 @@ int gemm_init_driver_api() {
   return M3PC_OK;
 }
 
-int gemm_bf16_tcgen05(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, int M, int N, int K, const GemmEpilogue& epi,
-                      cudaStream_t st) {
-  M3PC_REQUIRE(M > 0 && N > 0 && K > 0, "gemm_bf16: empty problem");
-  M3PC_REQUIRE(K % BK == 0, "gemm_bf16: K must be a multiple of 64");
-  M3PC_REQUIRE(N % 128 == 0, "gemm_bf16: N must be a multiple of 128");
-  M3PC_REQUIRE((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(W) & 15) == 0 &&
-                   (reinterpret_cast<uintptr_t>(C) & 15) == 0,
-               "gemm_bf16: operands must be 16-byte aligned");
-  M3PC_TRY(gemm_init_driver_api());
-  if (M <= 32 && static_cast<size_t>(M) * K * 2 <= 160 * 1024) return gemm_bf16_skinny(A, W, C, M, N, K, epi, st);
-  // CTA-pair kernel wherever a pair has two row tiles to work on and N splits into 256-wide tiles
-  if (N % 256 == 0 && M > BM) {
-    const GemmProblem q{A, W, C, M, N, K, epi};
-    return launch_2sm<4>(&q, 1, st);
-  }
-  // pick tile width and cluster size by the modelled time (ties: wider tile, larger cluster = less L2 traffic)
-  struct Cand { int bn, cl; } cands[] = {{256, 2}, {256, 1}, {128, 2}, {128, 1}};
-  int best = -1;
-  double best_t = 1e30;
-  for (int i = 0; i < 4; ++i) {
-    if (N % cands[i].bn != 0) continue;
-    const double t = model_time(M, N, K, cands[i].bn, cands[i].cl);
-    if (t < best_t * 0.98) { best_t = t; best = i; }
-  }
-  switch (best) {
-    case 0: return launch<256, 3, 2>(A, W, C, M, N, K, epi, st);
-    case 1: return launch<256, 3, 1>(A, W, C, M, N, K, epi, st);
-    case 2: return launch<128, 4, 2>(A, W, C, M, N, K, epi, st);
-    default: return launch<128, 4, 1>(A, W, C, M, N, K, epi, st);
-  }
-}
-
-// Several independent GEMMs in one launch (see GroupParams).  Falls back to one launch per problem where the CTA-pair
-// kernel does not apply (a problem with N % 256 != 0, only tiny M).
-int gemm_bf16_grouped(const GemmProblem* probs, int n, cudaStream_t st) {
-  M3PC_REQUIRE(n >= 1, "gemm_bf16_grouped: no problems");
-  M3PC_TRY(gemm_init_driver_api());
-  bool ok = n <= MAX_GROUP;
-  int max_m = 0;
-  for (int g = 0; g < n && ok; ++g) {
+// Problems are taken kMaxGroup at a time.  Several problems whose N all split into 256-wide tiles share one CTA-pair launch (small
+// ones included) once one of them gives a pair two row tiles to work on (see GroupParams); otherwise each problem gets its own.
+int gemm_bf16(const GemmProblem* probs, int n, cudaStream_t st) {
+  M3PC_REQUIRE(n >= 1, "gemm_bf16: no problems");
+  for (int g = 0; g < n; ++g) {
     const GemmProblem& q = probs[g];
-    ok = q.M > 0 && q.N > 0 && q.K > 0 && q.N % 256 == 0 && q.K % BK == 0 && (reinterpret_cast<uintptr_t>(q.A) & 15) == 0 &&
-         (reinterpret_cast<uintptr_t>(q.W) & 15) == 0 && (reinterpret_cast<uintptr_t>(q.C) & 15) == 0;
-    max_m = std::max(max_m, q.M);
+    M3PC_REQUIRE(q.M > 0 && q.N > 0 && q.K > 0, "gemm_bf16: empty problem");
+    M3PC_REQUIRE(q.K % BK == 0, "gemm_bf16: K must be a multiple of 64");
+    M3PC_REQUIRE(q.N % 128 == 0, "gemm_bf16: N must be a multiple of 128");
+    M3PC_REQUIRE(((reinterpret_cast<uintptr_t>(q.A) | reinterpret_cast<uintptr_t>(q.W) | reinterpret_cast<uintptr_t>(q.C)) & 15) == 0,
+                 "gemm_bf16: operands must be 16-byte aligned");
   }
-  if (ok && max_m > BM && n > 1) return launch_2sm<4>(probs, n, st);
-  for (int g = 0; g < n; ++g) M3PC_TRY(gemm_bf16_tcgen05(probs[g].A, probs[g].W, probs[g].C, probs[g].M, probs[g].N, probs[g].K, probs[g].epi, st));
+  M3PC_TRY(gemm_init_driver_api());
+  for (int i0 = 0; i0 < n; i0 += kMaxGroup) {
+    const GemmProblem* group = probs + i0;
+    const int m = std::min(kMaxGroup, n - i0);
+    bool pair = m > 1;
+    int max_m = 0;
+    for (int g = 0; g < m; ++g) {
+      pair = pair && group[g].N % 256 == 0;
+      max_m = std::max(max_m, group[g].M);
+    }
+    if (pair && max_m > BM) {
+      M3PC_TRY(launch_2sm<4>(group, m, st));
+    } else {
+      for (int g = 0; g < m; ++g) M3PC_TRY(gemm_bf16_one(group[g], st));
+    }
+  }
   return M3PC_OK;
 }
 

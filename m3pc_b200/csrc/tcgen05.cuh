@@ -197,8 +197,175 @@ __device__ __forceinline__ float gelu_erf_tanh(float x) {
   return fmaf(hx, t, hx);
 }
 
+// ---- the pipeline every tensor-core GEMM kernel runs -----------------------------------------------------------------------------
+// Warp 0 (one thread) streams the operands of each k-block through a STAGES-deep shared-memory ring (`full`: the stage's bytes have
+// landed; `empty`: the MMAs that read it have completed).  Warp 1 (one thread; the leader CTA's with a CTA pair) issues the MMAs of
+// a unit into one of NACC accumulators of ACC_COLS TMEM columns (`acc_full`: complete; `acc_empty`: every epilogue warp has read it),
+// so with NACC = 2 the epilogue of one unit runs under the MMAs of the next.  Every role walks the same units u_lo, u_lo + u_step,
+// ... < u_hi in order, which keeps their stage and accumulator indices in step.  CG is the MMAs' cta_group (2: a CTA pair shares
+// each MMA and its accumulator) and CL the CTAs of a cluster (CG = 1: CL CTAs multicast their operands to each other).
+template <int STAGES, int NACC, int ACC_COLS, int CG, int CL>
+struct TcPipeline {
+  static_assert(CG == 1 || CL == 2, "a CTA pair is a cluster of two");
+  static constexpr uint32_t kTmemCols = NACC * ACC_COLS;
+  static constexpr int kBarBytes = 8 * (2 * STAGES + 2 * NACC + 1);  // the barriers and the TMEM address slot
+  uint64_t* full;
+  uint64_t* empty;
+  uint64_t* acc_full;
+  uint64_t* acc_empty;
+  uint32_t acc_empty_leader;  // CG = 2: shared::cluster address of the leader's acc_empty
+  uint32_t tmem_base;
+
+  // Set-up, run by every thread of the CTA, with the kBarBytes of barriers at `bars`.  Thread 0 initialises them -- an accumulator
+  // is handed back by the `epi_warps` epilogue warps of each CTA of the MMA -- and runs init() (tensor-map prefetches, barriers of
+  // the kernel's own); warp 1 allocates the tensor memory.  Ends with PDL_PROLOGUE: everything before it is private to the CTA (or
+  // pair), operands of the previous kernel are touched only after it.
+  template <typename Init>
+  static __device__ __forceinline__ TcPipeline setup(uint8_t* bars, uint32_t epi_warps, Init&& init) {
+    TcPipeline p;
+    p.full = reinterpret_cast<uint64_t*>(bars);
+    p.empty = p.full + STAGES;
+    p.acc_full = p.empty + STAGES;
+    p.acc_empty = p.acc_full + NACC;
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(p.acc_empty + NACC);
+    if (threadIdx.x == 0) {
+#pragma unroll
+      for (int s = 0; s < STAGES; ++s) {
+        mbar_init(&p.full[s], 1);
+        mbar_init(&p.empty[s], CG == 2 ? 1 : CL);  // one tcgen05.commit arrival from every CTA whose MMAs read the stage
+      }
+#pragma unroll
+      for (int b = 0; b < NACC; ++b) {
+        mbar_init(&p.acc_full[b], 1);
+        mbar_init(&p.acc_empty[b], CG * epi_warps);
+      }
+      init();
+      fence_barrier_init();
+      fence_proxy_async();
+    }
+    if (threadIdx.x / 32 == 1) {
+      if (CG == 1) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+      } else {  // the same warp of both CTAs allocates
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTmemCols)
+                     : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+      }
+    }
+    tc_fence_before();
+    if (CL > 1) cluster_sync_all(); else __syncthreads();  // peers must see initialised barriers before any multicast or arrival lands
+    tc_fence_after();
+    p.tmem_base = *tmem_slot;
+    if (CG == 2) p.acc_empty_leader = mapa_u32(smem_u32(p.acc_empty), 0);
+    PDL_PROLOGUE();
+    return p;
+  }
+
+  // TMA producer (one thread): unit(u) prepares unit u and returns its number of k-blocks (returned as a reference into the kernel
+  // parameters, it is read again at every k-block, and the loop is not unrolled); load(kb, s) issues the loads of k-block kb into
+  // stage s, whose previous contents every MMA has read, and posts the bytes they bring on full[s].
+  template <typename Unit, typename Load>
+  __device__ __forceinline__ void produce(int u_lo, int u_hi, int u_step, Unit&& unit, Load&& load) const {
+    int s = 0;
+    uint32_t ph = 0;
+    for (int u = u_lo; u < u_hi; u += u_step) {
+      decltype(auto) num_kb = unit(u);
+      for (int kb = 0; kb < num_kb; ++kb) {
+        mbar_wait(&empty[s], ph ^ 1);
+        load(kb, s);
+        if (++s == STAGES) { s = 0; ph ^= 1; }
+      }
+    }
+  }
+
+  // MMA issuer (one thread): unit(u) returns unit u's number of k-blocks (as for produce); mma(d, kb, s) issues the MMAs of
+  // k-block kb from stage s into the accumulator at TMEM address d.  A stage is released once its MMAs have completed (in every
+  // CTA that reads it: the commit multicasts), the accumulator once the unit's last MMA has.
+  template <typename Unit, typename Mma>
+  __device__ __forceinline__ void issue(int u_lo, int u_hi, int u_step, Unit&& unit, Mma&& mma) const {
+    int s = 0;
+    uint32_t ph = 0, it = 0;
+    for (int u = u_lo; u < u_hi; u += u_step, ++it) {
+      const uint32_t a = it % NACC;
+      mbar_wait(&acc_empty[a], ((it / NACC) & 1u) ^ 1u);  // the epilogue has drained this accumulator (first use passes at once)
+      tc_fence_after();
+      const uint32_t d = tmem_base + a * ACC_COLS;
+      decltype(auto) num_kb = unit(u);
+      for (int kb = 0; kb < num_kb; ++kb) {
+        mbar_wait(&full[s], ph);
+        tc_fence_after();
+        mma(d, kb, s);
+        if (CG == 2) umma_commit_2sm(&empty[s]);
+        else if (CL > 1) umma_commit_mc(&empty[s], static_cast<uint16_t>((1u << CL) - 1u));
+        else umma_commit(&empty[s]);
+        if (++s == STAGES) { s = 0; ph ^= 1; }
+      }
+      if (CG == 2) umma_commit_2sm(&acc_full[a]); else umma_commit(&acc_full[a]);
+    }
+  }
+
+  // Epilogue: waits until the accumulator of this CTA's it-th unit is complete and returns its index.
+  __device__ __forceinline__ uint32_t acc_wait(uint32_t it) const {
+    const uint32_t a = it % NACC;
+    mbar_wait(&acc_full[a], (it / NACC) & 1u);
+    tc_fence_after();
+    return a;
+  }
+  // Epilogue: hands accumulator a back to the MMA issuer (on the leader's barrier with a CTA pair) once every TMEM read of this warp
+  // has completed (tcgen05.wait::ld).
+  __device__ __forceinline__ void acc_release(uint32_t a) const {
+    tc_fence_before();
+    if (threadIdx.x % 32 == 0) {
+      if (CG == 2) mbar_arrive_remote(acc_empty_leader + 8u * a); else mbar_arrive(&acc_empty[a]);
+    }
+  }
+
+  // Run by every thread: no CTA may exit while a peer can still multicast into / arrive on it.
+  __device__ __forceinline__ void teardown() const {
+    tc_fence_before();
+    if (CL > 1) cluster_sync_all(); else __syncthreads();
+    if (threadIdx.x / 32 == 1) {
+      tc_fence_after();
+      if (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
+      else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
+    }
+  }
+};
+
+// Problem of unit u in a grouped launch: P holds P.n <= kMaxGroup problems P.p[g], in the order of their first units P.p[g].unit0.
+template <typename Params>
+__device__ __forceinline__ int problem_of(const Params& P, int u) {
+  int g = 0;
+#pragma unroll
+  for (int i = 1; i < kMaxGroup; ++i)
+    if (i < P.n && u >= P.p[i].unit0) g = i;
+  return g;
+}
+
 // host: K-major bf16 operand map (box = 64 k x box_rows rows, SWIZZLE_128B) and output map (box = 32 rows x 64 bytes, SWIZZLE_64B)
 int make_tmap(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows);
 int make_tmap_out(CUtensorMap* map, void* ptr, uint64_t rows, uint64_t cols, bool f32);
+
+// host: one launch of a CTA-pair kernel over the problems of P.  Their units are numbered in problem order (P.p[g].unit0, P.n_units;
+// units(P.p[g]) each) and min(units, SMs / 2) pairs walk them; schedule(pairs) sets what depends on the number of pairs.
+// `smem_limit` belongs to the kernel instance (raise_smem_limit).
+template <typename Params, typename Units, typename Schedule>
+int launch_pair(void (*kernel)(Params), PerDevice<size_t>& smem_limit, int smem, int threads, Params& P, Units&& units,
+                Schedule&& schedule, cudaStream_t st) {
+  M3PC_CHECK_CUDA(raise_smem_limit(kernel, smem_limit, smem));
+  int n_units = 0;
+  for (int g = 0; g < P.n; ++g) {
+    P.p[g].unit0 = n_units;
+    n_units += units(P.p[g]);
+  }
+  P.n_units = n_units;
+  const int pairs = std::min(n_units, device_num_sms() / 2);
+  schedule(pairs);
+  M3PC_CHECK_CUDA(launch_k_cluster(2, kernel, dim3(2 * pairs), dim3(threads), smem, st, P));
+  M3PC_CHECK_LAUNCH();
+  return M3PC_OK;
+}
 
 }  // namespace m3pc
