@@ -37,6 +37,9 @@ extern "C" {
 
 #define M3PC_PREC_BF16 0 /* bf16 operands on tcgen05 tensor cores, fp32 accumulate, fp32 residual stream */
 #define M3PC_PREC_FP32 1 /* fp32 operands and accumulate on CUDA cores (reference-grade, 1e-5) */
+/* fp32 operands, activations and residual stream as M3PC_PREC_FP32; the contractions on tcgen05 tensor cores (kind::tf32) with
+ * each operand split into a tf32 high part and an fp32 remainder, three MMAs per product, fp32 accumulate: fp32-grade accuracy */
+#define M3PC_PREC_TF32X3 2
 
 /* modality order everywhere: the reference's dict order, finetune_omtm/learner.py:361-366 */
 #define M3PC_STATES 0
@@ -254,6 +257,11 @@ int m3pc_gemm_bf16(const void* A, const void* W, const float* bias, void* C, int
                    int32_t flags, void* stream);
 int m3pc_gemm_fp32(const float* A, const float* W, const float* bias, float* C, int32_t M, int32_t N, int32_t K,
                    int32_t flags, void* stream);
+/* m3pc_gemm_fp32's contract on the tensor cores with the 3xTF32 split (the GEMM of M3PC_PREC_TF32X3): problems of at most 128
+ * rows, with N not a multiple of 256 or with K not a multiple of 4 run on the CUDA-core fp32 kernel.  A, W, C and bias (when
+ * not NULL) must be 16-byte aligned; M3PC_ERR_INVALID otherwise. */
+int m3pc_gemm_tf32x3(const float* A, const float* W, const float* bias, float* C, int32_t M, int32_t N, int32_t K,
+                     int32_t flags, void* stream);
 /* n independent bf16 GEMMs (arrays of n operands / shapes / flags as in m3pc_gemm_bf16; bias may be NULL or hold NULLs)
  * in as few launches as possible: up to 4 problems whose N are multiples of 256 share one launch of the CTA-pair
  * tensor-core kernel -- how the engine issues the decoder-embedding runs, the decoder K/V + Q projections, the

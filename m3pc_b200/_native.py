@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(HERE, "libm3pc.so")
 CSRC = os.path.join(HERE, "csrc")
 
 OK = 0
-PREC_BF16, PREC_FP32 = 0, 1
+PREC_BF16, PREC_FP32, PREC_TF32X3 = 0, 1, 2
 GUIDE_RTG, GUIDE_CRITIC, GUIDE_NOISE_CRITIC, GUIDE_SAMPLING = 0, 1, 2, 3
 MAX_T, MAX_ACT, MAX_OBS = 16, 32, 128
 PARTIAL_FLOATS = 8 + 2 * MAX_ACT
@@ -32,7 +32,7 @@ GUIDANCE = {
 SYMBOLS = (
     "m3pc_last_error", "m3pc_version", "m3pc_create", "m3pc_destroy", "m3pc_set_param", "m3pc_finalize_params", "m3pc_set_option",
     "m3pc_forward", "m3pc_plan", "m3pc_merge_partials", "m3pc_exchange_local", "m3pc_exchange_connect", "m3pc_exchange_status", "m3pc_backward_plan", "m3pc_backward_plan_draws",
-    "m3pc_ring_reset", "m3pc_ring_append_slots", "m3pc_ring_windows_slots", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16", "m3pc_gemm_fp32",
+    "m3pc_ring_reset", "m3pc_ring_append_slots", "m3pc_ring_windows_slots", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16", "m3pc_gemm_fp32", "m3pc_gemm_tf32x3",
     "m3pc_layernorm", "m3pc_attention", "m3pc_embed_gather", "m3pc_decoder_scatter_embed", "m3pc_block_forward", "m3pc_heads", "m3pc_sample_candidates", "m3pc_twinq",
     "m3pc_score_select", "m3pc_last_device_ms", "m3pc_last_launch_count", "m3pc_set_profile", "m3pc_get_profile",
 )
@@ -111,6 +111,7 @@ def lib() -> C.CDLL:
     L.m3pc_gemm_bf16_grouped.argtypes = [i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.m3pc_gemm_ln_bf16.argtypes = [vp, vp, f32p, f32p, vp, f32p, f32p, f32p, i32, i32, i32, vp]
     L.m3pc_gemm_fp32.argtypes = [f32p, f32p, f32p, f32p, i32, i32, i32, i32, vp]
+    L.m3pc_gemm_tf32x3.argtypes = [f32p, f32p, f32p, f32p, i32, i32, i32, i32, vp]
     L.m3pc_layernorm.argtypes = [f32p, f32p, f32p, vp, i32, i32, i32, vp]
     L.m3pc_attention.argtypes = [vp, vp, i32, i32, i32, i32, vp]
     L.m3pc_embed_gather.argtypes = [vp, i32, f32p, f32p, f32p, f32p, vp, f32p, vp, vp]

@@ -297,5 +297,7 @@ int gemm_bf16(const GemmProblem* probs, int n, cudaStream_t st);
 int gemm_bf16_skinny(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, int M, int N, int K, const GemmEpilogue& epi, cudaStream_t st);
 // sgemm.cu
 int gemm_fp32(const float* A, const float* W, float* C, int M, int N, int K, const GemmEpilogue& epi, cudaStream_t st);
+// gemm_tf32x3.cu: the same contract as gemm_fp32, on the tensor cores with the 3xTF32 split (small problems: gemm_fp32)
+int gemm_tf32x3(const float* A, const float* W, float* C, int M, int N, int K, const GemmEpilogue& epi, cudaStream_t st);
 
 }  // namespace m3pc

@@ -103,6 +103,7 @@ struct m3pc_engine {
   int D = 0, H = 0, T = 0, F = 0, obs = 0, act = 0, Le = 0, Ld = 0, QH = 0;
   int dims[4] = {0, 0, 0, 0};
   bool bf16 = true;
+  bool tf32x3 = false;  // M3PC_PREC_TF32X3: the fp32 mode with its contractions on the tensor cores (gemm_tf32x3)
   int chunk = 0;
   bool finalized = false;
   std::map<std::string, std::vector<float>> staged;
@@ -440,8 +441,16 @@ int profiled(m3pc_engine* e, double flops, cudaStream_t st, Launch&& launch) {
   return M3PC_OK;
 }
 
-// Independent GEMMs C = epilogue(A W^T) with the weights in both precisions.  bf16 mode: kMaxGroup at a time, each such group one
-// launch of the CTA-pair tensor-core kernel where it applies (gemm_bf16) and booked as one profile entry; fp32 mode: one launch each.
+// C = epilogue(A W^T) on fp32 operands, with the kernel the precision mode runs fp32 contractions on: the 3xTF32 tensor-core kernel
+// in tf32x3 mode, the CUDA-core kernel otherwise (fp32 mode; the fp32 critic layers of bf16 mode, when its width is not a multiple
+// of 128).
+int gemm_f32(const m3pc_engine* e, const float* A, const float* W, float* C, int M, int N, int K, const GemmEpilogue& epi, cudaStream_t st) {
+  return e->tf32x3 ? gemm_tf32x3(A, W, C, M, N, K, epi, st) : gemm_fp32(A, W, C, M, N, K, epi, st);
+}
+
+// Independent GEMMs C = epilogue(A W^T) on activations of the mode's type, with the weights in both precisions.  bf16 mode:
+// kMaxGroup at a time, each such group one launch of the CTA-pair tensor-core kernel where it applies (gemm_bf16) and booked as one
+// profile entry; fp32 and tf32x3 modes: one launch each (gemm_f32).
 struct GemmJob {
   const void* A;
   const float* w32;
@@ -464,7 +473,7 @@ int gemm_group(m3pc_engine* e, const GemmJob* jobs, int n, cudaStream_t st) {
     const GemmJob& j = jobs[i0];
     M3PC_TRY(profiled(e, flops, st, [&] {
       return e->bf16 ? gemm_bf16(pr, m, st)
-                     : gemm_fp32(reinterpret_cast<const float*>(j.A), j.w32, reinterpret_cast<float*>(j.C), j.M, j.N, j.K, j.epi, st);
+                     : gemm_f32(e, reinterpret_cast<const float*>(j.A), j.w32, reinterpret_cast<float*>(j.C), j.M, j.N, j.K, j.epi, st);
     }));
   }
   return M3PC_OK;
@@ -1101,7 +1110,8 @@ int forward(m3pc_engine* e, const FwdIO& io, int B, cudaStream_t st) {
 
 // K7: TwinQ on all (candidate, step) rows at once (the reference calls it h times on N rows, learner.py:250-252).
 // bf16 mode: the two hidden layers run on the tcgen05 GEMM (bf16 operands, fp32 accumulate, second layer written in fp32);
-// fp32 mode: CUDA-core fp32 GEMMs.  The final 256 -> 1 layer and min(q1, q2) are fp32 in both.
+// otherwise (and in the fp32 / tf32x3 modes) fp32 GEMMs on the mode's fp32 kernel (gemm_f32).  The final 256 -> 1 layer and
+// min(q1, q2) are fp32 in all modes.
 int critic(m3pc_engine* e, int N, int h, cudaStream_t st, const float* states_pred = nullptr, const float* cand = nullptr, float* q_out = nullptr) {
   const int rows = N * h, in = e->obs + e->act, Hq = e->QH;
   float* qv = q_out != nullptr ? q_out : e->qvals.as<float>();
@@ -1139,9 +1149,9 @@ int critic(m3pc_engine* e, int N, int h, cudaStream_t st, const float* states_pr
     GemmEpilogue ge;
     ge.bias = e->q_b[q][0];
     ge.flags = EPI_RELU;
-    M3PC_TRY(gemm_fp32(e->sa.as<float>(), e->q_w[q][0], e->qa.as<float>(), rows, Hq, in, ge, st));
+    M3PC_TRY(profiled(e, 2.0 * rows * Hq * in, st, [&] { return gemm_f32(e, e->sa.as<float>(), e->q_w[q][0], e->qa.as<float>(), rows, Hq, in, ge, st); }));
     ge.bias = e->q_b[q][1];
-    M3PC_TRY(gemm_fp32(e->qa.as<float>(), e->q_w[q][1], outs[q], rows, Hq, Hq, ge, st));
+    M3PC_TRY(profiled(e, 2.0 * rows * Hq * Hq, st, [&] { return gemm_f32(e, e->qa.as<float>(), e->q_w[q][1], outs[q], rows, Hq, Hq, ge, st); }));
   }
   return launch_critic_out(outs[0], outs[1], e->q_w[0][2], e->q_b[0][2], e->q_w[1][2], e->q_b[1][2], qv, rows, Hq, st);
 }
@@ -1485,7 +1495,8 @@ int create(m3pc_handle_t* out, const m3pc_config_t* cfg) {
   M3PC_REQUIRE(cfg->traj_length >= 1 && cfg->traj_length <= M3PC_MAX_T, "traj_length out of range");
   M3PC_REQUIRE(cfg->obs_dim >= 1 && cfg->obs_dim <= M3PC_MAX_OBS && cfg->act_dim >= 1 && cfg->act_dim <= M3PC_MAX_ACT, "obs/act dim out of range");
   M3PC_REQUIRE(cfg->n_enc_layer >= 1 && cfg->n_dec_layer >= 1, "need at least one encoder and one decoder layer");
-  M3PC_REQUIRE(cfg->precision == M3PC_PREC_BF16 || cfg->precision == M3PC_PREC_FP32, "unknown precision");
+  M3PC_REQUIRE(cfg->precision == M3PC_PREC_BF16 || cfg->precision == M3PC_PREC_FP32 || cfg->precision == M3PC_PREC_TF32X3,
+               "unknown precision");
   M3PC_REQUIRE(cfg->max_batch >= 1, "max_batch must be positive");
   int dev = 0;
   M3PC_CHECK_CUDA(cudaGetDevice(&dev));
@@ -1502,9 +1513,10 @@ int create(m3pc_handle_t* out, const m3pc_config_t* cfg) {
   e->obs = cfg->obs_dim; e->act = cfg->act_dim; e->Le = cfg->n_enc_layer; e->Ld = cfg->n_dec_layer; e->QH = cfg->critic_hidden;
   e->dims[0] = e->obs; e->dims[1] = e->act; e->dims[2] = 1; e->dims[3] = 1;
   e->bf16 = cfg->precision == M3PC_PREC_BF16;
+  e->tf32x3 = cfg->precision == M3PC_PREC_TF32X3;
   e->chunk = cfg->chunk > 0 ? cfg->chunk : 8192;  // measured (profiles/r1e_chunk_sweep.txt, 8 x 1024 rows per step): 3.86 ms in chunks of 1024, 3.28 ms at 4096, 3.20 ms at 8192
   e->chunk = std::min(e->chunk, cfg->max_batch);
-  if (e->bf16) M3PC_TRY(gemm_init_driver_api());
+  if (e->bf16 || e->tf32x3) M3PC_TRY(gemm_init_driver_api());
   const size_t rows = static_cast<size_t>(4) * e->T * e->chunk + 128;  // +128: slack rows for tile tails
   const size_t ab = act_bytes(e.get()), D = e->D;
   M3PC_TRY(e->X.alloc(rows * D * 4));
@@ -1796,6 +1808,15 @@ int m3pc_gemm_fp32(const float* A, const float* W, const float* bias, float* C, 
   ep.bias = bias;
   ep.flags = flags;
   return m3pc::gemm_fp32(A, W, C, M, N, K, ep, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int m3pc_gemm_tf32x3(const float* A, const float* W, const float* bias, float* C, int32_t M, int32_t N, int32_t K, int32_t flags, void* stream) {
+  M3PC_REQUIRE(A && W && C, "null argument");
+  M3PC_REQUIRE((flags & ~7) == 0, "unknown flag");
+  m3pc::GemmEpilogue ep;
+  ep.bias = bias;
+  ep.flags = flags;
+  return m3pc::gemm_tf32x3(A, W, C, M, N, K, ep, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_layernorm(const float* x, const float* gamma, const float* beta, void* y, int32_t M, int32_t D, int32_t out_bf16, void* stream) {

@@ -454,12 +454,14 @@ __global__ void __launch_bounds__(GEMM_THREADS_2SM, 1) gemm_bf16_2sm_kernel(cons
 }
 
 }  // namespace
-int make_tmap(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows) {
+namespace {
+int make_tmap_operand(CUtensorMap* map, CUtensorMapDataType type, uint32_t elem_bytes, const void* ptr, uint64_t rows, uint64_t cols,
+                      uint32_t box_rows) {
   cuuint64_t gdim[2] = {cols, rows};
-  cuuint64_t gstride[1] = {cols * sizeof(__nv_bfloat16)};
-  cuuint32_t box[2] = {static_cast<cuuint32_t>(BK), box_rows};
+  cuuint64_t gstride[1] = {cols * elem_bytes};
+  cuuint32_t box[2] = {128u / elem_bytes, box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), gdim, gstride, box, estr,
+  CUresult r = g_encode_tiled(map, type, 2, const_cast<void*>(ptr), gdim, gstride, box, estr,
                               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -468,6 +470,13 @@ int make_tmap(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, u
     return M3PC_ERR_CUDA;
   }
   return M3PC_OK;
+}
+}  // namespace
+int make_tmap(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows) {
+  return make_tmap_operand(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, ptr, rows, cols, box_rows);
+}
+int make_tmap_f32(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows) {
+  return make_tmap_operand(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, ptr, rows, cols, box_rows);
 }
 namespace {
 

@@ -1,4 +1,4 @@
-// tcgen05 / TMA / mbarrier PTX wrappers shared by the sm_100a tensor-core kernels (gemm_tcgen05.cu, gemm_ln.cu).
+// tcgen05 / TMA / mbarrier PTX wrappers shared by the sm_100a tensor-core kernels (gemm_tcgen05.cu, gemm_ln.cu, gemm_tf32x3.cu).
 #pragma once
 #include <cuda.h>
 
@@ -154,6 +154,26 @@ __device__ __forceinline__ void umma_commit_2sm(uint64_t* bar) {
 __host__ __device__ constexpr uint32_t make_idesc_mn(int m, int n) {
   return (1u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(m >> 4) << 24);
 }
+// kind::tf32 instruction descriptor (cute::UMMA::InstrDescriptor): c_format [4,6) = F32 (1), a_format [7,10) = b_format [10,13) =
+// TF32 (2 in UMMA::F16F32Format), both K-major, N >> 3 at bit 17, M >> 4 at bit 24.
+__host__ __device__ constexpr uint32_t make_idesc_tf32(int m, int n) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(m >> 4) << 24);
+}
+// as umma_bf16_2sm, kind::tf32: K = 8 fp32 (32 bytes) per instruction
+__device__ __forceinline__ void umma_tf32_2sm(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t"
+      "}" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// arrive on a barrier of another CTA of the cluster, releasing this thread's prior writes at cluster scope
+__device__ __forceinline__ void mbar_arrive_remote_release(uint32_t bar_cluster_addr) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster_addr) : "memory");
+}
 
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile(
@@ -202,8 +222,10 @@ __device__ __forceinline__ float gelu_erf_tanh(float x) {
 // landed; `empty`: the MMAs that read it have completed).  Warp 1 (one thread; the leader CTA's with a CTA pair) issues the MMAs of
 // a unit into one of NACC accumulators of ACC_COLS TMEM columns (`acc_full`: complete; `acc_empty`: every epilogue warp has read it),
 // so with NACC = 2 the epilogue of one unit runs under the MMAs of the next.  Every role walks the same units u_lo, u_lo + u_step,
-// ... < u_hi in order, which keeps their stage and accumulator indices in step.  CG is the MMAs' cta_group (2: a CTA pair shares
-// each MMA and its accumulator) and CL the CTAs of a cluster (CG = 1: CL CTAs multicast their operands to each other).
+// ... < u_hi in order, which keeps their stage and accumulator indices in step.  The MMAs of a stage wait on `ready`, which is `full`
+// unless the kernel points it at barriers of its own (a stage that is transformed in shared memory before the MMAs read it).  CG is
+// the MMAs' cta_group (2: a CTA pair shares each MMA and its accumulator) and CL the CTAs of a cluster (CG = 1: CL CTAs multicast
+// their operands to each other).
 template <int STAGES, int NACC, int ACC_COLS, int CG, int CL>
 struct TcPipeline {
   static_assert(CG == 1 || CL == 2, "a CTA pair is a cluster of two");
@@ -213,6 +235,7 @@ struct TcPipeline {
   uint64_t* empty;
   uint64_t* acc_full;
   uint64_t* acc_empty;
+  uint64_t* ready;
   uint32_t acc_empty_leader;  // CG = 2: shared::cluster address of the leader's acc_empty
   uint32_t tmem_base;
 
@@ -227,6 +250,7 @@ struct TcPipeline {
     p.empty = p.full + STAGES;
     p.acc_full = p.empty + STAGES;
     p.acc_empty = p.acc_full + NACC;
+    p.ready = p.full;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(p.acc_empty + NACC);
     if (threadIdx.x == 0) {
 #pragma unroll
@@ -294,7 +318,7 @@ struct TcPipeline {
       const uint32_t d = tmem_base + a * ACC_COLS;
       decltype(auto) num_kb = unit(u);
       for (int kb = 0; kb < num_kb; ++kb) {
-        mbar_wait(&full[s], ph);
+        mbar_wait(&ready[s], ph);
         tc_fence_after();
         mma(d, kb, s);
         if (CG == 2) umma_commit_2sm(&empty[s]);
@@ -344,8 +368,10 @@ __device__ __forceinline__ int problem_of(const Params& P, int u) {
   return g;
 }
 
-// host: K-major bf16 operand map (box = 64 k x box_rows rows, SWIZZLE_128B) and output map (box = 32 rows x 64 bytes, SWIZZLE_64B)
+// host: K-major bf16 / fp32 operand maps (box = one 128-byte row of k -- 64 bf16 / 32 fp32 -- x box_rows rows, SWIZZLE_128B) and
+// output map (box = 32 rows x 64 bytes, SWIZZLE_64B)
 int make_tmap(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows);
+int make_tmap_f32(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t cols, uint32_t box_rows);
 int make_tmap_out(CUtensorMap* map, void* ptr, uint64_t rows, uint64_t cols, bool f32);
 
 // host: one launch of a CTA-pair kernel over the problems of P.  Their units are numbered in problem order (P.p[g].unit0, P.n_units;

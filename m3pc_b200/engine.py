@@ -31,6 +31,10 @@ def _dev_f32(t: torch.Tensor, what: str) -> torch.Tensor:
     return t
 
 
+#: ``precision`` names -> M3PC_PREC_* (include/m3pc.h): "bf16" tensor cores at bf16 operands; "fp32" IEEE fp32 FFMA on CUDA cores, the
+#: reference's arithmetic; "tf32x3" fp32 operands on the tensor cores with the 3xTF32 split, fp32-grade accuracy
+PRECISIONS = {"bf16": nat.PREC_BF16, "fp32": nat.PREC_FP32, "tf32x3": nat.PREC_TF32X3}
+
 class PlanEngine:
     """One engine per (process, device).  Mirrors ``m3pc_create`` .. ``m3pc_destroy``."""
 
@@ -41,6 +45,8 @@ class PlanEngine:
     def __init__(self, *, n_embd: int, n_head: int, n_enc_layer: int, n_dec_layer: int, traj_length: int, obs_dim: int,
                  act_dim: int, precision: str = "bf16", max_batch: int = 1024, chunk: int = 0, critic_hidden: int = 0,
                  device: Optional[torch.device] = None):
+        if precision not in PRECISIONS:
+            raise ValueError(f"unknown precision {precision!r}: one of {sorted(PRECISIONS)}")
         if not torch.cuda.is_available():
             raise RuntimeError("m3pc_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = nat.lib()
@@ -52,7 +58,7 @@ class PlanEngine:
         self.critic_hidden = int(critic_hidden)
         cfg = nat.Config(n_embd=n_embd, n_head=n_head, n_enc_layer=n_enc_layer, n_dec_layer=n_dec_layer,
                          traj_length=traj_length, obs_dim=obs_dim, act_dim=act_dim,
-                         precision={"bf16": nat.PREC_BF16, "fp32": nat.PREC_FP32}[precision],
+                         precision=PRECISIONS[precision],
                          max_batch=self.max_batch, chunk=int(chunk), critic_hidden=self.critic_hidden)
         self._h = C.c_void_p()
         with torch.cuda.device(self.device):

@@ -45,7 +45,8 @@ class PlannerMixin:
     #: global candidate id of this process's first candidate / total (candidate sharding across ranks)
     cand_offset: int = 0
 
-    #: precision of the shadow engine when ``self.mtm`` is the REFERENCE's trainable omtm (hybrid drop-in, INTEGRATION.md)
+    #: precision of the shadow engine when ``self.mtm`` is the REFERENCE's trainable omtm (hybrid drop-in, INTEGRATION.md):
+    #: "bf16", "fp32" or "tf32x3" (fp32-grade on the tensor cores)
     planner_precision: str = "bf16"
 
     @staticmethod

@@ -92,7 +92,8 @@ class omtmConfig:
     target_entropy: float = -3
     use_entropy: bool = True
     # engine options (not in the reference)
-    precision: str = "bf16"   # "bf16": tcgen05 tensor cores; "fp32": reference-grade CUDA-core path
+    precision: str = "bf16"   # "bf16": tcgen05 tensor cores; "fp32": reference-grade CUDA-core path;
+                              # "tf32x3": fp32-grade, the fp32 path with its GEMMs on the tensor cores (3xTF32 split)
     max_batch: int = 1024     # largest batch (candidates or envs) a forward / plan may carry
     chunk: int = 0            # batch rows per kernel sequence (0 = library default)
 
