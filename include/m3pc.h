@@ -278,6 +278,26 @@ int m3pc_layernorm(const float* x, const float* gamma, const float* beta, void* 
                    int32_t out_bf16, void* stream);
 /* Bidirectional attention over token-major qkv (S*B rows, 3*D cols), head_dim 128; out (S*B, D). */
 int m3pc_attention(const void* qkv, void* out, int32_t B, int32_t S, int32_t n_head, int32_t is_bf16, void* stream);
+/* One token of m3pc_attention_gather: its row for batch row b starts at ptr + (bdiv > 0 ? b / bdiv : b) * bstride elements
+ * (bstride 0: one row for the whole batch; bdiv > 0: one row per group of bdiv batch rows).  Head h is columns h*128 .. h*128+127. */
+typedef struct {
+  const void* ptr;
+  int32_t bstride;
+  int32_t bdiv;
+} m3pc_attn_tok_t;
+/* The token-gather attention the engine runs in pass 2 (queries, keys and values each from their own rows):
+ * out[i*B + b, h*128 + d] = softmax_j(q_i(b,h) . k_j(b,h) / sqrt(128)) v_j(b,h)[d], out (n_q*B, n_head*128) device, bf16
+ * (is_bf16) or fp32 like every operand.  q, k, v are HOST arrays of n_q, n_kv, n_kv headers; n_q, n_kv in [1, 64].
+ * n_kv_batch > 0 names keys [0, n_kv_batch) per-batch-row and keys [n_kv_batch, n_kv) shared: the bf16 path then takes the
+ * shared-key kernel (constant K / V staged once per CTA of 8 batch rows) when n_q <= 16, B >= 64, at least 8 shared keys, at
+ * most 32 per-batch and 48 shared keys, every per-batch key's K and V have one bstride and bdiv, and the shared keys are all
+ * batch-constant (bstride 0, bdiv 0) or all per-group with one common bdiv that is a multiple of 8; otherwise the per-row kernel.
+ * ptr and out must be 16-byte aligned and bstride a multiple of 8 (bf16) or 4 (fp32) elements; M3PC_ERR_INVALID otherwise.
+ * out_kernel: NULL, or HOST int32[4] that receives {kind, a, b, grid_x} of the launch: kind 0 = the fp32 kernel, 1 = the bf16
+ * per-row kernel with a = ceil(n_q/16) query and b = ceil(n_kv/16) key tiles, 2 = the shared-key kernel with a per-batch and b
+ * shared key tiles; grid_x < ceil(B/8) there means each CTA walked several blocks of 8 batch rows. */
+int m3pc_attention_gather(const m3pc_attn_tok_t* q, int32_t n_q, const m3pc_attn_tok_t* k, const m3pc_attn_tok_t* v, int32_t n_kv,
+                          int32_t n_kv_batch, int32_t B, int32_t n_head, void* out, int32_t is_bf16, int32_t* out_kernel, void* stream);
 
 /* ---- the fused memory-bound kernels of the path, one entry each (SURVEY.md section 8b K1, K4..K8) ----
  * The activation layout these expose is the library's internal one: token-major matrices, row = token * batch + b, fp32

@@ -33,7 +33,7 @@ SYMBOLS = (
     "m3pc_last_error", "m3pc_version", "m3pc_create", "m3pc_destroy", "m3pc_set_param", "m3pc_finalize_params", "m3pc_set_option",
     "m3pc_forward", "m3pc_plan", "m3pc_merge_partials", "m3pc_exchange_local", "m3pc_exchange_connect", "m3pc_exchange_status", "m3pc_backward_plan", "m3pc_backward_plan_draws",
     "m3pc_ring_reset", "m3pc_ring_append_slots", "m3pc_ring_windows_slots", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16", "m3pc_gemm_fp32", "m3pc_gemm_tf32x3",
-    "m3pc_layernorm", "m3pc_attention", "m3pc_embed_gather", "m3pc_decoder_scatter_embed", "m3pc_block_forward", "m3pc_heads", "m3pc_sample_candidates", "m3pc_twinq",
+    "m3pc_layernorm", "m3pc_attention", "m3pc_attention_gather", "m3pc_embed_gather", "m3pc_decoder_scatter_embed", "m3pc_block_forward", "m3pc_heads", "m3pc_sample_candidates", "m3pc_twinq",
     "m3pc_score_select", "m3pc_last_device_ms", "m3pc_last_launch_count", "m3pc_set_profile", "m3pc_get_profile",
 )
 
@@ -60,6 +60,11 @@ class PlanArgs(C.Structure):
         ("dbg_expect_return", C.c_void_p), ("dbg_candidates", C.c_void_p), ("dbg_indices", C.c_void_p),
         ("exchange", C.c_int32), ("reserved0", C.c_int32), ("env_horizons", C.c_void_p), ("reserved1", C.c_void_p * 2),
     ]
+
+
+class AttnTok(C.Structure):
+    """m3pc_attn_tok_t: one query / key / value token of m3pc_attention_gather."""
+    _fields_ = [("ptr", C.c_void_p), ("bstride", C.c_int32), ("bdiv", C.c_int32)]
 
 
 _lib: Optional[C.CDLL] = None
@@ -114,6 +119,8 @@ def lib() -> C.CDLL:
     L.m3pc_gemm_tf32x3.argtypes = [f32p, f32p, f32p, f32p, i32, i32, i32, i32, vp]
     L.m3pc_layernorm.argtypes = [f32p, f32p, f32p, vp, i32, i32, i32, vp]
     L.m3pc_attention.argtypes = [vp, vp, i32, i32, i32, i32, vp]
+    L.m3pc_attention_gather.argtypes = [C.POINTER(AttnTok), i32, C.POINTER(AttnTok), C.POINTER(AttnTok), i32, i32, i32, i32, vp, i32,
+                                        C.POINTER(i32), vp]
     L.m3pc_embed_gather.argtypes = [vp, i32, f32p, f32p, f32p, f32p, vp, f32p, vp, vp]
     L.m3pc_decoder_scatter_embed.argtypes = [vp, i32, vp, vp, f32p, vp]
     L.m3pc_heads.argtypes = [vp, i32, f32p, f32p, f32p, f32p, f32p, f32p, vp]

@@ -100,7 +100,14 @@ __global__ void __launch_bounds__(ATT_THREADS) attention_kernel(const __grid_con
   }
 }
 
-int launch_simple(const AttnParams& p, cudaStream_t st) {
+// {kind, a, b, grid_x} of the launch into `info` when it is not null (the kernel-level entry reports which instance ran):
+// kind 0 = attention_kernel, 1 = attention_mma_kernel<a, b>, 2 = attention_mma_shared_kernel<a, b>
+void report_launch(int* info, int kind, int a, int b, int grid_x) {
+  if (info == nullptr) return;
+  info[0] = kind; info[1] = a; info[2] = b; info[3] = grid_x;
+}
+
+int launch_simple(const AttnParams& p, cudaStream_t st, int* info) {
   const size_t smem = (static_cast<size_t>(p.n_q) * QS + static_cast<size_t>(p.n_kv) * QS + static_cast<size_t>(p.n_kv) * HD +
                        static_cast<size_t>(p.n_q) * (p.n_kv + 1)) * sizeof(float);
   M3PC_REQUIRE(smem <= 200 * 1024, "attention: sequence too long for the shared-memory resident kernel");
@@ -108,6 +115,7 @@ int launch_simple(const AttnParams& p, cudaStream_t st) {
   M3PC_CHECK_CUDA(raise_smem_limit(attention_kernel, smem_limit, smem));
   M3PC_CHECK_CUDA(launch_k(attention_kernel, dim3(p.B * p.n_head), dim3(ATT_THREADS), smem, st, p));
   M3PC_CHECK_LAUNCH();
+  report_launch(info, 0, 0, 0, p.B * p.n_head);
   return M3PC_OK;
 }
 
@@ -448,7 +456,7 @@ __global__ void __launch_bounds__(SH_WARPS * 32) attention_mma_shared_kernel(con
 }
 
 template <int NTB, int NTC>
-int launch_mma_shared(const AttnParams& p, cudaStream_t st) {
+int launch_mma_shared(const AttnParams& p, cudaStream_t st, int* info) {
   constexpr int smem = 2 * NTC * 16 * 256 + SH_WARPS * (16 + 2 * NTB * 16) * 256;
   static PerDevice<size_t> smem_limit;
   M3PC_CHECK_CUDA(raise_smem_limit(attention_mma_shared_kernel<NTB, NTC>, smem_limit, smem));
@@ -460,57 +468,62 @@ int launch_mma_shared(const AttnParams& p, cudaStream_t st) {
   const int gx = nblk >= 4 * wave ? wave : nblk;
   M3PC_CHECK_CUDA(launch_k(attention_mma_shared_kernel<NTB, NTC>, dim3(gx, p.n_head), dim3(SH_WARPS * 32), smem, st, p));
   M3PC_CHECK_LAUNCH();
+  report_launch(info, 2, NTB, NTC, gx);
   return M3PC_OK;
 }
 
 template <int NTQ, int NTK>
-int launch_mma(const AttnParams& p, cudaStream_t st) {
+int launch_mma(const AttnParams& p, cudaStream_t st, int* info) {
   constexpr int smem = MMA_WARPS * (NTQ + 2 * NTK) * 16 * 256;
   static PerDevice<size_t> smem_limit;
   M3PC_CHECK_CUDA(raise_smem_limit(attention_mma_kernel<NTQ, NTK>, smem_limit, smem));
-  M3PC_CHECK_CUDA(launch_k(attention_mma_kernel<NTQ, NTK>, dim3(ceil_div(p.B * p.n_head, MMA_WARPS)), dim3(MMA_WARPS * 32), smem, st, p));
+  const int gx = ceil_div(p.B * p.n_head, MMA_WARPS);
+  M3PC_CHECK_CUDA(launch_k(attention_mma_kernel<NTQ, NTK>, dim3(gx), dim3(MMA_WARPS * 32), smem, st, p));
   M3PC_CHECK_LAUNCH();
+  report_launch(info, 1, NTQ, NTK, gx);
   return M3PC_OK;
 }
 
 template <int NTK>
-int dispatch_q(const AttnParams& p, cudaStream_t st) {
+int dispatch_q(const AttnParams& p, cudaStream_t st, int* info) {
   switch ((p.n_q + 15) / 16) {
-    case 1: return launch_mma<1, NTK>(p, st);
-    case 2: return launch_mma<2, NTK>(p, st);
-    case 3: return launch_mma<3, NTK>(p, st);
-    default: return launch_mma<4, NTK>(p, st);
+    case 1: return launch_mma<1, NTK>(p, st, info);
+    case 2: return launch_mma<2, NTK>(p, st, info);
+    case 3: return launch_mma<3, NTK>(p, st, info);
+    default: return launch_mma<4, NTK>(p, st, info);
   }
 }
 
 }  // namespace
 
-int launch_attention_gather(const AttnParams& p, bool bf16, cudaStream_t st) {
+int launch_attention_gather(const AttnParams& p, bool bf16, cudaStream_t st, int* launched) {
   M3PC_REQUIRE(p.B > 0 && p.n_q > 0 && p.n_kv > 0 && p.n_q <= MAX_TOK && p.n_kv <= MAX_TOK && p.n_head > 0, "attention: bad shape (<= 64 tokens)");
-  if (!bf16) return launch_simple(p, st);
+  if (!bf16) return launch_simple(p, st, launched);
   if (p.n_kv_batch > 0 && p.n_q <= 16 && p.B >= 64) {  // batch keys first, constant keys after (see AttnParams)
     const int n_c = p.n_kv - p.n_kv_batch, ntb = (p.n_kv_batch + 15) / 16, ntc = (n_c + 15) / 16;
-    bool ok = n_c >= 8 && ntb <= 2 && ntc <= 3;
+    // The constant keys must all have one form: batch-constant, or per-group with one common bdiv (a multiple of SH_WARPS, so
+    // the 8 rows of a block share a group).  The kernel decides when to restage the shared tiles from the first constant key.
+    const int cdiv = n_c > 0 ? p.k[p.n_kv_batch].bdiv : 0;
+    bool ok = n_c >= 8 && ntb <= 2 && ntc <= 3 && cdiv % SH_WARPS == 0;
     for (int j = 0; j < p.n_kv && ok; ++j)
       ok = j < p.n_kv_batch ? (p.k[j].bstride == p.v[j].bstride && p.k[j].bdiv == p.v[j].bdiv)  // K and V of a token move together
-                            : ((p.k[j].bstride == 0 && p.v[j].bstride == 0 && p.k[j].bdiv == 0 && p.v[j].bdiv == 0) ||
-                                      (p.k[j].bdiv > 0 && p.k[j].bdiv % SH_WARPS == 0 && p.v[j].bdiv == p.k[j].bdiv));
+                            : (p.k[j].bdiv == cdiv && p.v[j].bdiv == cdiv && (cdiv > 0 || (p.k[j].bstride == 0 && p.v[j].bstride == 0)));
     if (ok) {
       switch (ntb * 10 + ntc) {
-        case 11: return launch_mma_shared<1, 1>(p, st);
-        case 12: return launch_mma_shared<1, 2>(p, st);
-        case 13: return launch_mma_shared<1, 3>(p, st);
-        case 21: return launch_mma_shared<2, 1>(p, st);
-        case 22: return launch_mma_shared<2, 2>(p, st);
-        default: return launch_mma_shared<2, 3>(p, st);
+        case 11: return launch_mma_shared<1, 1>(p, st, launched);
+        case 12: return launch_mma_shared<1, 2>(p, st, launched);
+        case 13: return launch_mma_shared<1, 3>(p, st, launched);
+        case 21: return launch_mma_shared<2, 1>(p, st, launched);
+        case 22: return launch_mma_shared<2, 2>(p, st, launched);
+        default: return launch_mma_shared<2, 3>(p, st, launched);
       }
     }
   }
   switch ((p.n_kv + 15) / 16) {
-    case 1: return dispatch_q<1>(p, st);
-    case 2: return dispatch_q<2>(p, st);
-    case 3: return dispatch_q<3>(p, st);
-    default: return dispatch_q<4>(p, st);
+    case 1: return dispatch_q<1>(p, st, launched);
+    case 2: return dispatch_q<2>(p, st, launched);
+    case 3: return dispatch_q<3>(p, st, launched);
+    default: return dispatch_q<4>(p, st, launched);
   }
 }
 

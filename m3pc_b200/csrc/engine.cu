@@ -1829,6 +1829,34 @@ int m3pc_attention(const void* qkv, void* out, int32_t B, int32_t S, int32_t n_h
   return m3pc::launch_attention(qkv, out, B, S, n_head, is_bf16 != 0, reinterpret_cast<cudaStream_t>(stream));
 }
 
+int m3pc_attention_gather(const m3pc_attn_tok_t* q, int32_t n_q, const m3pc_attn_tok_t* k, const m3pc_attn_tok_t* v, int32_t n_kv,
+                          int32_t n_kv_batch, int32_t B, int32_t n_head, void* out, int32_t is_bf16, int32_t* out_kernel, void* stream) {
+  M3PC_REQUIRE(q && k && v && out, "null argument");
+  M3PC_REQUIRE(n_q >= 1 && n_q <= m3pc::MAX_TOK && n_kv >= 1 && n_kv <= m3pc::MAX_TOK, "attention_gather: n_q and n_kv must be in [1, 64]");
+  M3PC_REQUIRE(n_kv_batch >= 0 && n_kv_batch <= n_kv, "attention_gather: n_kv_batch must be in [0, n_kv]");
+  M3PC_REQUIRE(B >= 1 && n_head >= 1 && static_cast<int64_t>(B) * n_head <= INT32_MAX, "attention_gather: bad B / n_head");
+  M3PC_REQUIRE(reinterpret_cast<uintptr_t>(out) % 16 == 0, "attention_gather: out must be 16-byte aligned");
+  const int align = is_bf16 ? 8 : 4;  // elements per 16-byte load: cp.async of bf16 rows, float4 of fp32 rows
+  m3pc::AttnParams p{};
+  const m3pc_attn_tok_t* const src[3] = {q, k, v};
+  m3pc::AttnTok* const dst[3] = {p.q, p.k, p.v};
+  for (int l = 0; l < 3; ++l)
+    for (int i = 0; i < (l == 0 ? n_q : n_kv); ++i) {
+      const m3pc_attn_tok_t& t = src[l][i];
+      M3PC_REQUIRE(t.ptr != nullptr, "null token pointer");
+      M3PC_REQUIRE(reinterpret_cast<uintptr_t>(t.ptr) % 16 == 0 && t.bstride >= 0 && t.bstride % align == 0 && t.bdiv >= 0,
+                   "attention_gather: a token's ptr must be 16-byte aligned and its bstride a non-negative multiple of 16 bytes");
+      dst[l][i] = m3pc::AttnTok{t.ptr, t.bstride, t.bdiv};
+    }
+  p.n_q = n_q;
+  p.n_kv = n_kv;
+  p.B = B;
+  p.n_head = n_head;
+  p.n_kv_batch = n_kv_batch;
+  p.out = out;
+  return m3pc::launch_attention_gather(p, is_bf16 != 0, reinterpret_cast<cudaStream_t>(stream), out_kernel);
+}
+
 // ---- kernel-level entries K1 / K4 / K5 / K6 / K7 / K8 (SURVEY.md section 8b): the same launchers m3pc_forward / m3pc_plan use ----
 int m3pc_embed_gather(m3pc_handle_t h, int32_t batch, const float* tok_states, const float* tok_actions, const float* tok_rewards,
                       const float* tok_returns, const uint8_t* masks, float* x_out, void* y_out, void* stream) {

@@ -132,11 +132,14 @@ struct AttnTok {
 struct AttnParams {
   AttnTok q[MAX_TOK], k[MAX_TOK], v[MAX_TOK];
   int n_q, n_kv, B, n_head;
-  int n_kv_batch;  // > 0: keys [0, n_kv_batch) are per-batch rows and keys [n_kv_batch, n_kv) are batch-constant (bstride 0);
-                   // the bf16 kernel then stages the constant keys / values once per CTA instead of once per batch row
+  int n_kv_batch;  // > 0: keys [0, n_kv_batch) are per-batch rows and keys [n_kv_batch, n_kv) are shared by batch rows, all
+                   // batch-constant (bstride 0) or all per-group with one bdiv; the bf16 kernel then stages them once per CTA instead
+                   // of once per batch row (any other key list runs on the per-row kernel)
   void* out;  // (n_q * B, n_head * 128), row = query token * B + b
 };
-int launch_attention_gather(const AttnParams& p, bool bf16, cudaStream_t st);
+// launched: null, or int[4] that receives {kind, a, b, grid_x} of the kernel it launched (kind 0 = fp32 attention_kernel,
+// 1 = attention_mma_kernel<a, b>, 2 = attention_mma_shared_kernel<a, b>)
+int launch_attention_gather(const AttnParams& p, bool bf16, cudaStream_t st, int* launched = nullptr);
 // self-attention over token-major qkv (S*B rows, [Q | K | V] columns)
 int launch_attention(const void* qkv, void* out, int B, int S, int n_head, bool bf16, cudaStream_t st);
 

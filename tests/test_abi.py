@@ -43,6 +43,7 @@ def test_constants_match_header():
     # struct sizes as the header lays them out (LP64)
     assert C.sizeof(nat.Config) == 16 * 4
     assert C.sizeof(nat.PlanArgs) == 8 * 4 + 6 * 8 + 8 + 6 * 8 + 4 * 8
+    assert C.sizeof(nat.AttnTok) == 8 + 2 * 4
 
 
 def test_version_and_error_strings(lib):
@@ -62,6 +63,7 @@ def test_invalid_arguments_are_rejected_without_a_gpu(lib):
     assert lib.m3pc_create(C.byref(h), C.byref(bad)) == -1
     assert lib.m3pc_forward(None, 1, None, None, None, None, None, None, None, None, None, None, None) == -1
     assert lib.m3pc_plan(None, None, None) == -1
+    assert lib.m3pc_attention_gather(None, 1, None, None, 1, 0, 1, 1, None, 1, None, None) == -1
     assert lib.m3pc_destroy(None) == 0
 
 

@@ -166,7 +166,7 @@ def test_layernorm(nat, D):
     assert rel(y, ref) < 1e-5 and rel(y16, ref) < 4e-3
 
 
-@pytest.mark.parametrize("B,S,H", [(5, 13, 4), (3, 32, 4), (2, 64, 8), (70, 17, 4), (1, 9, 4), (33, 10, 4)])
+@pytest.mark.parametrize("B,S,H", [(5, 13, 4), (3, 32, 4), (2, 64, 8), (70, 17, 4), (1, 9, 4), (33, 10, 4), (7, 40, 4), (66, 48, 4)])
 def test_attention(nat, B, S, H):
     torch.manual_seed(0)
     D = H * 128
