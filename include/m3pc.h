@@ -273,6 +273,51 @@ int m3pc_gemm_bf16_grouped(int32_t n, const void* const* A, const void* const* W
  * X = table[row / rows_per_group] + A W^T + bias; Y[M,512] (bf16) = LayerNorm(X; gamma, beta), eps 1e-5.  A, W bf16. */
 int m3pc_gemm_ln_bf16(const void* A, const void* W, const float* bias, float* X, void* Y, const float* gamma, const float* beta,
                       const float* table, int32_t rows_per_group, int32_t M, int32_t K, void* stream);
+
+/* Epilogue flags of m3pc_gemm_bf16_problems (the first three are those of m3pc_gemm_bf16). */
+#define M3PC_EPI_GELU 1      /* GELU(erf) */
+#define M3PC_EPI_RESIDUAL 2  /* C (fp32) += result, in place */
+#define M3PC_EPI_RELU 4      /* ReLU, after GELU when both are set */
+#define M3PC_EPI_ROWTABLE 8  /* add table[(row / rows_per_group) * N + col] before the activations */
+#define M3PC_EPI_OUT_F32 16  /* C is fp32 without a residual */
+/* One bf16 GEMM C[M,N] = act(A[M,K] W[N,K]^T + bias + table[row / rows_per_group]) (+ C with M3PC_EPI_RESIDUAL).  A, W, C device,
+ * 16-byte aligned; bias (N) fp32 or NULL; table (ceil(M / rows_per_group), N) fp32, given exactly when M3PC_EPI_ROWTABLE is set.
+ * bias and table must be 16-byte aligned (the epilogues read them with vector loads); rows_per_group >= 1; K % 64 == 0,
+ * N % 128 == 0.  M3PC_EPI_ROWTABLE and M3PC_EPI_RESIDUAL exclude each other. */
+typedef struct {
+  const void* A;
+  const void* W;
+  const float* bias;
+  const float* table;
+  void* C;
+  int32_t M, N, K;
+  int32_t rows_per_group;
+  int32_t flags;
+} m3pc_gemm_problem_t;
+/* The n >= 1 problems of the HOST array p, issued as the engine issues its grouped GEMMs: 4 at a time, a group of problems whose N
+ * are multiples of 256 as one launch of the CTA-pair kernel when one of them has more than 128 rows, every other problem on its own.
+ * Every argument is checked before any CUDA call; M3PC_ERR_INVALID otherwise.  out_kernel: NULL, or HOST int32[4n] that receives
+ * {kind, a, b, launch} per problem: kind 0 = the skinny CUDA-core kernel (M <= 32); 1 = the single-CTA tensor-core kernel with
+ * a = tile width BN and b = cluster size; 2 = the CTA-pair kernel with a = 1 when its pairs stride over the units (else 0) and
+ * b = the problems sharing that launch; launch = index of the kernel launch within this call. */
+int m3pc_gemm_bf16_problems(const m3pc_gemm_problem_t* p, int32_t n, int32_t* out_kernel, void* stream);
+/* One job of m3pc_gemm_ln_bf16_grouped: X[M,512] = residual + A[M,K] W[512,K]^T + bias, Y[M,512] (bf16) = LayerNorm(X).  The
+ * residual is table[row / rows_per_group] when table is set, else the fp32 rows R (left unchanged) when R is set, else X itself
+ * (in place).  A, W, X, Y, R and table 16-byte aligned; table and R exclude each other; rows_per_group >= 1. */
+typedef struct {
+  const void* A;
+  const void* W;
+  float* X;
+  void* Y;
+  const float* table;
+  const float* R;
+  int32_t rows_per_group;
+  int32_t M;
+} m3pc_ln_job_t;
+/* 1 .. 4 jobs of the fused residual GEMM + LayerNorm in one launch (shared K, bias (512) or NULL, gamma, beta).  out_kernel: NULL,
+ * or HOST int32[2] that receives {rows per CTA-pair unit (128 or 256), CTA pairs} of the launch. */
+int m3pc_gemm_ln_bf16_grouped(const m3pc_ln_job_t* jobs, int32_t n, const float* bias, const float* gamma, const float* beta, int32_t K,
+                              int32_t* out_kernel, void* stream);
 /* y = LayerNorm(x) over the last dim (eps 1e-5); x fp32 (M,D); y bf16 (out_bf16=1) or fp32. */
 int m3pc_layernorm(const float* x, const float* gamma, const float* beta, void* y, int32_t M, int32_t D,
                    int32_t out_bf16, void* stream);

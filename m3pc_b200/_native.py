@@ -32,7 +32,8 @@ GUIDANCE = {
 SYMBOLS = (
     "m3pc_last_error", "m3pc_version", "m3pc_create", "m3pc_destroy", "m3pc_set_param", "m3pc_finalize_params", "m3pc_set_option",
     "m3pc_forward", "m3pc_plan", "m3pc_merge_partials", "m3pc_exchange_local", "m3pc_exchange_connect", "m3pc_exchange_status", "m3pc_backward_plan", "m3pc_backward_plan_draws",
-    "m3pc_ring_reset", "m3pc_ring_append_slots", "m3pc_ring_windows_slots", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16", "m3pc_gemm_fp32", "m3pc_gemm_tf32x3",
+    "m3pc_ring_reset", "m3pc_ring_append_slots", "m3pc_ring_windows_slots", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16",
+    "m3pc_gemm_bf16_problems", "m3pc_gemm_ln_bf16_grouped", "m3pc_gemm_fp32", "m3pc_gemm_tf32x3",
     "m3pc_layernorm", "m3pc_attention", "m3pc_attention_gather", "m3pc_embed_gather", "m3pc_decoder_scatter_embed", "m3pc_block_forward", "m3pc_heads", "m3pc_sample_candidates", "m3pc_twinq",
     "m3pc_score_select", "m3pc_last_device_ms", "m3pc_last_launch_count", "m3pc_set_profile", "m3pc_get_profile",
 )
@@ -65,6 +66,21 @@ class PlanArgs(C.Structure):
 class AttnTok(C.Structure):
     """m3pc_attn_tok_t: one query / key / value token of m3pc_attention_gather."""
     _fields_ = [("ptr", C.c_void_p), ("bstride", C.c_int32), ("bdiv", C.c_int32)]
+
+
+EPI_GELU, EPI_RESIDUAL, EPI_RELU, EPI_ROWTABLE, EPI_OUT_F32 = 1, 2, 4, 8, 16
+
+
+class GemmProblem(C.Structure):
+    """m3pc_gemm_problem_t: one problem of m3pc_gemm_bf16_problems."""
+    _fields_ = [("A", C.c_void_p), ("W", C.c_void_p), ("bias", C.c_void_p), ("table", C.c_void_p), ("C", C.c_void_p),
+                ("M", C.c_int32), ("N", C.c_int32), ("K", C.c_int32), ("rows_per_group", C.c_int32), ("flags", C.c_int32)]
+
+
+class LnJob(C.Structure):
+    """m3pc_ln_job_t: one job of m3pc_gemm_ln_bf16_grouped."""
+    _fields_ = [("A", C.c_void_p), ("W", C.c_void_p), ("X", C.c_void_p), ("Y", C.c_void_p), ("table", C.c_void_p), ("R", C.c_void_p),
+                ("rows_per_group", C.c_int32), ("M", C.c_int32)]
 
 
 _lib: Optional[C.CDLL] = None
@@ -115,6 +131,8 @@ def lib() -> C.CDLL:
     L.m3pc_gemm_bf16.argtypes = [vp, vp, f32p, vp, i32, i32, i32, i32, vp]
     L.m3pc_gemm_bf16_grouped.argtypes = [i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.m3pc_gemm_ln_bf16.argtypes = [vp, vp, f32p, f32p, vp, f32p, f32p, f32p, i32, i32, i32, vp]
+    L.m3pc_gemm_bf16_problems.argtypes = [C.POINTER(GemmProblem), i32, C.POINTER(i32), vp]
+    L.m3pc_gemm_ln_bf16_grouped.argtypes = [C.POINTER(LnJob), i32, f32p, f32p, f32p, i32, C.POINTER(i32), vp]
     L.m3pc_gemm_fp32.argtypes = [f32p, f32p, f32p, f32p, i32, i32, i32, i32, vp]
     L.m3pc_gemm_tf32x3.argtypes = [f32p, f32p, f32p, f32p, i32, i32, i32, i32, vp]
     L.m3pc_layernorm.argtypes = [f32p, f32p, f32p, vp, i32, i32, i32, vp]

@@ -282,7 +282,9 @@ struct LnJob {
   int M;
   const float* R;       // residual rows when they are not X itself (and table is null), or null
 };
-int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const float* gamma, const float* beta, int K, cudaStream_t st);
+// report: null, or int[2] that receives {rows per CTA-pair unit, CTA pairs} of the launch
+int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const float* gamma, const float* beta, int K, cudaStream_t st,
+                         int* report = nullptr);
 // n >= 1 independent bf16 GEMMs C = epilogue(A W^T); up to kMaxGroup of them share one launch of the CTA-pair kernel where it
 // applies (decoder embedding runs, K/V + Q, heads, twin critics)
 struct GemmProblem {
@@ -292,7 +294,9 @@ struct GemmProblem {
   int M, N, K;
   GemmEpilogue epi;
 };
-int gemm_bf16(const GemmProblem* probs, int n, cudaStream_t st);
+// report: null, or int[4 n] that receives {kind, a, b, launch} per problem: kind 0 = the skinny kernel; 1 = gemm_bf16_kernel with
+// a = BN, b = CL; 2 = the CTA-pair kernel with a = strided, b = problems in its launch; launch = index of the launch within this call
+int gemm_bf16(const GemmProblem* probs, int n, cudaStream_t st, int* report = nullptr);
 // gemm_skinny.cu: M <= 32 rows (B = 1 passes): a latency-optimised CUDA-core kernel, same epilogues
 int gemm_bf16_skinny(const __nv_bfloat16* A, const __nv_bfloat16* W, void* C, int M, int N, int K, const GemmEpilogue& epi, cudaStream_t st);
 // sgemm.cu

@@ -1801,6 +1801,37 @@ int m3pc_gemm_ln_bf16(const void* A, const void* W, const float* bias, float* X,
   return m3pc::gemm_ln_bf16_grouped(&job, 1, bias, gamma, beta, K, reinterpret_cast<cudaStream_t>(stream));
 }
 
+int m3pc_gemm_bf16_problems(const m3pc_gemm_problem_t* p, int32_t n, int32_t* out_kernel, void* stream) {
+  static_assert(M3PC_EPI_GELU == m3pc::EPI_GELU && M3PC_EPI_RESIDUAL == m3pc::EPI_RESIDUAL && M3PC_EPI_RELU == m3pc::EPI_RELU &&
+                    M3PC_EPI_ROWTABLE == m3pc::EPI_ROWTABLE && M3PC_EPI_OUT_F32 == m3pc::EPI_OUT_F32,
+                "public epilogue flags");
+  M3PC_REQUIRE(p != nullptr && n >= 1 && n <= m3pc::MAX_TOK, "gemm_bf16_problems: 1 .. 64 problems");
+  m3pc::GemmProblem pr[m3pc::MAX_TOK];
+  for (int i = 0; i < n; ++i) {
+    const m3pc_gemm_problem_t& q = p[i];
+    M3PC_REQUIRE(q.A && q.W && q.C, "null operand");
+    m3pc::GemmEpilogue ep;
+    ep.bias = q.bias;
+    ep.table = q.table;
+    ep.rows_per_group = q.rows_per_group;
+    ep.flags = q.flags;
+    pr[i] = m3pc::GemmProblem{reinterpret_cast<const __nv_bfloat16*>(q.A), reinterpret_cast<const __nv_bfloat16*>(q.W), q.C, q.M, q.N, q.K, ep};
+  }
+  return m3pc::gemm_bf16(pr, n, reinterpret_cast<cudaStream_t>(stream), out_kernel);
+}
+
+int m3pc_gemm_ln_bf16_grouped(const m3pc_ln_job_t* jobs, int32_t n, const float* bias, const float* gamma, const float* beta, int32_t K,
+                              int32_t* out_kernel, void* stream) {
+  M3PC_REQUIRE(jobs != nullptr && n >= 1 && n <= m3pc::kMaxGroup, "gemm_ln_bf16_grouped: 1 .. 4 jobs");
+  m3pc::LnJob lj[m3pc::kMaxGroup];
+  for (int i = 0; i < n; ++i) {
+    const m3pc_ln_job_t& j = jobs[i];
+    lj[i] = m3pc::LnJob{reinterpret_cast<const __nv_bfloat16*>(j.A), reinterpret_cast<const __nv_bfloat16*>(j.W), j.X,
+                        reinterpret_cast<__nv_bfloat16*>(j.Y), j.table, j.rows_per_group, j.M, j.R};
+  }
+  return m3pc::gemm_ln_bf16_grouped(lj, n, bias, gamma, beta, K, reinterpret_cast<cudaStream_t>(stream), out_kernel);
+}
+
 int m3pc_gemm_fp32(const float* A, const float* W, const float* bias, float* C, int32_t M, int32_t N, int32_t K, int32_t flags, void* stream) {
   M3PC_REQUIRE(A && W && C, "null argument");
   M3PC_REQUIRE((flags & ~7) == 0, "unknown flag");

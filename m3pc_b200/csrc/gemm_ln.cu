@@ -100,8 +100,11 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
   constexpr uint32_t ACC_COLS = LN_N / NACC;        // TMEM columns of one accumulator
   constexpr int NSHARE = ROWS == 128 ? 8 : 4;       // warps that share a row
   constexpr int WCOLS = LN_N / NSHARE;              // output columns per warp
-  // Row statistics are accumulated in a CANONICAL order that does not depend on ROWS: (sum, sum of squares) over each group of 64
-  // consecutive columns, ascending, then the eight groups added in column order -- so both unit sizes produce identical bits.
+  // Row statistics are accumulated in a CANONICAL order that does not depend on ROWS, so both unit sizes produce identical bits: each
+  // group ("slice") of 64 consecutive columns gets its sum and its sum of squared deviations from its own mean, built from its four
+  // 16-column chunks in ascending order (Chan et al.'s pairwise update), and the row's variance adds the eight slices' deviations in
+  // column order around the row mean.  Centred sums, which m3pc_layernorm and nn.LayerNorm use as well, keep the variance accurate for
+  // rows whose mean is large against their spread, where E[x^2] - mean^2 cancels catastrophically in fp32.
   constexpr int NSLICE = 8;
   using Pipe = TcPipeline<STAGES, NACC, ACC_COLS, 2, 2>;
   extern __shared__ uint8_t smem_raw[];
@@ -244,10 +247,22 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
             v[4 * j + 3] = __uint_as_float(r[4 * j + 3]) + b4.w + res.w;
             *slot = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
           }
+          {
+            float c1 = 0.f;
 #pragma unroll
-          for (int j = 0; j < 16; ++j) {
-            s1 += v[j];
-            s2 = fmaf(v[j], v[j], s2);
+            for (int j = 0; j < 16; ++j) c1 += v[j];
+            const float cm = c1 * (1.0f / 16);
+            float c2 = 0.f;
+#pragma unroll
+            for (int j = 0; j < 16; ++j) c2 = fmaf(v[j] - cm, v[j] - cm, c2);
+            // merge this chunk (16 columns, mean cm) into the k = ci & 3 chunks of the slice so far (16 k columns, sum s1):
+            // M2 += c2 + d^2 * 16 k / (k + 1), d = cm - s1 / (16 k); constants selected instead of divided
+            const int k = ci & 3;
+            const float inv_n = k == 1 ? 1.0f / 16 : (k == 2 ? 1.0f / 32 : 1.0f / 48);
+            const float wgt = k == 1 ? 8.0f : (k == 2 ? 32.0f / 3 : 12.0f);
+            const float d = cm - s1 * inv_n;
+            s2 += k == 0 ? c2 : fmaf(d * d, wgt, c2);
+            s1 += c1;
           }
           if ((ci & 3) == 3) {  // a 64-column group is complete
             sstats[(rowq * 32 + lane) * NSLICE + slice + (ci >> 2)] = make_float2(s1, s2);
@@ -277,16 +292,18 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
       named_bar_sync(1 + rowq, 32 * NSHARE);
       float mean, rstd;
       {
-        float t1 = 0.f, t2 = 0.f;
+        const float2* rs = sstats + (rowq * 32 + lane) * NSLICE;
+        float t1 = 0.f;
+#pragma unroll
+        for (int g = 0; g < NSLICE; ++g) t1 += rs[g].x;
+        mean = t1 * (1.0f / LN_N);
+        float t2 = 0.f;
 #pragma unroll
         for (int g = 0; g < NSLICE; ++g) {
-          const float2 pq = sstats[(rowq * 32 + lane) * NSLICE + g];
-          t1 += pq.x;
-          t2 += pq.y;
+          const float d = rs[g].x * (1.0f / 64) - mean;
+          t2 += rs[g].y + 64.0f * d * d;
         }
-        mean = t1 * (1.0f / LN_N);
-        const float var = fmaxf(t2 * (1.0f / LN_N) - mean * mean, 0.f);
-        rstd = rsqrtf(var + kLnEps);
+        rstd = rsqrtf(t2 * (1.0f / LN_N) + kLnEps);
       }
       named_bar_sync(1 + rowq, 32 * NSHARE);  // everybody has read the statistics: the next unit may overwrite them
       if (live) {
@@ -331,13 +348,15 @@ __global__ void __launch_bounds__(LN_THREADS, 1) gemm_ln_2sm_kernel(const __grid
 }
 
 template <int ROWS, int STAGES, int NBOX>
-int launch_ln(LnGemmParams& P, cudaStream_t st) {
+int launch_ln(LnGemmParams& P, cudaStream_t st, int* report) {
   using L = SmemLn<ROWS, STAGES, NBOX>;
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
   static_assert(L::kStoreOffset % 1024 == 0, "operand stages must keep 1024-byte alignment");
   static PerDevice<size_t> smem_limit;
   return launch_pair(gemm_ln_2sm_kernel<ROWS, STAGES, NBOX>, smem_limit, L::kTotal, LN_THREADS, P,
-                     [](const LnProblem& Q) { return ceil_div(Q.M, ROWS); }, [](int) {}, st);
+                     [](const LnProblem& Q) { return ceil_div(Q.M, ROWS); }, [&](int pairs) {
+                       if (report != nullptr) { report[0] = ROWS; report[1] = pairs; }
+                     }, st);
 }
 
 }  // namespace
@@ -349,10 +368,21 @@ int launch_ln(LnGemmParams& P, cudaStream_t st) {
 //              (measured at 106 496 rows: 125 us vs 135 us with 256-row units; profiles/r2g_gemm_ln_variants.txt)
 //   K  > 512   256-row units feed the tensor pipe with 1/3 less operand traffic per FLOP (238 vs 264 us) -- unless the launch is so
 //              small that whole 256-row units quantise badly on the 74 CTA pairs (26 624 rows: 104 units = 2 rounds, vs 3 half rounds)
-int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const float* gamma, const float* beta, int K, cudaStream_t st) {
+int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const float* gamma, const float* beta, int K, cudaStream_t st,
+                         int* report) {
   M3PC_REQUIRE(n >= 1 && n <= kMaxGroup, "gemm_ln: 1 .. kMaxGroup problems per launch");
   M3PC_REQUIRE(K > 0 && K % BK == 0, "gemm_ln: K must be a positive multiple of 64");
   M3PC_REQUIRE(gamma && beta, "gemm_ln: null operand");
+  for (int g = 0; g < n; ++g) {
+    const LnJob& j = jobs[g];
+    M3PC_REQUIRE(j.M > 0 && j.A && j.W && j.X && j.Y, "gemm_ln: null operand or empty problem");
+    M3PC_REQUIRE(((reinterpret_cast<uintptr_t>(j.A) | reinterpret_cast<uintptr_t>(j.W) | reinterpret_cast<uintptr_t>(j.X) | reinterpret_cast<uintptr_t>(j.Y)) & 15) == 0,
+                 "gemm_ln: operands must be 16-byte aligned");
+    M3PC_REQUIRE(j.R == nullptr || j.table == nullptr, "gemm_ln: a residual source excludes a table");
+    // the epilogue reads table rows with 16-byte loads
+    M3PC_REQUIRE(((reinterpret_cast<uintptr_t>(j.R) | reinterpret_cast<uintptr_t>(j.table)) & 15) == 0, "gemm_ln: R and table must be 16-byte aligned");
+    M3PC_REQUIRE(j.rows_per_group >= 1, "gemm_ln: rows_per_group must be at least 1");
+  }
   M3PC_TRY(gemm_init_driver_api());
   int rows = g_ln_unit_rows;
   if (rows != 128 && rows != 256) {
@@ -370,23 +400,18 @@ int gemm_ln_bf16_grouped(const LnJob* jobs, int n, const float* bias, const floa
   for (int g = 0; g < n; ++g) {
     const LnJob& j = jobs[g];
     LnProblem& Q = P.p[g];
-    M3PC_REQUIRE(j.M > 0 && j.A && j.W && j.X && j.Y, "gemm_ln: null operand or empty problem");
-    M3PC_REQUIRE(((reinterpret_cast<uintptr_t>(j.A) | reinterpret_cast<uintptr_t>(j.W) | reinterpret_cast<uintptr_t>(j.X) | reinterpret_cast<uintptr_t>(j.Y)) & 15) == 0,
-                 "gemm_ln: operands must be 16-byte aligned");
-    M3PC_REQUIRE(j.R == nullptr || (j.table == nullptr && (reinterpret_cast<uintptr_t>(j.R) & 15) == 0),
-                 "gemm_ln: a residual source excludes a table and must be 16-byte aligned");
     M3PC_TRY(make_tmap(&Q.ta, j.A, static_cast<uint64_t>(j.M), static_cast<uint64_t>(K), rows / 2));
     M3PC_TRY(make_tmap(&Q.tw, j.W, static_cast<uint64_t>(LN_N), static_cast<uint64_t>(K), 128));
     M3PC_TRY(make_tmap_out(&Q.tx, j.X, static_cast<uint64_t>(j.M), LN_N, true));
     M3PC_TRY(make_tmap_out(&Q.tr, const_cast<float*>(j.R != nullptr ? j.R : j.X), static_cast<uint64_t>(j.M), LN_N, true));
     M3PC_TRY(make_tmap_out(&Q.ty, j.Y, static_cast<uint64_t>(j.M), LN_N, false));
     Q.table = j.table;
-    Q.rows_per_group = j.rows_per_group > 0 ? j.rows_per_group : 1;
+    Q.rows_per_group = j.rows_per_group;
     Q.M = j.M;
   }
   P.bias = bias; P.gamma = gamma; P.beta = beta;
   P.num_kb = K / BK;
-  return rows == 128 ? launch_ln<128, 3, 2>(P, st) : launch_ln<256, 3, 2>(P, st);
+  return rows == 128 ? launch_ln<128, 3, 2>(P, st, report) : launch_ln<256, 3, 2>(P, st, report);
 }
 
 }  // namespace m3pc

@@ -481,7 +481,7 @@ int make_tmap_f32(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t col
 namespace {
 
 template <int BN, int STAGES, int CL>
-int launch(const GemmProblem& q, cudaStream_t st) {
+int launch(const GemmProblem& q, cudaStream_t st, int* report) {
   using L = SmemLayout<BN, STAGES>;
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
   static PerDevice<size_t> smem_limit;
@@ -495,6 +495,7 @@ int launch(const GemmProblem& q, cudaStream_t st) {
   M3PC_CHECK_CUDA(launch_k_cluster(CL, gemm_bf16_kernel<BN, STAGES, CL>, dim3(clusters * CL), dim3(GEMM_THREADS), L::kTotal, st, ta, tw, q.C,
                                    q.M, q.N, q.K, ep));
   M3PC_CHECK_LAUNCH();
+  if (report != nullptr) { report[0] = 1; report[1] = BN; report[2] = CL; }
   return M3PC_OK;
 }
 
@@ -519,7 +520,7 @@ namespace {
 
 // One launch of the CTA-pair kernel over `n` problems (n <= kMaxGroup; every N a multiple of 256).
 template <int STAGES>
-int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
+int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st, int* report) {
   using L = Smem2<STAGES>;
   static_assert(L::kTotal <= 227 * 1024, "shared memory budget exceeded");
   static_assert(sizeof(GroupParams) <= 4000, "kernel parameter space");
@@ -541,11 +542,15 @@ int launch_2sm(const GemmProblem* probs, int n, cudaStream_t st) {
     P.n_tiles = q.N / 256;
     P.num_kb = q.K / BK;
   }
-  return launch_pair(gemm_bf16_2sm_kernel<STAGES>, smem_limit, L::kTotal, GEMM_THREADS_2SM, gp,
-                     [](const GroupProblem& P) { return P.n_tiles * ceil_div(P.M, 2 * BM); },
-                     [&](int pairs) {
-                       gp.strided = n == 1 && gp.p[0].n_tiles == 2 && probs[0].K >= 1024 && pairs % 2 == 0 && gp.n_units >= 2 * pairs;
-                     }, st);
+  M3PC_TRY(launch_pair(gemm_bf16_2sm_kernel<STAGES>, smem_limit, L::kTotal, GEMM_THREADS_2SM, gp,
+                       [](const GroupProblem& P) { return P.n_tiles * ceil_div(P.M, 2 * BM); },
+                       [&](int pairs) {
+                         gp.strided = n == 1 && gp.p[0].n_tiles == 2 && probs[0].K >= 1024 && pairs % 2 == 0 && gp.n_units >= 2 * pairs;
+                       }, st));
+  for (int g = 0; report != nullptr && g < n; ++g) {
+    report[4 * g] = 2; report[4 * g + 1] = gp.strided; report[4 * g + 2] = n;
+  }
+  return M3PC_OK;
 }
 
 // Modelled time of one configuration: the slower of the tensor pipe (rounds of the persistent grid x MMA cycles per tile)
@@ -563,9 +568,12 @@ double model_time(int M, int N, int K, int bn, int cl) {
 
 // One problem in a launch of its own: the skinny kernel for a few rows, the CTA-pair kernel wherever a pair has two row tiles to
 // work on and N splits into 256-wide tiles, else the single-CTA kernel.
-int gemm_bf16_one(const GemmProblem& q, cudaStream_t st) {
-  if (q.M <= 32 && static_cast<size_t>(q.M) * q.K * 2 <= 160 * 1024) return gemm_bf16_skinny(q.A, q.W, q.C, q.M, q.N, q.K, q.epi, st);
-  if (q.N % 256 == 0 && q.M > BM) return launch_2sm<4>(&q, 1, st);
+int gemm_bf16_one(const GemmProblem& q, cudaStream_t st, int* report) {
+  if (q.M <= 32 && static_cast<size_t>(q.M) * q.K * 2 <= 160 * 1024) {
+    if (report != nullptr) { report[0] = 0; report[1] = 0; report[2] = 0; }
+    return gemm_bf16_skinny(q.A, q.W, q.C, q.M, q.N, q.K, q.epi, st);
+  }
+  if (q.N % 256 == 0 && q.M > BM) return launch_2sm<4>(&q, 1, st, report);
   // pick tile width and cluster size by the modelled time (ties: wider tile, larger cluster = less L2 traffic)
   struct Cand { int bn, cl; } cands[] = {{256, 2}, {256, 1}, {128, 2}, {128, 1}};
   int best = -1;
@@ -576,10 +584,10 @@ int gemm_bf16_one(const GemmProblem& q, cudaStream_t st) {
     if (t < best_t * 0.98) { best_t = t; best = i; }
   }
   switch (best) {
-    case 0: return launch<256, 3, 2>(q, st);
-    case 1: return launch<256, 3, 1>(q, st);
-    case 2: return launch<128, 4, 2>(q, st);
-    default: return launch<128, 4, 1>(q, st);
+    case 0: return launch<256, 3, 2>(q, st, report);
+    case 1: return launch<256, 3, 1>(q, st, report);
+    case 2: return launch<128, 4, 2>(q, st, report);
+    default: return launch<128, 4, 1>(q, st, report);
   }
 }
 
@@ -600,19 +608,30 @@ int gemm_init_driver_api() {
 
 // Problems are taken kMaxGroup at a time.  Several problems whose N all split into 256-wide tiles share one CTA-pair launch (small
 // ones included) once one of them gives a pair two row tiles to work on (see GroupParams); otherwise each problem gets its own.
-int gemm_bf16(const GemmProblem* probs, int n, cudaStream_t st) {
+// Every argument is checked before the first CUDA call: a bias or table the epilogues read with vector loads must be 16-byte aligned.
+int gemm_bf16(const GemmProblem* probs, int n, cudaStream_t st, int* report) {
   M3PC_REQUIRE(n >= 1, "gemm_bf16: no problems");
   for (int g = 0; g < n; ++g) {
     const GemmProblem& q = probs[g];
+    const GemmEpilogue& ep = q.epi;
     M3PC_REQUIRE(q.M > 0 && q.N > 0 && q.K > 0, "gemm_bf16: empty problem");
     M3PC_REQUIRE(q.K % BK == 0, "gemm_bf16: K must be a multiple of 64");
     M3PC_REQUIRE(q.N % 128 == 0, "gemm_bf16: N must be a multiple of 128");
     M3PC_REQUIRE(((reinterpret_cast<uintptr_t>(q.A) | reinterpret_cast<uintptr_t>(q.W) | reinterpret_cast<uintptr_t>(q.C)) & 15) == 0,
                  "gemm_bf16: operands must be 16-byte aligned");
+    M3PC_REQUIRE((ep.flags & ~(EPI_GELU | EPI_RESIDUAL | EPI_RELU | EPI_ROWTABLE | EPI_OUT_F32)) == 0, "gemm_bf16: unknown flag");
+    M3PC_REQUIRE((ep.table != nullptr) == ((ep.flags & EPI_ROWTABLE) != 0), "gemm_bf16: a table goes with EPI_ROWTABLE and only with it");
+    M3PC_REQUIRE((ep.flags & (EPI_ROWTABLE | EPI_RESIDUAL)) != (EPI_ROWTABLE | EPI_RESIDUAL),
+                 "gemm_bf16: a row table and the in-place residual exclude each other");
+    M3PC_REQUIRE(ep.rows_per_group >= 1, "gemm_bf16: rows_per_group must be at least 1");
+    M3PC_REQUIRE(((reinterpret_cast<uintptr_t>(ep.bias) | reinterpret_cast<uintptr_t>(ep.table)) & 15) == 0,
+                 "gemm_bf16: bias and table must be 16-byte aligned");
   }
   M3PC_TRY(gemm_init_driver_api());
+  int launches = 0;
   for (int i0 = 0; i0 < n; i0 += kMaxGroup) {
     const GemmProblem* group = probs + i0;
+    int* rep = report != nullptr ? report + 4 * i0 : nullptr;
     const int m = std::min(kMaxGroup, n - i0);
     bool pair = m > 1;
     int max_m = 0;
@@ -621,9 +640,14 @@ int gemm_bf16(const GemmProblem* probs, int n, cudaStream_t st) {
       max_m = std::max(max_m, group[g].M);
     }
     if (pair && max_m > BM) {
-      M3PC_TRY(launch_2sm<4>(group, m, st));
+      M3PC_TRY(launch_2sm<4>(group, m, st, rep));
+      for (int g = 0; rep != nullptr && g < m; ++g) rep[4 * g + 3] = launches;
+      ++launches;
     } else {
-      for (int g = 0; g < m; ++g) M3PC_TRY(gemm_bf16_one(group[g], st));
+      for (int g = 0; g < m; ++g, ++launches) {
+        M3PC_TRY(gemm_bf16_one(group[g], st, rep != nullptr ? rep + 4 * g : nullptr));
+        if (rep != nullptr) rep[4 * g + 3] = launches;
+      }
     }
   }
   return M3PC_OK;

@@ -96,3 +96,82 @@ def test_product_never_imports_the_oracle():
             if f.endswith((".py", ".cu", ".cuh", ".h")):
                 txt = open(os.path.join(dirpath, f)).read()
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", txt, flags=re.M), f"{f} imports the oracle"
+
+
+def test_gemm_entry_structs_match_header():
+    assert C.sizeof(nat.GemmProblem) == 5 * 8 + 5 * 4 + 4  # padded to pointer alignment
+    assert C.sizeof(nat.LnJob) == 6 * 8 + 2 * 4
+    src = open(os.path.join(ROOT, "include", "m3pc.h")).read()
+    defs = dict(re.findall(r"#define\s+(M3PC_EPI_[A-Z0-9_]+)\s+(\d+)", src))
+    assert {k: int(v) for k, v in defs.items()} == {"M3PC_EPI_GELU": nat.EPI_GELU, "M3PC_EPI_RESIDUAL": nat.EPI_RESIDUAL, "M3PC_EPI_RELU": nat.EPI_RELU,
+                                                    "M3PC_EPI_ROWTABLE": nat.EPI_ROWTABLE, "M3PC_EPI_OUT_F32": nat.EPI_OUT_F32}
+
+
+# Pointer values below are never dereferenced: every rule is checked before the first CUDA call, so these run without a GPU.
+A16, W16, C16, T16, B16 = 0x10000, 0x20000, 0x30000, 0x40000, 0x50000
+
+
+def _gemm_rc(lib, n=1, **kw):
+    f = dict(A=A16, W=W16, bias=B16, table=None, C=C16, M=256, N=512, K=512, rows_per_group=1, flags=0)
+    f.update(kw)
+    arr = (nat.GemmProblem * max(n, 1))(*[nat.GemmProblem(**f)] * max(n, 1))
+    return lib.m3pc_gemm_bf16_problems(arr, n, None, None)
+
+
+@pytest.mark.parametrize("kw,msg", [
+    (dict(bias=B16 + 4), b"16-byte aligned"),                              # a bias slice at a 4-byte offset (float4 / float2 loads)
+    (dict(bias=B16 + 8), b"16-byte aligned"),
+    (dict(table=T16 + 4, flags=nat.EPI_ROWTABLE), b"16-byte aligned"),
+    (dict(table=T16), b"EPI_ROWTABLE"),                                     # a table without the flag
+    (dict(flags=nat.EPI_ROWTABLE), b"EPI_ROWTABLE"),                        # the flag without a table
+    (dict(table=T16, flags=nat.EPI_ROWTABLE, rows_per_group=0), b"rows_per_group"),
+    (dict(rows_per_group=-3), b"rows_per_group"),
+    (dict(table=T16, flags=nat.EPI_ROWTABLE | nat.EPI_RESIDUAL), b"exclude"),  # two residual sources
+    (dict(flags=32), b"unknown flag"),
+    (dict(C=C16 + 2), b"16-byte aligned"),
+    (dict(K=100), b"multiple of 64"),
+    (dict(N=200), b"multiple of 128"),
+    (dict(A=None), b"null"),
+])
+def test_gemm_bf16_problems_rejects_without_a_gpu(lib, kw, msg):
+    assert _gemm_rc(lib, **kw) == -1
+    assert msg in lib.m3pc_last_error(), lib.m3pc_last_error()
+
+
+def test_gemm_entries_reject_misaligned_bias_and_table_without_a_gpu(lib):
+    assert _gemm_rc(lib, n=0) == -1 and _gemm_rc(lib, n=65) == -1
+    assert lib.m3pc_gemm_bf16_problems(None, 1, None, None) == -1
+    # the older entries share the dispatcher's checks
+    assert lib.m3pc_gemm_bf16(A16, W16, B16 + 4, C16, 256, 512, 512, 0, None) == -1
+    assert b"16-byte aligned" in lib.m3pc_last_error()
+    bias = (C.c_void_p * 2)(B16, B16 + 4)
+    ptrs = lambda v: (C.c_void_p * 2)(v, v)
+    i32 = lambda *xs: (C.c_int32 * 2)(*xs)
+    assert lib.m3pc_gemm_bf16_grouped(2, ptrs(A16), ptrs(W16), bias, ptrs(C16), i32(256, 256), i32(512, 512), i32(512, 512), i32(0, 0), None) == -1
+    assert lib.m3pc_gemm_ln_bf16(A16, W16, B16, C16, C16 + 0x100000, B16, B16, T16 + 4, 8, 256, 512, None) == -1
+    assert b"16-byte aligned" in lib.m3pc_last_error()
+
+
+def _ln_rc(lib, n=1, K=512, gamma=B16, **kw):
+    f = dict(A=A16, W=W16, X=C16, Y=C16 + 0x100000, table=None, R=None, rows_per_group=1, M=256)
+    f.update(kw)
+    arr = (nat.LnJob * max(n, 1))(*[nat.LnJob(**f)] * max(n, 1))
+    return lib.m3pc_gemm_ln_bf16_grouped(arr, n, B16, gamma, B16, K, None, None)
+
+
+@pytest.mark.parametrize("kw,msg", [
+    (dict(table=T16 + 4, rows_per_group=8), b"16-byte aligned"),
+    (dict(R=T16 + 8), b"16-byte aligned"),
+    (dict(table=T16, R=T16 + 0x1000), b"excludes"),
+    (dict(table=T16, rows_per_group=0), b"rows_per_group"),
+    (dict(rows_per_group=0), b"rows_per_group"),
+    (dict(n=0), b"1 .. 4"),
+    (dict(n=5), b"1 .. 4"),
+    (dict(K=96), b"multiple of 64"),
+    (dict(gamma=None), b"null"),
+    (dict(Y=C16 + 2), b"16-byte aligned"),
+    (dict(M=0), b"empty"),
+])
+def test_gemm_ln_bf16_grouped_rejects_without_a_gpu(lib, kw, msg):
+    assert _ln_rc(lib, **kw) == -1
+    assert msg in lib.m3pc_last_error(), lib.m3pc_last_error()
