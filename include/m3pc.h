@@ -202,7 +202,8 @@ int m3pc_exchange_status(m3pc_handle_t h, uint64_t* out_epoch, uint64_t* out_fai
 int m3pc_merge_partials(m3pc_handle_t h, const float* partials, int32_t n_shards, float temperature,
                         float* out_eval_action, float* out_sample_action, int32_t* out_indices, void* stream);
 
-/* Zero-shot backward planners on E lock-step environments (zeroshot_omtm/learner.py:60-261).
+/* Zero-shot backward planners on E lock-step environments (zeroshot_omtm/learner.py:60-261); m3pc_backward_plan_env below plans
+ * environments at different points of their episodes.
  *   mode 0 = action_id_sample (one pass, gid mask); 1 = action_piid_sample (pi mask -> fill states -> fid mask).
  *   win_* as in m3pc_plan_args_t but with a leading E axis: (E,T,obs) etc.; eps (E,A) or NULL (mean only).
  *   out_eval_action / out_sample_action: device (E,A). */
@@ -222,6 +223,21 @@ int m3pc_backward_plan_draws(m3pc_handle_t h, int32_t mode, int32_t n_env, int32
                              const float* win_actions, const float* win_rewards, const float* win_returns_tok, const float* eps,
                              uint64_t seed, float* out_eval_action, float* out_sample_actions, void* stream);
 
+/* m3pc_backward_plan_draws with one planning horizon per environment (learner.py:342-345 clamps the horizon of an environment in
+ * its first T - h steps), the semantics of m3pc_plan_args_t.env_horizons:
+ *   env_horizons  HOST (n_env), each in [1, traj_length]; n_env <= 256 (and <= cfg.max_batch).  M3PC_ERR_INVALID otherwise, before
+ *                 any launch.
+ *   eps           device (E, C, A) injected N(0,1) noise or NULL (Philox keyed by (seed, environment, draw)); out_sample_actions
+ *                 device (E, C, A), (E, A) for C = 1; out_eval_action device (E, A).
+ * All entries equal: exactly m3pc_backward_plan_draws at that horizon.  Otherwise the environments are split into horizon classes:
+ * one launch gathers their windows, then each class runs the uniform sequence at n_env = E_c on its windows, so each class computes
+ * bit for bit what the uniform call on its windows (and its eps rows) computes.  Outputs land in the caller's rows and Philox is keyed
+ * by the caller's environment index, so an environment's draws do not depend on the other environments of the call.  The
+ * end-of-waypoints clamp (p + h > 1000) changes window contents only and needs no class of its own. */
+int m3pc_backward_plan_env(m3pc_handle_t h, int32_t mode, int32_t n_env, const int32_t* env_horizons, int32_t n_draws, const float* win_states,
+                           const float* win_actions, const float* win_rewards, const float* win_returns_tok, const float* eps, uint64_t seed,
+                           float* out_eval_action, float* out_sample_actions, void* stream);
+
 /* Device-resident episode histories of n_env environment slots (SURVEY.md section 8f rank 1): what the reference keeps as
  * `current_trajectory` numpy arrays (replay_buffer.py:192-205, learner.py:663-675) and re-slices on the host every step
  * (learner.py:346-366).  Each step uploads n*(obs+act+1) floats instead of n windows.
@@ -233,6 +249,11 @@ int m3pc_backward_plan_draws(m3pc_handle_t h, int32_t mode, int32_t n_env, int32
  *                            actions / rewards of the previous episode would show up in the windows of the next.
  *   m3pc_ring_append_slots   listed slot k = slots[k] writes obs row k at step t[slot] and (when non-NULL) prev_action row k /
  *                            prev_reward[k] at step t[slot] - 1; a slot with t outside [0, ring_len) writes nothing.
+ *   m3pc_ring_write_obs      writes only the observation columns of rows [first_row, first_row + n_rows) of each listed slot from
+ *                            obs_rows (device (n_slots, n_rows, obs)): the waypoint table of a zero-shot episode
+ *                            (zeroshot_omtm/learner.py:75-79), stored once after m3pc_ring_reset.  The appends that follow overwrite
+ *                            rows 0 .. path_length with the observations of the episode, so windows with future_obs see what the
+ *                            host builder sees on a history whose observations array holds the waypoints.
  *   m3pc_ring_windows_slots  window k of the (n_slots, T, .) planner windows is slot s = slots[k] at step p = path_length[s] with
  *                            horizon h = horizons[k] (HOST list, in [1, T]), exactly as learner.py:346-366 builds it: the states,
  *                            actions and rewards of steps p-T+h .. p (the last T-h+1 steps, zero where before step 0), zero padded
@@ -244,6 +265,8 @@ int m3pc_ring_reset(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_di
                     void* stream);
 int m3pc_ring_append_slots(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* t, const int32_t* slots,
                            int32_t n_slots, const float* obs, const float* prev_action, const float* prev_reward, void* stream);
+int m3pc_ring_write_obs(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* slots, int32_t n_slots,
+                        int32_t first_row, int32_t n_rows, const float* obs_rows, void* stream);
 int m3pc_ring_windows_slots(const float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* path_length,
                             const int32_t* slots, const int32_t* horizons, int32_t n_slots, int32_t traj_length, int32_t future_obs,
                             const float* rtg_tok, float* win_states, float* win_actions, float* win_rewards, float* win_returns_tok,

@@ -32,7 +32,7 @@ GUIDANCE = {
 SYMBOLS = (
     "m3pc_last_error", "m3pc_version", "m3pc_create", "m3pc_destroy", "m3pc_set_param", "m3pc_finalize_params", "m3pc_set_option",
     "m3pc_forward", "m3pc_plan", "m3pc_merge_partials", "m3pc_exchange_local", "m3pc_exchange_connect", "m3pc_exchange_status", "m3pc_backward_plan", "m3pc_backward_plan_draws",
-    "m3pc_ring_reset", "m3pc_ring_append_slots", "m3pc_ring_windows_slots", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16",
+    "m3pc_backward_plan_env", "m3pc_ring_reset", "m3pc_ring_append_slots", "m3pc_ring_write_obs", "m3pc_ring_windows_slots", "m3pc_gemm_bf16", "m3pc_gemm_bf16_grouped", "m3pc_gemm_ln_bf16",
     "m3pc_gemm_bf16_problems", "m3pc_gemm_ln_bf16_grouped", "m3pc_gemm_fp32", "m3pc_gemm_tf32x3",
     "m3pc_layernorm", "m3pc_attention", "m3pc_attention_gather", "m3pc_embed_gather", "m3pc_decoder_scatter_embed", "m3pc_block_forward", "m3pc_heads", "m3pc_sample_candidates", "m3pc_twinq",
     "m3pc_score_select", "m3pc_last_device_ms", "m3pc_last_launch_count", "m3pc_set_profile", "m3pc_get_profile",
@@ -125,6 +125,8 @@ def lib() -> C.CDLL:
     L.m3pc_exchange_status.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     L.m3pc_backward_plan.argtypes = [vp, i32, i32, i32, f32p, f32p, f32p, f32p, f32p, f32p, f32p, f32p, vp]
     L.m3pc_backward_plan_draws.argtypes = [vp, i32, i32, i32, i32, f32p, f32p, f32p, f32p, f32p, C.c_uint64, f32p, f32p, vp]
+    L.m3pc_backward_plan_env.argtypes = [vp, i32, i32, vp, i32, f32p, f32p, f32p, f32p, f32p, C.c_uint64, f32p, f32p, vp]
+    L.m3pc_ring_write_obs.argtypes = [f32p, i32, i32, i32, i32, vp, i32, i32, i32, f32p, vp]
     L.m3pc_ring_reset.argtypes = [f32p, i32, i32, i32, i32, vp, i32, vp]
     L.m3pc_ring_append_slots.argtypes = [f32p, i32, i32, i32, i32, vp, vp, i32, f32p, f32p, f32p, vp]
     L.m3pc_ring_windows_slots.argtypes = [f32p, i32, i32, i32, i32, vp, vp, vp, i32, i32, i32, f32p, f32p, f32p, f32p, f32p, vp]

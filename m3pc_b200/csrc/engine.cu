@@ -1294,6 +1294,21 @@ struct MixPlan {
   short src[MIX_MAX_ENV] = {};
 };
 
+// Splits E <= MIX_MAX_ENV environments with horizons hz[i] in [1, T] into their classes.
+void horizon_classes(const int32_t* hz, int E, int T, MixPlan& m) {
+  int n = 0;
+  for (int hh = 1; hh <= T; ++hh) {
+    const int start = n;
+    for (int i = 0; i < E; ++i)
+      if (hz[i] == hh) m.src[n++] = static_cast<short>(i);
+    if (n > start) {
+      m.h[m.n_class] = hh;
+      m.off[m.n_class++] = start;
+    }
+  }
+  m.off[m.n_class] = n;
+}
+
 // Validates env_horizons.  *mixed is false when it is null or all its entries are equal: the plan is then exactly the uniform one.
 int mix_classes(const m3pc_engine* e, const m3pc_plan_args_t* a, MixPlan& m, bool* mixed) {
   *mixed = false;
@@ -1312,17 +1327,7 @@ int mix_classes(const m3pc_engine* e, const m3pc_plan_args_t* a, MixPlan& m, boo
   M3PC_REQUIRE(a->horizon == hmax, "with env_horizons, horizon must equal its largest entry");
   if (equal) return M3PC_OK;
   M3PC_REQUIRE(E <= MIX_MAX_ENV, "env_horizons: more environments than one mixed plan takes (256)");
-  int n = 0;
-  for (int hh = 1; hh <= e->T; ++hh) {
-    const int start = n;
-    for (int i = 0; i < E; ++i)
-      if (a->env_horizons[i] == hh) m.src[n++] = static_cast<short>(i);
-    if (n > start) {
-      m.h[m.n_class] = hh;
-      m.off[m.n_class++] = start;
-    }
-  }
-  m.off[m.n_class] = n;
+  horizon_classes(a->env_horizons, E, e->T, m);
   *mixed = true;
   return M3PC_OK;
 }
@@ -1444,9 +1449,11 @@ int plan(m3pc_engine* e, const m3pc_plan_args_t* args, cudaStream_t st) {
   return M3PC_OK;
 }
 
+// env_id: null, or the device id table of a horizon class planned by backward_plan_env (local environment -> the caller's index):
+// outputs go to the caller's rows, Philox is keyed by the caller's index and eps is read from the caller's rows in place
 int backward_plan(m3pc_engine* e, int mode, int E, int h, const float* ws, const float* wa, const float* wr, const float* wrt,
                   const float* eps, float* out_eval, float* out_sample, float* dbg_filled, cudaStream_t st, int n_draws = 1,
-                  unsigned long long seed = 0ull) {
+                  unsigned long long seed = 0ull, const int* env_id = nullptr) {
   M3PC_REQUIRE(e->finalized, "backward_plan before m3pc_finalize_params");
   const int T = e->T, idx = T - h, A = e->act;
   M3PC_REQUIRE(mode == 0 || mode == 1, "mode must be 0 (id) or 1 (piid)");
@@ -1485,7 +1492,43 @@ int backward_plan(m3pc_engine* e, int mode, int E, int h, const float* ws, const
     io2.need_nt[M3PC_ACTIONS] = 1;
     M3PC_TRY(forward(e, io2, E, st));
   }
-  return launch_sampling_tail(e->e_mu.as<float>(), e->e_std.as<float>(), eps, T, h, A, E, out_eval, out_sample, seed, nullptr, st, n_draws);
+  return launch_sampling_tail(e->e_mu.as<float>(), e->e_std.as<float>(), eps, T, h, A, E, out_eval, out_sample, seed, nullptr, st, n_draws,
+                              env_id, env_id != nullptr);
+}
+
+// m3pc_backward_plan_env: one horizon per environment.  All equal: exactly the uniform call.  Otherwise one gather launch puts every
+// horizon class's windows side by side, then backward_plan runs once per class at n_env = E_c on its contiguous windows with the
+// class's id table.  The injected eps (E, C, A) is not gathered: it depends on no horizon, and E * C rows can exceed the gather buffer.
+int backward_plan_env(m3pc_engine* e, int mode, int E, const int32_t* hz, int n_draws, const float* ws, const float* wa, const float* wr,
+                      const float* wt, const float* eps, unsigned long long seed, float* out_eval, float* out_sample, cudaStream_t st) {
+  M3PC_REQUIRE(e->finalized, "backward_plan before m3pc_finalize_params");
+  M3PC_REQUIRE(mode == 0 || mode == 1, "mode must be 0 (id) or 1 (piid)");
+  M3PC_REQUIRE(E >= 1 && E <= MIX_MAX_ENV && E <= e->cfg.max_batch, "n_env must be in [1, min(256, cfg.max_batch)]");
+  bool equal = true;
+  for (int i = 0; i < E; ++i) {
+    M3PC_REQUIRE(hz[i] >= 1 && hz[i] <= e->T, "env_horizons entries must be in [1, traj_length]");
+    equal = equal && hz[i] == hz[0];
+  }
+  if (equal) return backward_plan(e, mode, E, hz[0], ws, wa, wr, wt, eps, out_eval, out_sample, nullptr, st, n_draws, seed);
+  MixPlan m;
+  horizon_classes(hz, E, e->T, m);
+  const int T = e->T, A = e->act;
+  MixGatherParams g{};
+  g.ws = ws; g.wa = wa; g.wr = wr; g.wt = wt;
+  g.gs = e->mix_ws.as<float>(); g.ga = e->mix_wa.as<float>(); g.gr = e->mix_wr.as<float>(); g.gt = e->mix_wt.as<float>();
+  g.env_id = e->mix_id.as<int>();
+  g.E = E; g.T = T; g.obs = e->obs; g.A = A;
+  for (int s = 0; s < E; ++s) {
+    g.src[s] = m.src[s];
+    g.slot_of[m.src[s]] = static_cast<short>(s);
+  }
+  M3PC_TRY(launch_mix_gather(g, st));
+  for (int c = 0; c < m.n_class; ++c) {
+    const size_t off = m.off[c];
+    M3PC_TRY(backward_plan(e, mode, m.off[c + 1] - m.off[c], m.h[c], g.gs + off * T * e->obs, g.ga + off * T * A, g.gr + off * T, g.gt + off * T,
+                           eps, out_eval, out_sample, nullptr, st, n_draws, seed, g.env_id + off));
+  }
+  return M3PC_OK;
 }
 
 int create(m3pc_handle_t* out, const m3pc_config_t* cfg) {
@@ -1750,6 +1793,19 @@ int m3pc_backward_plan_draws(m3pc_handle_t h, int32_t mode, int32_t n_env, int32
   });
 }
 
+int m3pc_backward_plan_env(m3pc_handle_t h, int32_t mode, int32_t n_env, const int32_t* env_horizons, int32_t n_draws, const float* win_states,
+                           const float* win_actions, const float* win_rewards, const float* win_returns_tok, const float* eps, uint64_t seed,
+                           float* out_eval_action, float* out_sample_actions, void* stream) {
+  M3PC_REQUIRE(h != nullptr && env_horizons && win_states && win_actions && win_rewards && win_returns_tok && out_eval_action && out_sample_actions,
+               "null argument");
+  M3PC_REQUIRE(n_draws >= 1 && n_draws <= (1 << 20), "n_draws out of range");
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  return m3pc::timed(h, st, [&] {
+    return m3pc::backward_plan_env(h, mode, n_env, env_horizons, n_draws, win_states, win_actions, win_rewards, win_returns_tok, eps, seed,
+                                   out_eval_action, out_sample_actions, st);
+  });
+}
+
 int m3pc_ring_reset(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* slots, int32_t n_slots,
                     void* stream) {
   return m3pc::launch_ring_reset(ring, n_env, ring_len, obs_dim, act_dim, slots, n_slots, reinterpret_cast<cudaStream_t>(stream));
@@ -1759,6 +1815,12 @@ int m3pc_ring_append_slots(float* ring, int32_t n_env, int32_t ring_len, int32_t
                            int32_t n_slots, const float* obs, const float* prev_action, const float* prev_reward, void* stream) {
   return m3pc::launch_ring_append_slots(ring, n_env, ring_len, obs_dim, act_dim, t, slots, n_slots, obs, prev_action, prev_reward,
                                         reinterpret_cast<cudaStream_t>(stream));
+}
+
+int m3pc_ring_write_obs(float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* slots, int32_t n_slots,
+                        int32_t first_row, int32_t n_rows, const float* obs_rows, void* stream) {
+  return m3pc::launch_ring_write_obs(ring, n_env, ring_len, obs_dim, act_dim, slots, n_slots, first_row, n_rows, obs_rows,
+                                     reinterpret_cast<cudaStream_t>(stream));
 }
 
 int m3pc_ring_windows_slots(const float* ring, int32_t n_env, int32_t ring_len, int32_t obs_dim, int32_t act_dim, const int32_t* path_length,

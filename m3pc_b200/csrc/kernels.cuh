@@ -234,9 +234,10 @@ int launch_merge(const float* partials, int n_shards, int A, float temperature, 
 // mtm_sampling tail (learner.py:103-115): eval = tanh(mu[T-h]), sample = tanh(mu[T-h] + std[T-h]*eps)
 // C > 1: C draws per environment, sample_action is (E, C, A) and eps (E, C, A)
 // env_id (E) or null: as CandParams::env_id (Philox keyed by, and outputs written to, the caller's environment index)
+// eps_at_env_id (needs env_id): eps is the caller's (E_caller, C, A) noise, read at the row of env_id[e] instead of row e
 int launch_sampling_tail(const float* mu, const float* std, const float* eps, int T, int h, int A, int E, float* eval_action,
                          float* sample_action, unsigned long long seed, const unsigned long long* seed_ptr, cudaStream_t st, int C = 1,
-                         const int* env_id = nullptr);
+                         const int* env_id = nullptr, bool eps_at_env_id = false);
 
 // ---- m3pc_plan with one horizon per environment: the environments of one horizon class are planned as one uniform sub-plan on
 // contiguous copies of their inputs.  One launch gathers every class at once (classes are disjoint, so nothing is overwritten
@@ -267,6 +268,8 @@ int launch_piid_fill(const float* win_states, const float* states_pred, const fl
 int launch_ring_reset(float* ring, int E, int L, int obs, int act, const int* slots, int n, cudaStream_t st);
 int launch_ring_append_slots(float* ring, int E, int L, int obs, int act, const int* t, const int* slots, int n, const float* o, const float* pa,
                              const float* pr, cudaStream_t st);
+int launch_ring_write_obs(float* ring, int E, int L, int obs, int act, const int* slots, int n, int first, int n_rows, const float* rows,
+                          cudaStream_t st);
 int launch_ring_windows_slots(const float* ring, int E, int L, int obs, int act, const int* pl, const int* slots, const int* horizons, int n,
                               int T, int future_obs, const float* rtg_tok, float* ws, float* wa, float* wr, float* wt, cudaStream_t st);
 

@@ -363,7 +363,7 @@ __global__ void set_seed_kernel(unsigned long long* dst, unsigned long long seed
 // C draws per environment: i = (e * C + c) * A + a.  C = 1 is the reference's single draw (zeroshot_omtm/learner.py:136-147).
 __global__ void sampling_tail_kernel(const float* __restrict__ mu, const float* __restrict__ std, const float* __restrict__ eps, int T, int h,
                                      int A, int E, int C, float* eval_action, float* sample_action, unsigned long long seed,
-                                     const unsigned long long* seed_ptr, const int* __restrict__ env_id) {
+                                     const unsigned long long* seed_ptr, const int* __restrict__ env_id, bool eps_at_env_id) {
   PDL_PROLOGUE();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= E * C * A) return;
@@ -372,7 +372,8 @@ __global__ void sampling_tail_kernel(const float* __restrict__ mu, const float* 
   const int oe = env_id ? env_id[e] : e;  // the caller's row of environment e
   const size_t src = (static_cast<size_t>(e) * T + (T - h)) * A + a;
   const float m = mu[src];
-  const float z = eps ? eps[i] : philox_normal(seed, static_cast<unsigned>(oe), static_cast<unsigned>(c * A + a), 2u);
+  const size_t ei = eps_at_env_id ? (static_cast<size_t>(oe) * C + c) * A + a : static_cast<size_t>(i);
+  const float z = eps ? eps[ei] : philox_normal(seed, static_cast<unsigned>(oe), static_cast<unsigned>(c * A + a), 2u);
   if (c == 0) eval_action[oe * A + a] = tanhf(m);
   sample_action[(static_cast<size_t>(oe) * C + c) * A + a] = tanhf(__fadd_rn(m, __fmul_rn(std[src], z)));
 }
@@ -427,6 +428,17 @@ __global__ void ring_append_slots_kernel(float* __restrict__ ring, int L, int ob
       row_p[c] = pr[k];
     }
   }
+}
+
+// observation c of row first + r of listed slot k = rows[k, r, c]; the action and reward columns are left as they are
+__global__ void ring_write_obs_kernel(float* __restrict__ ring, int L, int obs, int act, int first, int n_rows, const __grid_constant__ RingSlots s,
+                                      const float* __restrict__ rows) {
+  PDL_PROLOGUE();
+  const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const size_t per = static_cast<size_t>(n_rows) * obs;
+  if (i >= per * s.n) return;
+  const int k = static_cast<int>(i / per), r = static_cast<int>((i - k * per) / obs), c = static_cast<int>(i % obs);
+  ring[(static_cast<size_t>(s.slot[k]) * L + first + r) * (obs + act + 1) + c] = rows[i];
 }
 
 // element c of time step t of window k: listed slot e = slots[k] at its step pl[e] with horizon h[k]
@@ -528,6 +540,20 @@ int launch_ring_append_slots(float* ring, int E, int L, int obs, int act, const 
     return M3PC_OK;
   });
 }
+int launch_ring_write_obs(float* ring, int E, int L, int obs, int act, const int* slots, int n, int first, int n_rows, const float* rows,
+                          cudaStream_t st) {
+  M3PC_REQUIRE(ring && E >= 1 && L >= 1 && obs >= 1 && act >= 1 && n >= 0 && (n == 0 || slots), "ring_write_obs: bad shape");
+  M3PC_REQUIRE(first >= 0 && n_rows >= 0 && first + static_cast<long>(n_rows) <= L, "ring_write_obs: rows outside the ring");
+  M3PC_REQUIRE(n_rows == 0 || n == 0 || rows, "ring_write_obs: null rows");
+  if (n_rows == 0) return M3PC_OK;
+  return for_slot_chunks(slots, nullptr, n, E, 1, [&](const RingSlots& s, int k0) {
+    const size_t cnt = static_cast<size_t>(s.n) * n_rows * obs;
+    M3PC_CHECK_CUDA(launch_k(ring_write_obs_kernel, dim3(static_cast<unsigned>((cnt + 255) / 256)), dim3(256), 0, st, ring, L, obs, act,
+                             first, n_rows, s, rows + static_cast<size_t>(k0) * n_rows * obs));
+    M3PC_CHECK_LAUNCH();
+    return M3PC_OK;
+  });
+}
 int launch_ring_windows_slots(const float* ring, int E, int L, int obs, int act, const int* pl, const int* slots, const int* horizons, int n,
                               int T, int future_obs, const float* rtg_tok, float* ws, float* wa, float* wr, float* wt, cudaStream_t st) {
   M3PC_REQUIRE(ring && pl && rtg_tok && ws && wa && wr && wt && horizons && E >= 1 && L >= 1 && n >= 0 && (n == 0 || slots) && T >= 1 &&
@@ -592,10 +618,11 @@ int launch_merge(const float* partials, int n_shards, int A, float temperature, 
 }
 int launch_sampling_tail(const float* mu, const float* std, const float* eps, int T, int h, int A, int E, float* eval_action,
                          float* sample_action, unsigned long long seed, const unsigned long long* seed_ptr, cudaStream_t st, int C,
-                         const int* env_id) {
+                         const int* env_id, bool eps_at_env_id) {
   M3PC_REQUIRE(C >= 1, "sampling tail: n_draws must be >= 1");
+  M3PC_REQUIRE(env_id || !eps_at_env_id, "sampling tail: eps rows by environment id need the id table");
   M3PC_CHECK_CUDA(launch_k(sampling_tail_kernel, dim3(ceil_div(E * C * A, 128)), dim3(128), 0, st, mu, std, eps, T, h, A, E, C, eval_action, sample_action, seed, seed_ptr,
-                           env_id));
+                           env_id, eps_at_env_id));
   M3PC_CHECK_LAUNCH();
   return M3PC_OK;
 }

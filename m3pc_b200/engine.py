@@ -272,14 +272,37 @@ class PlanEngine:
 
     def backward_plan(self, *, mode: str, horizon: int, win_states: torch.Tensor, win_actions: torch.Tensor, win_rewards: torch.Tensor,
                       win_returns_tok: torch.Tensor, eps: Optional[torch.Tensor] = None, debug: bool = False, n_draws: Optional[int] = None,
-                      seed: int = 0):
+                      seed: int = 0, env_horizons: Optional[Sequence[int]] = None):
         """Zero-shot backward planners on E environments (zeroshot_omtm/learner.py:60-261). Windows have a leading E axis.
-        ``n_draws = C``: C action draws per environment from one set of forward passes -> sample actions (E, C, A); eps (E, C, A)."""
+        ``n_draws = C``: C action draws per environment from one set of forward passes -> sample actions (E, C, A); eps (E, C, A).
+
+        ``env_horizons``: one planning horizon per environment (environments at different points of their episodes); ``horizon``
+        must be the largest.  When the entries differ the call is ``m3pc_backward_plan_env``: row e is what the uniform call on the
+        environments of e's horizon returns for e (no ``states_filled`` debug output)."""
         if not self.finalized:
             self.finalize()
         ws = _dev_f32(win_states, "win_states")
         E = ws.shape[0]
         wa, wr, wt = _dev_f32(win_actions, "win_actions"), _dev_f32(win_rewards, "win_rewards"), _dev_f32(win_returns_tok, "win_returns_tok")
+        if env_horizons is not None:
+            hz = np.ascontiguousarray(np.asarray(env_horizons, dtype=np.int32).reshape(-1))
+            if hz.size != E:
+                raise ValueError(f"env_horizons has {hz.size} entries, expected n_env={E}")
+            if int(hz.max()) != int(horizon):
+                raise ValueError("with env_horizons, horizon must equal its largest entry")
+            if int(hz.min()) != int(hz.max()):
+                Cn = 1 if n_draws is None else int(n_draws)
+                ev = torch.empty(E, self.act, device=self.device)
+                sm = torch.empty((E, self.act) if n_draws is None else (E, Cn, self.act), device=self.device)
+                if eps is not None:
+                    eps = _dev_f32(eps, "eps")
+                    if eps.numel() != E * Cn * self.act:
+                        raise ValueError(f"eps has {eps.numel()} elements, expected (E={E}, C={Cn}, A={self.act})")
+                with torch.cuda.device(self.device):
+                    nat.check(self.lib.m3pc_backward_plan_env(self._h, {"id": 0, "piid": 1}[mode], E, hz.ctypes.data, Cn, ws.data_ptr(), wa.data_ptr(),
+                                                              wr.data_ptr(), wt.data_ptr(), _ptr(eps), int(seed) & (2 ** 64 - 1), ev.data_ptr(),
+                                                              sm.data_ptr(), _stream()), "m3pc_backward_plan_env")
+                return ev, sm, {}
         if n_draws is not None:
             Cn = int(n_draws)
             ev = torch.empty(E, self.act, device=self.device)
